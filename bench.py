@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: ViT forward, images/sec (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2|c3|c4|c5] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2|c3|c4|c5] [--impl reference] [--dump-outputs DIR]
 
 One process per GPU (torchrun sets RANK/LOCAL_RANK/WORLD_SIZE for N > 1).  A step = one forward
 of the per-GPU batch (c2 / c3: weak scaling, the per-GPU batch is fixed; c4 / c5: the named GLOBAL batch
@@ -24,6 +24,9 @@ Rank 0 prints ONE JSON line.
             `roofline.library_same_shape` (N = 1): every GEMM shape of the layer through our kernel and through
             cuBLASLt, back to back in the same process (same box, same power cap): the library comparison that
             does not depend on which peak figure the fraction is taken of
+  --dump-outputs DIR    after the timed steps, DIR/pooled.npy (float32) holds what the last timed step returned:
+            the pooled CLS embeddings, (global batch, hidden).  The weights and pixels are seeded, so two builds run
+            with the same arguments can be compared output for output
   gather_check (N > 1)  one untimed step: peer-store gather == NCCL gather == single-process forward
   other_configs         short untimed-side measurements of the other BASELINE configs on the same box
   cpu_baseline / --impl reference
@@ -492,6 +495,19 @@ def library_same_shape(dev, M, D, F, secs=0.3):
                     "cuBLASLt through torch.addmm", "shapes": out_rows}
 
 
+def dump_pooled(out_dir, rows):
+    """``out_dir``/pooled.npy: the rows in float32, or the same seeded sample of them on every run when all of
+    them would take more than 64 MB."""
+    import numpy as np
+    import torch
+    cap = ((64 << 20) - 4096) // (4 * rows.shape[1])      # 4 KB left for the .npy header
+    if rows.shape[0] > cap:
+        pick = torch.randperm(rows.shape[0], generator=torch.Generator().manual_seed(0))[:cap]
+        rows = rows[pick.sort().values]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pooled.npy"), rows.float().numpy())
+
+
 def gather_check(model, dp, x, global_batch, world, rank):
     """One untimed step three ways: peer-store kernel, NCCL all-gather, and (rank 0) the single-process
     forward of the first images of every rank's shard.  Returns a dict of verdicts (identical on all ranks)."""
@@ -528,7 +544,13 @@ def main():
     ap.add_argument("--profile-step", action="store_true",
                     help="bracket ONE extra eager step after the timed region with cudaProfilerStart/Stop "
                          "(ncu --profile-from-start off then captures exactly one forward)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the output of the last timed step to DIR/pooled.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the output of the B200 path; --impl reference has none to write")
     args.warmup = max(args.warmup, 3)
 
     arch, _, _, desc = CONFIGS[args.config]
@@ -598,6 +620,8 @@ def main():
         stop.record()
         sync_all()
         launches = run.launches(args.steps, _lib.launch_count - launches0)
+        # copied now: the passes below may reuse the buffers of the timed step
+        timed_rows = (last if last is not None else out).cpu() if args.dump_outputs else None
         # the same K steps again, eagerly, with a CUDA event before and after EVERY kernel launch (rooflines);
         # kept out of the region above because ~130 event records per step cost 2-4 %
         timer = KernelTimer()
@@ -712,6 +736,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_pooled(args.dump_outputs, timed_rows)
 
     ms_per_step = ms_total / args.steps
     value = global_batch * args.steps / (ms_total / 1e3)

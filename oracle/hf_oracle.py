@@ -6,6 +6,7 @@ from seeds; biases and LayerNorm affines are re-randomised because HF zero/one-i
 """
 import torch
 
+import hashlib
 import os
 import sys
 
@@ -40,3 +41,25 @@ def make_input(arch: str, batch: int, seed: int = 1234) -> torch.Tensor:
 @torch.no_grad()
 def hf_forward(model, x: torch.Tensor) -> torch.Tensor:
     return model(pixel_values=x).last_hidden_state
+
+
+def digest(t: torch.Tensor) -> str:
+    return hashlib.sha256(t.detach().contiguous().cpu().numpy().tobytes()).hexdigest()
+
+
+def build_hf_golden(gold: dict):
+    """The model a tests/golden/hf_<arch>.pt fixture was computed with: rebuilt from the fixture's seed and
+    checked tensor by tensor against the sha256 digests the fixture stores in place of the weights."""
+    model = build_hf(gold["arch"], seed=gold["model_seed"])
+    got = {k: digest(v) for k, v in model.state_dict().items()}
+    assert got == gold["state_dict_sha256"], (
+        f"the seed-{gold['model_seed']} {gold['arch']} weights differ from the fixture's (torch {torch.__version__}, "
+        f"fixture made with {gold['torch']}): regenerate tests/golden with oracle/make_golden.py")
+    return model
+
+
+def golden_input(gold: dict) -> torch.Tensor:
+    """The pixels of a golden fixture, regenerated from its seed and checked against its digest."""
+    x = make_input(gold["arch"], gold["batch"], seed=gold["input_seed"])
+    assert digest(x) == gold["input_digest"], f"seed-{gold['input_seed']} input differs from the fixture's"
+    return x

@@ -272,3 +272,24 @@ def test_zero_sum_layernorm_fold_packing(K, N):
     err_z = ((got_z - want).norm() / want.norm()).item()
     err_c = ((got_c - want).norm() / want.norm()).item()
     assert err_z <= 1.1 * err_c + 1e-5 and err_z <= 2e-3
+
+
+def test_bench_dump_outputs_float32_and_bounded(tmp_path):
+    """bench.py --dump-outputs: the rows exactly, in float32, while they fit in 64 MB; above that the same seeded
+    sample of rows on every run, and the file stays within 64 MB."""
+    import numpy as np
+    import bench
+    small = torch.randn(256, 768).bfloat16()
+    bench.dump_pooled(str(tmp_path / "small"), small)
+    got = np.load(tmp_path / "small" / "pooled.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, small.float().numpy())
+    big = torch.randn(24000, 768)
+    for d in ("a", "b"):
+        bench.dump_pooled(str(tmp_path / d), big)
+    a, b = np.load(tmp_path / "a" / "pooled.npy"), np.load(tmp_path / "b" / "pooled.npy")
+    assert os.path.getsize(tmp_path / "a" / "pooled.npy") <= 64 << 20
+    assert np.array_equal(a, b) and a.shape == (21844, 768)         # (64 MB - 4 KB of header) / 3 KB rows
+    # every stored row is one whole row of the output, each at most once, in the output's order
+    where = {r.tobytes(): i for i, r in enumerate(big.numpy())}
+    idx = [where.get(r.tobytes(), -1) for r in a]
+    assert min(idx) >= 0 and all(i < j for i, j in zip(idx, idx[1:]))

@@ -12,12 +12,10 @@ from vit.utils import transfer_pretrained_weights
 from vit.vit import VIT
 
 
-def _custom_state_dict(arch, hf_state_dict=None, hf_model=None):
+def _custom_state_dict(arch, hf_model=None):
     model = VIT(**hf_oracle.vit_kwargs(arch))
     if hf_model is None:
         hf_model = hf_oracle.build_hf(arch, seed=0)
-        if hf_state_dict is not None:
-            hf_model.load_state_dict(hf_state_dict)
     transfer_pretrained_weights(hf_model, model, verbose=False)
     return model.state_dict(), hf_model
 
@@ -25,11 +23,12 @@ def _custom_state_dict(arch, hf_state_dict=None, hf_model=None):
 @pytest.mark.parametrize("arch", ["tiny-b", "tiny-h"])
 def test_restatement_matches_golden_hf(arch, golden_dir):
     gold = torch.load(os.path.join(golden_dir, f"hf_{arch}.pt"))
-    sd, hf = _custom_state_dict(arch, gold["state_dict"])
+    sd, hf = _custom_state_dict(arch, hf_model=hf_oracle.build_hf_golden(gold))
+    x = hf_oracle.golden_input(gold)
     # the stored HF output is reproduced by HF itself here (pins transformers/torch numerics)
-    live = hf_oracle.hf_forward(hf, gold["input"])
+    live = hf_oracle.hf_forward(hf, x)
     assert torch.allclose(live, gold["output"], atol=1e-5, rtol=0)
-    out = restatement.vit_forward(sd, gold["input"])
+    out = restatement.vit_forward(sd, x)
     assert out.shape == gold["output"].shape
     assert (out - gold["output"]).abs().max().item() <= 2e-5
 
@@ -42,7 +41,7 @@ def test_restatement_matches_hf_vit_b16(golden_dir):
     out = restatement.vit_forward(sd, x)
     assert (out - live).abs().max().item() <= 2e-5
     if str(torch.__version__) == gold["torch"]:
-        assert (live - gold["output"]).abs().max().item() <= 1e-5
+        assert (live[:, gold["tokens"]] - gold["output"]).abs().max().item() <= 1e-5
 
 
 def test_restatement_edge_batch_sizes():

@@ -5,6 +5,7 @@
 #include <stdlib.h>
 
 #include "../../include/vitb200.h"
+#include "../../include/vitb200_resolution.h"
 
 namespace vt {
 int layernorm_rows(const void*, const void*, const void*, void*, long long, int, long long,
@@ -42,7 +43,8 @@ int gemm2_fp8_tcgen05(const void*, long long, const void*, long long, void*, lon
 int layernorm_e4m3(const void*, const void*, const void*, void*, long long, int, long long, long long, float, float,
                    cudaStream_t);
 int quantize_rows_e4m3(const void*, long long, void*, long long, float*, int, int, cudaStream_t);
-int patch_gather(const void*, int, void*, int, int, int, int, int, int, cudaStream_t);
+int patch_gather(const void*, int, void*, int, int, int, int, int, int, int, cudaStream_t);
+int pos_resample(const void*, int, float*, int, int, int, int, cudaStream_t);
 int gemm2_patch_tokens(const void*, long long, const void*, long long, void*, const float*, const void*, float*, int, int,
                        int, int, int, int, cudaStream_t);
 int ln_fold(const void*, long long, const float*, const float*, const float*, void*, long long, float*, float*, int,
@@ -230,16 +232,30 @@ int vt_ln_fold(const void* w, int64_t ldw, const float* bias, const float* gamma
 int vt_patch_embed_gemm(const void* pixels, int32_t pix_dtype, const void* w, int64_t ldw, const float* bias,
                         const void* posb, void* out, float* stats_out, void* workspace, int32_t B, int32_t C, int32_t S_,
                         int32_t P, int32_t D, void* stream) {
-  if (P <= 0 || S_ <= 0 || (S_ % P) || !workspace) return VT_ERR_ARG;
-  const int n = (S_ / P) * (S_ / P);
-  const int tokens = n + 1;
+  if (P <= 0 || S_ <= 0 || (S_ % P)) return VT_ERR_ARG;
+  return vt_patch_embed_gemm_hw(pixels, pix_dtype, w, ldw, bias, posb, out, stats_out, workspace, B, C, S_, S_, P, D,
+                                stream);
+}
+
+int vt_patch_embed_gemm_hw(const void* pixels, int32_t pix_dtype, const void* w, int64_t ldw, const float* bias,
+                           const void* posb, void* out, float* stats_out, void* workspace, int32_t B, int32_t C,
+                           int32_t H, int32_t W, int32_t P, int32_t D, void* stream) {
+  if (P <= 0 || H < P || W < P || !workspace) return VT_ERR_ARG;
+  const long long n = static_cast<long long>(H / P) * (W / P);
+  if (n + 32 > 0x7fffffffLL) return VT_ERR_UNSUPPORTED;
+  const int tokens = static_cast<int>(n) + 1;
   const int tok_pad = (tokens + 31) & ~31;
   const int K = C * P * P;
   if (ldw < K || (ldw % 8)) return VT_ERR_ALIGN;
-  const int rc = vt::patch_gather(pixels, pix_dtype, workspace, B, C, S_, P, tok_pad, static_cast<int>(ldw), S(stream));
+  const int rc = vt::patch_gather(pixels, pix_dtype, workspace, B, C, H, W, P, tok_pad, static_cast<int>(ldw), S(stream));
   if (rc) return rc;
   return vt::gemm2_patch_tokens(workspace, ldw, w, ldw, out, bias, posb, stats_out, B, tok_pad, tokens, D,
                                 static_cast<int>(ldw), next_direction(), S(stream));
+}
+
+int vt_pos_embed_resample(const void* pos, int32_t pos_dtype, float* out, int32_t D, int32_t g_in, int32_t gh,
+                          int32_t gw, void* stream) {
+  return vt::pos_resample(pos, pos_dtype, out, D, g_in, gh, gw, S(stream));
 }
 
 int vt_patching(const void* image, void* out, int32_t B, int32_t C, int32_t H, int32_t W, int32_t P,

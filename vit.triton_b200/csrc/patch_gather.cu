@@ -22,7 +22,7 @@ namespace {
 struct GatherParams {
   const void* pixels;
   __nv_bfloat16* out;
-  int B, C, S, P, grid_w, n_patches, K, Kpad, Tpad;
+  int B, C, H, W, P, grid_w, n_patches, K, Kpad, Tpad;
   long long total_chunks;    // B * Tpad * Kpad / 8
 };
 
@@ -44,7 +44,7 @@ patch_gather_kernel(const GatherParams p) {
   const int patch = t - 1;
   const int py = patch / p.grid_w, px = patch - py * p.grid_w;      // block-uniform
   const bool real_row = t >= 1 && t <= p.n_patches;
-  const TPix* img = static_cast<const TPix*>(p.pixels) + static_cast<long long>(b) * p.C * p.S * p.S;
+  const TPix* img = static_cast<const TPix*>(p.pixels) + static_cast<long long>(b) * p.C * p.H * p.W;
   uint4* out_row = reinterpret_cast<uint4*>(p.out) + (static_cast<long long>(b) * p.Tpad + t) * chunks_per_row;
   for (int kc = threadIdx.x; kc < chunks_per_row; kc += blockDim.x) {
     const int k0 = kc << 3;
@@ -54,7 +54,7 @@ patch_gather_kernel(const GatherParams p) {
         const int PC = p.P * p.C;                 // bytes of one patch row; PC % 8 == 0
         const int i = k0 / PC, rem = k0 - i * PC;
         const uint2 v = __ldg(reinterpret_cast<const uint2*>(
-            img + (static_cast<long long>(py * p.P + i) * p.S + px * p.P) * p.C + rem));
+            img + (static_cast<long long>(py * p.P + i) * p.W + px * p.P) * p.C + rem));
         auto f = [](uint32_t w, int s) { return static_cast<float>((w >> (8 * s)) & 0xFFu); };
         o = make_uint4(pack_bf16x2(f(v.x, 0), f(v.x, 1)), pack_bf16x2(f(v.x, 2), f(v.x, 3)),
                        pack_bf16x2(f(v.y, 0), f(v.y, 1)), pack_bf16x2(f(v.y, 2), f(v.y, 3)));
@@ -62,7 +62,7 @@ patch_gather_kernel(const GatherParams p) {
         const int PP = p.P * p.P;
         const int c = k0 / PP, rem = k0 - c * PP;
         const int i = rem / p.P, j = rem - i * p.P;   // P % 8 == 0: the 8 pixels stay inside one patch row
-        const TPix* src = img + (static_cast<long long>(c) * p.S + py * p.P + i) * p.S + px * p.P + j;
+        const TPix* src = img + (static_cast<long long>(c) * p.H + py * p.P + i) * p.W + px * p.P + j;
         if constexpr (sizeof(TPix) == 2) {
           o = __ldg(reinterpret_cast<const uint4*>(src));
         } else {
@@ -80,12 +80,12 @@ patch_gather_kernel(const GatherParams p) {
             if constexpr (kNHWC) {
               const int PC = p.P * p.C;
               const int i = k / PC, rem = k - i * PC;
-              e[u] = gpx(img[(static_cast<long long>(py * p.P + i) * p.S + px * p.P) * p.C + rem]);
+              e[u] = gpx(img[(static_cast<long long>(py * p.P + i) * p.W + px * p.P) * p.C + rem]);
             } else {
               const int PP = p.P * p.P;
               const int c = k / PP, rem = k - c * PP;
               const int i = rem / p.P, j = rem - i * p.P;
-              e[u] = gpx(img[(static_cast<long long>(c) * p.S + py * p.P + i) * p.S + px * p.P + j]);
+              e[u] = gpx(img[(static_cast<long long>(c) * p.H + py * p.P + i) * p.W + px * p.P + j]);
             }
           }
         }
@@ -105,27 +105,31 @@ int launch_gather(const GatherParams& p, cudaStream_t stream) {
 
 }  // namespace
 
+// pixels: [B, C, H, W] (f32 | bf16) or [B, H, W, C] (VT_U8); the patch grid is (H / P) x (W / P) rounded down, the
+// pixels of the last H % P rows and W % P columns belong to no patch (a stride-P convolution drops them too).
 // out: bf16 [B, Tpad, Kpad] (Kpad % 8 == 0, Tpad >= n_patches + 1), 16-byte aligned.
-int patch_gather(const void* pixels, int pix_dtype, void* out, int B, int C, int S, int P, int Tpad, int Kpad,
+int patch_gather(const void* pixels, int pix_dtype, void* out, int B, int C, int H, int W, int P, int Tpad, int Kpad,
                  cudaStream_t stream) {
-  if (!pixels || !out || B <= 0 || C <= 0 || S <= 0 || P <= 0 || (S % P)) return VT_ERR_ARG;
+  if (!pixels || !out || B <= 0 || C <= 0 || P <= 0 || H < P || W < P) return VT_ERR_ARG;
   GatherParams p;
   p.pixels = pixels;
   p.out = static_cast<__nv_bfloat16*>(out);
-  p.B = B; p.C = C; p.S = S; p.P = P;
-  p.grid_w = S / P;
-  p.n_patches = p.grid_w * p.grid_w;
+  p.B = B; p.C = C; p.H = H; p.W = W; p.P = P;
+  p.grid_w = W / P;
+  p.n_patches = (H / P) * p.grid_w;
   p.K = C * P * P;
   p.Kpad = Kpad;
   p.Tpad = Tpad;
   if ((Kpad % 8) || Kpad < p.K || Tpad < p.n_patches + 1) return VT_ERR_ARG;
   if ((reinterpret_cast<uintptr_t>(pixels) | reinterpret_cast<uintptr_t>(out)) & 15) return VT_ERR_ALIGN;
   p.total_chunks = static_cast<long long>(B) * Tpad * (Kpad / 8);
+  // vector loads need every 8-element chunk inside one patch row and 8-element aligned: image rows of a multiple of
+  // 8 elements (W * C bytes for NHWC, W for NCHW) then keep every row, plane and image start aligned too
   if (pix_dtype == VT_U8) {
-    const bool vec = ((P * C) % 8 == 0) && ((S * C) % 8 == 0);
+    const bool vec = ((P * C) % 8 == 0) && ((W * C) % 8 == 0);
     return vec ? launch_gather<uint8_t, true>(p, stream) : launch_gather<uint8_t, false>(p, stream);
   }
-  const bool vec = (P % 8 == 0) && (S % 8 == 0);
+  const bool vec = (P % 8 == 0) && (W % 8 == 0);
   if (pix_dtype == VT_BF16)
     return vec ? launch_gather<__nv_bfloat16, true>(p, stream) : launch_gather<__nv_bfloat16, false>(p, stream);
   if (pix_dtype == VT_F32) return vec ? launch_gather<float, true>(p, stream) : launch_gather<float, false>(p, stream);

@@ -1,4 +1,4 @@
-"""ctypes binding of libvitb200.so (C ABI declared in include/vitb200.h).
+"""ctypes binding of libvitb200.so (C ABI declared in include/vitb200.h and include/vitb200_resolution.h).
 
 There is deliberately no fallback: if the shared library is missing or a tensor is not on a CUDA
 device the entry points raise.  The oracle under /oracle is test infrastructure and is never
@@ -65,6 +65,14 @@ SIGNATURES = {
                               _c_ptr, _c_ptr, _c_i32, _c_i32, _c_ptr],
 }
 
+# name -> argtypes of the any-resolution entry points; mirrors include/vitb200_resolution.h one to one
+# (tests/test_abi_resolution.py checks both directions)
+RESOLUTION_SIGNATURES = {
+    "vt_patch_embed_gemm_hw": [_c_ptr, _c_i32, _c_ptr, _c_i64, _c_ptr, _c_ptr, _c_ptr, _c_ptr, _c_ptr, _c_i32, _c_i32,
+                               _c_i32, _c_i32, _c_i32, _c_i32, _c_ptr],
+    "vt_pos_embed_resample": [_c_ptr, _c_i32, _c_ptr, _c_i32, _c_i32, _c_i32, _c_i32, _c_ptr],
+}
+
 
 def lib_path() -> str:
     # VT_LIB selects an alternative build of the same library (A/B measurements of kernel variants)
@@ -85,7 +93,7 @@ def load() -> ctypes.CDLL:
             f"{_LIB_NAME} not found at {path}: build it with `make -C vit.triton_b200` "
             "(or `python -c 'import __graft_entry__ as g; g.build()'`). There is no CPU fallback.")
     lib = ctypes.CDLL(path)
-    for name, argtypes in SIGNATURES.items():
+    for name, argtypes in list(SIGNATURES.items()) + list(RESOLUTION_SIGNATURES.items()):
         fn = getattr(lib, name)
         fn.argtypes = argtypes
         fn.restype = ctypes.c_int

@@ -11,6 +11,8 @@ source parameter's storage pointer or version counter changes (in-place ops, opt
 bump no version counter and cannot be seen without reading the device: call ``VIT.invalidate_packed()``
 after them.
 """
+import math
+from collections import OrderedDict
 from types import SimpleNamespace
 from typing import Optional
 
@@ -234,17 +236,9 @@ def pack_embeddings_u8(emb, image_mean, image_std, rescale_factor: float) -> Sim
                            posb16=_posb16(pos, emb.cls_token, bias32))
 
 
-def patch_embed_u8(emb, x: torch.Tensor, image_mean, image_std, rescale_factor: float,
-                   stats: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """Raw uint8 NHWC pixels (B, S, S, C) -> token embeddings (B, n+1, D), rescale + normalise + patch
-    projection + CLS + position embeddings in ONE kernel (bf16 models on the tensor-core path)."""
-    w = emb.projection.weight
-    assert x.is_cuda and x.dtype == torch.uint8 and x.dim() == 4, \
-        f"Raw pixels need to be a CUDA uint8 (B, H, W, C) tensor, provided: {x.dtype}, {tuple(x.shape)}"
-    assert w.dtype == torch.bfloat16 and emb.hidden_dim % 8 == 0, \
-        "The fused uint8 input path runs on the bf16 tensor-core kernels only"
-    B, S, S2, C = x.shape
-    assert S == S2 and C == emb.channels, f"Image size {tuple(x.shape[1:])} not matching with the model input size"
+def u8_pack(emb, image_mean, image_std, rescale_factor: float) -> tuple:
+    """(key, pack) of ``pack_embeddings_u8`` for these image-processor constants, cached on the module (one set of
+    constants at a time) and rebuilt when a source parameter's storage pointer or version counter changes."""
     key = (tuple(float(m) for m in image_mean), tuple(float(v) for v in image_std), float(rescale_factor))
     cache = emb.__dict__.setdefault("_u8_pack", {})
     params = emb._packed_sources()
@@ -255,18 +249,45 @@ def patch_embed_u8(emb, x: torch.Tensor, image_mean, image_std, rescale_factor: 
             hit = (stamp, pack_embeddings_u8(emb, image_mean, image_std, rescale_factor))
         cache.clear()
         cache[key] = hit
-    pk = hit[1]
+    return key, hit[1]
+
+
+def patch_embed_u8(emb, x: torch.Tensor, image_mean, image_std, rescale_factor: float,
+                   stats: Optional[torch.Tensor] = None, interpolate: bool = False) -> torch.Tensor:
+    """Raw uint8 NHWC pixels (B, S, S, C) -> token embeddings (B, n+1, D), rescale + normalise + patch
+    projection + CLS + position embeddings in ONE kernel (bf16 models on the tensor-core path).
+    ``interpolate``: any (B, H, W, C) with H, W >= patch size, position table resampled to its patch grid
+    (``pos_grid``)."""
+    w = emb.projection.weight
+    assert x.is_cuda and x.dtype == torch.uint8 and x.dim() == 4, \
+        f"Raw pixels need to be a CUDA uint8 (B, H, W, C) tensor, provided: {x.dtype}, {tuple(x.shape)}"
+    assert w.dtype == torch.bfloat16 and emb.hidden_dim % 8 == 0, \
+        "The fused uint8 input path runs on the bf16 tensor-core kernels only"
+    B, S, S2, C = x.shape
+    if interpolate:
+        check_any_size(emb, C, S, S2)
+    else:
+        assert S == S2 and C == emb.channels, f"Image size {tuple(x.shape[1:])} not matching with the model input size"
+    _, pk = u8_pack(emb, image_mean, image_std, rescale_factor)
     x = x.contiguous()
-    n_tok = emb.num_patches + 1
+    n = emb.num_patches
+    hw = posb16 = None
+    if interpolate:
+        grid = patch_grid(emb, S, S2)
+        n = grid[0] * grid[1]
+        hw = (S, S2)
+        if grid != native_grid(emb):
+            posb16 = pos_grid(emb, *grid).token_table_u8(emb, image_mean, image_std, rescale_factor)
+    n_tok = n + 1
     out = torch.empty((B, n_tok, emb.hidden_dim), device=x.device, dtype=w.dtype)
     if B == 0:
         return out
     stream = _lib.stream_ptr(x)
-    step = 65535 * 128 // emb.num_patches
+    step = _embed_batch_step(n)
     for b0 in range(0, B, step):
         nb = min(step, B - b0)
         _embed_call(stats, b0, n_tok, emb.hidden_dim, pk, x[b0:].data_ptr(), _lib.VT_U8, out[b0:].data_ptr(), nb, C, S,
-                    emb.patch_size, stream, x.device)
+                    emb.patch_size, stream, x.device, hw=hw, posb16=posb16)
     return out
 
 
@@ -369,15 +390,30 @@ def split_weight(w_nk: torch.Tensor, pieces: int) -> torch.Tensor:
     return value
 
 
+def _embed_batch_step(n_patches: int) -> int:
+    """Images per patch-embedding launch: the gather's grid is (token rows, images), at most 65535 images."""
+    return min(65535, 65535 * 128 // n_patches)
+
+
 def _two_launch_embed() -> bool:
     """Gather + token-mode GEMM (default) or round 1's single kernel (VT_PATCH_EMBED=1, A/B measurements)."""
     return os.environ.get("VT_PATCH_EMBED", "2") != "1"
 
 
-def _embed_call(stats, b0, n_tok, dim, pk, pixels_ptr, pix_code, out_ptr, nb, C, S, P, stream, device):
+def _embed_call(stats, b0, n_tok, dim, pk, pixels_ptr, pix_code, out_ptr, nb, C, S, P, stream, device, hw=None,
+                posb16=None):
     """Patch embedding of images b0 .. b0 + nb: ``vt_patch_embed_gemm`` (gather + 2-CTA GEMM in token mode), or the
-    single-kernel ``vt_patch_embed[_stats]``; row statistics of those images go into ``stats`` when given."""
+    single-kernel ``vt_patch_embed[_stats]``; row statistics of those images go into ``stats`` when given.
+    ``hw`` = (H, W): an input at any resolution, ``vt_patch_embed_gemm_hw`` with the position table ``posb16``
+    (None: the packed one) — always the two-launch form, the single kernel takes square native inputs only."""
     s_ptr = None if stats is None else stats.data_ptr() + b0 * n_tok * (dim // STATS_COLS) * 2 * 4
+    if hw is not None:
+        tok_pad = (n_tok + 31) // 32 * 32
+        work = torch.empty((nb, tok_pad, pk.ldw), device=device, dtype=torch.bfloat16)
+        posb16 = pk.posb16 if posb16 is None else posb16
+        _lib.call("vt_patch_embed_gemm_hw", pixels_ptr, pix_code, pk.w.data_ptr(), pk.ldw, pk.bias32.data_ptr(),
+                  posb16.data_ptr(), out_ptr, s_ptr, work.data_ptr(), nb, C, hw[0], hw[1], P, dim, stream)
+        return
     if _two_launch_embed():
         tok_pad = (n_tok + 31) // 32 * 32
         work = torch.empty((nb, tok_pad, pk.ldw), device=device, dtype=torch.bfloat16)
@@ -392,16 +428,24 @@ def _embed_call(stats, b0, n_tok, dim, pk, pixels_ptr, pix_code, out_ptr, nb, C,
                   _lib.VT_BF16, s_ptr, nb, C, S, P, dim, stream)
 
 
-def patch_embed(emb, x: torch.Tensor, stats: Optional[torch.Tensor] = None) -> torch.Tensor:
+def patch_embed(emb, x: torch.Tensor, stats: Optional[torch.Tensor] = None, interpolate: bool = False) -> torch.Tensor:
     """Pixels (B, C, S, S) -> token embeddings (B, n+1, D) including CLS and position embeddings.
     ``stats``: optional (B * (n+1), D/128, 2) fp32 buffer for the row statistics the LayerNorm folded
-    into the first QKV GEMM consumes (bf16 tensor-core path only)."""
+    into the first QKV GEMM consumes (bf16 tensor-core path only).  ``interpolate``: pixels (B, C, H, W) at any
+    H, W >= patch size, n = (H // P) * (W // P), position table resampled to that grid (``pos_grid``)."""
     pk = emb.packed()
     w = emb.projection.weight
-    B, C, S, _ = x.shape
+    B, C, S, S2 = x.shape
     P = emb.patch_size
     D = emb.hidden_dim
-    n_tok = emb.num_patches + 1
+    n = emb.num_patches
+    grid = None                                            # resampled tables, None = the model's own
+    if interpolate:
+        gh, gw = patch_grid(emb, S, S2)
+        n = gh * gw
+        if (gh, gw) != native_grid(emb):
+            grid = pos_grid(emb, gh, gw)
+    n_tok = n + 1
     x = x.contiguous()
     out = torch.empty((B, n_tok, D), device=x.device, dtype=w.dtype)
     if B == 0:
@@ -409,11 +453,13 @@ def patch_embed(emb, x: torch.Tensor, stats: Optional[torch.Tensor] = None) -> t
     stream = _lib.stream_ptr(x)
 
     if w.dtype == torch.bfloat16 and D % 8 == 0 and x.dtype in (torch.float32, torch.bfloat16):
-        step = 65535 * 128 // emb.num_patches
+        hw = (S, S2) if interpolate else None
+        posb16 = None if grid is None else grid.token_table(emb)
+        step = _embed_batch_step(n)
         for b0 in range(0, B, step):
             nb = min(step, B - b0)
             _embed_call(stats, b0, n_tok, D, pk, x[b0:].data_ptr(), _lib.dtype_code(x), out[b0:].data_ptr(), nb, C, S, P,
-                        stream, x.device)
+                        stream, x.device, hw=hw, posb16=posb16)
         return out
     assert stats is None, "Row statistics come out of the bf16 tensor-core patch embedding only"
 
@@ -422,8 +468,9 @@ def patch_embed(emb, x: torch.Tensor, stats: Optional[torch.Tensor] = None) -> t
     from .kernels.patching import patching
     if x.dtype != w.dtype:
         x = x.to(w.dtype)
+    if interpolate and (S % P or S2 % P):
+        x = x[:, :, :S // P * P, :S2 // P * P]             # the pixels no patch covers (patching() copies)
     patches = patching(x, P)
-    n = emb.num_patches
     K = pk.K
     code = _lib.dtype_code(out)
     es = out.element_size()
@@ -442,6 +489,106 @@ def patch_embed(emb, x: torch.Tensor, stats: Optional[torch.Tensor] = None) -> t
         kk = a.shape[2]
         bg.bgemm(a.data_ptr(), wp.data_ptr(), out, out.data_ptr() + D * es, n, D, kk, B, 1, (n * kk, 0, kk),
                  (0, 0, kk), (n_tok * D, 0, D), bias32=pk.bias32)
-    _lib.call("vt_embed_finalize", out.data_ptr(), emb.position_embeddings.data_ptr(),
-              emb.cls_token.data_ptr(), B, n_tok, D, code, stream)
+    pos = emb.position_embeddings if grid is None else grid.pos
+    _lib.call("vt_embed_finalize", out.data_ptr(), pos.data_ptr(), emb.cls_token.data_ptr(), B, n_tok, D, code, stream)
     return out
+
+
+# ------------------------------------------------------------------------------------------------ any input resolution
+POS_GRIDS_KEPT = 4     # resampled position tables kept per Embeddings module, least recently used dropped first
+
+
+def patch_grid(emb, height: int, width: int) -> tuple:
+    """(gh, gw) patch grid of an input: a stride-P convolution drops the last H % P rows and W % P columns."""
+    return height // emb.patch_size, width // emb.patch_size
+
+
+def native_grid(emb) -> tuple:
+    """(g0, g0): the patch grid the position table was trained for."""
+    g0 = math.isqrt(emb.num_patches)
+    assert g0 * g0 == emb.num_patches, f"Position table of {emb.num_patches} patches is not a square grid"
+    return g0, g0
+
+
+def check_any_size(emb, channels: int, height: int, width: int) -> None:
+    P = emb.patch_size
+    assert channels == emb.channels and height >= P and width >= P, \
+        f"Image size {(channels, height, width)} needs {emb.channels} channels and sides of at least the patch size {P}"
+
+
+def resample_pos_table(pos: torch.Tensor, g_in: int, gh: int, gw: int) -> torch.Tensor:
+    """[1 + g_in^2, D] position table (fp32 | bf16, CUDA) -> fp32 [1 + gh * gw, D]: row 0 copied, the grid resampled
+    bicubically like HF ``ViTEmbeddings.interpolate_pos_encoding`` (one ``vt_pos_embed_resample`` launch)."""
+    assert pos.is_cuda and pos.dim() == 2 and pos.shape[0] == 1 + g_in * g_in, \
+        f"Expected a CUDA [1 + {g_in}^2, D] position table, provided: {tuple(pos.shape)} on {pos.device}"
+    pos = pos.contiguous()
+    out = torch.empty((1 + gh * gw, pos.shape[1]), device=pos.device, dtype=torch.float32)
+    _lib.call("vt_pos_embed_resample", pos.data_ptr(), _lib.dtype_code(pos), out.data_ptr(), pos.shape[1], g_in, gh, gw,
+              _lib.stream_ptr(pos))
+    return out
+
+
+class PosGrid:
+    """Position tables of one non-native patch grid, all derived from one resample of the model's table:
+    ``pos32`` fp32 [1 + n, D]; ``pos`` (1, 1 + n, D) in the model's dtype (``Embeddings.interpolate_pos_encoding``,
+    and ``vt_embed_finalize`` of the fp32 / unfused paths); ``token_table`` / ``token_table_u8`` the bf16 tables of
+    the two-launch patch embedding (row 0 = cls + pos[0] - the pack's bias).  A table, once built, is never replaced
+    while this object lives: CUDA graphs keep reading it (see ``pos_grid``)."""
+
+    def __init__(self, emb, gh: int, gw: int):
+        source = emb.position_embeddings.detach()
+        self.pos32 = resample_pos_table(source[0], native_grid(emb)[0], gh, gw)
+        self.pos = self.pos32.to(source.dtype)[None]
+        self._plain = None
+        self._u8 = {}
+
+    def token_table(self, emb) -> torch.Tensor:
+        """bf16 table for pixels in NCHW (the pack ``emb.packed()``)."""
+        if self._plain is None:
+            _assert_not_capturing()
+            with torch.no_grad():
+                self._plain = _posb16(self.pos32, emb.cls_token, emb.packed().bias32)
+        return self._plain
+
+    def token_table_u8(self, emb, image_mean, image_std, rescale_factor: float) -> torch.Tensor:
+        """bf16 table for raw uint8 NHWC pixels with these image-processor constants (the pack ``u8_pack``)."""
+        key, pk = u8_pack(emb, image_mean, image_std, rescale_factor)
+        table = self._u8.get(key)
+        if table is None:
+            _assert_not_capturing()
+            with torch.no_grad():
+                table = self._u8[key] = _posb16(self.pos32, emb.cls_token, pk.bias32)
+        return table
+
+
+def _assert_not_capturing() -> None:
+    assert not torch.cuda.is_current_stream_capturing(), \
+        "the position tables of a new input resolution are built outside CUDA-graph capture: run the interpolated " \
+        "forward once at that resolution first (capture_cuda_graph's warm-up does)"
+
+
+def pos_grid(emb, gh: int, gw: int) -> PosGrid:
+    """Cached ``PosGrid`` of the (gh, gw) patch grid.  Dropped with the module's packs (``_apply``, ``load_state_dict``,
+    ``VIT.invalidate_packed``) and rebuilt when a source parameter's storage pointer or version counter changes; the
+    last ``POS_GRIDS_KEPT`` grids are kept.
+
+    A CUDA graph captured at a resolution holds the raw addresses of that grid's tables, so a ``PosGrid`` read during
+    capture is also referenced from ``_pos_grids_in_graphs`` for the life of the module: dropping it from the cache
+    (eviction, invalidation) never frees memory a captured graph still reads."""
+    cache = emb.__dict__.setdefault("_pos_grids", OrderedDict())
+    stamp = emb._packed_key(emb._packed_sources())
+    hit = cache.get((gh, gw))
+    if hit is not None and hit[0] == stamp:
+        cache.move_to_end((gh, gw))
+        if torch.cuda.is_current_stream_capturing():
+            emb.__dict__.setdefault("_pos_grids_in_graphs", {})[id(hit[1])] = hit[1]
+        return hit[1]
+    if hit is not None:
+        cache.clear()                                      # every entry was derived from the old parameters
+    _assert_not_capturing()
+    with torch.no_grad():
+        value = PosGrid(emb, gh, gw)
+    cache[(gh, gw)] = (stamp, value)
+    while len(cache) > POS_GRIDS_KEPT:
+        cache.popitem(last=False)
+    return value

@@ -129,7 +129,7 @@ class DataParallelVIT(torch.nn.Module):
     the gathered (B, D) pooled embeddings."""
 
     def __init__(self, model: torch.nn.Module, group=None, peer_gather: Optional[bool] = None,
-                 output: str = "pooled"):
+                 output: str = "pooled", interpolate_pos_encoding: bool = False):
         """``output``: "pooled" gathers the CLS embeddings (B, D); "pooler" the HF pooler output
         tanh(dense(CLS)) (B, D) of a model built with ``add_pooling_layer=True``; "logits" the class
         logits (B, num_labels) of a model built with a classifier head (``VIT(num_labels=...)``).
@@ -138,13 +138,17 @@ class DataParallelVIT(torch.nn.Module):
         require it, False = always all-gather through torch.distributed.  Which one runs is decided
         COLLECTIVELY the first time a (local batch, global batch, dtype) combination is seen: every rank
         contributes what it wants and what it holds to one all-reduce, so either all ranks use the
-        peer-store kernel with identical shapes or none does."""
+        peer-store kernel with identical shapes or none does.
+        ``interpolate_pos_encoding``: passed to every model call (``VIT.forward``'s flag: inputs at any resolution,
+        the position table resampled to their patch grid); the gathered rows keep their width, so the collective is
+        the same."""
         super().__init__()
         self.model = model
         self.group = group
         self.peer_gather = peer_gather
         assert output in ("pooled", "pooler", "logits"), f"output must be 'pooled', 'pooler' or 'logits', provided: {output}"
         self.output = output
+        self.interpolate_pos_encoding = bool(interpolate_pos_encoding)
         self._peer = None          # PeerGather of the current plan
         self._plans = {}           # (B_local, global_batch, dtype) -> PeerGather | None (= torch.distributed)
         self._pending = False      # a put() whose rows have not been collected yet (pipelined form)
@@ -164,17 +168,23 @@ class DataParallelVIT(torch.nn.Module):
     def forward_local(self, x_local: torch.Tensor) -> torch.Tensor:
         """Pooled embeddings (or pooler output / logits) of this rank's images, (B_local, D | num_labels); no
         communication."""
+        kw = self._model_kwargs()
         if self.output == "logits":
-            return self.model.logits(x_local)
+            return self.model.logits(x_local, **kw)
         if self.output == "pooler":
-            return self.model.pooler_output(x_local)
-        return self.model.pooled(x_local)
+            return self.model.pooler_output(x_local, **kw)
+        return self.model.pooled(x_local, **kw)
+
+    def _model_kwargs(self) -> dict:
+        # the keyword only when set: the wrapper also takes models whose methods have no such parameter
+        return dict(interpolate_pos_encoding=True) if self.interpolate_pos_encoding else {}
 
     def _rows(self, x_local: torch.Tensor) -> torch.Tensor:
         """(B_local, *, D) tensor whose [:, 0, :] rows this rank contributes: the final hidden states for
         "pooled" (the gather kernel pools them itself), the head's output as a one-token sequence otherwise."""
         if self.output == "pooled":
-            return self.model.forward_uint8(x_local) if x_local.dtype == torch.uint8 else self.model(x_local)
+            kw = self._model_kwargs()
+            return self.model.forward_uint8(x_local, **kw) if x_local.dtype == torch.uint8 else self.model(x_local, **kw)
         return self.forward_local(x_local).unsqueeze(1)
 
     def forward(self, x_local: torch.Tensor, global_batch: Optional[int] = None) -> torch.Tensor:

@@ -301,27 +301,53 @@ class Embeddings(packing.PackedMixin, nn.Module):
             kernel_size=(self.patch_size, self.patch_size)
         )
 
-    def forward(self, x, stats_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def forward(self, x, stats_out: Optional[torch.Tensor] = None, interpolate_pos_encoding: bool = False) -> torch.Tensor:
         """``stats_out`` (optional, fused bf16 path only): (B * N, D/128, 2) fp32 buffer that receives the
-        row statistics of the output for the LayerNorm folded into block 0's QKV GEMM."""
+        row statistics of the output for the LayerNorm folded into block 0's QKV GEMM.
+        ``interpolate_pos_encoding``: (B, C, H, W) at any H, W >= patch size, N = 1 + (H // P) * (W // P), the
+        position table resampled to that grid (``interpolate_pos_encoding(H, W)``), like HF ``ViTEmbeddings``."""
         if not (_FUSED and x.is_cuda):
             assert stats_out is None
+            pos = self.position_embeddings
+            if interpolate_pos_encoding:
+                H, W = x.shape[2], x.shape[3]
+                x = x[:, :, :H // self.patch_size * self.patch_size, :W // self.patch_size * self.patch_size]
+                pos = self.interpolate_pos_encoding(H, W)
             tokens = self.projection(x.to(self.projection.weight.dtype)).flatten(2).transpose(1, 2)
-            out = torch.empty((x.shape[0], self.num_patches + 1, self.hidden_dim), device=x.device,
+            out = torch.empty((x.shape[0], pos.shape[1], self.hidden_dim), device=x.device,
                               dtype=tokens.dtype)
             out[:, 1:, :] = tokens
-            _lib.call("vt_embed_finalize", out.data_ptr(), self.position_embeddings.data_ptr(),
+            _lib.call("vt_embed_finalize", out.data_ptr(), pos.data_ptr(),
                       self.cls_token.data_ptr(), out.shape[0], out.shape[1], out.shape[2],
                       _lib.dtype_code(out), _lib.stream_ptr(out))
             return out
-        return packing.patch_embed(self, x, stats_out)
+        return packing.patch_embed(self, x, stats_out, interpolate=interpolate_pos_encoding)
 
     def forward_uint8(self, x, image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
-                      rescale_factor: float = 1.0 / 255.0, stats_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+                      rescale_factor: float = 1.0 / 255.0, stats_out: Optional[torch.Tensor] = None,
+                      interpolate_pos_encoding: bool = False) -> torch.Tensor:
         """Raw uint8 NHWC pixels (B, H, W, C) -> embeddings: the image processor's rescale and
         normalisation (defaults: HF ``ViTImageProcessor`` of google/vit-base-patch16-224) are folded
-        into the patch projection, see ``packing.pack_embeddings_u8``."""
-        return packing.patch_embed_u8(self, x, image_mean, image_std, rescale_factor, stats_out)
+        into the patch projection, see ``packing.pack_embeddings_u8``.  ``interpolate_pos_encoding`` as for
+        ``forward``."""
+        return packing.patch_embed_u8(self, x, image_mean, image_std, rescale_factor, stats_out,
+                                      interpolate=interpolate_pos_encoding)
+
+    def interpolate_pos_encoding(self, height: int, width: int) -> torch.Tensor:
+        """(1, 1 + gh * gw, D) position table for a (height, width) input, gh = height // P, gw = width // P:
+        HF ``ViTEmbeddings.interpolate_pos_encoding``.  The stored parameter itself at the trained grid; otherwise
+        its patch grid resampled bicubically (align_corners=False) by one ``vt_pos_embed_resample`` launch, cached
+        per grid for the last few grids (``packing.pos_grid``) with the tables the patch embedding derives from it.
+        A new grid's tables are built outside CUDA-graph capture."""
+        grid = packing.patch_grid(self, height, width)
+        assert grid[0] >= 1 and grid[1] >= 1, f"Image size {(height, width)} is smaller than one {self.patch_size}-pixel patch"
+        if grid == packing.native_grid(self):
+            return self.position_embeddings
+        return packing.pos_grid(self, *grid).pos
+
+    def invalidate_packed(self):
+        super().invalidate_packed()
+        self.__dict__.pop("_pos_grids", None)
 
     def _packed_sources(self):
         return [self.cls_token, self.position_embeddings, self.projection.weight, self.projection.bias]
@@ -437,17 +463,28 @@ class VIT(nn.Module):
     def dtype(self) -> torch.dtype:
         return self.layernorm.weight.dtype
 
-    def forward(self, x):
-        assert x.shape[1:] == (self.channels, self.height, self.width), f"Image size {x.shape[1:]} not matching with the model input size: {self.channels, self.height, self.width}"
-        stats = self._embed_stats(x)
-        x = self.embeddings(x, stats) if stats is not None else self.embeddings(x)
+    def forward(self, x, interpolate_pos_encoding: bool = False):
+        """(B, C, H, W) -> final hidden states (B, N, D).  ``interpolate_pos_encoding`` (HF ``ViTModel``'s flag): any
+        H, W >= patch size, square or not; N = 1 + (H // P) * (W // P), the position table resampled bicubically to
+        that grid (``Embeddings.interpolate_pos_encoding``).  Without it the input must be the model's size."""
+        if interpolate_pos_encoding:
+            assert x.dim() == 4, f"Expected (B, C, H, W) pixels, provided: {tuple(x.shape)}"
+            packing.check_any_size(self.embeddings, *x.shape[1:])
+            n_tok = 1 + math.prod(packing.patch_grid(self.embeddings, x.shape[2], x.shape[3]))
+        else:
+            assert x.shape[1:] == (self.channels, self.height, self.width), f"Image size {x.shape[1:]} not matching with the model input size: {self.channels, self.height, self.width}"
+            n_tok = None
+        stats = self._embed_stats(x, n_tok)
+        kw = dict(interpolate_pos_encoding=True) if interpolate_pos_encoding else {}
+        x = self.embeddings(x, stats, **kw) if stats is not None else self.embeddings(x, **kw)
         x = self.encoder(x, stats) if stats is not None else self.encoder(x)
         x = self.layernorm(x)
         return x
 
-    def _embed_stats(self, x: torch.Tensor) -> Optional[torch.Tensor]:
+    def _embed_stats(self, x: torch.Tensor, n_tok: Optional[int] = None) -> Optional[torch.Tensor]:
         """Buffer for the row statistics of the embeddings when block 0's layernorm_before is folded
-        into its QKV GEMM (fused bf16 tensor-core path, hidden size a multiple of 128); None otherwise."""
+        into its QKV GEMM (fused bf16 tensor-core path, hidden size a multiple of 128); None otherwise.
+        ``n_tok``: tokens per image (default: the model's own, num_patches + 1)."""
         w = self.embeddings.projection.weight
         batch = x.shape[0]
         if not (x.is_cuda and w.is_cuda and w.dtype == torch.bfloat16 and batch > 0 and self.hidden_dim % 8 == 0
@@ -456,41 +493,54 @@ class VIT(nn.Module):
         probe = torch.empty((1,), device=x.device, dtype=w.dtype)
         if not self.encoder.folding_active(probe):
             return None
-        n_tok = self.embeddings.num_patches + 1
+        n_tok = self.embeddings.num_patches + 1 if n_tok is None else n_tok
         return torch.empty((batch * n_tok, self.hidden_dim // packing.STATS_COLS, 2), device=x.device,
                            dtype=torch.float32)
 
     def forward_uint8(self, x, image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
-                      rescale_factor: float = 1.0 / 255.0):
+                      rescale_factor: float = 1.0 / 255.0, interpolate_pos_encoding: bool = False):
         """Forward from RAW uint8 NHWC pixels (B, H, W, C) — the step in front of the reference's
         ``forward``: rescale + normalise (HF ``ViTImageProcessor``) run inside the patch-embedding
-        kernel, so the host -> device copy is one byte per pixel value."""
-        assert tuple(x.shape[1:]) == (self.height, self.width, self.channels), f"Image size {x.shape[1:]} not matching with the model input size: {self.height, self.width, self.channels}"
-        stats = self._embed_stats(x)
-        x = self.embeddings.forward_uint8(x, image_mean, image_std, rescale_factor, stats)
+        kernel, so the host -> device copy is one byte per pixel value.  ``interpolate_pos_encoding`` as for
+        ``forward``."""
+        if interpolate_pos_encoding:
+            assert x.dim() == 4, f"Expected (B, H, W, C) pixels, provided: {tuple(x.shape)}"
+            packing.check_any_size(self.embeddings, x.shape[3], x.shape[1], x.shape[2])
+            n_tok = 1 + math.prod(packing.patch_grid(self.embeddings, x.shape[1], x.shape[2]))
+        else:
+            assert tuple(x.shape[1:]) == (self.height, self.width, self.channels), f"Image size {x.shape[1:]} not matching with the model input size: {self.height, self.width, self.channels}"
+            n_tok = None
+        stats = self._embed_stats(x, n_tok)
+        x = self.embeddings.forward_uint8(x, image_mean, image_std, rescale_factor, stats,
+                                          interpolate_pos_encoding=interpolate_pos_encoding)
         x = self.encoder(x, stats) if stats is not None else self.encoder(x)
         x = self.layernorm(x)
         return x
 
-    def pooler_output(self, x) -> torch.Tensor:
+    def _hidden(self, x, interpolate_pos_encoding: bool) -> torch.Tensor:
+        """Final hidden states of pixels (B, C, H, W) or raw uint8 (B, H, W, C)."""
+        kw = dict(interpolate_pos_encoding=True) if interpolate_pos_encoding else {}
+        return self.forward_uint8(x, **kw) if x.dtype == torch.uint8 else self.forward(x, **kw)
+
+    def pooler_output(self, x, interpolate_pos_encoding: bool = False) -> torch.Tensor:
         """HF ``ViTModel(...).pooler_output``: tanh(dense(final hidden state of CLS)), (B, D)."""
         assert self.pooler is not None, "Model was built without add_pooling_layer=True"
-        hidden = self.forward_uint8(x) if x.dtype == torch.uint8 else self.forward(x)
+        hidden = self._hidden(x, interpolate_pos_encoding)
         return self.pooler(hidden)
 
-    def logits(self, x) -> torch.Tensor:
+    def logits(self, x, interpolate_pos_encoding: bool = False) -> torch.Tensor:
         """Class logits (B, num_labels) = classifier(final hidden states[:, 0]) — HF
         ``ViTForImageClassification(...).logits``; needs ``VIT(..., num_labels=...)``.  One tensor-core
         launch over the CLS rows of the final hidden states."""
         assert self.classifier is not None, "VIT was built without a classifier head (num_labels)"
-        hidden = self.forward_uint8(x) if x.dtype == torch.uint8 else self.forward(x)
+        hidden = self._hidden(x, interpolate_pos_encoding)
         from .kernels import bgemm as bg
         return _head_on_cls(hidden, self.classifier, bg.ACT_NONE)
 
-    def pooled(self, x) -> torch.Tensor:
+    def pooled(self, x, interpolate_pos_encoding: bool = False) -> torch.Tensor:
         """CLS row of the final hidden states, (B, D): the tensor the data-parallel wrapper gathers.
         uint8 (B, H, W, C) inputs take the fused raw-pixel path."""
-        hidden = self.forward_uint8(x) if x.dtype == torch.uint8 else self.forward(x)
+        hidden = self._hidden(x, interpolate_pos_encoding)
         out = torch.empty((hidden.shape[0], hidden.shape[2]), device=hidden.device, dtype=hidden.dtype)
         _lib.call("vt_pool_cls", hidden.data_ptr(), out.data_ptr(), hidden.shape[0], hidden.shape[2],
                   hidden.stride(0), _lib.dtype_code(hidden), _lib.stream_ptr(hidden))

@@ -83,13 +83,15 @@ def test_c2_vit_b16_bf16_matches_hf():
 
 def test_batch_independence_full_batch_c2():
     """Full C2 batch (256): every image's output equals the output it gets in a batch of 4 —
-    a size-independent property standing in for the oracle at sizes it cannot reach quickly."""
+    a size-independent property standing in for the oracle at sizes it cannot reach quickly.  All 64
+    slices: at 256 images every GEMM group and attention CTA walks many tiles, so a wrong later tile
+    shows up here as one slice that differs."""
     model, _ = _build("vit-b16-224", torch.bfloat16)
     g = torch.Generator().manual_seed(5)
     x = torch.randn(256, 3, 224, 224, generator=g).to(DEV, torch.bfloat16)
     with torch.no_grad():
         full = model(x)
-        for lo in (0, 124, 252):
+        for lo in range(0, 256, 4):
             part = model(x[lo:lo + 4].contiguous())
             assert torch.equal(full[lo:lo + 4], part), f"images {lo}..{lo+3} differ between batch 256 and batch 4"
 

@@ -135,7 +135,8 @@ int vt_quantize_rows_fp8(const void* w, int64_t ldw, void* out, int64_t ldo, flo
  * A: bf16 [M, K] per batch, K contiguous; element strides sA = {outer, inner, row}.
  * B: bf16; b_mn_major == 0: [N, K] per batch, K contiguous; != 0: [K, N] per batch, N contiguous (the layout
  *    matmul3 receives) — consumed in place as an MN-major UMMA operand; sB = {outer, inner, row}.
- *    Both batch strides 0 = one matrix shared by all batches (weights).
+ *    A batch stride of 0 broadcasts the operand along that level (A and B alike); both batch strides 0 =
+ *    one matrix shared by all batches (weights).
  * C / residual: out_dtype (bf16 | f32) [M, N] per batch, sC = {outer, inner, row}; bias f32 [N] (nullable);
  * act: 0 none, 1 exact-erf GELU, 2 tanh.  Any M, N, K; every A / B stride a multiple of 8 elements and
  * both bases 16-byte aligned (pack with vt_pack_bf16 otherwise).

@@ -40,7 +40,8 @@ struct BgemmParams {
   int M, N, K;
   int num_m_tiles, num_n_tiles;
   int batch_inner, batch_total;
-  int a_batched, b_batched;      // operand has its own data per batch (else batch coordinates are 0)
+  int a_inner, a_outer;          // operand has its own data per inner / outer batch (else that coordinate is 0)
+  int b_inner, b_outer;
   void* C;
   long long sCo, sCi, ldc;       // element strides of C: outer batch, inner batch, row (column stride 1)
   const void* residual;          // same dtype and strides as C, nullable
@@ -139,8 +140,8 @@ bgemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_con
       int z, m_blk, n_blk;
       decode(t, z, m_blk, n_blk);
       const int zo = z / p.batch_inner, zi = z - zo * p.batch_inner;
-      const int azi = p.a_batched ? zi : 0, azo = p.a_batched ? zo : 0;
-      const int bzi = p.b_batched ? zi : 0, bzo = p.b_batched ? zo : 0;
+      const int azi = p.a_inner ? zi : 0, azo = p.a_outer ? zo : 0;
+      const int bzi = p.b_inner ? zi : 0, bzo = p.b_outer ? zo : 0;
       for (int kb = 0; kb < num_kb; ++kb) {
         mbar_wait(empty_bar(s), phase ^ 1u);
         if (elect_one_sync()) {
@@ -324,7 +325,8 @@ int launch_bgemm(const CUtensorMap& ta, const CUtensorMap& tb, const BgemmParams
 
 // A: bf16 [bo, bi, M, K] K-major (strides sA = {outer, inner, row}, column stride 1).
 // B: bf16; b_mn == 0: [bo, bi, N, K] K-major; b_mn != 0: [bo, bi, K, N] with N contiguous (sB = {outer, inner, row}).
-// A batch stride of 0 on BOTH levels marks an operand shared by all batches (weights).
+// A batch stride of 0 broadcasts the operand along that level; 0 on both levels shares one matrix with all
+// batches (weights).
 // C / residual: bf16 | f32 [bo, bi, M, N] (sC = {outer, inner, row}); bias f32 [N].
 int bgemm_tcgen05(const void* A, const void* B, void* C, const float* bias, const void* residual, int M, int N, int K,
                   int batch_outer, int batch_inner, const long long* sA, const long long* sB, const long long* sC,
@@ -344,8 +346,8 @@ int bgemm_tcgen05(const void* A, const void* B, void* C, const float* bias, cons
   p.M = M; p.N = N; p.K = K;
   p.batch_inner = batch_inner;
   p.batch_total = batch_outer * batch_inner;
-  p.a_batched = (sA[0] != 0 || sA[1] != 0) ? 1 : 0;
-  p.b_batched = (sB[0] != 0 || sB[1] != 0) ? 1 : 0;
+  p.a_inner = sA[1] != 0; p.a_outer = sA[0] != 0;
+  p.b_inner = sB[1] != 0; p.b_outer = sB[0] != 0;
   p.C = C;
   p.sCo = sC[0]; p.sCi = sC[1]; p.ldc = sC[2];
   p.residual = residual;
@@ -361,8 +363,8 @@ int bgemm_tcgen05(const void* A, const void* B, void* C, const float* bias, cons
   p.num_m_tiles = (M + GB_BM - 1) / GB_BM;
 
   CUtensorMap ta, tb;
-  const uint64_t abi = p.a_batched ? batch_inner : 1, abo = p.a_batched ? batch_outer : 1;
-  const uint64_t bbi = p.b_batched ? batch_inner : 1, bbo = p.b_batched ? batch_outer : 1;
+  const uint64_t abi = p.a_inner ? batch_inner : 1, abo = p.a_outer ? batch_outer : 1;
+  const uint64_t bbi = p.b_inner ? batch_inner : 1, bbo = p.b_outer ? batch_outer : 1;
   int rc = make_tmap_bf16_4d(&ta, A, K, M, abi, abo, sA[2], sA[1], sA[0], GB_BK, GB_BM);
   if (rc) return rc;
   if (b_mn) {

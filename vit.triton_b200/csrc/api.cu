@@ -1,4 +1,5 @@
-// extern "C" surface of libvitb200.so (declared in include/vitb200.h).  Thin: argument plumbing
+// extern "C" surface of libvitb200.so (declared in include/vitb200.h and its companions
+// vitb200_resolution.h, vitb200_ragged.h).  Thin: argument plumbing
 // only, all kernels live in the other translation units.
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -6,6 +7,7 @@
 
 #include "../../include/vitb200.h"
 #include "../../include/vitb200_resolution.h"
+#include "../../include/vitb200_ragged.h"
 
 namespace vt {
 int layernorm_rows(const void*, const void*, const void*, void*, long long, int, long long,
@@ -45,6 +47,8 @@ int layernorm_e4m3(const void*, const void*, const void*, void*, long long, int,
 int quantize_rows_e4m3(const void*, long long, void*, long long, float*, int, int, cudaStream_t);
 int patch_gather(const void*, int, void*, int, int, int, int, int, int, int, cudaStream_t);
 int pos_resample(const void*, int, float*, int, int, int, int, cudaStream_t);
+int patch_gather_ragged(const void*, int, int, int, int, void*, long long, void*, int, long long, cudaStream_t);
+int gather_rows(const void*, long long, const long long*, void*, long long, int, int, int, cudaStream_t);
 int gemm2_patch_tokens(const void*, long long, const void*, long long, void*, const float*, const void*, float*, int, int,
                        int, int, int, int, cudaStream_t);
 int ln_fold(const void*, long long, const float*, const float*, const float*, void*, long long, float*, float*, int,
@@ -256,6 +260,17 @@ int vt_patch_embed_gemm_hw(const void* pixels, int32_t pix_dtype, const void* w,
 int vt_pos_embed_resample(const void* pos, int32_t pos_dtype, float* out, int32_t D, int32_t g_in, int32_t gh,
                           int32_t gw, void* stream) {
   return vt::pos_resample(pos, pos_dtype, out, D, g_in, gh, gw, S(stream));
+}
+
+int vt_patch_embed_ragged_gather(const vt_ragged_image* images, int32_t n_images, int32_t pix_dtype, int32_t C,
+                                 int32_t P, void* patches, int64_t ldw, void* table, int32_t D, int64_t M,
+                                 void* stream) {
+  return vt::patch_gather_ragged(images, n_images, pix_dtype, C, P, patches, ldw, table, D, M, S(stream));
+}
+
+int vt_gather_rows(const void* x, int64_t ldx, const int64_t* idx, void* out, int64_t ldo, int32_t rows, int32_t cols,
+                   int32_t dtype, void* stream) {
+  return vt::gather_rows(x, ldx, reinterpret_cast<const long long*>(idx), out, ldo, rows, cols, dtype, S(stream));
 }
 
 int vt_patching(const void* image, void* out, int32_t B, int32_t C, int32_t H, int32_t W, int32_t P,

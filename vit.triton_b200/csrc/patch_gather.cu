@@ -14,6 +14,7 @@
 // Replaces the patch extraction inside conv2d_kernel (vit/kernels/conv2d.py:19-97) / patching_kernel
 // (vit/kernels/patching.py:54-92).
 #include "common.cuh"
+#include "../../include/vitb200_ragged.h"
 
 namespace vt {
 
@@ -30,6 +31,56 @@ __device__ __forceinline__ float gpx(float v) { return v; }
 __device__ __forceinline__ float gpx(__nv_bfloat16 v) { return __bfloat162float(v); }
 __device__ __forceinline__ float gpx(uint8_t v) { return static_cast<float>(v); }
 
+// One 16-byte chunk of a patch row: elements k0 .. k0 + 7 (k0 < K, k0 % 8 == 0) of patch (py, px) of one image, the
+// elements >= K zero.  The addressing of both gathers (the batched one below and the ragged one of
+// vt_patch_embed_ragged_gather).  kVec: 8-element loads, which need P % 8 == 0 and W % 8 == 0 (NCHW) / P * C and
+// W * C multiples of 8 (NHWC), and a 16-byte aligned image.
+template <typename TPix, bool kVec>
+__device__ __forceinline__ uint4 gather_chunk(const TPix* img, int C, int H, int W, int P, int K, int py, int px,
+                                              int k0) {
+  constexpr bool kNHWC = sizeof(TPix) == 1;
+  if constexpr (kVec && kNHWC) {
+    const int PC = P * C;                     // bytes of one patch row; PC % 8 == 0
+    const int i = k0 / PC, rem = k0 - i * PC;
+    const uint2 v = __ldg(reinterpret_cast<const uint2*>(img + (static_cast<long long>(py * P + i) * W + px * P) * C + rem));
+    auto f = [](uint32_t w, int s) { return static_cast<float>((w >> (8 * s)) & 0xFFu); };
+    return make_uint4(pack_bf16x2(f(v.x, 0), f(v.x, 1)), pack_bf16x2(f(v.x, 2), f(v.x, 3)),
+                      pack_bf16x2(f(v.y, 0), f(v.y, 1)), pack_bf16x2(f(v.y, 2), f(v.y, 3)));
+  } else if constexpr (kVec) {
+    const int PP = P * P;
+    const int c = k0 / PP, rem = k0 - c * PP;
+    const int i = rem / P, j = rem - i * P;   // P % 8 == 0: the 8 pixels stay inside one patch row
+    const TPix* src = img + (static_cast<long long>(c) * H + py * P + i) * W + px * P + j;
+    if constexpr (sizeof(TPix) == 2) {
+      return __ldg(reinterpret_cast<const uint4*>(src));
+    } else {
+      const float4 a = __ldg(reinterpret_cast<const float4*>(src));
+      const float4 c4 = __ldg(reinterpret_cast<const float4*>(src) + 1);
+      return make_uint4(pack_bf16x2(a.x, a.y), pack_bf16x2(a.z, a.w), pack_bf16x2(c4.x, c4.y), pack_bf16x2(c4.z, c4.w));
+    }
+  } else {
+    float e[8];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) {
+      const int k = k0 + u;
+      e[u] = 0.f;
+      if (k < K) {
+        if constexpr (kNHWC) {
+          const int PC = P * C;
+          const int i = k / PC, rem = k - i * PC;
+          e[u] = gpx(img[(static_cast<long long>(py * P + i) * W + px * P) * C + rem]);
+        } else {
+          const int PP = P * P;
+          const int c = k / PP, rem = k - c * PP;
+          const int i = rem / P, j = rem - i * P;
+          e[u] = gpx(img[(static_cast<long long>(c) * H + py * P + i) * W + px * P + j]);
+        }
+      }
+    }
+    return make_uint4(pack_bf16x2(e[0], e[1]), pack_bf16x2(e[2], e[3]), pack_bf16x2(e[4], e[5]), pack_bf16x2(e[6], e[7]));
+  }
+}
+
 // one thread = one 16-byte chunk (8 bf16) of A; blockIdx.x = token row, blockIdx.y = image: no division by the row
 // length or the token count (the first version decoded a flat 64-bit chunk index with four 64-bit divisions per
 // chunk and ran at 44 us for the C2 batch, issue-bound: 77 % issue slots, DRAM 35 %; now ~40.  Staging whole image
@@ -37,7 +88,6 @@ __device__ __forceinline__ float gpx(uint8_t v) { return static_cast<float>(v); 
 template <typename TPix, bool kVec>
 __global__ void __launch_bounds__(128)
 patch_gather_kernel(const GatherParams p) {
-  constexpr bool kNHWC = sizeof(TPix) == 1;
   const int chunks_per_row = p.Kpad >> 3;
   const int t = blockIdx.x;
   const int b = blockIdx.y;
@@ -49,49 +99,7 @@ patch_gather_kernel(const GatherParams p) {
   for (int kc = threadIdx.x; kc < chunks_per_row; kc += blockDim.x) {
     const int k0 = kc << 3;
     uint4 o = make_uint4(0u, 0u, 0u, 0u);
-    if (real_row && k0 < p.K) {
-      if constexpr (kVec && kNHWC) {
-        const int PC = p.P * p.C;                 // bytes of one patch row; PC % 8 == 0
-        const int i = k0 / PC, rem = k0 - i * PC;
-        const uint2 v = __ldg(reinterpret_cast<const uint2*>(
-            img + (static_cast<long long>(py * p.P + i) * p.W + px * p.P) * p.C + rem));
-        auto f = [](uint32_t w, int s) { return static_cast<float>((w >> (8 * s)) & 0xFFu); };
-        o = make_uint4(pack_bf16x2(f(v.x, 0), f(v.x, 1)), pack_bf16x2(f(v.x, 2), f(v.x, 3)),
-                       pack_bf16x2(f(v.y, 0), f(v.y, 1)), pack_bf16x2(f(v.y, 2), f(v.y, 3)));
-      } else if constexpr (kVec) {
-        const int PP = p.P * p.P;
-        const int c = k0 / PP, rem = k0 - c * PP;
-        const int i = rem / p.P, j = rem - i * p.P;   // P % 8 == 0: the 8 pixels stay inside one patch row
-        const TPix* src = img + (static_cast<long long>(c) * p.H + py * p.P + i) * p.W + px * p.P + j;
-        if constexpr (sizeof(TPix) == 2) {
-          o = __ldg(reinterpret_cast<const uint4*>(src));
-        } else {
-          const float4 a = __ldg(reinterpret_cast<const float4*>(src));
-          const float4 c4 = __ldg(reinterpret_cast<const float4*>(src) + 1);
-          o = make_uint4(pack_bf16x2(a.x, a.y), pack_bf16x2(a.z, a.w), pack_bf16x2(c4.x, c4.y), pack_bf16x2(c4.z, c4.w));
-        }
-      } else {
-        float e[8];
-#pragma unroll
-        for (int u = 0; u < 8; ++u) {
-          const int k = k0 + u;
-          e[u] = 0.f;
-          if (k < p.K) {
-            if constexpr (kNHWC) {
-              const int PC = p.P * p.C;
-              const int i = k / PC, rem = k - i * PC;
-              e[u] = gpx(img[(static_cast<long long>(py * p.P + i) * p.W + px * p.P) * p.C + rem]);
-            } else {
-              const int PP = p.P * p.P;
-              const int c = k / PP, rem = k - c * PP;
-              const int i = rem / p.P, j = rem - i * p.P;
-              e[u] = gpx(img[(static_cast<long long>(c) * p.H + py * p.P + i) * p.W + px * p.P + j]);
-            }
-          }
-        }
-        o = make_uint4(pack_bf16x2(e[0], e[1]), pack_bf16x2(e[2], e[3]), pack_bf16x2(e[4], e[5]), pack_bf16x2(e[6], e[7]));
-      }
-    }
+    if (real_row && k0 < p.K) o = gather_chunk<TPix, kVec>(img, p.C, p.H, p.W, p.P, p.K, py, px, k0);
     out_row[kc] = o;
   }
 }
@@ -134,6 +142,101 @@ int patch_gather(const void* pixels, int pix_dtype, void* out, int B, int C, int
     return vec ? launch_gather<__nv_bfloat16, true>(p, stream) : launch_gather<__nv_bfloat16, false>(p, stream);
   if (pix_dtype == VT_F32) return vec ? launch_gather<float, true>(p, stream) : launch_gather<float, false>(p, stream);
   return VT_ERR_DTYPE;
+}
+
+// ------------------------------------------------------------------------------------------------ ragged batch
+// Images of different sizes in one launch (vt_patch_embed_ragged_gather): one block per packed output row.  The row's
+// image is found by a binary search over the descriptors' first rows (log2(images) cached loads, block-uniform); the
+// block writes the row's patch pixels (gather_chunk, the batched kernel's addressing) and the image's position row, the
+// residual of the embedding GEMM.  No row padding: the GEMM runs in plain mode over the packed rows, whose epilogue
+// adds bias + residual in the same order as token mode, so every image comes out as it does from its own call.
+namespace {
+
+struct RaggedParams {
+  const vt_ragged_image* images;
+  __nv_bfloat16* patches;
+  __nv_bfloat16* table;
+  int n_images, C, P, K, Kpad, D;
+};
+
+template <typename TPix>
+__global__ void __launch_bounds__(128)
+patch_gather_ragged_kernel(const RaggedParams p) {
+  constexpr bool kNHWC = sizeof(TPix) == 1;
+  const long long row = blockIdx.x;
+  int lo = 0, hi = p.n_images - 1;                  // last image with row0 <= row
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (__ldg(&p.images[mid].row0) <= row) lo = mid; else hi = mid - 1;
+  }
+  const vt_ragged_image* d = p.images + lo;
+  const long long row0 = __ldg(&d->row0);
+  const int H = __ldg(&d->height), W = __ldg(&d->width);
+  const long long t64 = row - row0;
+  const bool covered = t64 >= 0 && t64 < __ldg(&d->tokens);
+  const int t = covered ? static_cast<int>(t64) : 0;
+  const int grid_w = W / p.P;
+  const int n_patches = (H / p.P) * grid_w;
+  const bool real_row = covered && t >= 1 && t <= n_patches;
+  const int patch = real_row ? t - 1 : 0;
+  const int py = patch / grid_w, px = patch - py * grid_w;
+  const TPix* img = static_cast<const TPix*>(d->pixels);
+  const bool aligned = (reinterpret_cast<uintptr_t>(img) & 15) == 0;
+  const bool vec = aligned && (kNHWC ? ((p.P * p.C) % 8 == 0 && (W * p.C) % 8 == 0) : (p.P % 8 == 0 && W % 8 == 0));
+
+  const int chunks_per_row = p.Kpad >> 3;
+  uint4* out_row = reinterpret_cast<uint4*>(p.patches) + row * chunks_per_row;
+  for (int kc = threadIdx.x; kc < chunks_per_row; kc += blockDim.x) {
+    const int k0 = kc << 3;
+    uint4 o = make_uint4(0u, 0u, 0u, 0u);
+    if (real_row && k0 < p.K)
+      o = vec ? gather_chunk<TPix, true>(img, p.C, H, W, p.P, p.K, py, px, k0)
+              : gather_chunk<TPix, false>(img, p.C, H, W, p.P, p.K, py, px, k0);
+    out_row[kc] = o;
+  }
+
+  const int dchunks = p.D >> 3;
+  const __nv_bfloat16* pos = static_cast<const __nv_bfloat16*>(d->pos) + static_cast<long long>(t) * p.D;
+  uint4* tab_row = reinterpret_cast<uint4*>(p.table) + row * dchunks;
+  const bool pos_aligned = (reinterpret_cast<uintptr_t>(d->pos) & 15) == 0;
+  for (int c = threadIdx.x; c < dchunks; c += blockDim.x) {
+    uint4 o = make_uint4(0u, 0u, 0u, 0u);
+    if (covered) {
+      if (pos_aligned) {
+        o = __ldg(reinterpret_cast<const uint4*>(pos) + c);
+      } else {
+        const unsigned short* s = reinterpret_cast<const unsigned short*>(pos) + (c << 3);
+        uint32_t w[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) w[u] = static_cast<uint32_t>(__ldg(s + 2 * u)) | (static_cast<uint32_t>(__ldg(s + 2 * u + 1)) << 16);
+        o = make_uint4(w[0], w[1], w[2], w[3]);
+      }
+    }
+    tab_row[c] = o;
+  }
+}
+
+}  // namespace
+
+int patch_gather_ragged(const void* images, int n_images, int pix_dtype, int C, int P, void* patches, long long ldw,
+                        void* table, int D, long long M, cudaStream_t stream) {
+  if (!images || !patches || !table || n_images <= 0 || C <= 0 || P <= 0 || D <= 0 || M <= 0) return VT_ERR_ARG;
+  if (M > 0x7fffffffLL) return VT_ERR_UNSUPPORTED;
+  const long long K = static_cast<long long>(C) * P * P;
+  if (ldw < K || ldw > 0x7fffffffLL) return VT_ERR_ARG;
+  if ((ldw % 8) || (D % 8)) return VT_ERR_ALIGN;
+  if ((reinterpret_cast<uintptr_t>(patches) | reinterpret_cast<uintptr_t>(table)) & 15) return VT_ERR_ALIGN;
+  RaggedParams p;
+  p.images = static_cast<const vt_ragged_image*>(images);
+  p.patches = static_cast<__nv_bfloat16*>(patches);
+  p.table = static_cast<__nv_bfloat16*>(table);
+  p.n_images = n_images; p.C = C; p.P = P; p.K = static_cast<int>(K); p.Kpad = static_cast<int>(ldw); p.D = D;
+  const dim3 grid(static_cast<unsigned int>(M));
+  if (pix_dtype == VT_U8) patch_gather_ragged_kernel<uint8_t><<<grid, 128, 0, stream>>>(p);
+  else if (pix_dtype == VT_BF16) patch_gather_ragged_kernel<__nv_bfloat16><<<grid, 128, 0, stream>>>(p);
+  else if (pix_dtype == VT_F32) patch_gather_ragged_kernel<float><<<grid, 128, 0, stream>>>(p);
+  else return VT_ERR_DTYPE;
+  return static_cast<int>(cudaGetLastError());
 }
 
 }  // namespace vt

@@ -572,4 +572,31 @@ int pool_cls(const void* x, void* out, int batch, int dim, long long batch_strid
   return static_cast<int>(cudaGetLastError());
 }
 
+// Row gather (vt_gather_rows): out[i, :] = x[idx[i], :] — the CLS rows of a ragged batch, whose images start at
+// arbitrary packed rows.  One block per output row, element copies (a few hundred rows per call).
+template <typename T>
+__global__ void __launch_bounds__(256)
+gather_rows_kernel(const T* __restrict__ x, long long ldx, const long long* __restrict__ idx, T* __restrict__ out,
+                   long long ldo, int cols) {
+  const long long src = __ldg(idx + blockIdx.x);
+  const T* in = x + src * ldx;
+  T* o = out + static_cast<long long>(blockIdx.x) * ldo;
+  for (int c = threadIdx.x; c < cols; c += blockDim.x) o[c] = in[c];
+}
+
+int gather_rows(const void* x, long long ldx, const long long* idx, void* out, long long ldo, int rows, int cols,
+                int dtype, cudaStream_t stream) {
+  if (!x || !idx || !out || rows < 0 || cols <= 0 || ldx < cols || ldo < cols) return VT_ERR_ARG;
+  if (rows == 0) return VT_OK;
+  if (dtype == VT_F32)
+    gather_rows_kernel<float><<<rows, 256, 0, stream>>>(static_cast<const float*>(x), ldx, idx,
+                                                        static_cast<float*>(out), ldo, cols);
+  else if (dtype == VT_BF16)
+    gather_rows_kernel<__nv_bfloat16><<<rows, 256, 0, stream>>>(static_cast<const __nv_bfloat16*>(x), ldx, idx,
+                                                                static_cast<__nv_bfloat16*>(out), ldo, cols);
+  else
+    return VT_ERR_DTYPE;
+  return static_cast<int>(cudaGetLastError());
+}
+
 }  // namespace vt

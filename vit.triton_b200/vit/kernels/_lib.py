@@ -1,4 +1,5 @@
-"""ctypes binding of libvitb200.so (C ABI declared in include/vitb200.h and include/vitb200_resolution.h).
+"""ctypes binding of libvitb200.so (C ABI declared in include/vitb200.h, include/vitb200_resolution.h and
+include/vitb200_ragged.h).
 
 There is deliberately no fallback: if the shared library is missing or a tensor is not on a CUDA
 device the entry points raise.  The oracle under /oracle is test infrastructure and is never
@@ -73,6 +74,20 @@ RESOLUTION_SIGNATURES = {
     "vt_pos_embed_resample": [_c_ptr, _c_i32, _c_ptr, _c_i32, _c_i32, _c_i32, _c_i32, _c_ptr],
 }
 
+# name -> argtypes of the ragged-batch entry points; mirrors include/vitb200_ragged.h one to one
+# (tests/test_abi_ragged.py checks both directions)
+RAGGED_SIGNATURES = {
+    "vt_patch_embed_ragged_gather": [_c_ptr, _c_i32, _c_i32, _c_i32, _c_i32, _c_ptr, _c_i64, _c_ptr, _c_i32, _c_i64,
+                                     _c_ptr],
+    "vt_gather_rows": [_c_ptr, _c_i64, _c_ptr, _c_ptr, _c_i64, _c_i32, _c_i32, _c_i32, _c_ptr],
+}
+
+
+class RaggedImage(ctypes.Structure):
+    """``vt_ragged_image`` of include/vitb200_ragged.h: one image of a ragged batch."""
+    _fields_ = [("pixels", _c_ptr), ("pos", _c_ptr), ("row0", _c_i64), ("height", _c_i32), ("width", _c_i32),
+                ("tokens", _c_i32), ("reserved", _c_i32)]
+
 
 def lib_path() -> str:
     # VT_LIB selects an alternative build of the same library (A/B measurements of kernel variants)
@@ -93,7 +108,8 @@ def load() -> ctypes.CDLL:
             f"{_LIB_NAME} not found at {path}: build it with `make -C vit.triton_b200` "
             "(or `python -c 'import __graft_entry__ as g; g.build()'`). There is no CPU fallback.")
     lib = ctypes.CDLL(path)
-    for name, argtypes in list(SIGNATURES.items()) + list(RESOLUTION_SIGNATURES.items()):
+    for name, argtypes in (list(SIGNATURES.items()) + list(RESOLUTION_SIGNATURES.items())
+                           + list(RAGGED_SIGNATURES.items())):
         fn = getattr(lib, name)
         fn.argtypes = argtypes
         fn.restype = ctypes.c_int

@@ -14,9 +14,11 @@ import os
 from . import _lib, bgemm as bg
 
 
-def flash_attention(qkv: torch.Tensor, num_heads: int, scale: Optional[float] = None) -> torch.Tensor:
+def flash_attention(qkv: torch.Tensor, num_heads: int, scale: Optional[float] = None,
+                    out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """qkv: (B, N, 3*D) with columns [Q | K | V], head h at columns h*dh:(h+1)*dh of each third.
-    Returns softmax(scale * Q K^T) V per head, concatenated: (B, N, D)."""
+    Returns softmax(scale * Q K^T) V per head, concatenated: (B, N, D), written into ``out`` when given (a contiguous
+    (B, N, D) tensor of qkv's dtype, e.g. a row range of a larger buffer)."""
     assert qkv.is_cuda, "Input is not on GPU"
     assert len(qkv.shape) == 3 and qkv.shape[2] % (3 * num_heads) == 0, \
         f"qkv needs to be (B, N, 3*D) with D divisible by num_heads, provided: {qkv.shape}, {num_heads}"
@@ -26,7 +28,10 @@ def flash_attention(qkv: torch.Tensor, num_heads: int, scale: Optional[float] = 
     dh = D // num_heads
     if scale is None:
         scale = 1.0 / math.sqrt(dh)
-    out = torch.empty((B, N, D), device=qkv.device, dtype=qkv.dtype)
+    if out is None:
+        out = torch.empty((B, N, D), device=qkv.device, dtype=qkv.dtype)
+    assert out.shape == (B, N, D) and out.dtype == qkv.dtype and out.is_contiguous(), \
+        f"out needs to be a contiguous {(B, N, D)} {qkv.dtype} tensor, provided: {tuple(out.shape)} {out.dtype}"
     if out.numel() == 0:
         return out
     es = qkv.element_size()

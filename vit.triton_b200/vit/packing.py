@@ -11,6 +11,7 @@ source parameter's storage pointer or version counter changes (in-place ops, opt
 bump no version counter and cannot be seen without reading the device: call ``VIT.invalidate_packed()``
 after them.
 """
+import ctypes
 import math
 from collections import OrderedDict
 from types import SimpleNamespace
@@ -567,10 +568,11 @@ def _assert_not_capturing() -> None:
         "forward once at that resolution first (capture_cuda_graph's warm-up does)"
 
 
-def pos_grid(emb, gh: int, gw: int) -> PosGrid:
+def pos_grid(emb, gh: int, gw: int, keep: int = POS_GRIDS_KEPT) -> PosGrid:
     """Cached ``PosGrid`` of the (gh, gw) patch grid.  Dropped with the module's packs (``_apply``, ``load_state_dict``,
     ``VIT.invalidate_packed``) and rebuilt when a source parameter's storage pointer or version counter changes; the
-    last ``POS_GRIDS_KEPT`` grids are kept.
+    last ``keep`` grids are kept (a ragged batch passes the number of grids it uses, so that repeating the list finds
+    every table in the cache).
 
     A CUDA graph captured at a resolution holds the raw addresses of that grid's tables, so a ``PosGrid`` read during
     capture is also referenced from ``_pos_grids_in_graphs`` for the life of the module: dropping it from the cache
@@ -589,6 +591,168 @@ def pos_grid(emb, gh: int, gw: int) -> PosGrid:
     with torch.no_grad():
         value = PosGrid(emb, gh, gw)
     cache[(gh, gw)] = (stamp, value)
-    while len(cache) > POS_GRIDS_KEPT:
+    while len(cache) > keep:
         cache.popitem(last=False)
     return value
+
+
+# ------------------------------------------------------------------------------------------------ ragged batches
+RAGGED_MAX_ROWS = 2 ** 31 - 1    # packed rows per embedding launch: the GEMM's row count is a 32-bit integer
+
+
+class RaggedLayout:
+    """Where the images of a ragged batch go in the packed (M, D) activation.  Images are grouped by token count, so
+    that images with the same count occupy one contiguous row range (one attention call each); inside a group they keep
+    the caller's order.  ``order``: caller indices in packed order; ``row0[i]`` / ``tokens[i]``: first row (CLS) and
+    token count of caller image i; ``groups``: (first row, images, tokens) per distinct token count; ``rows`` = M."""
+
+    def __init__(self, grids):
+        self.grids = [tuple(g) for g in grids]
+        self.tokens = [1 + gh * gw for gh, gw in self.grids]
+        self.order = sorted(range(len(self.grids)), key=lambda i: (self.tokens[i], i))
+        self.row0 = [0] * len(self.grids)
+        self.groups = []
+        row = 0
+        for i in self.order:
+            n = self.tokens[i]
+            self.row0[i] = row
+            if self.groups and self.groups[-1][2] == n:
+                r0, count, _ = self.groups[-1]
+                self.groups[-1] = (r0, count + 1, n)
+            else:
+                self.groups.append((row, 1, n))
+            row += n
+        self.rows = row
+
+    def chunks(self, max_rows: int = RAGGED_MAX_ROWS) -> list:
+        """Consecutive runs of ``order`` of at most ``max_rows`` packed rows each: one patch-embedding launch pair each
+        (the gather and the embedding GEMM take a 32-bit row count).  This covers the embedding only; the encoder runs
+        over all M rows at once, like a batched forward of M rows."""
+        out, cur, rows = [], [], 0
+        for i in self.order:
+            n = self.tokens[i]
+            assert n <= max_rows, f"an image of {n} tokens exceeds {max_rows} rows"
+            if cur and rows + n > max_rows:
+                out.append(cur)
+                cur, rows = [], 0
+            cur.append(i)
+            rows += n
+        if cur:
+            out.append(cur)
+        return out
+
+
+def check_ragged(emb, images) -> tuple:
+    """Host-side checks of a ragged batch, before anything is launched: a non-empty list of (C, H, W) float32 / bfloat16
+    or (H, W, C) uint8 tensors of one dtype, on one device, with the model's channel count and sides of at least one
+    patch.  Returns (patch grids, uint8?)."""
+    assert isinstance(images, (list, tuple)), f"A ragged batch is a list of images, provided: {type(images)}"
+    assert len(images) > 0, "A ragged batch needs at least one image"
+    dtype, device = images[0].dtype, images[0].device
+    assert dtype in (torch.float32, torch.bfloat16, torch.uint8), \
+        f"Images need to be float32 / bfloat16 (C, H, W) or uint8 (H, W, C), provided: {dtype}"
+    u8 = dtype == torch.uint8
+    grids = []
+    for i, img in enumerate(images):
+        assert isinstance(img, torch.Tensor) and img.dtype == dtype, \
+            f"All images of a ragged batch need one dtype: image 0 is {dtype}, image {i} {getattr(img, 'dtype', type(img))}"
+        assert img.device == device, f"All images of a ragged batch need one device: image {i} is on {img.device}"
+        assert img.dim() == 3, f"Image {i}: expected {'(H, W, C)' if u8 else '(C, H, W)'}, provided: {tuple(img.shape)}"
+        C, H, W = (img.shape[2], img.shape[0], img.shape[1]) if u8 else tuple(img.shape)
+        assert C == emb.channels, f"Image {i} has {C} channels, the model {emb.channels}"
+        assert H >= emb.patch_size and W >= emb.patch_size, \
+            f"Image {i} of size {(H, W)} is smaller than one {emb.patch_size}-pixel patch"
+        grids.append(patch_grid(emb, H, W))
+    return grids, u8
+
+
+def _ragged_table(emb, grid, u8: bool, image_mean, image_std, rescale_factor: float, keep: int) -> torch.Tensor:
+    """bf16 [1 + gh * gw, D] position table of one grid for the ragged gather: the one the image's own
+    interpolate_pos_encoding=True call reads (the packed table at the trained grid).  ``keep``: grids ``pos_grid``
+    keeps."""
+    if u8:
+        if grid == native_grid(emb):
+            return u8_pack(emb, image_mean, image_std, rescale_factor)[1].posb16
+        return pos_grid(emb, *grid, keep=keep).token_table_u8(emb, image_mean, image_std, rescale_factor)
+    if grid == native_grid(emb):
+        return emb.packed().posb16
+    return pos_grid(emb, *grid, keep=keep).token_table(emb)
+
+
+def _to_device_async(host_bytes: bytes, device) -> torch.Tensor:
+    """Bytes -> a device uint8 tensor: staged in pinned host memory, one cudaMemcpyAsync on the current stream (the
+    pinned block is not reused before the copy has run)."""
+    pinned = torch.empty((len(host_bytes),), dtype=torch.uint8, pin_memory=True)
+    ctypes.memmove(pinned.data_ptr(), host_bytes, len(host_bytes))
+    dev = torch.empty((len(host_bytes),), dtype=torch.uint8, device=device)
+    dev.copy_(pinned, non_blocking=True)
+    return dev
+
+
+def patch_embed_ragged(emb, images, layout: RaggedLayout, stats: Optional[torch.Tensor] = None, u8: bool = False,
+                       image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
+                       rescale_factor: float = 1.0 / 255.0) -> torch.Tensor:
+    """Images of different sizes -> packed token embeddings (1, M, D) in ``layout``'s row order: per chunk of at most
+    ``RAGGED_MAX_ROWS`` rows one ``vt_patch_embed_ragged_gather`` (patch rows + per-row position table) and one
+    ``vt_gemm_bf16_ln`` over the packed rows with the table as its residual (and ``stats``, (M, D/128, 2) fp32, the row
+    statistics for block 0's folded LayerNorm).  Every image's rows equal its own ``interpolate_pos_encoding=True``
+    call's bit for bit (bf16 tensor-core path only)."""
+    w = emb.projection.weight
+    D = emb.hidden_dim
+    assert w.is_cuda and w.dtype == torch.bfloat16 and D % 8 == 0, \
+        "The ragged patch embedding runs on the bf16 tensor-core kernels only"
+    pk = u8_pack(emb, image_mean, image_std, rescale_factor)[1] if u8 else emb.packed()
+    device = images[0].device
+    # every grid's table is held here until the launches are enqueued, and the cache keeps at least this list's grids:
+    # a list of many aspect ratios, run again, finds all of its tables instead of resampling each one per call
+    grids = list(dict.fromkeys(layout.grids))
+    keep = max(POS_GRIDS_KEPT, len(grids))
+    tables = {g: _ragged_table(emb, g, u8, image_mean, image_std, rescale_factor, keep) for g in grids}
+    pixels = [img.contiguous() for img in images]
+    code = _lib.VT_U8 if u8 else _lib.dtype_code(pixels[0])
+    out = torch.empty((1, layout.rows, D), device=device, dtype=w.dtype)
+    stream = _lib.stream_ptr(out)
+    for chunk in layout.chunks():
+        base = layout.row0[chunk[0]]
+        rows = sum(layout.tokens[i] for i in chunk)
+        desc = (_lib.RaggedImage * len(chunk))()
+        for j, i in enumerate(chunk):
+            shape = pixels[i].shape
+            h, wd = (shape[0], shape[1]) if u8 else (shape[1], shape[2])
+            desc[j] = _lib.RaggedImage(pixels[i].data_ptr(), tables[layout.grids[i]].data_ptr(),
+                                       layout.row0[i] - base, h, wd, layout.tokens[i], 0)
+        desc_dev = _to_device_async(bytes(desc), device)
+        patches = torch.empty((rows, pk.ldw), device=device, dtype=torch.bfloat16)
+        table = torch.empty((rows, D), device=device, dtype=torch.bfloat16)
+        _lib.call("vt_patch_embed_ragged_gather", desc_dev.data_ptr(), len(chunk), code, emb.channels, emb.patch_size,
+                  patches.data_ptr(), pk.ldw, table.data_ptr(), D, rows, stream)
+        s_ptr = None if stats is None else stats[base:].data_ptr()
+        _lib.call("vt_gemm_bf16_ln", patches.data_ptr(), pk.ldw, pk.w.data_ptr(), pk.ldw, out[0, base:].data_ptr(), D,
+                  pk.bias32.data_ptr(), table.data_ptr(), D, rows, D, pk.ldw, 0, None, None, 0, 0.0, s_ptr, stream)
+    return out
+
+
+def ragged_attention(qkv: torch.Tensor, num_heads: int, scale: float, groups) -> torch.Tensor:
+    """Attention of a packed ragged batch (1, M, 3D): one ``flash_attention`` per group of images with the same token
+    count ((first row, images, tokens), ``RaggedLayout.groups``), each over its contiguous row range."""
+    from .kernels import flash_attention
+    _, M, D3 = qkv.shape
+    out = torch.empty((1, M, D3 // 3), device=qkv.device, dtype=qkv.dtype)
+    for row0, count, n_tok in groups:
+        rows = slice(row0, row0 + count * n_tok)
+        flash_attention(qkv[0, rows].view(count, n_tok, D3), num_heads, scale,
+                        out=out[0, rows].view(count, n_tok, D3 // 3))
+    return out
+
+
+def gather_rows(x: torch.Tensor, rows) -> torch.Tensor:
+    """(len(rows), D) = x[rows, :] of a (M, D) CUDA tensor: one ``vt_gather_rows`` launch (index list uploaded like the
+    ragged descriptors)."""
+    assert x.is_cuda and x.dim() == 2 and x.stride(1) == 1
+    out = torch.empty((len(rows), x.shape[1]), device=x.device, dtype=x.dtype)
+    if not rows:
+        return out
+    idx = _to_device_async(bytes((ctypes.c_int64 * len(rows))(*rows)), x.device)
+    _lib.call("vt_gather_rows", x.data_ptr(), x.stride(0), idx.data_ptr(), out.data_ptr(), out.stride(0), len(rows),
+              x.shape[1], _lib.dtype_code(x), _lib.stream_ptr(x))
+    return out

@@ -118,6 +118,13 @@ class SelfAttention(nn.Module):
         return matmul3(probs, v)
 
 
+def _attention(qkv: torch.Tensor, num_heads: int, scale: float, groups=None) -> torch.Tensor:
+    """Fused attention of (B, N, 3D) rows, or of a packed ragged batch (1, M, 3D) when ``groups`` is given."""
+    if groups is None:
+        return flash_attention(qkv, num_heads, scale)
+    return packing.ragged_attention(qkv, num_heads, scale, groups)
+
+
 class MultiHeadAttention(packing.PackedMixin, nn.Module):
     """All heads + output projection (reference vit.py:77-111)."""
 
@@ -131,8 +138,9 @@ class MultiHeadAttention(packing.PackedMixin, nn.Module):
         self.attention = nn.ModuleList([SelfAttention(d_in=d_in, d_out=d_out) for _ in range(self.num_heads)])
         self.output = LinearWithBias(self.d_in, self.d_in)
 
-    def forward(self, x: torch.Tensor, residual: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """x: (B, N, D).  ``residual`` (fused path only) is added in the out-projection epilogue."""
+    def forward(self, x: torch.Tensor, residual: Optional[torch.Tensor] = None, groups=None) -> torch.Tensor:
+        """x: (B, N, D).  ``residual`` (fused path only) is added in the out-projection epilogue.  ``groups`` (fused path
+        only): x is a packed ragged batch (1, M, D), attention per group of images (``packing.RaggedLayout.groups``)."""
         if not (_FUSED and x.is_cuda):
             assert residual is None
             heads_out = torch.empty_like(x)
@@ -144,7 +152,7 @@ class MultiHeadAttention(packing.PackedMixin, nn.Module):
         B, N, D = x.shape
         x = x.contiguous()
         qkv = packing.linear(x, pk.wqkv, pk.bqkv)
-        ctx = flash_attention(qkv, self.num_heads, 1.0 / math.sqrt(self.d_out))
+        ctx = _attention(qkv, self.num_heads, 1.0 / math.sqrt(self.d_out), groups)
         return packing.linear(ctx, pk.wo, pk.bo, residual=residual)
 
     def _build_packed(self):
@@ -168,15 +176,16 @@ class Transformer(packing.PackedMixin, nn.Module):
         self.output = LinearWithBias(self.mlp_dim, self.d_in)
         self.layernorm_after = LayerNormTriton(self.d_in, eps=1e-12)
 
-    def forward(self, x):
+    def forward(self, x, groups=None):
         if not (_FUSED and x.is_cuda):
+            assert groups is None
             res = add(self.attention(self.layernorm_before(x)), x)
             out = self.output(self.intermediate(self.layernorm_after(res)))
             return add(out, res)
 
         pk = self.packed()
         x = x.contiguous()
-        res = self.attention(self.layernorm_before(x), residual=x)
+        res = self.attention(self.layernorm_before(x), residual=x, groups=groups)
         mid = packing.linear(self.layernorm_after(res), pk.w1, pk.b1, gelu=True)
         return packing.linear(mid, pk.w2, pk.b2, residual=res)
 
@@ -198,26 +207,27 @@ class Transformer(packing.PackedMixin, nn.Module):
     def _build_packed_fp8(self):
         return packing.pack_block_fp8(self)
 
-    def forward_fp8(self, x: torch.Tensor) -> torch.Tensor:
-        """Block forward with the QKV / fc1 / fc2 GEMMs on e4m3 operands (7 launches; see the note at _FP8)."""
+    def forward_fp8(self, x: torch.Tensor, groups=None) -> torch.Tensor:
+        """Block forward with the QKV / fc1 / fc2 GEMMs on e4m3 operands (7 launches; see the note at _FP8).
+        ``groups``: as for ``MultiHeadAttention.forward``."""
         att = self.attention.packed()
         mlp = self.packed()
         q8 = self.packed("fp8")
         x = x.contiguous()
         qkv = packing.linear_fp8(packing.layernorm_fp8(x, self.layernorm_before), q8.wqkv8, q8.cqkv, att.bqkv)
-        ctx = flash_attention(qkv, self.num_heads, 1.0 / math.sqrt(self.d_out))
+        ctx = _attention(qkv, self.num_heads, 1.0 / math.sqrt(self.d_out), groups)
         res = packing.linear(ctx, att.wo, att.bo, residual=x)
         mid8 = packing.linear_fp8(packing.layernorm_fp8(res, self.layernorm_after), q8.w18, q8.c1, mlp.b1, gelu=True,
                                   out_fp8=True, out_scale=packing.FP8_MID_SCALE)
         return packing.linear_fp8(mid8, q8.w28, q8.c2, mlp.b2, residual=res)
 
-    def forward_folded(self, x: torch.Tensor, ln1_stats: Optional[torch.Tensor]):
+    def forward_folded(self, x: torch.Tensor, ln1_stats: Optional[torch.Tensor], groups=None):
         """Block forward with layernorm_before folded into the QKV GEMM (bf16 only).
 
         ``ln1_stats``: (M, D/128, 2) fp32 per-128-column (sum, M2) partials of x's rows, written by the
         previous block's last GEMM (None for the first block: layernorm_before then runs as a
         kernel).  Returns (output, statistics of the output rows).  5 launches per block (layernorm_after folded into
-        fc1 as well, the default) instead of 7."""
+        fc1 as well, the default) instead of 7.  ``groups``: as for ``MultiHeadAttention.forward``."""
         att = self.attention.packed()
         mlp = self.packed()
         x = x.contiguous()
@@ -226,7 +236,7 @@ class Transformer(packing.PackedMixin, nn.Module):
         else:
             pk = self.packed("folded")
             qkv = packing.linear_ln(x, pk.wqkv, pk.bqkv, pk.cqkv, ln1_stats, self.layernorm_before.eps)
-        ctx = flash_attention(qkv, self.num_heads, 1.0 / math.sqrt(self.d_out))
+        ctx = _attention(qkv, self.num_heads, 1.0 / math.sqrt(self.d_out), groups)
         if _FOLD_LN_MLP:
             pk = self.packed("folded")
             stats2 = torch.empty((x.shape[0] * x.shape[1], self.d_in // packing.STATS_COLS, 2), device=x.device,
@@ -264,21 +274,22 @@ class Encoder(nn.Module):
         return bool(_FUSED and _FOLD_LN and not self.fp8_active(x) and len(self.layer) > 0 and x.numel() > 0 and
                     packing.folding_supported(x, self.hidden_dim, self.layer[0].mlp_dim))
 
-    def forward(self, x, ln1_stats: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def forward(self, x, ln1_stats: Optional[torch.Tensor] = None, groups=None) -> torch.Tensor:
         """``ln1_stats``: row statistics of x written by the patch-embedding epilogue (see
-        ``Embeddings.forward``); without them block 0's layernorm_before runs as a kernel."""
+        ``Embeddings.forward``); without them block 0's layernorm_before runs as a kernel.  ``groups``: x is a
+        packed ragged batch (1, M, D) whose attention runs per group of images (``VIT.forward_ragged``)."""
         if self.fp8_active(x):
             for layer in self.layer:
-                x = layer.forward_fp8(x)
+                x = layer.forward_fp8(x, groups)
             return x
         if self.folding_active(x):
             # layernorm_before folded into the QKV GEMM; row statistics of each block's output are
             # produced by its last GEMM's epilogue
             for layer in self.layer:
-                x, ln1_stats = layer.forward_folded(x, ln1_stats)
+                x, ln1_stats = layer.forward_folded(x, ln1_stats, groups)
             return x
         for layer in self.layer:
-            x = layer(x)
+            x = layer(x, groups)
         return x
 
 
@@ -517,29 +528,81 @@ class VIT(nn.Module):
         x = self.layernorm(x)
         return x
 
+    def forward_ragged(self, images, image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
+                       rescale_factor: float = 1.0 / 255.0) -> list:
+        """Images of different resolutions in one batch: a list of (C, H_i, W_i) float32 / bfloat16 or raw (H_i, W_i, C)
+        uint8 tensors (one dtype, the model's channel count, sides of at least one patch) -> the list of final hidden
+        states (N_i, D), N_i = 1 + (H_i // P) * (W_i // P), in the caller's order.  Image i gives what
+        ``self(images[i][None], interpolate_pos_encoding=True)[0]`` (``forward_uint8`` for uint8, with these image-processor
+        constants) gives, bit for bit: each image takes its own patch grid and position table.
+
+        On the fused bf16 path (LayerNorm fold on, only ``layernorm_before`` folded, fold off, FP8) the images' tokens
+        are packed into one (sum N_i, D) activation, grouped by token count: one ragged patch gather and one embedding
+        GEMM for the list, one launch per dense layer of every block over all rows, one attention launch per distinct
+        token count; the returned tensors are views into that buffer.  fp32 models and ``set_fused(False)`` run the list
+        image by image through ``forward`` / ``forward_uint8`` (correct, not fast).  Not capturable into a CUDA graph:
+        the per-image descriptors are uploaded from the host on every call."""
+        hidden, layout = self._ragged_hidden(images, image_mean, image_std, rescale_factor)
+        return [hidden[r:r + n] for r, n in zip(layout.row0, layout.tokens)]
+
+    def _ragged_hidden(self, images, image_mean, image_std, rescale_factor) -> tuple:
+        """(packed final hidden states (M, D), ``packing.RaggedLayout``) of a ragged batch."""
+        grids, u8 = packing.check_ragged(self.embeddings, images)
+        assert not torch.cuda.is_current_stream_capturing(), "A ragged batch cannot be captured into a CUDA graph"
+        layout = packing.RaggedLayout(grids)
+        first = images[0]
+        if not (_FUSED and first.is_cuda and self.dtype == torch.bfloat16 and self.hidden_dim % 8 == 0):
+            hidden = None
+            for i in layout.order:
+                if u8:
+                    h = self.forward_uint8(images[i][None], image_mean, image_std, rescale_factor,
+                                           interpolate_pos_encoding=True)
+                else:
+                    h = self.forward(images[i][None], interpolate_pos_encoding=True)
+                if hidden is None:
+                    hidden = torch.empty((layout.rows, h.shape[2]), device=h.device, dtype=h.dtype)
+                hidden[layout.row0[i]:layout.row0[i] + layout.tokens[i]].copy_(h[0])
+            return hidden, layout
+        stats = self._embed_stats(first[None], layout.rows)       # one "image" of M rows
+        x = packing.patch_embed_ragged(self.embeddings, images, layout, stats, u8, image_mean, image_std,
+                                       rescale_factor)
+        x = self.encoder(x, stats, groups=layout.groups)
+        x = self.layernorm(x)
+        return x[0], layout
+
+    def _ragged_cls(self, images) -> torch.Tensor:
+        """(B, D) CLS rows of the final hidden states of a ragged batch, in the caller's order (``vt_gather_rows``)."""
+        hidden, layout = self._ragged_hidden(images, (0.5, 0.5, 0.5), (0.5, 0.5, 0.5), 1.0 / 255.0)
+        return packing.gather_rows(hidden, layout.row0)
+
     def _hidden(self, x, interpolate_pos_encoding: bool) -> torch.Tensor:
         """Final hidden states of pixels (B, C, H, W) or raw uint8 (B, H, W, C)."""
         kw = dict(interpolate_pos_encoding=True) if interpolate_pos_encoding else {}
         return self.forward_uint8(x, **kw) if x.dtype == torch.uint8 else self.forward(x, **kw)
 
     def pooler_output(self, x, interpolate_pos_encoding: bool = False) -> torch.Tensor:
-        """HF ``ViTModel(...).pooler_output``: tanh(dense(final hidden state of CLS)), (B, D)."""
+        """HF ``ViTModel(...).pooler_output``: tanh(dense(final hidden state of CLS)), (B, D).  ``x`` may also be a list
+        of images of different sizes (``forward_ragged``), each with its own patch grid."""
         assert self.pooler is not None, "Model was built without add_pooling_layer=True"
-        hidden = self._hidden(x, interpolate_pos_encoding)
+        hidden = self._ragged_cls(x)[:, None, :] if isinstance(x, (list, tuple)) else self._hidden(x, interpolate_pos_encoding)
         return self.pooler(hidden)
 
     def logits(self, x, interpolate_pos_encoding: bool = False) -> torch.Tensor:
         """Class logits (B, num_labels) = classifier(final hidden states[:, 0]) — HF
         ``ViTForImageClassification(...).logits``; needs ``VIT(..., num_labels=...)``.  One tensor-core
-        launch over the CLS rows of the final hidden states."""
+        launch over the CLS rows of the final hidden states.  ``x`` may also be a list of images of different sizes
+        (``forward_ragged``), each with its own patch grid."""
         assert self.classifier is not None, "VIT was built without a classifier head (num_labels)"
-        hidden = self._hidden(x, interpolate_pos_encoding)
+        hidden = self._ragged_cls(x)[:, None, :] if isinstance(x, (list, tuple)) else self._hidden(x, interpolate_pos_encoding)
         from .kernels import bgemm as bg
         return _head_on_cls(hidden, self.classifier, bg.ACT_NONE)
 
     def pooled(self, x, interpolate_pos_encoding: bool = False) -> torch.Tensor:
         """CLS row of the final hidden states, (B, D): the tensor the data-parallel wrapper gathers.
-        uint8 (B, H, W, C) inputs take the fused raw-pixel path."""
+        uint8 (B, H, W, C) inputs take the fused raw-pixel path.  ``x`` may also be a list of images of different sizes
+        (``forward_ragged``), each with its own patch grid."""
+        if isinstance(x, (list, tuple)):
+            return self._ragged_cls(x)
         hidden = self._hidden(x, interpolate_pos_encoding)
         out = torch.empty((hidden.shape[0], hidden.shape[2]), device=hidden.device, dtype=hidden.dtype)
         _lib.call("vt_pool_cls", hidden.data_ptr(), out.data_ptr(), hidden.shape[0], hidden.shape[2],

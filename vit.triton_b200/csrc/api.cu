@@ -1,5 +1,5 @@
 // extern "C" surface of libvitb200.so (declared in include/vitb200.h and its companions
-// vitb200_resolution.h, vitb200_ragged.h).  Thin: argument plumbing
+// vitb200_resolution.h, vitb200_ragged.h, vitb200_mask.h).  Thin: argument plumbing
 // only, all kernels live in the other translation units.
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -8,6 +8,7 @@
 #include "../../include/vitb200.h"
 #include "../../include/vitb200_resolution.h"
 #include "../../include/vitb200_ragged.h"
+#include "../../include/vitb200_mask.h"
 
 namespace vt {
 int layernorm_rows(const void*, const void*, const void*, void*, long long, int, long long,
@@ -54,6 +55,11 @@ int gemm2_patch_tokens(const void*, long long, const void*, long long, void*, co
 int ln_fold(const void*, long long, const float*, const float*, const float*, void*, long long, float*, float*, int,
             int, int, cudaStream_t);
 int embed_finalize(void*, const void*, const void*, int, int, int, int, cudaStream_t);
+int patch_gather_masked(const void*, int, const void*, const void*, const void*, void*, long long, void*, int, int, int,
+                        int, int, int, cudaStream_t);
+int embed_finalize_masked(void*, const void*, const void*, const void*, const void*, int, int, int, int, cudaStream_t);
+int mim_reconstruct(const void*, void*, int, int, int, int, int, int, const void*, int, const float*, float, const void*,
+                    float*, float*, cudaStream_t);
 int conv2d_nchw(const void*, const void*, const void*, void*, int, int, int, int, int, int, int,
                 int, cudaStream_t);
 }  // namespace vt
@@ -281,6 +287,24 @@ int vt_patching(const void* image, void* out, int32_t B, int32_t C, int32_t H, i
 int vt_embed_finalize(void* x, const void* pos, const void* cls, int32_t B, int32_t N, int32_t D,
                       int32_t dtype, void* stream) {
   return vt::embed_finalize(x, pos, cls, B, N, D, dtype, S(stream));
+}
+
+int vt_patch_embed_masked_gather(const void* pixels, int32_t pix_dtype, const void* mask, const void* pos,
+                                 const void* posm, void* patches, int64_t ldw, void* table, int32_t B, int32_t C,
+                                 int32_t H, int32_t W, int32_t P, int32_t D, void* stream) {
+  return vt::patch_gather_masked(pixels, pix_dtype, mask, pos, posm, patches, ldw, table, B, C, H, W, P, D, S(stream));
+}
+
+int vt_embed_finalize_masked(void* x, const void* pos, const void* cls, const void* mask_token, const void* mask,
+                             int32_t B, int32_t N, int32_t D, int32_t dtype, void* stream) {
+  return vt::embed_finalize_masked(x, pos, cls, mask_token, mask, B, N, D, dtype, S(stream));
+}
+
+int vt_mim_reconstruct(const void* dec, void* rec, int32_t dtype, int32_t B, int32_t C, int32_t gh, int32_t gw,
+                       int32_t s, const void* pixels, int32_t pix_dtype, const float* norm, float rescale,
+                       const void* mask, float* partial, float* loss, void* stream) {
+  return vt::mim_reconstruct(dec, rec, dtype, B, C, gh, gw, s, pixels, pix_dtype, norm, rescale, mask, partial, loss,
+                             S(stream));
 }
 
 int vt_conv2d(const void* input, const void* weight, const void* bias, void* out, int32_t B,

@@ -48,6 +48,26 @@ __global__ void embed_finalize_kernel(T* __restrict__ x, const T* __restrict__ p
   stf(x + idx, v + pv);
 }
 
+// embed_finalize with bool_masked_pos: a masked patch's projection is replaced by the mask token before pos is added
+template <typename T>
+__global__ void embed_finalize_masked_kernel(T* __restrict__ x, const T* __restrict__ pos, const T* __restrict__ cls,
+                                             const T* __restrict__ mask_token, const uint8_t* __restrict__ mask,
+                                             int B, int N, int D) {
+  const long long total = static_cast<long long>(B) * N * D;
+  const long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (idx >= total) return;
+  const int d = static_cast<int>(idx % D);
+  const long long bt = idx / D;
+  const int t = static_cast<int>(bt % N);
+  const long long b = bt / N;
+  const float pv = ldf(pos + static_cast<long long>(t) * D + d);
+  float v;
+  if (t == 0) v = ldf(cls + d);
+  else if (mask[b * (N - 1) + t - 1]) v = ldf(mask_token + d);
+  else v = ldf(x + idx);
+  stf(x + idx, v + pv);
+}
+
 // One thread per output element; weights are read with k fastest within a thread so consecutive
 // output channels do not coalesce — this entry point exists for API parity, the model path uses
 // patch_embed_tcgen05 (bf16) or patching + simt_gemm (fp32).
@@ -106,6 +126,26 @@ int embed_finalize(void* x, const void* pos, const void* cls, int B, int N, int 
     embed_finalize_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(
         static_cast<__nv_bfloat16*>(x), static_cast<const __nv_bfloat16*>(pos),
         static_cast<const __nv_bfloat16*>(cls), B, N, D);
+  else
+    return VT_ERR_DTYPE;
+  return static_cast<int>(cudaGetLastError());
+}
+
+int embed_finalize_masked(void* x, const void* pos, const void* cls, const void* mask_token, const void* mask, int B,
+                          int N, int D, int dtype, cudaStream_t stream) {
+  if (!x || !pos || !cls || !mask_token || !mask || B < 0 || N <= 0 || D <= 0) return VT_ERR_ARG;
+  const long long total = static_cast<long long>(B) * N * D;
+  if (total == 0) return VT_OK;
+  const unsigned grid = static_cast<unsigned>((total + 255) / 256);
+  const uint8_t* m = static_cast<const uint8_t*>(mask);
+  if (dtype == VT_F32)
+    embed_finalize_masked_kernel<float><<<grid, 256, 0, stream>>>(
+        static_cast<float*>(x), static_cast<const float*>(pos), static_cast<const float*>(cls),
+        static_cast<const float*>(mask_token), m, B, N, D);
+  else if (dtype == VT_BF16)
+    embed_finalize_masked_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(
+        static_cast<__nv_bfloat16*>(x), static_cast<const __nv_bfloat16*>(pos),
+        static_cast<const __nv_bfloat16*>(cls), static_cast<const __nv_bfloat16*>(mask_token), m, B, N, D);
   else
     return VT_ERR_DTYPE;
   return static_cast<int>(cudaGetLastError());

@@ -239,4 +239,95 @@ int patch_gather_ragged(const void* images, int n_images, int pix_dtype, int C, 
   return static_cast<int>(cudaGetLastError());
 }
 
+// ------------------------------------------------------------------------------------------------ masked batch
+// bool_masked_pos (vt_patch_embed_masked_gather): one block per unpadded output row (blockIdx.x = token, blockIdx.y =
+// image).  A masked patch's row is zero and its table row carries mask_token + pos - bias, so the plain-mode GEMM's
+// bias + residual epilogue turns it into mask_token + pos; an unmasked row is the batched gather's row and pos[t].
+namespace {
+
+struct MaskedParams {
+  const void* pixels;
+  const uint8_t* mask;
+  const uint4* pos;
+  const uint4* posm;
+  uint4* patches;
+  uint4* table;
+  int C, H, W, P, grid_w, n_patches, K, Kpad, D;
+};
+
+template <typename TPix, bool kVec>
+__global__ void __launch_bounds__(128)
+patch_gather_masked_kernel(const MaskedParams p) {
+  const int t = blockIdx.x;
+  const int b = blockIdx.y;
+  const int N = p.n_patches + 1;
+  const int patch = t > 0 ? t - 1 : 0;
+  const bool masked = t > 0 && p.mask[static_cast<long long>(b) * p.n_patches + patch] != 0;   // block-uniform
+  const bool real_row = t > 0 && !masked;
+  const int py = patch / p.grid_w, px = patch - py * p.grid_w;
+  const TPix* img = static_cast<const TPix*>(p.pixels) + static_cast<long long>(b) * p.C * p.H * p.W;
+  const long long row = static_cast<long long>(b) * N + t;
+
+  const int chunks_per_row = p.Kpad >> 3;
+  uint4* out_row = p.patches + row * chunks_per_row;
+  for (int kc = threadIdx.x; kc < chunks_per_row; kc += blockDim.x) {
+    const int k0 = kc << 3;
+    uint4 o = make_uint4(0u, 0u, 0u, 0u);
+    if (real_row && k0 < p.K) o = gather_chunk<TPix, kVec>(img, p.C, p.H, p.W, p.P, p.K, py, px, k0);
+    out_row[kc] = o;
+  }
+
+  const int dchunks = p.D >> 3;
+  const uint4* src = (masked ? p.posm : p.pos) + static_cast<long long>(t) * dchunks;
+  uint4* tab_row = p.table + row * dchunks;
+  for (int c = threadIdx.x; c < dchunks; c += blockDim.x) tab_row[c] = __ldg(src + c);
+}
+
+template <typename TPix, bool kVec>
+int launch_masked(const MaskedParams& p, int B, cudaStream_t stream) {
+  patch_gather_masked_kernel<TPix, kVec><<<dim3(p.n_patches + 1, B), 128, 0, stream>>>(p);
+  return static_cast<int>(cudaGetLastError());
+}
+
+}  // namespace
+
+int patch_gather_masked(const void* pixels, int pix_dtype, const void* mask, const void* pos, const void* posm,
+                        void* patches, long long ldw, void* table, int B, int C, int H, int W, int P, int D,
+                        cudaStream_t stream) {
+  if (!pixels || !mask || !pos || !posm || !patches || !table || B <= 0 || C <= 0 || P <= 0 || D <= 0 || H < P ||
+      W < P)
+    return VT_ERR_ARG;
+  const long long K = static_cast<long long>(C) * P * P;
+  if (ldw < K || ldw > 0x7fffffffLL) return VT_ERR_ARG;
+  if ((ldw % 8) || (D % 8)) return VT_ERR_ALIGN;
+  const long long n = static_cast<long long>(H / P) * (W / P);
+  if (B > 65535 || static_cast<long long>(B) * (n + 1) > 0x7fffffffLL) return VT_ERR_UNSUPPORTED;
+  if ((reinterpret_cast<uintptr_t>(pixels) | reinterpret_cast<uintptr_t>(patches) | reinterpret_cast<uintptr_t>(table) |
+       reinterpret_cast<uintptr_t>(pos) | reinterpret_cast<uintptr_t>(posm)) & 15)
+    return VT_ERR_ALIGN;
+  MaskedParams p;
+  p.pixels = pixels;
+  p.mask = static_cast<const uint8_t*>(mask);
+  p.pos = static_cast<const uint4*>(pos);
+  p.posm = static_cast<const uint4*>(posm);
+  p.patches = static_cast<uint4*>(patches);
+  p.table = static_cast<uint4*>(table);
+  p.C = C; p.H = H; p.W = W; p.P = P;
+  p.grid_w = W / P;
+  p.n_patches = static_cast<int>(n);
+  p.K = static_cast<int>(K);
+  p.Kpad = static_cast<int>(ldw);
+  p.D = D;
+  // the vector-load conditions of patch_gather
+  if (pix_dtype == VT_U8) {
+    const bool vec = ((P * C) % 8 == 0) && ((W * C) % 8 == 0);
+    return vec ? launch_masked<uint8_t, true>(p, B, stream) : launch_masked<uint8_t, false>(p, B, stream);
+  }
+  const bool vec = (P % 8 == 0) && (W % 8 == 0);
+  if (pix_dtype == VT_BF16)
+    return vec ? launch_masked<__nv_bfloat16, true>(p, B, stream) : launch_masked<__nv_bfloat16, false>(p, B, stream);
+  if (pix_dtype == VT_F32) return vec ? launch_masked<float, true>(p, B, stream) : launch_masked<float, false>(p, B, stream);
+  return VT_ERR_DTYPE;
+}
+
 }  // namespace vt

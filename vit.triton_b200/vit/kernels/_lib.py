@@ -1,5 +1,5 @@
-"""ctypes binding of libvitb200.so (C ABI declared in include/vitb200.h, include/vitb200_resolution.h and
-include/vitb200_ragged.h).
+"""ctypes binding of libvitb200.so (C ABI declared in include/vitb200.h, include/vitb200_resolution.h,
+include/vitb200_ragged.h and include/vitb200_mask.h).
 
 There is deliberately no fallback: if the shared library is missing or a tensor is not on a CUDA
 device the entry points raise.  The oracle under /oracle is test infrastructure and is never
@@ -82,6 +82,16 @@ RAGGED_SIGNATURES = {
     "vt_gather_rows": [_c_ptr, _c_i64, _c_ptr, _c_ptr, _c_i64, _c_i32, _c_i32, _c_i32, _c_ptr],
 }
 
+# name -> argtypes of the masked-input / masked-image-modeling entry points; mirrors include/vitb200_mask.h one to one
+# (tests/test_abi_mask.py checks both directions)
+MASK_SIGNATURES = {
+    "vt_patch_embed_masked_gather": [_c_ptr, _c_i32, _c_ptr, _c_ptr, _c_ptr, _c_ptr, _c_i64, _c_ptr, _c_i32, _c_i32,
+                                     _c_i32, _c_i32, _c_i32, _c_i32, _c_ptr],
+    "vt_embed_finalize_masked": [_c_ptr, _c_ptr, _c_ptr, _c_ptr, _c_ptr, _c_i32, _c_i32, _c_i32, _c_i32, _c_ptr],
+    "vt_mim_reconstruct": [_c_ptr, _c_ptr, _c_i32, _c_i32, _c_i32, _c_i32, _c_i32, _c_i32, _c_ptr, _c_i32, _c_ptr,
+                           _c_f32, _c_ptr, _c_ptr, _c_ptr, _c_ptr],
+}
+
 
 class RaggedImage(ctypes.Structure):
     """``vt_ragged_image`` of include/vitb200_ragged.h: one image of a ragged batch."""
@@ -109,7 +119,7 @@ def load() -> ctypes.CDLL:
             "(or `python -c 'import __graft_entry__ as g; g.build()'`). There is no CPU fallback.")
     lib = ctypes.CDLL(path)
     for name, argtypes in (list(SIGNATURES.items()) + list(RESOLUTION_SIGNATURES.items())
-                           + list(RAGGED_SIGNATURES.items())):
+                           + list(RAGGED_SIGNATURES.items()) + list(MASK_SIGNATURES.items())):
         fn = getattr(lib, name)
         fn.argtypes = argtypes
         fn.restype = ctypes.c_int

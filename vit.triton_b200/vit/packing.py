@@ -192,6 +192,15 @@ def _posb16(pos32: torch.Tensor, cls_token: torch.Tensor, bias32: torch.Tensor) 
     return t.to(torch.bfloat16).contiguous()
 
 
+def _posm16(pos32: torch.Tensor, mask_token: Optional[torch.Tensor], bias32: torch.Tensor) -> Optional[torch.Tensor]:
+    """bf16 [N, D] table of masked patches (``vt_patch_embed_masked_gather``): a masked patch's row is zero, so the GEMM
+    gives bias + this row, which must come out as mask_token + pos.  One rounding from fp32; row 0 is not read.  None
+    for a model without a mask token."""
+    if mask_token is None:
+        return None
+    return (pos32 + mask_token.detach().float().reshape(-1) - bias32).to(torch.bfloat16).contiguous()
+
+
 def pack_embeddings(emb) -> SimpleNamespace:
     w = emb.projection.weight.detach()
     D = w.shape[0]
@@ -205,7 +214,7 @@ def pack_embeddings(emb) -> SimpleNamespace:
     posb[1:] += emb.projection.bias.detach().float()
     bias32 = emb.projection.bias.detach().float().contiguous()
     return SimpleNamespace(w=w2d, ldw=kpad, K=K, posb=posb.contiguous(), bias32=bias32,
-                           posb16=_posb16(pos, emb.cls_token, bias32))
+                           posb16=_posb16(pos, emb.cls_token, bias32), posm16=_posm16(pos, emb.mask_token, bias32))
 
 
 def pack_embeddings_u8(emb, image_mean, image_std, rescale_factor: float) -> SimpleNamespace:
@@ -234,7 +243,7 @@ def pack_embeddings_u8(emb, image_mean, image_std, rescale_factor: float) -> Sim
     posb[1:] += emb.projection.bias.detach().float() - offset
     bias32 = (emb.projection.bias.detach().float() - offset).contiguous()
     return SimpleNamespace(w=w2d, ldw=kpad, K=K, posb=posb.contiguous(), bias32=bias32,
-                           posb16=_posb16(pos, emb.cls_token, bias32))
+                           posb16=_posb16(pos, emb.cls_token, bias32), posm16=_posm16(pos, emb.mask_token, bias32))
 
 
 def u8_pack(emb, image_mean, image_std, rescale_factor: float) -> tuple:
@@ -254,11 +263,12 @@ def u8_pack(emb, image_mean, image_std, rescale_factor: float) -> tuple:
 
 
 def patch_embed_u8(emb, x: torch.Tensor, image_mean, image_std, rescale_factor: float,
-                   stats: Optional[torch.Tensor] = None, interpolate: bool = False) -> torch.Tensor:
+                   stats: Optional[torch.Tensor] = None, interpolate: bool = False,
+                   mask: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Raw uint8 NHWC pixels (B, S, S, C) -> token embeddings (B, n+1, D), rescale + normalise + patch
     projection + CLS + position embeddings in ONE kernel (bf16 models on the tensor-core path).
     ``interpolate``: any (B, H, W, C) with H, W >= patch size, position table resampled to its patch grid
-    (``pos_grid``)."""
+    (``pos_grid``).  ``mask``: checked bool_masked_pos (B, n), masked patches take the mask token (``embed_masked``)."""
     w = emb.projection.weight
     assert x.is_cuda and x.dtype == torch.uint8 and x.dim() == 4, \
         f"Raw pixels need to be a CUDA uint8 (B, H, W, C) tensor, provided: {x.dtype}, {tuple(x.shape)}"
@@ -273,15 +283,22 @@ def patch_embed_u8(emb, x: torch.Tensor, image_mean, image_std, rescale_factor: 
     x = x.contiguous()
     n = emb.num_patches
     hw = posb16 = None
+    posm16 = pk.posm16
     if interpolate:
         grid = patch_grid(emb, S, S2)
         n = grid[0] * grid[1]
         hw = (S, S2)
         if grid != native_grid(emb):
-            posb16 = pos_grid(emb, *grid).token_table_u8(emb, image_mean, image_std, rescale_factor)
+            pg = pos_grid(emb, *grid)
+            posb16 = pg.token_table_u8(emb, image_mean, image_std, rescale_factor)
+            if mask is not None:
+                posm16 = pg.mask_table_u8(emb, image_mean, image_std, rescale_factor)
     n_tok = n + 1
     out = torch.empty((B, n_tok, emb.hidden_dim), device=x.device, dtype=w.dtype)
     if B == 0:
+        return out
+    if mask is not None:
+        embed_masked(emb, x, _lib.VT_U8, S, S2, mask, pk, pk.posb16 if posb16 is None else posb16, posm16, out, stats)
         return out
     stream = _lib.stream_ptr(x)
     step = _embed_batch_step(n)
@@ -429,11 +446,14 @@ def _embed_call(stats, b0, n_tok, dim, pk, pixels_ptr, pix_code, out_ptr, nb, C,
                   _lib.VT_BF16, s_ptr, nb, C, S, P, dim, stream)
 
 
-def patch_embed(emb, x: torch.Tensor, stats: Optional[torch.Tensor] = None, interpolate: bool = False) -> torch.Tensor:
+def patch_embed(emb, x: torch.Tensor, stats: Optional[torch.Tensor] = None, interpolate: bool = False,
+                mask: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Pixels (B, C, S, S) -> token embeddings (B, n+1, D) including CLS and position embeddings.
     ``stats``: optional (B * (n+1), D/128, 2) fp32 buffer for the row statistics the LayerNorm folded
     into the first QKV GEMM consumes (bf16 tensor-core path only).  ``interpolate``: pixels (B, C, H, W) at any
-    H, W >= patch size, n = (H // P) * (W // P), position table resampled to that grid (``pos_grid``)."""
+    H, W >= patch size, n = (H // P) * (W // P), position table resampled to that grid (``pos_grid``).
+    ``mask``: checked bool_masked_pos (B, n): masked patches take the mask token (``embed_masked`` on the bf16
+    tensor-core path, ``vt_embed_finalize_masked`` on the others)."""
     pk = emb.packed()
     w = emb.projection.weight
     B, C, S, S2 = x.shape
@@ -454,6 +474,10 @@ def patch_embed(emb, x: torch.Tensor, stats: Optional[torch.Tensor] = None, inte
     stream = _lib.stream_ptr(x)
 
     if w.dtype == torch.bfloat16 and D % 8 == 0 and x.dtype in (torch.float32, torch.bfloat16):
+        if mask is not None:
+            pos, posm = (pk.posb16, pk.posm16) if grid is None else (grid.token_table(emb), grid.mask_table(emb))
+            embed_masked(emb, x, _lib.dtype_code(x), S, S2, mask, pk, pos, posm, out, stats)
+            return out
         hw = (S, S2) if interpolate else None
         posb16 = None if grid is None else grid.token_table(emb)
         step = _embed_batch_step(n)
@@ -491,8 +515,84 @@ def patch_embed(emb, x: torch.Tensor, stats: Optional[torch.Tensor] = None, inte
         bg.bgemm(a.data_ptr(), wp.data_ptr(), out, out.data_ptr() + D * es, n, D, kk, B, 1, (n * kk, 0, kk),
                  (0, 0, kk), (n_tok * D, 0, D), bias32=pk.bias32)
     pos = emb.position_embeddings if grid is None else grid.pos
-    _lib.call("vt_embed_finalize", out.data_ptr(), pos.data_ptr(), emb.cls_token.data_ptr(), B, n_tok, D, code, stream)
+    finalize_embeddings(emb, out, pos, mask)
     return out
+
+
+def finalize_embeddings(emb, out: torch.Tensor, pos: torch.Tensor, mask: Optional[torch.Tensor]) -> None:
+    """CLS row and position add of embeddings (B, N, D) whose rows 1.. hold the patch projections, in place:
+    ``vt_embed_finalize``, or ``vt_embed_finalize_masked`` (masked patches take the mask token) with a mask."""
+    B, n_tok, D = out.shape
+    code, stream = _lib.dtype_code(out), _lib.stream_ptr(out)
+    if mask is None:
+        _lib.call("vt_embed_finalize", out.data_ptr(), pos.data_ptr(), emb.cls_token.data_ptr(), B, n_tok, D, code,
+                  stream)
+    else:
+        _lib.call("vt_embed_finalize_masked", out.data_ptr(), pos.data_ptr(), emb.cls_token.data_ptr(),
+                  emb.mask_token.data_ptr(), mask.contiguous().data_ptr(), B, n_tok, D, code, stream)
+
+
+# ------------------------------------------------------------------------------------------------ bool_masked_pos
+def check_mask(emb, mask, x, n_patches: int) -> None:
+    """Host-side checks of a ``bool_masked_pos`` for pixels ``x`` with ``n_patches`` patches per image, before anything
+    is launched."""
+    assert getattr(emb, "mask_token", None) is not None, \
+        "bool_masked_pos needs a model built with use_mask_token=True (or add_decoder=True)"
+    assert not isinstance(x, (list, tuple)), "bool_masked_pos is not supported with a list of images (ragged batch)"
+    assert isinstance(mask, torch.Tensor) and mask.dtype == torch.bool, \
+        f"bool_masked_pos must be a torch.bool tensor, provided: {getattr(mask, 'dtype', type(mask))}"
+    assert tuple(mask.shape) == (x.shape[0], n_patches), \
+        f"bool_masked_pos must be (batch, patches) = {(x.shape[0], n_patches)}, provided: {tuple(mask.shape)}"
+    assert mask.device == x.device, f"bool_masked_pos is on {mask.device}, the pixels on {x.device}"
+
+
+def embed_masked(emb, x: torch.Tensor, pix_code: int, H: int, W: int, mask: torch.Tensor, pk, pos: torch.Tensor,
+                 posm: torch.Tensor, out: torch.Tensor, stats: Optional[torch.Tensor]) -> None:
+    """Patch embedding with bool_masked_pos into ``out`` (B, N, D) (bf16 tensor-core path): per chunk of images one
+    ``vt_patch_embed_masked_gather`` (unpadded patch rows, masked ones zero, and a per-row table of ``pos`` / ``posm``
+    rows) and one plain-mode ``vt_gemm_bf16_ln`` with that table as its residual (and the row statistics into
+    ``stats``): the epilogue of the token-mode GEMM, so an all-false mask gives the unmasked call's output bit for
+    bit."""
+    B, n_tok, D = out.shape
+    x = x.contiguous()
+    mask = mask.contiguous()
+    stream = _lib.stream_ptr(out)
+    step = min(65535, RAGGED_MAX_ROWS // n_tok)           # the gather's grid.y and the GEMM's 32-bit row count
+    for b0 in range(0, B, step):
+        nb = min(step, B - b0)
+        rows = nb * n_tok
+        patches = torch.empty((rows, pk.ldw), device=out.device, dtype=torch.bfloat16)
+        table = torch.empty((rows, D), device=out.device, dtype=torch.bfloat16)
+        _lib.call("vt_patch_embed_masked_gather", x[b0:].data_ptr(), pix_code, mask[b0:].data_ptr(), pos.data_ptr(),
+                  posm.data_ptr(), patches.data_ptr(), pk.ldw, table.data_ptr(), nb, emb.channels, H, W,
+                  emb.patch_size, D, stream)
+        s_ptr = None if stats is None else stats[b0 * n_tok:].data_ptr()
+        _lib.call("vt_gemm_bf16_ln", patches.data_ptr(), pk.ldw, pk.w.data_ptr(), pk.ldw, out[b0:].data_ptr(), D,
+                  pk.bias32.data_ptr(), table.data_ptr(), D, rows, D, pk.ldw, 0, None, None, 0, 0.0, s_ptr, stream)
+
+
+def mim_reconstruct(dec: torch.Tensor, gh: int, gw: int, s: int, channels: int, pixels: Optional[torch.Tensor] = None,
+                    pix_code: int = 0, norm: Optional[torch.Tensor] = None, rescale: float = 1.0,
+                    mask: Optional[torch.Tensor] = None) -> tuple:
+    """Decoder output (B, 1 + gh * gw, s * s * C) -> (loss or None, reconstruction (B, C, gh * s, gw * s)) with one
+    ``vt_mim_reconstruct`` (PixelShuffle(s) of the patch rows; with ``mask`` also the masked L1 loss against
+    ``pixels``, a 0-dim fp32 device tensor, reduced in a fixed order)."""
+    B = dec.shape[0]
+    dec = dec.contiguous()
+    rec = torch.empty((B, channels, gh * s, gw * s), device=dec.device, dtype=dec.dtype)
+    loss = partial = None
+    if mask is not None:
+        loss = torch.empty((), device=dec.device, dtype=torch.float32)
+        partial = torch.empty((B * gh * gw,), device=dec.device, dtype=torch.float32)
+        pixels = pixels.contiguous()
+        mask = mask.contiguous()
+    if B:
+        _lib.call("vt_mim_reconstruct", dec.data_ptr(), rec.data_ptr(), _lib.dtype_code(dec), B, channels, gh, gw, s,
+                  _lib.ptr(pixels), pix_code, _lib.ptr(norm), float(rescale), _lib.ptr(mask), _lib.ptr(partial),
+                  _lib.ptr(loss), _lib.stream_ptr(dec))
+    elif loss is not None:
+        loss.zero_()
+    return loss, rec
 
 
 # ------------------------------------------------------------------------------------------------ any input resolution
@@ -533,7 +633,8 @@ class PosGrid:
     """Position tables of one non-native patch grid, all derived from one resample of the model's table:
     ``pos32`` fp32 [1 + n, D]; ``pos`` (1, 1 + n, D) in the model's dtype (``Embeddings.interpolate_pos_encoding``,
     and ``vt_embed_finalize`` of the fp32 / unfused paths); ``token_table`` / ``token_table_u8`` the bf16 tables of
-    the two-launch patch embedding (row 0 = cls + pos[0] - the pack's bias).  A table, once built, is never replaced
+    the two-launch patch embedding (row 0 = cls + pos[0] - the pack's bias); ``mask_table`` / ``mask_table_u8`` those
+    of masked patches (mask_token + pos - the pack's bias, ``embed_masked``).  A table, once built, is never replaced
     while this object lives: CUDA graphs keep reading it (see ``pos_grid``)."""
 
     def __init__(self, emb, gh: int, gw: int):
@@ -542,6 +643,8 @@ class PosGrid:
         self.pos = self.pos32.to(source.dtype)[None]
         self._plain = None
         self._u8 = {}
+        self._plain_masked = None
+        self._u8_masked = {}
 
     def token_table(self, emb) -> torch.Tensor:
         """bf16 table for pixels in NCHW (the pack ``emb.packed()``)."""
@@ -559,6 +662,24 @@ class PosGrid:
             _assert_not_capturing()
             with torch.no_grad():
                 table = self._u8[key] = _posb16(self.pos32, emb.cls_token, pk.bias32)
+        return table
+
+    def mask_table(self, emb) -> torch.Tensor:
+        """bf16 table of masked patches for pixels in NCHW (the pack ``emb.packed()``)."""
+        if self._plain_masked is None:
+            _assert_not_capturing()
+            with torch.no_grad():
+                self._plain_masked = _posm16(self.pos32, emb.mask_token, emb.packed().bias32)
+        return self._plain_masked
+
+    def mask_table_u8(self, emb, image_mean, image_std, rescale_factor: float) -> torch.Tensor:
+        """bf16 table of masked patches for raw uint8 NHWC pixels with these image-processor constants."""
+        key, pk = u8_pack(emb, image_mean, image_std, rescale_factor)
+        table = self._u8_masked.get(key)
+        if table is None:
+            _assert_not_capturing()
+            with torch.no_grad():
+                table = self._u8_masked[key] = _posm16(self.pos32, emb.mask_token, pk.bias32)
         return table
 
 

@@ -40,6 +40,9 @@ def _dense_mapping(num_layers: int) -> dict:
         'pooler.dense.bias': 'pooler.dense.bias',
         'classifier.weight': 'classifier.weight',     # ViTForImageClassification head, VIT(num_labels=...)
         'classifier.bias': 'classifier.bias',
+        'embeddings.mask_token': 'embeddings.mask_token',   # ViTModel(use_mask_token=True), VIT(use_mask_token=True)
+        'decoder.0.weight': 'decoder.0.weight',             # ViTForMaskedImageModeling, VIT(add_decoder=True)
+        'decoder.0.bias': 'decoder.0.bias',
     }
     for i in range(num_layers):
         pre = f'encoder.layer.{i}.'
@@ -59,7 +62,7 @@ def transfer_pretrained_weights(pretrained_model: torch.nn.Module, custom_model:
     """Copy every weight of a HuggingFace ``ViTModel`` into ``custom_model`` (a ``vit.vit.VIT``).
 
     Same call and result as the reference (utils.py:45-113); the layer count comes from the models.
-    Keys of the source may carry a ``vit.`` prefix (``ViTForImageClassification``).
+    Keys of the source may carry a ``vit.`` prefix (``ViTForImageClassification``, ``ViTForMaskedImageModeling``).
     """
     source = {(k[4:] if k.startswith('vit.') else k): v for k, v in pretrained_model.state_dict().items()}
     dest = custom_model.state_dict()

@@ -20,6 +20,7 @@ width can be set, and dtype / device follow the parameters instead of module-lev
 """
 import math
 import os
+from types import SimpleNamespace
 from typing import Optional
 
 import torch
@@ -296,7 +297,7 @@ class Encoder(nn.Module):
 class Embeddings(packing.PackedMixin, nn.Module):
     """Patch projection + CLS token + position embeddings (reference vit.py:173-200)."""
 
-    def __init__(self, patch_size, num_patches, patch_dim, hidden_dim, channels: int = 3):
+    def __init__(self, patch_size, num_patches, patch_dim, hidden_dim, channels: int = 3, use_mask_token: bool = False):
         super().__init__()
         self.patch_size = patch_size
         self.num_patches = num_patches
@@ -305,6 +306,8 @@ class Embeddings(packing.PackedMixin, nn.Module):
         self.channels = channels
 
         self.cls_token = nn.Parameter(torch.zeros((1, 1, hidden_dim)))
+        # HF ViTEmbeddings(use_mask_token=True): the embedding of a patch masked by bool_masked_pos
+        self.mask_token = nn.Parameter(torch.zeros(1, 1, hidden_dim)) if use_mask_token else None
         self.position_embeddings = nn.Parameter(torch.zeros(1, num_patches + 1, hidden_dim))
         self.projection = Conv2DTriton(
             in_channels=channels,
@@ -312,11 +315,16 @@ class Embeddings(packing.PackedMixin, nn.Module):
             kernel_size=(self.patch_size, self.patch_size)
         )
 
-    def forward(self, x, stats_out: Optional[torch.Tensor] = None, interpolate_pos_encoding: bool = False) -> torch.Tensor:
+    def forward(self, x, stats_out: Optional[torch.Tensor] = None, interpolate_pos_encoding: bool = False,
+                bool_masked_pos: Optional[torch.Tensor] = None) -> torch.Tensor:
         """``stats_out`` (optional, fused bf16 path only): (B * N, D/128, 2) fp32 buffer that receives the
         row statistics of the output for the LayerNorm folded into block 0's QKV GEMM.
         ``interpolate_pos_encoding``: (B, C, H, W) at any H, W >= patch size, N = 1 + (H // P) * (W // P), the
-        position table resampled to that grid (``interpolate_pos_encoding(H, W)``), like HF ``ViTEmbeddings``."""
+        position table resampled to that grid (``interpolate_pos_encoding(H, W)``), like HF ``ViTEmbeddings``.
+        ``bool_masked_pos``: bool (B, N - 1), needs ``use_mask_token=True``: a masked patch's embedding is the mask token
+        (plus its position embedding), like HF ``ViTEmbeddings``."""
+        if bool_masked_pos is not None:
+            self.check_mask(bool_masked_pos, x, x.shape[2], x.shape[3], interpolate_pos_encoding)
         if not (_FUSED and x.is_cuda):
             assert stats_out is None
             pos = self.position_embeddings
@@ -328,21 +336,27 @@ class Embeddings(packing.PackedMixin, nn.Module):
             out = torch.empty((x.shape[0], pos.shape[1], self.hidden_dim), device=x.device,
                               dtype=tokens.dtype)
             out[:, 1:, :] = tokens
-            _lib.call("vt_embed_finalize", out.data_ptr(), pos.data_ptr(),
-                      self.cls_token.data_ptr(), out.shape[0], out.shape[1], out.shape[2],
-                      _lib.dtype_code(out), _lib.stream_ptr(out))
+            packing.finalize_embeddings(self, out, pos, bool_masked_pos)
             return out
-        return packing.patch_embed(self, x, stats_out, interpolate=interpolate_pos_encoding)
+        return packing.patch_embed(self, x, stats_out, interpolate=interpolate_pos_encoding, mask=bool_masked_pos)
 
     def forward_uint8(self, x, image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
                       rescale_factor: float = 1.0 / 255.0, stats_out: Optional[torch.Tensor] = None,
-                      interpolate_pos_encoding: bool = False) -> torch.Tensor:
+                      interpolate_pos_encoding: bool = False,
+                      bool_masked_pos: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Raw uint8 NHWC pixels (B, H, W, C) -> embeddings: the image processor's rescale and
         normalisation (defaults: HF ``ViTImageProcessor`` of google/vit-base-patch16-224) are folded
-        into the patch projection, see ``packing.pack_embeddings_u8``.  ``interpolate_pos_encoding`` as for
-        ``forward``."""
+        into the patch projection, see ``packing.pack_embeddings_u8``.  ``interpolate_pos_encoding`` and
+        ``bool_masked_pos`` as for ``forward``."""
+        if bool_masked_pos is not None:
+            self.check_mask(bool_masked_pos, x, x.shape[1], x.shape[2], interpolate_pos_encoding)
         return packing.patch_embed_u8(self, x, image_mean, image_std, rescale_factor, stats_out,
-                                      interpolate=interpolate_pos_encoding)
+                                      interpolate=interpolate_pos_encoding, mask=bool_masked_pos)
+
+    def check_mask(self, bool_masked_pos, x, height: int, width: int, interpolate_pos_encoding: bool) -> None:
+        """AssertionError, before anything is launched, unless ``bool_masked_pos`` fits pixels ``x`` of that size."""
+        grid = packing.patch_grid(self, height, width)
+        packing.check_mask(self, bool_masked_pos, x, grid[0] * grid[1] if interpolate_pos_encoding else self.num_patches)
 
     def interpolate_pos_encoding(self, height: int, width: int) -> torch.Tensor:
         """(1, 1 + gh * gw, D) position table for a (height, width) input, gh = height // P, gw = width // P:
@@ -361,7 +375,8 @@ class Embeddings(packing.PackedMixin, nn.Module):
         self.__dict__.pop("_pos_grids", None)
 
     def _packed_sources(self):
-        return [self.cls_token, self.position_embeddings, self.projection.weight, self.projection.bias]
+        sources = [self.cls_token, self.position_embeddings, self.projection.weight, self.projection.bias]
+        return sources if self.mask_token is None else sources + [self.mask_token]
 
     def _build_packed(self):
         return packing.pack_embeddings(self)
@@ -406,6 +421,21 @@ class Pooler(nn.Module):
         return torch.tanh(self.dense(hidden_states[:, :1, :].contiguous())[:, 0, :])
 
 
+class DecoderConv(packing.PackedMixin, nn.Module):
+    """Parameters of HF ``ViTForMaskedImageModeling.decoder[0]``, the 1x1 ``Conv2d(D, s * s * C)`` in front of the
+    PixelShuffle: weight (s * s * C, D, 1, 1), bias (s * s * C,).  ``VIT.masked_image_modeling`` runs it as one GEMM over
+    the final hidden states (the weight reshaped to (s * s * C, D) is already K-major)."""
+
+    def __init__(self, hidden_dim: int, out_channels: int):
+        super().__init__()
+        self.weight = nn.Parameter(torch.zeros(out_channels, hidden_dim, 1, 1))
+        self.bias = nn.Parameter(torch.zeros(out_channels))
+
+    def _build_packed(self):
+        return SimpleNamespace(w=self.weight.detach().reshape(self.weight.shape[0], -1).contiguous(),
+                               b32=self.bias.detach().float().contiguous())
+
+
 class VIT(nn.Module):
     """ViT encoder returning the final-LayerNorm hidden states (B, N, D) — no pooler, like the
     reference (vit.py:203-247) and HF ``ViTModel(add_pooling_layer=False).last_hidden_state``."""
@@ -422,6 +452,9 @@ class VIT(nn.Module):
         mlp_dim: Optional[int] = None,
         add_pooling_layer: bool = False,
         num_labels: Optional[int] = None,
+        use_mask_token: bool = False,
+        add_decoder: bool = False,
+        encoder_stride: Optional[int] = None,
     ):
         super().__init__()
         assert height == width, "Height and width should be the same"
@@ -443,7 +476,8 @@ class VIT(nn.Module):
         d_out = self.hidden_dim // self.num_heads
 
         self.embeddings = Embeddings(patch_size=self.patch_size, num_patches=num_patches, patch_dim=patch_dim,
-                                     hidden_dim=self.hidden_dim, channels=self.channels)
+                                     hidden_dim=self.hidden_dim, channels=self.channels,
+                                     use_mask_token=use_mask_token or add_decoder)
         self.encoder = Encoder(num_layers=self.num_layers, num_heads=self.num_heads, hidden_dim=self.hidden_dim,
                                d_out=d_out, mlp_dim=mlp_dim)
         self.layernorm = LayerNormTriton(dim=self.hidden_dim, eps=1e-12)
@@ -452,6 +486,13 @@ class VIT(nn.Module):
         # optional HF ViTForImageClassification head (Linear on the CLS row of the final hidden states):
         # state-dict keys classifier.{weight,bias}
         self.classifier = LinearWithBias(self.hidden_dim, num_labels) if num_labels else None
+        # optional HF ViTForMaskedImageModeling (SimMIM) decoder, Conv2d(D, s^2 C, 1) + PixelShuffle(s) with s =
+        # encoder_stride (default: the patch size): state-dict keys decoder.0.{weight,bias}; implies the mask token
+        self.encoder_stride = patch_size if encoder_stride is None else encoder_stride
+        self.decoder = None
+        if add_decoder:
+            s = self.encoder_stride
+            self.decoder = nn.Sequential(DecoderConv(self.hidden_dim, s * s * self.channels), nn.PixelShuffle(s))
 
     def invalidate_packed(self) -> None:
         """Drop every derived weight (packed / LayerNorm-folded / uint8-scaled operands of all sub-modules
@@ -474,10 +515,15 @@ class VIT(nn.Module):
     def dtype(self) -> torch.dtype:
         return self.layernorm.weight.dtype
 
-    def forward(self, x, interpolate_pos_encoding: bool = False):
+    def forward(self, x, interpolate_pos_encoding: bool = False, bool_masked_pos: Optional[torch.Tensor] = None):
         """(B, C, H, W) -> final hidden states (B, N, D).  ``interpolate_pos_encoding`` (HF ``ViTModel``'s flag): any
         H, W >= patch size, square or not; N = 1 + (H // P) * (W // P), the position table resampled bicubically to
-        that grid (``Embeddings.interpolate_pos_encoding``).  Without it the input must be the model's size."""
+        that grid (``Embeddings.interpolate_pos_encoding``).  Without it the input must be the model's size.
+        ``bool_masked_pos`` (HF ``ViTModel``'s argument, needs ``use_mask_token=True``): bool (B, N - 1) on x's device,
+        True = the patch's embedding is replaced by the mask token.  Masked inputs take the gather + GEMM patch
+        embedding (``packing.embed_masked``); an all-false mask gives the unmasked result bit for bit."""
+        if bool_masked_pos is not None:
+            assert not isinstance(x, (list, tuple)), "bool_masked_pos is not supported with a list of images"
         if interpolate_pos_encoding:
             assert x.dim() == 4, f"Expected (B, C, H, W) pixels, provided: {tuple(x.shape)}"
             packing.check_any_size(self.embeddings, *x.shape[1:])
@@ -485,8 +531,12 @@ class VIT(nn.Module):
         else:
             assert x.shape[1:] == (self.channels, self.height, self.width), f"Image size {x.shape[1:]} not matching with the model input size: {self.channels, self.height, self.width}"
             n_tok = None
+        if bool_masked_pos is not None:
+            self.embeddings.check_mask(bool_masked_pos, x, x.shape[2], x.shape[3], interpolate_pos_encoding)
         stats = self._embed_stats(x, n_tok)
         kw = dict(interpolate_pos_encoding=True) if interpolate_pos_encoding else {}
+        if bool_masked_pos is not None:
+            kw["bool_masked_pos"] = bool_masked_pos
         x = self.embeddings(x, stats, **kw) if stats is not None else self.embeddings(x, **kw)
         x = self.encoder(x, stats) if stats is not None else self.encoder(x)
         x = self.layernorm(x)
@@ -509,11 +559,14 @@ class VIT(nn.Module):
                            dtype=torch.float32)
 
     def forward_uint8(self, x, image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
-                      rescale_factor: float = 1.0 / 255.0, interpolate_pos_encoding: bool = False):
+                      rescale_factor: float = 1.0 / 255.0, interpolate_pos_encoding: bool = False,
+                      bool_masked_pos: Optional[torch.Tensor] = None):
         """Forward from RAW uint8 NHWC pixels (B, H, W, C) — the step in front of the reference's
         ``forward``: rescale + normalise (HF ``ViTImageProcessor``) run inside the patch-embedding
-        kernel, so the host -> device copy is one byte per pixel value.  ``interpolate_pos_encoding`` as for
-        ``forward``."""
+        kernel, so the host -> device copy is one byte per pixel value.  ``interpolate_pos_encoding`` and
+        ``bool_masked_pos`` as for ``forward``."""
+        if bool_masked_pos is not None:
+            assert not isinstance(x, (list, tuple)), "bool_masked_pos is not supported with a list of images"
         if interpolate_pos_encoding:
             assert x.dim() == 4, f"Expected (B, H, W, C) pixels, provided: {tuple(x.shape)}"
             packing.check_any_size(self.embeddings, x.shape[3], x.shape[1], x.shape[2])
@@ -521,9 +574,12 @@ class VIT(nn.Module):
         else:
             assert tuple(x.shape[1:]) == (self.height, self.width, self.channels), f"Image size {x.shape[1:]} not matching with the model input size: {self.height, self.width, self.channels}"
             n_tok = None
+        if bool_masked_pos is not None:
+            self.embeddings.check_mask(bool_masked_pos, x, x.shape[1], x.shape[2], interpolate_pos_encoding)
         stats = self._embed_stats(x, n_tok)
         x = self.embeddings.forward_uint8(x, image_mean, image_std, rescale_factor, stats,
-                                          interpolate_pos_encoding=interpolate_pos_encoding)
+                                          interpolate_pos_encoding=interpolate_pos_encoding,
+                                          bool_masked_pos=bool_masked_pos)
         x = self.encoder(x, stats) if stats is not None else self.encoder(x)
         x = self.layernorm(x)
         return x
@@ -575,36 +631,99 @@ class VIT(nn.Module):
         hidden, layout = self._ragged_hidden(images, (0.5, 0.5, 0.5), (0.5, 0.5, 0.5), 1.0 / 255.0)
         return packing.gather_rows(hidden, layout.row0)
 
-    def _hidden(self, x, interpolate_pos_encoding: bool) -> torch.Tensor:
-        """Final hidden states of pixels (B, C, H, W) or raw uint8 (B, H, W, C)."""
+    def _hidden(self, x, interpolate_pos_encoding: bool, bool_masked_pos: Optional[torch.Tensor] = None,
+                image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
+                rescale_factor: float = 1.0 / 255.0) -> torch.Tensor:
+        """Final hidden states of pixels (B, C, H, W) or raw uint8 (B, H, W, C); a list of images (ragged batch) is
+        refused when a mask is given."""
+        assert bool_masked_pos is None or not isinstance(x, (list, tuple)), \
+            "bool_masked_pos is not supported with a list of images"
         kw = dict(interpolate_pos_encoding=True) if interpolate_pos_encoding else {}
-        return self.forward_uint8(x, **kw) if x.dtype == torch.uint8 else self.forward(x, **kw)
+        if bool_masked_pos is not None:
+            kw["bool_masked_pos"] = bool_masked_pos
+        if x.dtype == torch.uint8:
+            return self.forward_uint8(x, image_mean, image_std, rescale_factor, **kw)
+        return self.forward(x, **kw)
 
-    def pooler_output(self, x, interpolate_pos_encoding: bool = False) -> torch.Tensor:
+    def _cls_hidden(self, x, interpolate_pos_encoding: bool, bool_masked_pos) -> torch.Tensor:
+        """(B, N, D) final hidden states, or (B, 1, D) CLS rows of a list of images (ragged batch)."""
+        if isinstance(x, (list, tuple)):
+            assert bool_masked_pos is None, "bool_masked_pos is not supported with a list of images"
+            return self._ragged_cls(x)[:, None, :]
+        return self._hidden(x, interpolate_pos_encoding, bool_masked_pos)
+
+    def pooler_output(self, x, interpolate_pos_encoding: bool = False,
+                      bool_masked_pos: Optional[torch.Tensor] = None) -> torch.Tensor:
         """HF ``ViTModel(...).pooler_output``: tanh(dense(final hidden state of CLS)), (B, D).  ``x`` may also be a list
-        of images of different sizes (``forward_ragged``), each with its own patch grid."""
+        of images of different sizes (``forward_ragged``), each with its own patch grid (without a mask)."""
         assert self.pooler is not None, "Model was built without add_pooling_layer=True"
-        hidden = self._ragged_cls(x)[:, None, :] if isinstance(x, (list, tuple)) else self._hidden(x, interpolate_pos_encoding)
-        return self.pooler(hidden)
+        return self.pooler(self._cls_hidden(x, interpolate_pos_encoding, bool_masked_pos))
 
-    def logits(self, x, interpolate_pos_encoding: bool = False) -> torch.Tensor:
+    def logits(self, x, interpolate_pos_encoding: bool = False,
+               bool_masked_pos: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Class logits (B, num_labels) = classifier(final hidden states[:, 0]) — HF
         ``ViTForImageClassification(...).logits``; needs ``VIT(..., num_labels=...)``.  One tensor-core
         launch over the CLS rows of the final hidden states.  ``x`` may also be a list of images of different sizes
-        (``forward_ragged``), each with its own patch grid."""
+        (``forward_ragged``), each with its own patch grid (without a mask)."""
         assert self.classifier is not None, "VIT was built without a classifier head (num_labels)"
-        hidden = self._ragged_cls(x)[:, None, :] if isinstance(x, (list, tuple)) else self._hidden(x, interpolate_pos_encoding)
+        hidden = self._cls_hidden(x, interpolate_pos_encoding, bool_masked_pos)
         from .kernels import bgemm as bg
         return _head_on_cls(hidden, self.classifier, bg.ACT_NONE)
 
-    def pooled(self, x, interpolate_pos_encoding: bool = False) -> torch.Tensor:
+    def pooled(self, x, interpolate_pos_encoding: bool = False,
+               bool_masked_pos: Optional[torch.Tensor] = None) -> torch.Tensor:
         """CLS row of the final hidden states, (B, D): the tensor the data-parallel wrapper gathers.
         uint8 (B, H, W, C) inputs take the fused raw-pixel path.  ``x`` may also be a list of images of different sizes
-        (``forward_ragged``), each with its own patch grid."""
+        (``forward_ragged``), each with its own patch grid (without a mask)."""
         if isinstance(x, (list, tuple)):
+            assert bool_masked_pos is None, "bool_masked_pos is not supported with a list of images"
             return self._ragged_cls(x)
-        hidden = self._hidden(x, interpolate_pos_encoding)
+        hidden = self._hidden(x, interpolate_pos_encoding, bool_masked_pos)
         out = torch.empty((hidden.shape[0], hidden.shape[2]), device=hidden.device, dtype=hidden.dtype)
         _lib.call("vt_pool_cls", hidden.data_ptr(), out.data_ptr(), hidden.shape[0], hidden.shape[2],
                   hidden.stride(0), _lib.dtype_code(hidden), _lib.stream_ptr(hidden))
         return out
+
+    def masked_image_modeling(self, x, bool_masked_pos: Optional[torch.Tensor] = None,
+                              interpolate_pos_encoding: bool = False, image_mean=(0.5, 0.5, 0.5),
+                              image_std=(0.5, 0.5, 0.5), rescale_factor: float = 1.0 / 255.0) -> tuple:
+        """HF ``ViTForMaskedImageModeling`` (SimMIM): (loss or None, reconstruction (B, C, gh * s, gw * s)) like its
+        ``MaskedImageModelingOutput``; needs ``VIT(..., add_decoder=True)``, s = ``encoder_stride``.  ``x``: pixels
+        (B, C, H, W) or raw uint8 (B, H, W, C) (normalised with these image-processor constants, as ``forward_uint8``).
+
+        The decoder's 1x1 convolution is one GEMM over the final hidden states (CLS rows included), and one
+        ``vt_mim_reconstruct`` launch pixel-shuffles its patch rows into the reconstruction in the model's dtype; with
+        ``bool_masked_pos`` the same pass computes the masked L1 loss against the (normalised) input pixels, a 0-dim
+        fp32 device tensor reduced in a fixed order (no host synchronisation, the same bits on every call).  The loss
+        needs s == P and H, W multiples of P; the reconstruction works on any grid (HF only defines square ones)."""
+        assert self.decoder is not None, "VIT was built without the masked image modeling decoder (add_decoder=True)"
+        assert not isinstance(x, (list, tuple)), "masked_image_modeling takes a batch tensor, not a list of images"
+        u8 = x.dtype == torch.uint8
+        H, W = (x.shape[1], x.shape[2]) if u8 else (x.shape[2], x.shape[3])
+        s = self.encoder_stride
+        P = self.patch_size
+        if bool_masked_pos is not None:
+            assert s == P, f"The masked image modeling loss needs encoder_stride == patch_size, got {s} and {P}"
+            assert H % P == 0 and W % P == 0, f"The masked image modeling loss needs H, W multiples of {P}, got {(H, W)}"
+        hidden = self._hidden(x, interpolate_pos_encoding, bool_masked_pos, image_mean, image_std, rescale_factor)
+        gh, gw = packing.patch_grid(self.embeddings, H, W)
+        pk = self.decoder[0].packed()
+        dec = packing.linear(hidden, pk.w, pk.b32)
+        if bool_masked_pos is None:
+            return packing.mim_reconstruct(dec, gh, gw, s, self.channels)
+        norm = self._pixel_norm(image_mean, image_std, x.device) if u8 else None
+        pix_code = _lib.VT_U8 if u8 else _lib.dtype_code(x)
+        return packing.mim_reconstruct(dec, gh, gw, s, self.channels, x, pix_code, norm, rescale_factor,
+                                       bool_masked_pos)
+
+    def _pixel_norm(self, image_mean, image_std, device) -> torch.Tensor:
+        """fp32 [2C] device tensor (mean, std) of the image processor for the uint8 loss, built once per constants
+        (outside CUDA-graph capture: run the call once before capturing it)."""
+        key = (tuple(float(m) for m in image_mean), tuple(float(v) for v in image_std), str(device))
+        cache = self.__dict__.setdefault("_pixel_norms", {})
+        if key not in cache:
+            assert not torch.cuda.is_current_stream_capturing(), \
+                "new image-processor constants are uploaded outside CUDA-graph capture: run the call once first"
+            assert len(key[0]) == self.channels and len(key[1]) == self.channels
+            cache[key] = torch.tensor(key[0] + key[1], dtype=torch.float32, device=device)
+        return cache[key]

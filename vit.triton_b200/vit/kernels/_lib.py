@@ -1,5 +1,5 @@
 """ctypes binding of libvitb200.so (C ABI declared in include/vitb200.h, include/vitb200_resolution.h,
-include/vitb200_ragged.h and include/vitb200_mask.h).
+include/vitb200_ragged.h, include/vitb200_mask.h and include/vitb200_attn.h).
 
 There is deliberately no fallback: if the shared library is missing or a tensor is not on a CUDA
 device the entry points raise.  The oracle under /oracle is test infrastructure and is never
@@ -92,6 +92,12 @@ MASK_SIGNATURES = {
                            _c_f32, _c_ptr, _c_ptr, _c_ptr, _c_ptr],
 }
 
+# name -> argtypes of the attention-probabilities entry point; mirrors include/vitb200_attn.h one to one
+# (tests/test_abi_attn.py checks both directions)
+ATTN_SIGNATURES = {
+    "vt_attn_probs": [_c_ptr, _c_ptr, _c_ptr, _c_i32, _c_i32, _c_i32, _c_i32, _c_i64, _c_i64, _c_f32, _c_ptr],
+}
+
 
 class RaggedImage(ctypes.Structure):
     """``vt_ragged_image`` of include/vitb200_ragged.h: one image of a ragged batch."""
@@ -119,7 +125,8 @@ def load() -> ctypes.CDLL:
             "(or `python -c 'import __graft_entry__ as g; g.build()'`). There is no CPU fallback.")
     lib = ctypes.CDLL(path)
     for name, argtypes in (list(SIGNATURES.items()) + list(RESOLUTION_SIGNATURES.items())
-                           + list(RAGGED_SIGNATURES.items()) + list(MASK_SIGNATURES.items())):
+                           + list(RAGGED_SIGNATURES.items()) + list(MASK_SIGNATURES.items())
+                           + list(ATTN_SIGNATURES.items())):
         fn = getattr(lib, name)
         fn.argtypes = argtypes
         fn.restype = ctypes.c_int

@@ -21,7 +21,7 @@ width can be set, and dtype / device follow the parameters instead of module-lev
 import math
 import os
 from types import SimpleNamespace
-from typing import Optional
+from typing import NamedTuple, Optional, Tuple
 
 import torch
 from torch import nn
@@ -111,18 +111,23 @@ class SelfAttention(nn.Module):
         self.key = LinearWithBias(self.d_in, self.d_out)
         self.value = LinearWithBias(self.d_in, self.d_out)
 
-    def forward(self, x: torch.Tensor) -> torch.Tensor:
+    def forward(self, x: torch.Tensor, probs: Optional[list] = None) -> torch.Tensor:
+        """``probs``: a list that receives this head's attention probabilities (B, N, N)."""
         q = self.query(x)
         k_t = self.key(x).transpose(1, 2).contiguous()
         v = self.value(x)
-        probs = softmax(matmul3(q, k_t, apply_scaling=True, scale_factor=1 / math.sqrt(self.d_out)))
-        return matmul3(probs, v)
+        p = softmax(matmul3(q, k_t, apply_scaling=True, scale_factor=1 / math.sqrt(self.d_out)))
+        if probs is not None:
+            probs.append(p)
+        return matmul3(p, v)
 
 
-def _attention(qkv: torch.Tensor, num_heads: int, scale: float, groups=None) -> torch.Tensor:
-    """Fused attention of (B, N, 3D) rows, or of a packed ragged batch (1, M, 3D) when ``groups`` is given."""
+def _attention(qkv: torch.Tensor, num_heads: int, scale: float, groups=None, attn: Optional[list] = None) -> torch.Tensor:
+    """Fused attention of (B, N, 3D) rows, or of a packed ragged batch (1, M, 3D) when ``groups`` is given.  ``attn``: a
+    list that receives the attention probabilities (B, H, N, N) (not with ``groups``)."""
     if groups is None:
-        return flash_attention(qkv, num_heads, scale)
+        return flash_attention(qkv, num_heads, scale, probs=attn)
+    assert attn is None, "attention probabilities are not supported for a list of images"
     return packing.ragged_attention(qkv, num_heads, scale, groups)
 
 
@@ -139,21 +144,26 @@ class MultiHeadAttention(packing.PackedMixin, nn.Module):
         self.attention = nn.ModuleList([SelfAttention(d_in=d_in, d_out=d_out) for _ in range(self.num_heads)])
         self.output = LinearWithBias(self.d_in, self.d_in)
 
-    def forward(self, x: torch.Tensor, residual: Optional[torch.Tensor] = None, groups=None) -> torch.Tensor:
+    def forward(self, x: torch.Tensor, residual: Optional[torch.Tensor] = None, groups=None,
+                attn: Optional[list] = None) -> torch.Tensor:
         """x: (B, N, D).  ``residual`` (fused path only) is added in the out-projection epilogue.  ``groups`` (fused path
-        only): x is a packed ragged batch (1, M, D), attention per group of images (``packing.RaggedLayout.groups``)."""
+        only): x is a packed ragged batch (1, M, D), attention per group of images (``packing.RaggedLayout.groups``).
+        ``attn``: a list that receives the attention probabilities of all heads, (B, H, N, N)."""
         if not (_FUSED and x.is_cuda):
             assert residual is None
             heads_out = torch.empty_like(x)
+            heads_probs = None if attn is None else []
             for i, head in enumerate(self.attention):
-                heads_out[:, :, i * self.d_out:(i + 1) * self.d_out] = head(x)
+                heads_out[:, :, i * self.d_out:(i + 1) * self.d_out] = head(x, heads_probs)
+            if attn is not None:
+                attn.append(torch.stack(heads_probs, dim=1))
             return self.output(heads_out)
 
         pk = self.packed()
         B, N, D = x.shape
         x = x.contiguous()
         qkv = packing.linear(x, pk.wqkv, pk.bqkv)
-        ctx = _attention(qkv, self.num_heads, 1.0 / math.sqrt(self.d_out), groups)
+        ctx = _attention(qkv, self.num_heads, 1.0 / math.sqrt(self.d_out), groups, attn)
         return packing.linear(ctx, pk.wo, pk.bo, residual=residual)
 
     def _build_packed(self):
@@ -177,16 +187,17 @@ class Transformer(packing.PackedMixin, nn.Module):
         self.output = LinearWithBias(self.mlp_dim, self.d_in)
         self.layernorm_after = LayerNormTriton(self.d_in, eps=1e-12)
 
-    def forward(self, x, groups=None):
+    def forward(self, x, groups=None, attn: Optional[list] = None):
+        """``attn``: a list that receives the block's attention probabilities (B, H, N, N)."""
         if not (_FUSED and x.is_cuda):
             assert groups is None
-            res = add(self.attention(self.layernorm_before(x)), x)
+            res = add(self.attention(self.layernorm_before(x), attn=attn), x)
             out = self.output(self.intermediate(self.layernorm_after(res)))
             return add(out, res)
 
         pk = self.packed()
         x = x.contiguous()
-        res = self.attention(self.layernorm_before(x), residual=x, groups=groups)
+        res = self.attention(self.layernorm_before(x), residual=x, groups=groups, attn=attn)
         mid = packing.linear(self.layernorm_after(res), pk.w1, pk.b1, gelu=True)
         return packing.linear(mid, pk.w2, pk.b2, residual=res)
 
@@ -208,27 +219,28 @@ class Transformer(packing.PackedMixin, nn.Module):
     def _build_packed_fp8(self):
         return packing.pack_block_fp8(self)
 
-    def forward_fp8(self, x: torch.Tensor, groups=None) -> torch.Tensor:
+    def forward_fp8(self, x: torch.Tensor, groups=None, attn: Optional[list] = None) -> torch.Tensor:
         """Block forward with the QKV / fc1 / fc2 GEMMs on e4m3 operands (7 launches; see the note at _FP8).
-        ``groups``: as for ``MultiHeadAttention.forward``."""
+        ``groups``, ``attn``: as for ``MultiHeadAttention.forward``."""
         att = self.attention.packed()
         mlp = self.packed()
         q8 = self.packed("fp8")
         x = x.contiguous()
         qkv = packing.linear_fp8(packing.layernorm_fp8(x, self.layernorm_before), q8.wqkv8, q8.cqkv, att.bqkv)
-        ctx = _attention(qkv, self.num_heads, 1.0 / math.sqrt(self.d_out), groups)
+        ctx = _attention(qkv, self.num_heads, 1.0 / math.sqrt(self.d_out), groups, attn)
         res = packing.linear(ctx, att.wo, att.bo, residual=x)
         mid8 = packing.linear_fp8(packing.layernorm_fp8(res, self.layernorm_after), q8.w18, q8.c1, mlp.b1, gelu=True,
                                   out_fp8=True, out_scale=packing.FP8_MID_SCALE)
         return packing.linear_fp8(mid8, q8.w28, q8.c2, mlp.b2, residual=res)
 
-    def forward_folded(self, x: torch.Tensor, ln1_stats: Optional[torch.Tensor], groups=None):
+    def forward_folded(self, x: torch.Tensor, ln1_stats: Optional[torch.Tensor], groups=None,
+                       attn: Optional[list] = None):
         """Block forward with layernorm_before folded into the QKV GEMM (bf16 only).
 
         ``ln1_stats``: (M, D/128, 2) fp32 per-128-column (sum, M2) partials of x's rows, written by the
         previous block's last GEMM (None for the first block: layernorm_before then runs as a
         kernel).  Returns (output, statistics of the output rows).  5 launches per block (layernorm_after folded into
-        fc1 as well, the default) instead of 7.  ``groups``: as for ``MultiHeadAttention.forward``."""
+        fc1 as well, the default) instead of 7.  ``groups``, ``attn``: as for ``MultiHeadAttention.forward``."""
         att = self.attention.packed()
         mlp = self.packed()
         x = x.contiguous()
@@ -237,7 +249,7 @@ class Transformer(packing.PackedMixin, nn.Module):
         else:
             pk = self.packed("folded")
             qkv = packing.linear_ln(x, pk.wqkv, pk.bqkv, pk.cqkv, ln1_stats, self.layernorm_before.eps)
-        ctx = _attention(qkv, self.num_heads, 1.0 / math.sqrt(self.d_out), groups)
+        ctx = _attention(qkv, self.num_heads, 1.0 / math.sqrt(self.d_out), groups, attn)
         if _FOLD_LN_MLP:
             pk = self.packed("folded")
             stats2 = torch.empty((x.shape[0] * x.shape[1], self.d_in // packing.STATS_COLS, 2), device=x.device,
@@ -275,22 +287,33 @@ class Encoder(nn.Module):
         return bool(_FUSED and _FOLD_LN and not self.fp8_active(x) and len(self.layer) > 0 and x.numel() > 0 and
                     packing.folding_supported(x, self.hidden_dim, self.layer[0].mlp_dim))
 
-    def forward(self, x, ln1_stats: Optional[torch.Tensor] = None, groups=None) -> torch.Tensor:
+    def forward(self, x, ln1_stats: Optional[torch.Tensor] = None, groups=None, hidden: Optional[list] = None,
+                attn: Optional[list] = None) -> torch.Tensor:
         """``ln1_stats``: row statistics of x written by the patch-embedding epilogue (see
         ``Embeddings.forward``); without them block 0's layernorm_before runs as a kernel.  ``groups``: x is a
-        packed ragged batch (1, M, D) whose attention runs per group of images (``VIT.forward_ragged``)."""
+        packed ragged batch (1, M, D) whose attention runs per group of images (``VIT.forward_ragged``).
+        ``hidden``: a list that receives x and every block's output (the tensors themselves: each block writes a fresh
+        one); ``attn``: a list that receives every block's attention probabilities (B, H, N, N)."""
+        if hidden is not None:
+            hidden.append(x)
         if self.fp8_active(x):
             for layer in self.layer:
-                x = layer.forward_fp8(x, groups)
+                x = layer.forward_fp8(x, groups, attn)
+                if hidden is not None:
+                    hidden.append(x)
             return x
         if self.folding_active(x):
             # layernorm_before folded into the QKV GEMM; row statistics of each block's output are
             # produced by its last GEMM's epilogue
             for layer in self.layer:
-                x, ln1_stats = layer.forward_folded(x, ln1_stats, groups)
+                x, ln1_stats = layer.forward_folded(x, ln1_stats, groups, attn)
+                if hidden is not None:
+                    hidden.append(x)
             return x
         for layer in self.layer:
-            x = layer(x, groups)
+            x = layer(x, groups, attn)
+            if hidden is not None:
+                hidden.append(x)
         return x
 
 
@@ -436,6 +459,21 @@ class DecoderConv(packing.PackedMixin, nn.Module):
                                b32=self.bias.detach().float().contiguous())
 
 
+class VITOutput(NamedTuple):
+    """What ``VIT.forward`` / ``forward_uint8`` return when ``output_hidden_states`` or ``output_attentions`` is set, like
+    HF ``BaseModelOutput``; an unrequested field is None.  ``hidden_states``: num_layers + 1 tensors (B, N, D), the
+    embeddings and every block's output before the final LayerNorm.  ``attentions``: num_layers contiguous tensors
+    (B, H, N, N) of the model's dtype, softmax(scale * Q K^T) per head."""
+    last_hidden_state: torch.Tensor
+    hidden_states: Optional[Tuple[torch.Tensor, ...]] = None
+    attentions: Optional[Tuple[torch.Tensor, ...]] = None
+
+
+def _refuse_outputs(what: str, output_hidden_states: bool, output_attentions: bool) -> None:
+    assert not (output_hidden_states or output_attentions), \
+        f"output_hidden_states / output_attentions are not supported by {what}: call the model itself with them"
+
+
 class VIT(nn.Module):
     """ViT encoder returning the final-LayerNorm hidden states (B, N, D) — no pooler, like the
     reference (vit.py:203-247) and HF ``ViTModel(add_pooling_layer=False).last_hidden_state``."""
@@ -515,13 +553,21 @@ class VIT(nn.Module):
     def dtype(self) -> torch.dtype:
         return self.layernorm.weight.dtype
 
-    def forward(self, x, interpolate_pos_encoding: bool = False, bool_masked_pos: Optional[torch.Tensor] = None):
+    def forward(self, x, interpolate_pos_encoding: bool = False, bool_masked_pos: Optional[torch.Tensor] = None,
+                output_hidden_states: bool = False, output_attentions: bool = False):
         """(B, C, H, W) -> final hidden states (B, N, D).  ``interpolate_pos_encoding`` (HF ``ViTModel``'s flag): any
         H, W >= patch size, square or not; N = 1 + (H // P) * (W // P), the position table resampled bicubically to
         that grid (``Embeddings.interpolate_pos_encoding``).  Without it the input must be the model's size.
         ``bool_masked_pos`` (HF ``ViTModel``'s argument, needs ``use_mask_token=True``): bool (B, N - 1) on x's device,
         True = the patch's embedding is replaced by the mask token.  Masked inputs take the gather + GEMM patch
-        embedding (``packing.embed_masked``); an all-false mask gives the unmasked result bit for bit."""
+        embedding (``packing.embed_masked``); an all-false mask gives the unmasked result bit for bit.
+
+        ``output_hidden_states`` / ``output_attentions`` (HF ``ViTModel``'s flags): return a ``VITOutput`` instead of the
+        tensor, with every layer's hidden states and / or attention probabilities; the final hidden states are the
+        same bits as without them.  The hidden states are the tensors the forward computes anyway; on the fused bf16
+        path with head dim 64 or 80 each block's probabilities take one ``vt_attn_probs`` launch, elsewhere they are
+        the ones the attention materialises.  Not for a list of images."""
+        self._check_outputs(x, output_hidden_states, output_attentions)
         if bool_masked_pos is not None:
             assert not isinstance(x, (list, tuple)), "bool_masked_pos is not supported with a list of images"
         if interpolate_pos_encoding:
@@ -538,9 +584,28 @@ class VIT(nn.Module):
         if bool_masked_pos is not None:
             kw["bool_masked_pos"] = bool_masked_pos
         x = self.embeddings(x, stats, **kw) if stats is not None else self.embeddings(x, **kw)
-        x = self.encoder(x, stats) if stats is not None else self.encoder(x)
+        return self._encode(x, stats, output_hidden_states, output_attentions)
+
+    @staticmethod
+    def _check_outputs(x, output_hidden_states: bool, output_attentions: bool) -> None:
+        if output_hidden_states or output_attentions:
+            assert not isinstance(x, (list, tuple)), \
+                "output_hidden_states / output_attentions are not supported with a list of images"
+
+    def _encode(self, x: torch.Tensor, stats: Optional[torch.Tensor], output_hidden_states: bool,
+                output_attentions: bool):
+        """Encoder + final LayerNorm over the embeddings x: the final hidden states, or a ``VITOutput`` when a flag is set."""
+        kw = {}
+        if output_hidden_states:
+            kw["hidden"] = []
+        if output_attentions:
+            kw["attn"] = []
+        x = self.encoder(x, stats, **kw) if stats is not None else self.encoder(x, **kw)
         x = self.layernorm(x)
-        return x
+        if not kw:
+            return x
+        return VITOutput(x, tuple(kw["hidden"]) if output_hidden_states else None,
+                         tuple(kw["attn"]) if output_attentions else None)
 
     def _embed_stats(self, x: torch.Tensor, n_tok: Optional[int] = None) -> Optional[torch.Tensor]:
         """Buffer for the row statistics of the embeddings when block 0's layernorm_before is folded
@@ -560,11 +625,13 @@ class VIT(nn.Module):
 
     def forward_uint8(self, x, image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
                       rescale_factor: float = 1.0 / 255.0, interpolate_pos_encoding: bool = False,
-                      bool_masked_pos: Optional[torch.Tensor] = None):
+                      bool_masked_pos: Optional[torch.Tensor] = None, output_hidden_states: bool = False,
+                      output_attentions: bool = False):
         """Forward from RAW uint8 NHWC pixels (B, H, W, C) — the step in front of the reference's
         ``forward``: rescale + normalise (HF ``ViTImageProcessor``) run inside the patch-embedding
-        kernel, so the host -> device copy is one byte per pixel value.  ``interpolate_pos_encoding`` and
-        ``bool_masked_pos`` as for ``forward``."""
+        kernel, so the host -> device copy is one byte per pixel value.  ``interpolate_pos_encoding``,
+        ``bool_masked_pos``, ``output_hidden_states`` and ``output_attentions`` as for ``forward``."""
+        self._check_outputs(x, output_hidden_states, output_attentions)
         if bool_masked_pos is not None:
             assert not isinstance(x, (list, tuple)), "bool_masked_pos is not supported with a list of images"
         if interpolate_pos_encoding:
@@ -580,9 +647,7 @@ class VIT(nn.Module):
         x = self.embeddings.forward_uint8(x, image_mean, image_std, rescale_factor, stats,
                                           interpolate_pos_encoding=interpolate_pos_encoding,
                                           bool_masked_pos=bool_masked_pos)
-        x = self.encoder(x, stats) if stats is not None else self.encoder(x)
-        x = self.layernorm(x)
-        return x
+        return self._encode(x, stats, output_hidden_states, output_attentions)
 
     def forward_ragged(self, images, image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
                        rescale_factor: float = 1.0 / 255.0) -> list:
@@ -653,28 +718,34 @@ class VIT(nn.Module):
         return self._hidden(x, interpolate_pos_encoding, bool_masked_pos)
 
     def pooler_output(self, x, interpolate_pos_encoding: bool = False,
-                      bool_masked_pos: Optional[torch.Tensor] = None) -> torch.Tensor:
+                      bool_masked_pos: Optional[torch.Tensor] = None, output_hidden_states: bool = False,
+                      output_attentions: bool = False) -> torch.Tensor:
         """HF ``ViTModel(...).pooler_output``: tanh(dense(final hidden state of CLS)), (B, D).  ``x`` may also be a list
         of images of different sizes (``forward_ragged``), each with its own patch grid (without a mask)."""
+        _refuse_outputs("pooler_output", output_hidden_states, output_attentions)
         assert self.pooler is not None, "Model was built without add_pooling_layer=True"
         return self.pooler(self._cls_hidden(x, interpolate_pos_encoding, bool_masked_pos))
 
     def logits(self, x, interpolate_pos_encoding: bool = False,
-               bool_masked_pos: Optional[torch.Tensor] = None) -> torch.Tensor:
+               bool_masked_pos: Optional[torch.Tensor] = None, output_hidden_states: bool = False,
+               output_attentions: bool = False) -> torch.Tensor:
         """Class logits (B, num_labels) = classifier(final hidden states[:, 0]) — HF
         ``ViTForImageClassification(...).logits``; needs ``VIT(..., num_labels=...)``.  One tensor-core
         launch over the CLS rows of the final hidden states.  ``x`` may also be a list of images of different sizes
         (``forward_ragged``), each with its own patch grid (without a mask)."""
+        _refuse_outputs("logits", output_hidden_states, output_attentions)
         assert self.classifier is not None, "VIT was built without a classifier head (num_labels)"
         hidden = self._cls_hidden(x, interpolate_pos_encoding, bool_masked_pos)
         from .kernels import bgemm as bg
         return _head_on_cls(hidden, self.classifier, bg.ACT_NONE)
 
     def pooled(self, x, interpolate_pos_encoding: bool = False,
-               bool_masked_pos: Optional[torch.Tensor] = None) -> torch.Tensor:
+               bool_masked_pos: Optional[torch.Tensor] = None, output_hidden_states: bool = False,
+               output_attentions: bool = False) -> torch.Tensor:
         """CLS row of the final hidden states, (B, D): the tensor the data-parallel wrapper gathers.
         uint8 (B, H, W, C) inputs take the fused raw-pixel path.  ``x`` may also be a list of images of different sizes
         (``forward_ragged``), each with its own patch grid (without a mask)."""
+        _refuse_outputs("pooled", output_hidden_states, output_attentions)
         if isinstance(x, (list, tuple)):
             assert bool_masked_pos is None, "bool_masked_pos is not supported with a list of images"
             return self._ragged_cls(x)
@@ -686,7 +757,8 @@ class VIT(nn.Module):
 
     def masked_image_modeling(self, x, bool_masked_pos: Optional[torch.Tensor] = None,
                               interpolate_pos_encoding: bool = False, image_mean=(0.5, 0.5, 0.5),
-                              image_std=(0.5, 0.5, 0.5), rescale_factor: float = 1.0 / 255.0) -> tuple:
+                              image_std=(0.5, 0.5, 0.5), rescale_factor: float = 1.0 / 255.0,
+                              output_hidden_states: bool = False, output_attentions: bool = False) -> tuple:
         """HF ``ViTForMaskedImageModeling`` (SimMIM): (loss or None, reconstruction (B, C, gh * s, gw * s)) like its
         ``MaskedImageModelingOutput``; needs ``VIT(..., add_decoder=True)``, s = ``encoder_stride``.  ``x``: pixels
         (B, C, H, W) or raw uint8 (B, H, W, C) (normalised with these image-processor constants, as ``forward_uint8``).
@@ -696,6 +768,7 @@ class VIT(nn.Module):
         ``bool_masked_pos`` the same pass computes the masked L1 loss against the (normalised) input pixels, a 0-dim
         fp32 device tensor reduced in a fixed order (no host synchronisation, the same bits on every call).  The loss
         needs s == P and H, W multiples of P; the reconstruction works on any grid (HF only defines square ones)."""
+        _refuse_outputs("masked_image_modeling", output_hidden_states, output_attentions)
         assert self.decoder is not None, "VIT was built without the masked image modeling decoder (add_decoder=True)"
         assert not isinstance(x, (list, tuple)), "masked_image_modeling takes a batch tensor, not a list of images"
         u8 = x.dtype == torch.uint8

@@ -427,3 +427,48 @@ def test_fp8_path_parity_vs_hf(arch):
     cos, err = _cos(fp8, want), (fp8 - want).abs().max().item()
     print(f"fp8 {arch}: cosine {cos:.6f} max-abs {err:.4f} (bf16 path: {_cos(bf16, want):.6f} / {(bf16 - want).abs().max().item():.4f})")
     assert cos >= 0.995 and err <= 0.5, f"cosine {cos}, max-abs {err}"
+
+
+def _wide_model(dim, layers=2, seed=0):
+    """A VIT of width `dim` (64-wide heads, 32x32 images, 16-pixel patches) with the oracle's initialisation:
+    weights 0.02 randn, biases 0.02 randn, LayerNorm gamma 1 + 0.02 randn."""
+    from vit.vit import VIT
+    model = VIT(height=32, width=32, channels=3, patch_size=16, hidden_dim=dim, num_heads=dim // 64,
+                num_layers=layers, mlp_dim=4 * dim)
+    g = torch.Generator().manual_seed(seed)
+    with torch.no_grad():
+        for name, p in model.named_parameters():
+            noise = 0.02 * torch.randn(p.shape, generator=g)
+            p.copy_(1.0 + noise if "layernorm" in name and name.endswith("weight") else noise)
+    return model.to(DEV, torch.bfloat16).eval()
+
+
+def _fp8_and_bf16(model, x):
+    from vit import vit as vit_mod
+    try:
+        with torch.no_grad():
+            bf16 = model(x).float().cpu()
+            vit_mod.set_fp8(True)
+            fp8 = model(x).float().cpu()
+    finally:
+        vit_mod.set_fp8(False)
+    return fp8, bf16
+
+
+def test_fp8_path_at_width_1664():
+    """D = 1664 (ViT-bigG's width): vt_layernorm_fp8 runs at 7 vectors per lane; the FP8 forward meets the FP8 gate
+    (cosine >= 0.995, max-abs <= 0.5) against the bf16 forward of the same model."""
+    model = _wide_model(1664)
+    x = torch.randn(3, 3, 32, 32, generator=torch.Generator().manual_seed(1)).to(DEV, torch.bfloat16)
+    fp8, bf16 = _fp8_and_bf16(model, x)
+    assert torch.isfinite(fp8).all() and not torch.equal(fp8, bf16)
+    cos, err = _cos(fp8, bf16), (fp8 - bf16).abs().max().item()
+    assert cos >= 0.995 and err <= 0.5, f"cosine {cos}, max-abs {err}"
+
+
+def test_fp8_path_above_width_2048_takes_the_bf16_path():
+    """D > 2048 has no e4m3 LayerNorm: set_fp8(True) runs the bf16 forward, bit for bit."""
+    model = _wide_model(2176)
+    x = torch.randn(2, 3, 32, 32, generator=torch.Generator().manual_seed(2)).to(DEV, torch.bfloat16)
+    fp8, bf16 = _fp8_and_bf16(model, x)
+    assert torch.equal(fp8, bf16)

@@ -3,6 +3,7 @@ data-parallel gather over a 2-process gloo group (the same code path NCCL drives
 import os
 import socket
 import sys
+from types import SimpleNamespace
 
 import pytest
 import torch
@@ -272,6 +273,43 @@ def test_zero_sum_layernorm_fold_packing(K, N):
     err_z = ((got_z - want).norm() / want.norm()).item()
     err_c = ((got_c - want).norm() / want.norm()).item()
     assert err_z <= 1.1 * err_c + 1e-5 and err_z <= 2e-3
+
+
+@pytest.mark.parametrize("arch", ["vit-b16-224", "vit-l16-224", "vit-h14-224"])
+def test_fp8_layernorm_scale_never_saturates(arch):
+    """packing.fp8_ln_scale on the oracle's LayerNorms (bf16, as the FP8 path stores them): every output element of
+    e4m3(LN(x) * scale) is at most B * scale <= 448 with B = max|gamma| sqrt(D - 1) + max|beta|; the scale is the
+    largest power of two <= 16 that allows it, so a LayerNorm with B <= 28 / (1 + 2^-10) keeps 16."""
+    import math
+    hf = hf_oracle.build_hf(arch)
+    lns = [m for name, m in hf.named_modules() if isinstance(m, torch.nn.LayerNorm)]
+    assert len(lns) == 2 * hf.config.num_hidden_layers + 1
+    margin = 1 + 2.0 ** -10
+    for ln in lns:
+        ln16 = torch.nn.LayerNorm(ln.normalized_shape, eps=ln.eps).bfloat16()
+        with torch.no_grad():
+            ln16.weight.copy_(ln.weight)
+            ln16.bias.copy_(ln.bias)
+        D = ln16.weight.numel()
+        B = ln16.weight.double().abs().max().item() * math.sqrt(D - 1) + ln16.bias.double().abs().max().item()
+        scale = packing.fp8_ln_scale(ln16)
+        assert scale <= 16 and math.log2(scale).is_integer()
+        assert B * margin * scale <= 448 and (scale == 16 or B * margin * scale * 2 > 448)
+        if B <= 28 / margin:
+            assert scale == 16
+    # gamma = 1, beta = 0 at D = 768: B = sqrt(767) = 27.7 keeps 16; a tenth more gamma halves it
+    unit = torch.nn.LayerNorm(768).bfloat16()
+    assert packing.fp8_ln_scale(unit) == 16
+    with torch.no_grad():
+        unit.weight.fill_(1.1)
+    assert packing.fp8_ln_scale(unit) == 8
+
+
+def test_fp8_path_limited_to_layernorm_rows_in_registers():
+    """vt_layernorm_fp8 has instances up to D = 2048: wider models take the bf16 path."""
+    x = SimpleNamespace(is_cuda=True, dtype=torch.bfloat16)      # fp8_supported reads only these two
+    for dim, ok in ((768, True), (1664, True), (2048, True), (2064, False), (4096, False)):
+        assert packing.fp8_supported(x, dim, 4 * dim) == ok, dim
 
 
 def test_bench_dump_outputs_float32_and_bounded(tmp_path):

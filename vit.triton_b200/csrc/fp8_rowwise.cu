@@ -5,8 +5,9 @@
 //                    vit/kernels/layernorm.py:51-85, with the quantisation of the GEMM operand fused in)
 //   quantize_rows    w8[n,:] = e4m3( w[n,:] / s_n ),  s_n = amax_k |w[n,k]| / 448   (pack time, per output channel)
 //
-// |LN(x)| <= sqrt(dim - 1) < 448 / 16 for dim <= 785, so out_scale = 16 uses the e4m3 range without ever saturating
-// for ViT-B; the cast saturates anyway (satfinite).
+// |LN(x)_i| <= sqrt(dim - 1) (Samuelson), so |gamma_i LN(x)_i + beta_i| <= max|gamma| sqrt(dim - 1) + max|beta|; the
+// host picks out_scale per LayerNorm from that bound (packing.fp8_ln_scale: a power of two, at most 16) so that no
+// element saturates.  The cast saturates anyway (satfinite).  dim <= 2048 (VPL <= 8).
 #include "common.cuh"
 
 namespace vt {
@@ -91,7 +92,10 @@ quantize_rows_e4m3_kernel(const __nv_bfloat16* __restrict__ w, long long ldw, ui
   float amax = 0.f;
   for (int k = lane; k < K; k += 32) amax = fmaxf(amax, fabsf(__bfloat162float(wr[k])));
   amax = warp_max(amax);
-  const float s = amax > 0.f ? amax / 448.0f : 1.0f;
+  // a zero or subnormal amax / 448 has no usable reciprocal (1 / s overflows to inf, 0 * inf = NaN); such a row
+  // (amax < 448 * 2^-126) quantises to zero codes with s = 1
+  const float s0 = amax / 448.0f;
+  const float s = s0 >= 0x1p-126f ? s0 : 1.0f;
   const float inv = 1.0f / s;
   if (lane == 0) scales[n] = s;
   uint8_t* orow = out + static_cast<long long>(n) * ldo;
@@ -124,7 +128,7 @@ int layernorm_e4m3(const void* x, const void* gamma, const void* beta, void* out
                                                        out_scale);                                                \
     break;
   switch (vpl) {
-    VT_LN8_CASE(1) VT_LN8_CASE(2) VT_LN8_CASE(3) VT_LN8_CASE(4) VT_LN8_CASE(5) VT_LN8_CASE(6) VT_LN8_CASE(8)
+    VT_LN8_CASE(1) VT_LN8_CASE(2) VT_LN8_CASE(3) VT_LN8_CASE(4) VT_LN8_CASE(5) VT_LN8_CASE(6) VT_LN8_CASE(7) VT_LN8_CASE(8)
     default: return VT_ERR_UNSUPPORTED;
   }
 #undef VT_LN8_CASE

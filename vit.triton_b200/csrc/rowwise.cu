@@ -83,19 +83,23 @@ layernorm_rows_kernel(const T* __restrict__ x, const T* __restrict__ gamma,
       for (int e = 0; e < EV; ++e) sum += d[i].v[e];
     }
   }
-  const float mean = warp_sum(sum) / static_cast<float>(dim);
-  float sq = 0.f;
+  const float mean0 = warp_sum(sum) / static_cast<float>(dim);
+  float sq = 0.f, sc = 0.f;
 #pragma unroll
   for (int i = 0; i < VPL; ++i) {
     const int vi = lane + i * 32;
     if (vi < nvec) {
 #pragma unroll
       for (int e = 0; e < EV; ++e) {
-        const float c = d[i].v[e] - mean;
+        const float c = d[i].v[e] - mean0;
+        sc += c;
         sq += c * c;
       }
     }
   }
+  // sum / dim of fp32 values is not exact: the centred sum corrects it, so that a row of one repeated value gives
+  // x - mean = 0 exactly (beta) instead of beta + gamma * (rounding residue) * rstd
+  const float mean = mean0 + warp_sum(sc) / static_cast<float>(dim);
   const float var = warp_sum(sq) / static_cast<float>(dim);
   const float rstd = 1.0f / sqrtf(var + eps);
 
@@ -207,12 +211,14 @@ layernorm_generic_kernel(const T* __restrict__ x, const T* __restrict__ gamma,
   const T* xr = x + row * in_stride;
   float sum = 0.f;
   for (int i = lane; i < dim; i += 32) sum += to_f(xr[i]);
-  const float mean = warp_sum(sum) / static_cast<float>(dim);
-  float sq = 0.f;
+  const float mean0 = warp_sum(sum) / static_cast<float>(dim);
+  float sq = 0.f, sc = 0.f;
   for (int i = lane; i < dim; i += 32) {
-    const float c = to_f(xr[i]) - mean;
+    const float c = to_f(xr[i]) - mean0;
+    sc += c;
     sq += c * c;
   }
+  const float mean = mean0 + warp_sum(sc) / static_cast<float>(dim);   // as in layernorm_rows_kernel
   const float rstd = 1.0f / sqrtf(warp_sum(sq) / static_cast<float>(dim) + eps);
   TO* orow = out + row * out_stride;
   for (int i = lane; i < dim; i += 32)

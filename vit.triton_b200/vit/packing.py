@@ -130,12 +130,28 @@ def pack_block_folded(block) -> SimpleNamespace:
 
 
 # ------------------------------------------------------------------------------------------------ FP8 (optional)
-FP8_ACT_SCALE = 16.0     # LayerNorm outputs are quantised as e4m3(y * 16): |LN(x)| <= sqrt(dim - 1), 448 / 16 = 28
+FP8_ACT_SCALE = 16.0     # LayerNorm outputs are quantised as e4m3(y * scale), scale <= 16 (fp8_ln_scale)
 FP8_MID_SCALE = 8.0      # GELU outputs (fc2's operand) as e4m3(g * 8), saturating at |g| = 56
+FP8_LN_MAX_DIM = 2048    # vt_layernorm_fp8 keeps a row in registers: at most 8 16-byte vectors per lane
 
 
 def fp8_supported(x: torch.Tensor, dim: int, mlp_dim: int) -> bool:
-    return x.is_cuda and x.dtype == torch.bfloat16 and dim % 16 == 0 and mlp_dim % 128 == 0
+    return (x.is_cuda and x.dtype == torch.bfloat16 and dim % 16 == 0 and dim <= FP8_LN_MAX_DIM
+            and mlp_dim % 128 == 0)
+
+
+def fp8_ln_scale(ln) -> float:
+    """Activation scale of the e4m3 output of LayerNorm ``ln``: the largest power of two <= FP8_ACT_SCALE at which no
+    element can saturate.  Every output element satisfies |gamma_i y_i + beta_i| <= B = max|gamma| sqrt(D - 1) +
+    max|beta|, because a normalised row has |y_i| <= sqrt(D - 1) (Samuelson's inequality); B * (1 + 2^-10) * scale
+    <= 448 leaves room for the kernel's fp32 rounding of y.  A power of two changes no e4m3 code that stays in the
+    normal range, so a LayerNorm with B <= 28 / (1 + 2^-10) keeps the scale 16."""
+    gamma = ln.weight.detach().double()
+    beta = ln.bias.detach().double()
+    bound = gamma.abs().max().item() * math.sqrt(gamma.numel() - 1) + beta.abs().max().item()
+    if bound == 0.0:
+        return FP8_ACT_SCALE
+    return min(FP8_ACT_SCALE, 2.0 ** math.floor(math.log2(448.0 / (bound * (1.0 + 2.0 ** -10)))))
 
 
 def quantize_weight_fp8(w_nk: torch.Tensor) -> tuple:
@@ -151,14 +167,18 @@ def quantize_weight_fp8(w_nk: torch.Tensor) -> tuple:
 
 def pack_block_fp8(block) -> SimpleNamespace:
     """e4m3 weights of the QKV / fc1 / fc2 layers of one block with their per-channel dequantisation scales,
-    the activation scales already divided out (the GEMM epilogue is acc * colscale + bias)."""
+    the activation scales already divided out (the GEMM epilogue is acc * colscale + bias); ``ln1_scale`` /
+    ``ln2_scale`` are the e4m3 scales of layernorm_before / layernorm_after (fp8_ln_scale)."""
     att = block.attention.packed()
     mlp = block.packed()
     wqkv8, sqkv = quantize_weight_fp8(att.wqkv)
     w18, s1 = quantize_weight_fp8(mlp.w1)
     w28, s2 = quantize_weight_fp8(mlp.w2)
-    return SimpleNamespace(wqkv8=wqkv8, cqkv=(sqkv / FP8_ACT_SCALE).contiguous(), w18=w18,
-                           c1=(s1 / FP8_ACT_SCALE).contiguous(), w28=w28, c2=(s2 / FP8_MID_SCALE).contiguous())
+    ln1_scale = fp8_ln_scale(block.layernorm_before)
+    ln2_scale = fp8_ln_scale(block.layernorm_after)
+    return SimpleNamespace(wqkv8=wqkv8, cqkv=(sqkv / ln1_scale).contiguous(), w18=w18,
+                           c1=(s1 / ln2_scale).contiguous(), w28=w28, c2=(s2 / FP8_MID_SCALE).contiguous(),
+                           ln1_scale=ln1_scale, ln2_scale=ln2_scale)
 
 
 def layernorm_fp8(x: torch.Tensor, ln, scale: float = FP8_ACT_SCALE) -> torch.Tensor:

@@ -226,11 +226,12 @@ class Transformer(packing.PackedMixin, nn.Module):
         mlp = self.packed()
         q8 = self.packed("fp8")
         x = x.contiguous()
-        qkv = packing.linear_fp8(packing.layernorm_fp8(x, self.layernorm_before), q8.wqkv8, q8.cqkv, att.bqkv)
+        qkv = packing.linear_fp8(packing.layernorm_fp8(x, self.layernorm_before, q8.ln1_scale), q8.wqkv8, q8.cqkv,
+                                 att.bqkv)
         ctx = _attention(qkv, self.num_heads, 1.0 / math.sqrt(self.d_out), groups, attn)
         res = packing.linear(ctx, att.wo, att.bo, residual=x)
-        mid8 = packing.linear_fp8(packing.layernorm_fp8(res, self.layernorm_after), q8.w18, q8.c1, mlp.b1, gelu=True,
-                                  out_fp8=True, out_scale=packing.FP8_MID_SCALE)
+        mid8 = packing.linear_fp8(packing.layernorm_fp8(res, self.layernorm_after, q8.ln2_scale), q8.w18, q8.c1,
+                                  mlp.b1, gelu=True, out_fp8=True, out_scale=packing.FP8_MID_SCALE)
         return packing.linear_fp8(mid8, q8.w28, q8.c2, mlp.b2, residual=res)
 
     def forward_folded(self, x: torch.Tensor, ln1_stats: Optional[torch.Tensor], groups=None,

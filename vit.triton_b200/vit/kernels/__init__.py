@@ -9,6 +9,7 @@ from .layernorm import LayerNormTriton, LayerNormB200, layernorm
 from .matmul3 import matmul3
 from .conv2d import Conv2DTriton, Conv2DB200, conv2d
 from .attention import flash_attention
+from .resize import resize_uint8
 
 # reference-style aliases (the reference imports e.g. `matmul_triton as matmul`)
 matmul_triton = matmul

@@ -1,5 +1,5 @@
 """ctypes binding of libvitb200.so (C ABI declared in include/vitb200.h, include/vitb200_resolution.h,
-include/vitb200_ragged.h, include/vitb200_mask.h and include/vitb200_attn.h).
+include/vitb200_ragged.h, include/vitb200_mask.h, include/vitb200_attn.h and include/vitb200_preprocess.h).
 
 There is deliberately no fallback: if the shared library is missing or a tensor is not on a CUDA
 device the entry points raise.  The oracle under /oracle is test infrastructure and is never
@@ -98,11 +98,25 @@ ATTN_SIGNATURES = {
     "vt_attn_probs": [_c_ptr, _c_ptr, _c_ptr, _c_i32, _c_i32, _c_i32, _c_i32, _c_i64, _c_i64, _c_f32, _c_ptr],
 }
 
+# name -> argtypes of the image-processor resize entry points; mirrors include/vitb200_preprocess.h one to one
+# (tests/test_abi_preprocess.py checks both directions)
+PREPROCESS_SIGNATURES = {
+    "vt_resize_u8": [_c_ptr, _c_i32, _c_i32, _c_i32, _c_i32, _c_i64, _c_ptr, _c_i32, _c_ptr, _c_i32, _c_ptr, _c_i32,
+                     _c_i32, _c_ptr],
+    "vt_resize_u8_list": [_c_ptr, _c_i32, _c_i32, _c_ptr, _c_ptr, _c_i32, _c_i32, _c_ptr],
+}
+
 
 class RaggedImage(ctypes.Structure):
     """``vt_ragged_image`` of include/vitb200_ragged.h: one image of a ragged batch."""
     _fields_ = [("pixels", _c_ptr), ("pos", _c_ptr), ("row0", _c_i64), ("height", _c_i32), ("width", _c_i32),
                 ("tokens", _c_i32), ("reserved", _c_i32)]
+
+
+class ResizeImage(ctypes.Structure):
+    """``vt_resize_image`` of include/vitb200_preprocess.h: one image of a resize list."""
+    _fields_ = [("pixels", _c_ptr), ("htab", _c_i64), ("vtab", _c_i64), ("height", _c_i32), ("width", _c_i32),
+                ("hk", _c_i32), ("vk", _c_i32)]
 
 
 def lib_path() -> str:
@@ -126,7 +140,7 @@ def load() -> ctypes.CDLL:
     lib = ctypes.CDLL(path)
     for name, argtypes in (list(SIGNATURES.items()) + list(RESOLUTION_SIGNATURES.items())
                            + list(RAGGED_SIGNATURES.items()) + list(MASK_SIGNATURES.items())
-                           + list(ATTN_SIGNATURES.items())):
+                           + list(ATTN_SIGNATURES.items()) + list(PREPROCESS_SIGNATURES.items())):
         fn = getattr(lib, name)
         fn.argtypes = argtypes
         fn.restype = ctypes.c_int

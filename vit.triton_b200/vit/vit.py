@@ -627,11 +627,17 @@ class VIT(nn.Module):
     def forward_uint8(self, x, image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
                       rescale_factor: float = 1.0 / 255.0, interpolate_pos_encoding: bool = False,
                       bool_masked_pos: Optional[torch.Tensor] = None, output_hidden_states: bool = False,
-                      output_attentions: bool = False):
+                      output_attentions: bool = False, do_resize: bool = False, resample: int = 2):
         """Forward from RAW uint8 NHWC pixels (B, H, W, C) — the step in front of the reference's
         ``forward``: rescale + normalise (HF ``ViTImageProcessor``) run inside the patch-embedding
         kernel, so the host -> device copy is one byte per pixel value.  ``interpolate_pos_encoding``,
-        ``bool_masked_pos``, ``output_hidden_states`` and ``output_attentions`` as for ``forward``."""
+        ``bool_masked_pos``, ``output_hidden_states`` and ``output_attentions`` as for ``forward``.
+
+        ``do_resize`` / ``resample`` (HF ``ViTImageProcessor``'s names): first resize x, a uint8 (B, H, W, C) batch of any
+        size or a list of (H_i, W_i, C) images of any sizes, to the model's size like ``PIL.Image.resize`` (2 = BILINEAR,
+        3 = BICUBIC; ``kernels.resize_uint8``), then run on that (B, height, width, C) batch: the call equals
+        ``forward_uint8(resize_uint8(x, height, width, resample), ...)`` bit for bit."""
+        x = self._resized(x, do_resize, resample)
         self._check_outputs(x, output_hidden_states, output_attentions)
         if bool_masked_pos is not None:
             assert not isinstance(x, (list, tuple)), "bool_masked_pos is not supported with a list of images"
@@ -649,6 +655,19 @@ class VIT(nn.Module):
                                           interpolate_pos_encoding=interpolate_pos_encoding,
                                           bool_masked_pos=bool_masked_pos)
         return self._encode(x, stats, output_hidden_states, output_attentions)
+
+    def _resized(self, x, do_resize: bool, resample: int):
+        """x itself, or with ``do_resize`` the uint8 (B, height, width, C) batch ``resize_uint8`` makes of x (a batch already
+        of the model's size is x itself).  AssertionError, before anything is launched, for pixels that are not uint8,
+        another channel count than the model's, an empty list, mixed devices, a side < 1 or an unsupported filter."""
+        if not do_resize:
+            return x
+        from .kernels.resize import check_images, check_resample, resize_uint8
+        resample = check_resample(resample)
+        is_list, _ = check_images(x, self.channels)
+        if not is_list and tuple(x.shape[1:3]) == (self.height, self.width):
+            return x
+        return resize_uint8(x, self.height, self.width, resample)
 
     def forward_ragged(self, images, image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
                        rescale_factor: float = 1.0 / 255.0) -> list:
@@ -720,33 +739,43 @@ class VIT(nn.Module):
 
     def pooler_output(self, x, interpolate_pos_encoding: bool = False,
                       bool_masked_pos: Optional[torch.Tensor] = None, output_hidden_states: bool = False,
-                      output_attentions: bool = False) -> torch.Tensor:
+                      output_attentions: bool = False, do_resize: bool = False,
+                      resample: int = 2) -> torch.Tensor:
         """HF ``ViTModel(...).pooler_output``: tanh(dense(final hidden state of CLS)), (B, D).  ``x`` may also be a list
-        of images of different sizes (``forward_ragged``), each with its own patch grid (without a mask)."""
+        of images of different sizes (``forward_ragged``), each with its own patch grid (without a mask).  ``do_resize`` /
+        ``resample`` as for ``forward_uint8``: the images are resized to the model's size first (a list then runs as
+        one batch, not ragged)."""
         _refuse_outputs("pooler_output", output_hidden_states, output_attentions)
         assert self.pooler is not None, "Model was built without add_pooling_layer=True"
+        x = self._resized(x, do_resize, resample)
         return self.pooler(self._cls_hidden(x, interpolate_pos_encoding, bool_masked_pos))
 
     def logits(self, x, interpolate_pos_encoding: bool = False,
                bool_masked_pos: Optional[torch.Tensor] = None, output_hidden_states: bool = False,
-               output_attentions: bool = False) -> torch.Tensor:
+               output_attentions: bool = False, do_resize: bool = False,
+               resample: int = 2) -> torch.Tensor:
         """Class logits (B, num_labels) = classifier(final hidden states[:, 0]) — HF
         ``ViTForImageClassification(...).logits``; needs ``VIT(..., num_labels=...)``.  One tensor-core
         launch over the CLS rows of the final hidden states.  ``x`` may also be a list of images of different sizes
-        (``forward_ragged``), each with its own patch grid (without a mask)."""
+        (``forward_ragged``), each with its own patch grid (without a mask).  ``do_resize`` / ``resample`` as for
+        ``forward_uint8``: the images are resized to the model's size first (a list then runs as one batch, not ragged)."""
         _refuse_outputs("logits", output_hidden_states, output_attentions)
         assert self.classifier is not None, "VIT was built without a classifier head (num_labels)"
+        x = self._resized(x, do_resize, resample)
         hidden = self._cls_hidden(x, interpolate_pos_encoding, bool_masked_pos)
         from .kernels import bgemm as bg
         return _head_on_cls(hidden, self.classifier, bg.ACT_NONE)
 
     def pooled(self, x, interpolate_pos_encoding: bool = False,
                bool_masked_pos: Optional[torch.Tensor] = None, output_hidden_states: bool = False,
-               output_attentions: bool = False) -> torch.Tensor:
+               output_attentions: bool = False, do_resize: bool = False,
+               resample: int = 2) -> torch.Tensor:
         """CLS row of the final hidden states, (B, D): the tensor the data-parallel wrapper gathers.
         uint8 (B, H, W, C) inputs take the fused raw-pixel path.  ``x`` may also be a list of images of different sizes
-        (``forward_ragged``), each with its own patch grid (without a mask)."""
+        (``forward_ragged``), each with its own patch grid (without a mask).  ``do_resize`` / ``resample`` as for
+        ``forward_uint8``: the images are resized to the model's size first (a list then runs as one batch, not ragged)."""
         _refuse_outputs("pooled", output_hidden_states, output_attentions)
+        x = self._resized(x, do_resize, resample)
         if isinstance(x, (list, tuple)):
             assert bool_masked_pos is None, "bool_masked_pos is not supported with a list of images"
             return self._ragged_cls(x)

@@ -31,7 +31,7 @@ typedef enum {
   VT_ERR_DRIVER = -5       /* cuTensorMapEncodeTiled unavailable / failed */
 } vt_status;
 
-typedef enum { VT_F32 = 0, VT_BF16 = 1, VT_U8 = 2 /* pixels of vt_patch_embed only */, VT_E4M3 = 3 /* FP8 path only */ } vt_dtype;
+typedef enum { VT_F32 = 0, VT_BF16 = 1, VT_U8 = 2 /* raw NHWC pixel inputs only */, VT_E4M3 = 3 /* FP8 path only */ } vt_dtype;
 
 /* Library version (major*10000 + minor*100 + patch). */
 int vt_version(void);
@@ -168,31 +168,20 @@ int vt_flash_attn(const void* q, const void* k, const void* v, void* out, int32_
                   int32_t N, int32_t dh, int64_t qkv_row_stride, int64_t qkv_batch_stride,
                   int64_t out_row_stride, int64_t out_batch_stride, float scale, void* stream);
 
-/* K2 — patch embedding (im2col-free tcgen05 GEMM) with CLS + position embedding fused:
+/* K2 — patch embedding with CLS + position embedding fused, as two launches: a bandwidth-bound gather of the pixels
+ * into padded bf16 patch rows — every pixel read once — followed by the 2-CTA tcgen05 GEMM in token mode, whose
+ * epilogue adds the conv bias and the position table.
  * pixels [B,C,S,S] (pix_dtype f32|bf16) with w [D, C*P*P] bf16 in (c,i,j) order (row stride ldw), or
- * pixels [B,S,S,C] (pix_dtype VT_U8: raw NHWC bytes) with w in (i,j,c) order — the caller folds the
- * image processor's rescale / mean / std into w and posb (vit/packing.py:pack_embeddings_u8);
- * posb [n+1, D] f32 = pos + (row 0: cls, rows >= 1: conv bias); out [B, n+1, D] (out_dtype).
- * Replaces Conv2DTriton.forward + Embeddings.forward glue (conv2d.py:100-167, vit/vit.py:188-200);
- * the uint8 form also replaces the HF ViTImageProcessor rescale + normalise step in front of it. */
-int vt_patch_embed(const void* pixels, int32_t pix_dtype, const void* w, int64_t ldw,
-                   const float* posb, void* out, int32_t out_dtype, int32_t B, int32_t C, int32_t S,
-                   int32_t P, int32_t D, void* stream);
-
-/* The same, also writing the (sum, M2 about the group mean) of every 128-column group of every output row (CLS rows
- * included) to stats_out[(row*(D/128) + group)*2 .. +1] — the rowstats layout of vt_gemm_bf16_ln, so the
- * first block's layernorm_before folds into its QKV GEMM too.  D % 128 == 0. */
-int vt_patch_embed_stats(const void* pixels, int32_t pix_dtype, const void* w, int64_t ldw,
-                         const float* posb, void* out, int32_t out_dtype, float* stats_out, int32_t B,
-                         int32_t C, int32_t S, int32_t P, int32_t D, void* stream);
-
-/* K2 as two launches (the default for bf16 models): a bandwidth-bound gather of the pixels into padded bf16 patch
- * rows — every pixel read once — followed by the 2-CTA tcgen05 GEMM in token mode, whose epilogue adds the conv bias
- * and the position table and (stats_out != NULL, D % 128 == 0) writes the row statistics like vt_patch_embed_stats.
- * pixels / pix_dtype / w / ldw as for vt_patch_embed (ldw >= C*P*P, multiple of 8: the K padding of w must be zero);
- * bias f32 [D] = conv bias (uint8 pixels: minus the folded mean term); posb bf16 [n+1, D] = position embeddings with
- * row 0 = cls + pos[0] - bias; out bf16 [B, n+1, D]; workspace: bf16 [B, roundup(n+1, 32), ldw] scratch owned by the
- * caller (the gathered patch rows).  Same reference entry points replaced as vt_patch_embed. */
+ * pixels [B,S,S,C] (pix_dtype VT_U8: raw NHWC bytes) with w in (i,j,c) order — the caller folds the image processor's
+ * rescale / mean / std into w and bias (vit/packing.py:pack_embeddings); ldw >= C*P*P, multiple of 8: the K padding
+ * of w must be zero.  bias f32 [D] = conv bias (uint8 pixels: minus the folded mean term); posb bf16 [n+1, D] =
+ * position embeddings with row 0 = cls + pos[0] - bias; out bf16 [B, n+1, D]; workspace: bf16
+ * [B, roundup(n+1, 32), ldw] scratch owned by the caller (the gathered patch rows).
+ * stats_out != NULL (D % 128 == 0): also writes the (sum, M2 about the group mean) of every 128-column group of every
+ * output row (CLS rows included) to stats_out[(row*(D/128) + group)*2 .. +1] — the rowstats layout of
+ * vt_gemm_bf16_ln, so the first block's layernorm_before folds into its QKV GEMM too.
+ * Replaces Conv2DTriton.forward + Embeddings.forward glue (conv2d.py:100-167, vit/vit.py:188-200); the uint8 form
+ * also replaces the HF ViTImageProcessor rescale + normalise step in front of it. */
 int vt_patch_embed_gemm(const void* pixels, int32_t pix_dtype, const void* w, int64_t ldw, const float* bias,
                         const void* posb, void* out, float* stats_out, void* workspace, int32_t B, int32_t C, int32_t S,
                         int32_t P, int32_t D, void* stream);

@@ -2,7 +2,7 @@
  * vitb200_preprocess.h — entry points of libvitb200.so for the first step of HF's ViT image processor: the resize of
  * raw uint8 HWC images of any size to the model's size, byte for byte what PIL's Image.resize gives for BILINEAR and
  * BICUBIC (transformers ViTImageProcessorPil.resize; libImaging/Resample.c).  Rescale and normalisation are folded into
- * the patch embedding of the uint8 path (vt_patch_embed*, VT_U8), so resize + forward is the whole processor.
+ * the patch embedding of the uint8 path (VT_U8 pixels), so resize + forward is the whole processor.
  *
  * Same conventions as vitb200.h (device pointers, void* stream, 0 / negative vt_status / positive cudaError_t, no
  * synchronisation, no device allocation, safe inside CUDA-graph capture: the tables and descriptors are read on the

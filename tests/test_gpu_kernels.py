@@ -668,7 +668,7 @@ def test_gemm_layernorm_fold_outliers(case, K, N, gelu):
 
 
 @pytest.mark.parametrize("case", ["massive_channels", "large_mean_100", "mixed"])
-def test_patch_embed_stats_outliers(case):
+def test_patch_embed_stats_outliers_against_parameters(case):
     """Row statistics written by the patch-embedding epilogue when the position / bias table carries large
     offsets and planted channels (the rows of block 0's folded layernorm_before)."""
     from vit.vit import Embeddings
@@ -692,7 +692,10 @@ def test_patch_embed_stats_outliers(case):
     from vit.kernels.patching import patching
     patches = patching(x, P).float()                                     # (B, n, K)
     tok = patches @ pk.w[:, :pk.K].float().t()                           # (B, n, D)
-    full = torch.cat([torch.zeros(B, 1, D, device=dev()), tok], dim=1) + pk.posb[None]
+    posb = emb.position_embeddings.detach().float()[0].clone()           # pos + (row 0: cls, rows >= 1: conv bias)
+    posb[0] += emb.cls_token.detach().float().reshape(-1)
+    posb[1:] += emb.projection.bias.detach().float()
+    full = torch.cat([torch.zeros(B, 1, D, device=dev()), tok], dim=1) + posb[None]
     ref = _group_stats(full.reshape(B * (n + 1), D))
     st, rf = stats.view(B, n + 1, -1, 2), ref.view(B, n + 1, -1, 2)
     assert torch.allclose(st[:, 1:, :, 0], rf[:, 1:, :, 0], rtol=1e-4, atol=5e-2)

@@ -31,7 +31,7 @@ def test_shard_bounds_cover_and_partition():
 
 
 @pytest.mark.parametrize("arch", ["tiny-b", "tiny-h"])
-def test_packed_qkv_layout_matches_hf(arch):
+def test_packed_layouts_match_hf(arch):
     """pack_attention rebuilds HF's fused (out, in) Q/K/V matrices from the per-head parameters."""
     hf = hf_oracle.build_hf(arch, seed=0)
     model = VIT(**hf_oracle.vit_kwargs(arch))
@@ -53,13 +53,20 @@ def test_packed_qkv_layout_matches_hf(arch):
     assert torch.equal(emb.w[:, :K], hsd["embeddings.patch_embeddings.projection.weight"].reshape(-1, K))
     assert torch.count_nonzero(emb.w[:, K:]) == 0
     pos = hsd["embeddings.position_embeddings"][0]
-    assert torch.allclose(emb.posb[0], pos[0] + hsd["embeddings.cls_token"].reshape(-1))
-    assert torch.allclose(emb.posb[1:], pos[1:] + hsd["embeddings.patch_embeddings.projection.bias"])
+    assert torch.equal(pos[1:] + emb.bias32, pos[1:] + hsd["embeddings.patch_embeddings.projection.bias"])
+    _assert_cls_row(emb, pos[0] + hsd["embeddings.cls_token"].reshape(-1))
+
+
+def _assert_cls_row(pk, want):
+    """The patch-embedding GEMM adds the bias to row 0 of the bf16 table (a zero patch row): cls + pos[0] within the one
+    bf16 rounding of posb16[0] = bf16(cls + pos[0] - bias)."""
+    got = pk.posb16[0].float() + pk.bias32
+    assert torch.all((got - want).abs() <= 2.0 ** -8 * (want - pk.bias32).abs() + 1e-6), (got - want).abs().max()
 
 
 @pytest.mark.parametrize("arch", ["tiny-b", "tiny-h"])
-def test_uint8_packing_folds_the_image_processor(arch):
-    """pack_embeddings_u8: raw bytes against the re-ordered, scaled weight + shifted bias table equal
+def test_uint8_pack_folds_the_image_processor(arch):
+    """pack_embeddings for uint8 pixels: raw bytes against the re-ordered, scaled weight + shifted bias table equal
     the patch projection of the rescaled / normalised pixels (what the uint8 kernel path computes)."""
     a = hf_oracle.ARCHS[arch]
     model = VIT(**hf_oracle.vit_kwargs(arch))
@@ -68,20 +75,20 @@ def test_uint8_packing_folds_the_image_processor(arch):
             p_.copy_(torch.randn_like(p_) * 0.05)
     emb = model.embeddings
     mean, std, r = (0.485, 0.456, 0.406), (0.229, 0.224, 0.225), 1.0 / 255.0
-    pk = packing.pack_embeddings_u8(emb, mean, std, r)
+    pk = packing.pack_embeddings(emb, packing.pixel_format(mean, std, r))
     S, P, D = a["image_size"], a["patch_size"], a["hidden_size"]
     g = torch.Generator().manual_seed(5)
     x = torch.randint(0, 256, (2, S, S, 3), generator=g, dtype=torch.uint8)
     # patches of the NHWC bytes in (i, j, c) order: [B, n, P*P*3]
     n = S // P
     patches = x.float().reshape(2, n, P, n, P, 3).permute(0, 1, 3, 2, 4, 5).reshape(2, n * n, P * P * 3)
-    got = patches @ pk.w[:, :pk.K].float().t() + pk.posb[1:]
+    got = patches @ pk.w[:, :pk.K].float().t() + (emb.position_embeddings.float()[0, 1:] + pk.bias32)
     xn = (x.float() * r - torch.tensor(mean)) / torch.tensor(std)
     want = torch.nn.functional.conv2d(xn.permute(0, 3, 1, 2), emb.projection.weight.float(),
                                       emb.projection.bias.float(), stride=P).flatten(2).transpose(1, 2)
     want = want + emb.position_embeddings.float()[0, 1:]
     assert torch.allclose(got, want, atol=2e-3, rtol=1e-4), (got - want).abs().max()
-    assert torch.allclose(pk.posb[0], (emb.cls_token.float().reshape(-1) + emb.position_embeddings.float()[0, 0]))
+    _assert_cls_row(pk, emb.cls_token.float().reshape(-1) + emb.position_embeddings.float()[0, 0])
 
 
 def test_pooler_weights_load_transposed():

@@ -90,7 +90,7 @@ def new_grid_cost_ms(model, grids) -> list:
     for gh, gw in grids:
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        packing.pos_grid(emb, gh, gw).token_table(emb)
+        packing.pos_grid(emb, gh, gw).table(emb, None, False)
         torch.cuda.synchronize()
         out.append(round((time.perf_counter() - t0) * 1e3, 3))
     return out

@@ -34,8 +34,6 @@ int attn5_fwd_tcgen05(const void*, const void*, const void*, void*, int, int, in
                       long long, long long, long long, float, int, cudaStream_t);
 int attn5mb_fwd_tcgen05(const void*, const void*, const void*, void*, int, int, int, int, long long,
                         long long, long long, long long, float, int, cudaStream_t);
-int patch_embed_tcgen05(const void*, int, const void*, long long, const float*, void*, int, float*, int,
-                        int, int, int, int, cudaStream_t);
 int patching(const void*, void*, int, int, int, int, int, int, cudaStream_t);
 int bgemm_tcgen05(const void*, const void*, void*, const float*, const void*, int, int, int, int, int, const long long*,
                   const long long*, const long long*, int, float, int, int, cudaStream_t);
@@ -218,20 +216,6 @@ int vt_flash_attn(const void* q, const void* k, const void* v, void* out, int32_
     return vt::attn5mb_fwd_tcgen05(q, k, v, out, B, H, N, dh, qkv_row_stride, qkv_batch_stride,
                                    out_row_stride, out_batch_stride, scale, next_direction(), S(stream));
   return VT_ERR_UNSUPPORTED;
-}
-
-int vt_patch_embed(const void* pixels, int32_t pix_dtype, const void* w, int64_t ldw,
-                   const float* posb, void* out, int32_t out_dtype, int32_t B, int32_t C, int32_t S_,
-                   int32_t P, int32_t D, void* stream) {
-  return vt::patch_embed_tcgen05(pixels, pix_dtype, w, ldw, posb, out, out_dtype, nullptr, B, C, S_, P, D,
-                                 S(stream));
-}
-
-int vt_patch_embed_stats(const void* pixels, int32_t pix_dtype, const void* w, int64_t ldw,
-                         const float* posb, void* out, int32_t out_dtype, float* stats_out, int32_t B,
-                         int32_t C, int32_t S_, int32_t P, int32_t D, void* stream) {
-  return vt::patch_embed_tcgen05(pixels, pix_dtype, w, ldw, posb, out, out_dtype, stats_out, B, C, S_, P, D,
-                                 S(stream));
 }
 
 int vt_ln_fold(const void* w, int64_t ldw, const float* bias, const float* gamma, const float* beta, void* w_out,

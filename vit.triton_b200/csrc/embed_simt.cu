@@ -70,7 +70,7 @@ __global__ void embed_finalize_masked_kernel(T* __restrict__ x, const T* __restr
 
 // One thread per output element; weights are read with k fastest within a thread so consecutive
 // output channels do not coalesce — this entry point exists for API parity, the model path uses
-// patch_embed_tcgen05 (bf16) or patching + simt_gemm (fp32).
+// vt_patch_embed_gemm (bf16) or patching + a GEMM (fp32).
 template <typename T>
 __global__ void conv2d_nchw_kernel(const T* __restrict__ in, const T* __restrict__ w,
                                    const T* __restrict__ bias, T* __restrict__ out, int B, int C,

@@ -7,10 +7,9 @@
 //   A[b, t, :]        = 0 for n < t < Tpad,  A[.., k] = 0 for K <= k < Kpad
 //
 // Tpad = tokens rounded up to 32: no 32-row tile of the GEMM's epilogue straddles two images, so its output and
-// position-table coordinates are (token, image) and TMA clips the padding rows.  Round 1's single kernel
-// (patch_embed_sm100.cu, kept for head widths that are not a multiple of 8 and as the A/B baseline) gathered the
-// pixels once per 256-column block of the output — three times for ViT-B — and ran at 172 us (tensor pipe 17 %,
-// DRAM 8 %); gather + GEMM need one pass over the pixels and one tensor-bound GEMM.
+// position-table coordinates are (token, image) and TMA clips the padding rows.  Gather + GEMM need one pass over the
+// pixels and one tensor-bound GEMM; a single fused kernel that gathered the pixels once per 256-column block of the
+// output — three times for ViT-B — ran at 172 us (tensor pipe 17 %, DRAM 8 %).
 // Replaces the patch extraction inside conv2d_kernel (vit/kernels/conv2d.py:19-97) / patching_kernel
 // (vit/kernels/patching.py:54-92).
 #include "common.cuh"

@@ -16,7 +16,7 @@ _lib: Optional[ctypes.CDLL] = None
 
 VT_F32 = 0
 VT_BF16 = 1
-VT_U8 = 2     # raw NHWC pixels of vt_patch_embed
+VT_U8 = 2     # raw NHWC pixels (patch embeddings, masked-image-modeling loss)
 VT_E4M3 = 3   # FP8 path (vt_gemm_fp8 / vt_layernorm_fp8)
 VT_PG_PUT = 1  # vt_pool_cls_allgather modes
 VT_PG_GET = 2
@@ -49,10 +49,6 @@ SIGNATURES = {
                      _c_i32, _c_ptr],
     "vt_flash_attn": [_c_ptr, _c_ptr, _c_ptr, _c_ptr, _c_i32, _c_i32, _c_i32, _c_i32, _c_i64, _c_i64,
                       _c_i64, _c_i64, _c_f32, _c_ptr],
-    "vt_patch_embed": [_c_ptr, _c_i32, _c_ptr, _c_i64, _c_ptr, _c_ptr, _c_i32, _c_i32, _c_i32,
-                       _c_i32, _c_i32, _c_i32, _c_ptr],
-    "vt_patch_embed_stats": [_c_ptr, _c_i32, _c_ptr, _c_i64, _c_ptr, _c_ptr, _c_i32, _c_ptr, _c_i32, _c_i32,
-                             _c_i32, _c_i32, _c_i32, _c_ptr],
     "vt_ln_fold": [_c_ptr, _c_i64, _c_ptr, _c_ptr, _c_ptr, _c_ptr, _c_i64, _c_ptr, _c_ptr, _c_i32, _c_i32, _c_i32,
                    _c_ptr],
     "vt_patch_embed_gemm": [_c_ptr, _c_i32, _c_ptr, _c_i64, _c_ptr, _c_ptr, _c_ptr, _c_ptr, _c_ptr, _c_i32, _c_i32,

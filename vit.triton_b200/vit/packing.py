@@ -25,10 +25,11 @@ from .kernels import _lib, bgemm as bg
 
 
 class PackedMixin:
-    """Gives a module lazily built, automatically invalidated ``packed(kind)`` namespaces.
+    """Gives a module lazily built, automatically invalidated ``packed(kind, *args)`` namespaces.
 
     ``kind`` selects a builder ``_build_packed[_<kind>]`` and its source list
-    ``_packed_sources[_<kind>]`` (default: every parameter of the module)."""
+    ``_packed_sources[_<kind>]`` (default: every parameter of the module).  ``args`` go to the builder and are part of
+    the cache key: one namespace per kind is kept, built for the last ``args``."""
 
     def _packed_sources(self):
         return list(self.parameters())
@@ -37,18 +38,18 @@ class PackedMixin:
     def _packed_key(params):
         return tuple((p.data_ptr(), p._version) for p in params)
 
-    def packed(self, kind: str = ""):
+    def packed(self, kind: str = "", *args):
         states = self.__dict__.setdefault("_packed_states", {})
         state = states.get(kind)
         if state is not None:
             params, key, value = state
-            if self._packed_key(params) == key:
+            if key == (args, self._packed_key(params)):
                 return value
         suffix = f"_{kind}" if kind else ""
         params = getattr(self, "_packed_sources" + suffix, self._packed_sources)()
         with torch.no_grad():
-            value = getattr(self, "_build_packed" + suffix)()
-        states[kind] = (params, self._packed_key(params), value)
+            value = getattr(self, "_build_packed" + suffix)(*args)
+        states[kind] = (params, (args, self._packed_key(params)), value)
         return value
 
     def invalidate_packed(self):
@@ -221,112 +222,56 @@ def _posm16(pos32: torch.Tensor, mask_token: Optional[torch.Tensor], bias32: tor
     return (pos32 + mask_token.detach().float().reshape(-1) - bias32).to(torch.bfloat16).contiguous()
 
 
-def pack_embeddings(emb) -> SimpleNamespace:
-    w = emb.projection.weight.detach()
-    D = w.shape[0]
-    K = w[0].numel()
-    kpad = (K + 7) // 8 * 8
-    w2d = torch.zeros((D, kpad), device=w.device, dtype=w.dtype)
-    w2d[:, :K] = w.reshape(D, K)
-    pos = emb.position_embeddings.detach().float()[0]          # [N, D]
-    posb = pos.clone()
-    posb[0] += emb.cls_token.detach().float().reshape(-1)
-    posb[1:] += emb.projection.bias.detach().float()
-    bias32 = emb.projection.bias.detach().float().contiguous()
-    return SimpleNamespace(w=w2d, ldw=kpad, K=K, posb=posb.contiguous(), bias32=bias32,
-                           posb16=_posb16(pos, emb.cls_token, bias32), posm16=_posm16(pos, emb.mask_token, bias32))
+def pixel_format(image_mean, image_std, rescale_factor: float) -> tuple:
+    """The pixel format of raw uint8 NHWC pixels with these image-processor constants: (mean, std, rescale) as floats.
+    Every embedding function takes a format ``fmt``: None for float NCHW pixels, or this key."""
+    return tuple(float(m) for m in image_mean), tuple(float(v) for v in image_std), float(rescale_factor)
 
 
-def pack_embeddings_u8(emb, image_mean, image_std, rescale_factor: float) -> SimpleNamespace:
-    """Patch projection for RAW uint8 NHWC pixels: the image processor's
-    ``(x * rescale_factor - mean_c) / std_c`` (HF ViTImageProcessor: 1/255, 0.5, 0.5) is folded into
-    the operands, so the kernel multiplies bytes:
+def pixel_dims(x: torch.Tensor, fmt: Optional[tuple]) -> tuple:
+    """(B, C, H, W) of a pixel batch of format ``fmt``: (B, C, H, W) float pixels, or (B, H, W, C) raw uint8 ones."""
+    if fmt is None:
+        return tuple(x.shape)
+    B, H, W, C = x.shape
+    return B, C, H, W
+
+
+def pack_embeddings(emb, fmt: Optional[tuple] = None) -> SimpleNamespace:
+    """Patch-projection operands for pixels of format ``fmt``: the bf16 | fp32 weight ``w`` [D, ldw] (K = C*P*P columns,
+    zero padding to a multiple of 8), the fp32 bias ``bias32`` [D] and the bf16 position tables ``posb16`` /
+    ``posm16`` of the trained grid.  Float pixels: the conv weight in the reference's (c, i, j) order and the conv bias.
+
+    Raw uint8 NHWC pixels (``fmt`` = ``pixel_format``): the image processor's ``(x * rescale - mean_c) / std_c`` (HF
+    ViTImageProcessor: 1/255, 0.5, 0.5) is folded into the operands, so the kernel multiplies bytes:
 
         sum_k w[d,k] * (x_k * r - mean_c) / std_c  =  sum_k (w[d,k] * r / std_c) * x_k  -  sum_k w[d,k] * mean_c / std_c
 
-    The weight is re-ordered from the reference's (c, i, j) to (i, j, c) — a patch row of an NHWC
-    image is P*C contiguous bytes — and scaled in fp32 before the single rounding to bf16; the
-    constant term joins the conv bias in the fp32 position/bias table."""
-    w = emb.projection.weight.detach().float()                 # [D, C, P, P]
+    The weight is re-ordered from the reference's (c, i, j) to (i, j, c) — a patch row of an NHWC image is P*C
+    contiguous bytes — and scaled in fp32 before the single rounding to the model's dtype; the constant term is
+    subtracted from the conv bias."""
+    w = emb.projection.weight.detach()                         # [D, C, P, P]
     D, C = w.shape[0], w.shape[1]
-    mean = torch.as_tensor(image_mean, dtype=torch.float32, device=w.device).reshape(1, C, 1, 1)
-    std = torch.as_tensor(image_std, dtype=torch.float32, device=w.device).reshape(1, C, 1, 1)
-    w_scaled = w * (float(rescale_factor) / std)
-    offset = (w * (mean / std)).sum(dim=(1, 2, 3))              # [D]
     K = w[0].numel()
     kpad = (K + 7) // 8 * 8
-    w2d = torch.zeros((D, kpad), device=w.device, dtype=emb.projection.weight.dtype)
-    w2d[:, :K] = w_scaled.permute(0, 2, 3, 1).reshape(D, K).to(w2d.dtype)
-    pos = emb.position_embeddings.detach().float()[0]
-    posb = pos.clone()
-    posb[0] += emb.cls_token.detach().float().reshape(-1)
-    posb[1:] += emb.projection.bias.detach().float() - offset
-    bias32 = (emb.projection.bias.detach().float() - offset).contiguous()
-    return SimpleNamespace(w=w2d, ldw=kpad, K=K, posb=posb.contiguous(), bias32=bias32,
-                           posb16=_posb16(pos, emb.cls_token, bias32), posm16=_posm16(pos, emb.mask_token, bias32))
+    bias32 = emb.projection.bias.detach().float().contiguous()
+    if fmt is not None:
+        image_mean, image_std, rescale_factor = fmt
+        w32 = w.float()
+        mean = torch.as_tensor(image_mean, dtype=torch.float32, device=w.device).reshape(1, C, 1, 1)
+        std = torch.as_tensor(image_std, dtype=torch.float32, device=w.device).reshape(1, C, 1, 1)
+        bias32 = (bias32 - (w32 * (mean / std)).sum(dim=(1, 2, 3))).contiguous()
+        w = (w32 * (rescale_factor / std)).permute(0, 2, 3, 1).to(w.dtype)
+    w2d = torch.zeros((D, kpad), device=w.device, dtype=w.dtype)
+    w2d[:, :K] = w.reshape(D, K)
+    pos = emb.position_embeddings.detach().float()[0]          # [N, D]
+    return SimpleNamespace(w=w2d, ldw=kpad, K=K, bias32=bias32, posb16=_posb16(pos, emb.cls_token, bias32),
+                           posm16=_posm16(pos, emb.mask_token, bias32))
 
 
-def u8_pack(emb, image_mean, image_std, rescale_factor: float) -> tuple:
-    """(key, pack) of ``pack_embeddings_u8`` for these image-processor constants, cached on the module (one set of
-    constants at a time) and rebuilt when a source parameter's storage pointer or version counter changes."""
-    key = (tuple(float(m) for m in image_mean), tuple(float(v) for v in image_std), float(rescale_factor))
-    cache = emb.__dict__.setdefault("_u8_pack", {})
-    params = emb._packed_sources()
-    stamp = emb._packed_key(params)
-    hit = cache.get(key)
-    if hit is None or hit[0] != stamp:
-        with torch.no_grad():
-            hit = (stamp, pack_embeddings_u8(emb, image_mean, image_std, rescale_factor))
-        cache.clear()
-        cache[key] = hit
-    return key, hit[1]
-
-
-def patch_embed_u8(emb, x: torch.Tensor, image_mean, image_std, rescale_factor: float,
-                   stats: Optional[torch.Tensor] = None, interpolate: bool = False,
-                   mask: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """Raw uint8 NHWC pixels (B, S, S, C) -> token embeddings (B, n+1, D), rescale + normalise + patch
-    projection + CLS + position embeddings in ONE kernel (bf16 models on the tensor-core path).
-    ``interpolate``: any (B, H, W, C) with H, W >= patch size, position table resampled to its patch grid
-    (``pos_grid``).  ``mask``: checked bool_masked_pos (B, n), masked patches take the mask token (``embed_masked``)."""
-    w = emb.projection.weight
-    assert x.is_cuda and x.dtype == torch.uint8 and x.dim() == 4, \
-        f"Raw pixels need to be a CUDA uint8 (B, H, W, C) tensor, provided: {x.dtype}, {tuple(x.shape)}"
-    assert w.dtype == torch.bfloat16 and emb.hidden_dim % 8 == 0, \
-        "The fused uint8 input path runs on the bf16 tensor-core kernels only"
-    B, S, S2, C = x.shape
-    if interpolate:
-        check_any_size(emb, C, S, S2)
-    else:
-        assert S == S2 and C == emb.channels, f"Image size {tuple(x.shape[1:])} not matching with the model input size"
-    _, pk = u8_pack(emb, image_mean, image_std, rescale_factor)
-    x = x.contiguous()
-    n = emb.num_patches
-    hw = posb16 = None
-    posm16 = pk.posm16
-    if interpolate:
-        grid = patch_grid(emb, S, S2)
-        n = grid[0] * grid[1]
-        hw = (S, S2)
-        if grid != native_grid(emb):
-            pg = pos_grid(emb, *grid)
-            posb16 = pg.token_table_u8(emb, image_mean, image_std, rescale_factor)
-            if mask is not None:
-                posm16 = pg.mask_table_u8(emb, image_mean, image_std, rescale_factor)
-    n_tok = n + 1
-    out = torch.empty((B, n_tok, emb.hidden_dim), device=x.device, dtype=w.dtype)
-    if B == 0:
-        return out
-    if mask is not None:
-        embed_masked(emb, x, _lib.VT_U8, S, S2, mask, pk, pk.posb16 if posb16 is None else posb16, posm16, out, stats)
-        return out
-    stream = _lib.stream_ptr(x)
-    step = _embed_batch_step(n)
-    for b0 in range(0, B, step):
-        nb = min(step, B - b0)
-        _embed_call(stats, b0, n_tok, emb.hidden_dim, pk, x[b0:].data_ptr(), _lib.VT_U8, out[b0:].data_ptr(), nb, C, S,
-                    emb.patch_size, stream, x.device, hw=hw, posb16=posb16)
-    return out
+def embed_pack(emb, fmt: Optional[tuple] = None) -> SimpleNamespace:
+    """``pack_embeddings(emb, fmt)``, cached on the module (``PackedMixin.packed``): the float pack and the pack of one
+    set of uint8 constants at a time, rebuilt when a source parameter's storage pointer or version counter changes."""
+    return emb.packed() if fmt is None else emb.packed("u8", fmt)
 
 
 STATS_COLS = 128   # columns per (sum, M2) partial of the row statistics (VT_LN_STATS_COLS in include/vitb200.h)
@@ -433,59 +378,60 @@ def _embed_batch_step(n_patches: int) -> int:
     return min(65535, 65535 * 128 // n_patches)
 
 
-def _two_launch_embed() -> bool:
-    """Gather + token-mode GEMM (default) or round 1's single kernel (VT_PATCH_EMBED=1, A/B measurements)."""
-    return os.environ.get("VT_PATCH_EMBED", "2") != "1"
-
-
-def _embed_call(stats, b0, n_tok, dim, pk, pixels_ptr, pix_code, out_ptr, nb, C, S, P, stream, device, hw=None,
-                posb16=None):
-    """Patch embedding of images b0 .. b0 + nb: ``vt_patch_embed_gemm`` (gather + 2-CTA GEMM in token mode), or the
-    single-kernel ``vt_patch_embed[_stats]``; row statistics of those images go into ``stats`` when given.
-    ``hw`` = (H, W): an input at any resolution, ``vt_patch_embed_gemm_hw`` with the position table ``posb16``
-    (None: the packed one) — always the two-launch form, the single kernel takes square native inputs only."""
+def _embed_call(stats, b0, n_tok, dim, pk, pos, pixels_ptr, pix_code, out_ptr, nb, C, H, W, P, stream, device,
+                interpolate):
+    """Patch embedding of images b0 .. b0 + nb: gather + 2-CTA GEMM in token mode with the bf16 position table ``pos``;
+    row statistics of those images go into ``stats`` when given.  ``vt_patch_embed_gemm`` for a square input at the
+    model's size, ``vt_patch_embed_gemm_hw`` for any (H, W) with ``interpolate``."""
     s_ptr = None if stats is None else stats.data_ptr() + b0 * n_tok * (dim // STATS_COLS) * 2 * 4
-    if hw is not None:
-        tok_pad = (n_tok + 31) // 32 * 32
-        work = torch.empty((nb, tok_pad, pk.ldw), device=device, dtype=torch.bfloat16)
-        posb16 = pk.posb16 if posb16 is None else posb16
+    tok_pad = (n_tok + 31) // 32 * 32
+    work = torch.empty((nb, tok_pad, pk.ldw), device=device, dtype=torch.bfloat16)
+    if interpolate:
         _lib.call("vt_patch_embed_gemm_hw", pixels_ptr, pix_code, pk.w.data_ptr(), pk.ldw, pk.bias32.data_ptr(),
-                  posb16.data_ptr(), out_ptr, s_ptr, work.data_ptr(), nb, C, hw[0], hw[1], P, dim, stream)
-        return
-    if _two_launch_embed():
-        tok_pad = (n_tok + 31) // 32 * 32
-        work = torch.empty((nb, tok_pad, pk.ldw), device=device, dtype=torch.bfloat16)
-        _lib.call("vt_patch_embed_gemm", pixels_ptr, pix_code, pk.w.data_ptr(), pk.ldw, pk.bias32.data_ptr(),
-                  pk.posb16.data_ptr(), out_ptr, s_ptr, work.data_ptr(), nb, C, S, P, dim, stream)
-        return
-    if stats is None:
-        _lib.call("vt_patch_embed", pixels_ptr, pix_code, pk.w.data_ptr(), pk.ldw, pk.posb.data_ptr(), out_ptr,
-                  _lib.VT_BF16, nb, C, S, P, dim, stream)
+                  pos.data_ptr(), out_ptr, s_ptr, work.data_ptr(), nb, C, H, W, P, dim, stream)
     else:
-        _lib.call("vt_patch_embed_stats", pixels_ptr, pix_code, pk.w.data_ptr(), pk.ldw, pk.posb.data_ptr(), out_ptr,
-                  _lib.VT_BF16, s_ptr, nb, C, S, P, dim, stream)
+        _lib.call("vt_patch_embed_gemm", pixels_ptr, pix_code, pk.w.data_ptr(), pk.ldw, pk.bias32.data_ptr(),
+                  pos.data_ptr(), out_ptr, s_ptr, work.data_ptr(), nb, C, H, P, dim, stream)
 
 
-def patch_embed(emb, x: torch.Tensor, stats: Optional[torch.Tensor] = None, interpolate: bool = False,
-                mask: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """Pixels (B, C, S, S) -> token embeddings (B, n+1, D) including CLS and position embeddings.
+def patch_embed(emb, x: torch.Tensor, fmt: Optional[tuple] = None, stats: Optional[torch.Tensor] = None,
+                interpolate: bool = False, mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Pixels of format ``fmt`` -> token embeddings (B, n+1, D) including CLS and position embeddings.  ``fmt`` None:
+    float pixels (B, C, S, S); ``pixel_format``: raw uint8 NHWC pixels (B, S, S, C), rescale + normalise + patch
+    projection in the same launches (bf16 models on the tensor-core path only).
     ``stats``: optional (B * (n+1), D/128, 2) fp32 buffer for the row statistics the LayerNorm folded
-    into the first QKV GEMM consumes (bf16 tensor-core path only).  ``interpolate``: pixels (B, C, H, W) at any
+    into the first QKV GEMM consumes (bf16 tensor-core path only).  ``interpolate``: pixels at any
     H, W >= patch size, n = (H // P) * (W // P), position table resampled to that grid (``pos_grid``).
     ``mask``: checked bool_masked_pos (B, n): masked patches take the mask token (``embed_masked`` on the bf16
     tensor-core path, ``vt_embed_finalize_masked`` on the others)."""
-    pk = emb.packed()
     w = emb.projection.weight
-    B, C, S, S2 = x.shape
-    P = emb.patch_size
     D = emb.hidden_dim
+    if fmt is None:
+        B, C, H, W = x.shape
+    else:
+        assert x.is_cuda and x.dtype == torch.uint8 and x.dim() == 4, \
+            f"Raw pixels need to be a CUDA uint8 (B, H, W, C) tensor, provided: {x.dtype}, {tuple(x.shape)}"
+        assert w.dtype == torch.bfloat16 and D % 8 == 0, \
+            "The fused uint8 input path runs on the bf16 tensor-core kernels only"
+        B, C, H, W = pixel_dims(x, fmt)
+        if interpolate:
+            check_any_size(emb, C, H, W)
+        else:
+            assert H == W and C == emb.channels, f"Image size {tuple(x.shape[1:])} not matching with the model input size"
+    pk = embed_pack(emb, fmt)
+    P = emb.patch_size
     n = emb.num_patches
-    grid = None                                            # resampled tables, None = the model's own
+    grid = None                                            # patch grid of an interpolated input, None = the model's own
     if interpolate:
-        gh, gw = patch_grid(emb, S, S2)
-        n = gh * gw
-        if (gh, gw) != native_grid(emb):
-            grid = pos_grid(emb, gh, gw)
+        grid = patch_grid(emb, H, W)
+        n = grid[0] * grid[1]
+    tensor_core = fmt is not None or (w.dtype == torch.bfloat16 and D % 8 == 0
+                                      and x.dtype in (torch.float32, torch.bfloat16))
+    if tensor_core:
+        pos = grid_table(emb, grid, fmt, False)
+        posm = None if mask is None else grid_table(emb, grid, fmt, True)
+    else:
+        pos = emb.position_embeddings if grid is None or grid == native_grid(emb) else pos_grid(emb, *grid).pos
     n_tok = n + 1
     x = x.contiguous()
     out = torch.empty((B, n_tok, D), device=x.device, dtype=w.dtype)
@@ -493,18 +439,16 @@ def patch_embed(emb, x: torch.Tensor, stats: Optional[torch.Tensor] = None, inte
         return out
     stream = _lib.stream_ptr(x)
 
-    if w.dtype == torch.bfloat16 and D % 8 == 0 and x.dtype in (torch.float32, torch.bfloat16):
+    if tensor_core:
+        code = _lib.dtype_code(x) if fmt is None else _lib.VT_U8
         if mask is not None:
-            pos, posm = (pk.posb16, pk.posm16) if grid is None else (grid.token_table(emb), grid.mask_table(emb))
-            embed_masked(emb, x, _lib.dtype_code(x), S, S2, mask, pk, pos, posm, out, stats)
+            embed_masked(emb, x, code, H, W, mask, pk, pos, posm, out, stats)
             return out
-        hw = (S, S2) if interpolate else None
-        posb16 = None if grid is None else grid.token_table(emb)
         step = _embed_batch_step(n)
         for b0 in range(0, B, step):
             nb = min(step, B - b0)
-            _embed_call(stats, b0, n_tok, D, pk, x[b0:].data_ptr(), _lib.dtype_code(x), out[b0:].data_ptr(), nb, C, S, P,
-                        stream, x.device, hw=hw, posb16=posb16)
+            _embed_call(stats, b0, n_tok, D, pk, pos, x[b0:].data_ptr(), code, out[b0:].data_ptr(), nb, C, H, W, P,
+                        stream, x.device, interpolate)
         return out
     assert stats is None, "Row statistics come out of the bf16 tensor-core patch embedding only"
 
@@ -513,8 +457,8 @@ def patch_embed(emb, x: torch.Tensor, stats: Optional[torch.Tensor] = None, inte
     from .kernels.patching import patching
     if x.dtype != w.dtype:
         x = x.to(w.dtype)
-    if interpolate and (S % P or S2 % P):
-        x = x[:, :, :S // P * P, :S2 // P * P]             # the pixels no patch covers (patching() copies)
+    if interpolate and (H % P or W % P):
+        x = x[:, :, :H // P * P, :W // P * P]               # the pixels no patch covers (patching() copies)
     patches = patching(x, P)
     K = pk.K
     code = _lib.dtype_code(out)
@@ -534,7 +478,6 @@ def patch_embed(emb, x: torch.Tensor, stats: Optional[torch.Tensor] = None, inte
         kk = a.shape[2]
         bg.bgemm(a.data_ptr(), wp.data_ptr(), out, out.data_ptr() + D * es, n, D, kk, B, 1, (n * kk, 0, kk),
                  (0, 0, kk), (n_tok * D, 0, D), bias32=pk.bias32)
-    pos = emb.position_embeddings if grid is None else grid.pos
     finalize_embeddings(emb, out, pos, mask)
     return out
 
@@ -652,54 +595,30 @@ def resample_pos_table(pos: torch.Tensor, g_in: int, gh: int, gw: int) -> torch.
 class PosGrid:
     """Position tables of one non-native patch grid, all derived from one resample of the model's table:
     ``pos32`` fp32 [1 + n, D]; ``pos`` (1, 1 + n, D) in the model's dtype (``Embeddings.interpolate_pos_encoding``,
-    and ``vt_embed_finalize`` of the fp32 / unfused paths); ``token_table`` / ``token_table_u8`` the bf16 tables of
-    the two-launch patch embedding (row 0 = cls + pos[0] - the pack's bias); ``mask_table`` / ``mask_table_u8`` those
-    of masked patches (mask_token + pos - the pack's bias, ``embed_masked``).  A table, once built, is never replaced
-    while this object lives: CUDA graphs keep reading it (see ``pos_grid``)."""
+    and ``vt_embed_finalize`` of the fp32 / unfused paths); ``table`` the bf16 tables of the tensor-core patch
+    embedding for each pixel format.  A table, once built, is never replaced while this object lives: CUDA graphs keep
+    reading it (see ``pos_grid``)."""
 
     def __init__(self, emb, gh: int, gw: int):
         source = emb.position_embeddings.detach()
         self.pos32 = resample_pos_table(source[0], native_grid(emb)[0], gh, gw)
         self.pos = self.pos32.to(source.dtype)[None]
-        self._plain = None
-        self._u8 = {}
-        self._plain_masked = None
-        self._u8_masked = {}
+        self._tables = {}
 
-    def token_table(self, emb) -> torch.Tensor:
-        """bf16 table for pixels in NCHW (the pack ``emb.packed()``)."""
-        if self._plain is None:
-            _assert_not_capturing()
-            with torch.no_grad():
-                self._plain = _posb16(self.pos32, emb.cls_token, emb.packed().bias32)
-        return self._plain
-
-    def token_table_u8(self, emb, image_mean, image_std, rescale_factor: float) -> torch.Tensor:
-        """bf16 table for raw uint8 NHWC pixels with these image-processor constants (the pack ``u8_pack``)."""
-        key, pk = u8_pack(emb, image_mean, image_std, rescale_factor)
-        table = self._u8.get(key)
+    def table(self, emb, fmt: Optional[tuple], masked: bool) -> torch.Tensor:
+        """bf16 table for pixels of format ``fmt`` (the pack ``embed_pack(emb, fmt)``): of every token (row 0 = cls +
+        pos[0] - the pack's bias), or with ``masked`` of masked patches (mask_token + pos - the pack's bias,
+        ``embed_masked``)."""
+        table = self._tables.get((fmt, masked))
         if table is None:
             _assert_not_capturing()
+            bias32 = embed_pack(emb, fmt).bias32
             with torch.no_grad():
-                table = self._u8[key] = _posb16(self.pos32, emb.cls_token, pk.bias32)
-        return table
-
-    def mask_table(self, emb) -> torch.Tensor:
-        """bf16 table of masked patches for pixels in NCHW (the pack ``emb.packed()``)."""
-        if self._plain_masked is None:
-            _assert_not_capturing()
-            with torch.no_grad():
-                self._plain_masked = _posm16(self.pos32, emb.mask_token, emb.packed().bias32)
-        return self._plain_masked
-
-    def mask_table_u8(self, emb, image_mean, image_std, rescale_factor: float) -> torch.Tensor:
-        """bf16 table of masked patches for raw uint8 NHWC pixels with these image-processor constants."""
-        key, pk = u8_pack(emb, image_mean, image_std, rescale_factor)
-        table = self._u8_masked.get(key)
-        if table is None:
-            _assert_not_capturing()
-            with torch.no_grad():
-                table = self._u8_masked[key] = _posm16(self.pos32, emb.mask_token, pk.bias32)
+                if masked:
+                    table = _posm16(self.pos32, emb.mask_token, bias32)
+                else:
+                    table = _posb16(self.pos32, emb.cls_token, bias32)
+            self._tables[(fmt, masked)] = table
         return table
 
 
@@ -735,6 +654,17 @@ def pos_grid(emb, gh: int, gw: int, keep: int = POS_GRIDS_KEPT) -> PosGrid:
     while len(cache) > keep:
         cache.popitem(last=False)
     return value
+
+
+def grid_table(emb, grid: Optional[tuple], fmt: Optional[tuple], masked: bool,
+               keep: int = POS_GRIDS_KEPT) -> torch.Tensor:
+    """bf16 [1 + gh * gw, D] position table of the tensor-core patch embedding for patch grid ``grid`` (None: the
+    model's own) and pixels of format ``fmt``; with ``masked`` the table of masked patches.  The pack's ``posb16`` /
+    ``posm16`` at the trained grid, else ``PosGrid.table`` of the resampled grid; ``keep``: grids ``pos_grid`` keeps."""
+    if grid is None or grid == native_grid(emb):
+        pk = embed_pack(emb, fmt)
+        return pk.posm16 if masked else pk.posb16
+    return pos_grid(emb, *grid, keep=keep).table(emb, fmt, masked)
 
 
 # ------------------------------------------------------------------------------------------------ ragged batches
@@ -807,19 +737,6 @@ def check_ragged(emb, images) -> tuple:
     return grids, u8
 
 
-def _ragged_table(emb, grid, u8: bool, image_mean, image_std, rescale_factor: float, keep: int) -> torch.Tensor:
-    """bf16 [1 + gh * gw, D] position table of one grid for the ragged gather: the one the image's own
-    interpolate_pos_encoding=True call reads (the packed table at the trained grid).  ``keep``: grids ``pos_grid``
-    keeps."""
-    if u8:
-        if grid == native_grid(emb):
-            return u8_pack(emb, image_mean, image_std, rescale_factor)[1].posb16
-        return pos_grid(emb, *grid, keep=keep).token_table_u8(emb, image_mean, image_std, rescale_factor)
-    if grid == native_grid(emb):
-        return emb.packed().posb16
-    return pos_grid(emb, *grid, keep=keep).token_table(emb)
-
-
 def _to_device_async(host_bytes: bytes, device) -> torch.Tensor:
     """Bytes -> a device uint8 tensor: staged in pinned host memory, one cudaMemcpyAsync on the current stream (the
     pinned block is not reused before the copy has run)."""
@@ -833,7 +750,8 @@ def _to_device_async(host_bytes: bytes, device) -> torch.Tensor:
 def patch_embed_ragged(emb, images, layout: RaggedLayout, stats: Optional[torch.Tensor] = None, u8: bool = False,
                        image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
                        rescale_factor: float = 1.0 / 255.0) -> torch.Tensor:
-    """Images of different sizes -> packed token embeddings (1, M, D) in ``layout``'s row order: per chunk of at most
+    """Images of different sizes (raw uint8 ones with these image-processor constants when ``u8``) -> packed token
+    embeddings (1, M, D) in ``layout``'s row order: per chunk of at most
     ``RAGGED_MAX_ROWS`` rows one ``vt_patch_embed_ragged_gather`` (patch rows + per-row position table) and one
     ``vt_gemm_bf16_ln`` over the packed rows with the table as its residual (and ``stats``, (M, D/128, 2) fp32, the row
     statistics for block 0's folded LayerNorm).  Every image's rows equal its own ``interpolate_pos_encoding=True``
@@ -842,15 +760,16 @@ def patch_embed_ragged(emb, images, layout: RaggedLayout, stats: Optional[torch.
     D = emb.hidden_dim
     assert w.is_cuda and w.dtype == torch.bfloat16 and D % 8 == 0, \
         "The ragged patch embedding runs on the bf16 tensor-core kernels only"
-    pk = u8_pack(emb, image_mean, image_std, rescale_factor)[1] if u8 else emb.packed()
+    fmt = pixel_format(image_mean, image_std, rescale_factor) if u8 else None
+    pk = embed_pack(emb, fmt)
     device = images[0].device
     # every grid's table is held here until the launches are enqueued, and the cache keeps at least this list's grids:
     # a list of many aspect ratios, run again, finds all of its tables instead of resampling each one per call
     grids = list(dict.fromkeys(layout.grids))
     keep = max(POS_GRIDS_KEPT, len(grids))
-    tables = {g: _ragged_table(emb, g, u8, image_mean, image_std, rescale_factor, keep) for g in grids}
+    tables = {g: grid_table(emb, g, fmt, False, keep) for g in grids}
     pixels = [img.contiguous() for img in images]
-    code = _lib.VT_U8 if u8 else _lib.dtype_code(pixels[0])
+    code = _lib.dtype_code(pixels[0]) if fmt is None else _lib.VT_U8
     out = torch.empty((1, layout.rows, D), device=device, dtype=w.dtype)
     stream = _lib.stream_ptr(out)
     for chunk in layout.chunks():
@@ -858,8 +777,7 @@ def patch_embed_ragged(emb, images, layout: RaggedLayout, stats: Optional[torch.
         rows = sum(layout.tokens[i] for i in chunk)
         desc = (_lib.RaggedImage * len(chunk))()
         for j, i in enumerate(chunk):
-            shape = pixels[i].shape
-            h, wd = (shape[0], shape[1]) if u8 else (shape[1], shape[2])
+            _, _, h, wd = pixel_dims(pixels[i][None], fmt)
             desc[j] = _lib.RaggedImage(pixels[i].data_ptr(), tables[layout.grids[i]].data_ptr(),
                                        layout.row0[i] - base, h, wd, layout.tokens[i], 0)
         desc_dev = _to_device_async(bytes(desc), device)

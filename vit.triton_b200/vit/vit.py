@@ -347,9 +347,27 @@ class Embeddings(packing.PackedMixin, nn.Module):
         position table resampled to that grid (``interpolate_pos_encoding(H, W)``), like HF ``ViTEmbeddings``.
         ``bool_masked_pos``: bool (B, N - 1), needs ``use_mask_token=True``: a masked patch's embedding is the mask token
         (plus its position embedding), like HF ``ViTEmbeddings``."""
+        return self._embed(x, None, stats_out, interpolate_pos_encoding, bool_masked_pos)
+
+    def forward_uint8(self, x, image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
+                      rescale_factor: float = 1.0 / 255.0, stats_out: Optional[torch.Tensor] = None,
+                      interpolate_pos_encoding: bool = False,
+                      bool_masked_pos: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Raw uint8 NHWC pixels (B, H, W, C) -> embeddings: the image processor's rescale and
+        normalisation (defaults: HF ``ViTImageProcessor`` of google/vit-base-patch16-224) are folded
+        into the patch projection, see ``packing.pack_embeddings``.  ``interpolate_pos_encoding`` and
+        ``bool_masked_pos`` as for ``forward``."""
+        return self._embed(x, packing.pixel_format(image_mean, image_std, rescale_factor), stats_out,
+                           interpolate_pos_encoding, bool_masked_pos)
+
+    def _embed(self, x, fmt, stats_out: Optional[torch.Tensor], interpolate_pos_encoding: bool,
+               bool_masked_pos: Optional[torch.Tensor]) -> torch.Tensor:
+        """Embeddings of pixels of format ``fmt`` (``packing.patch_embed``): uint8 pixels always take the fused patch
+        embedding, float pixels when the fused execution is on and they are on the GPU."""
         if bool_masked_pos is not None:
-            self.check_mask(bool_masked_pos, x, x.shape[2], x.shape[3], interpolate_pos_encoding)
-        if not (_FUSED and x.is_cuda):
+            _, _, H, W = packing.pixel_dims(x, fmt)
+            self.check_mask(bool_masked_pos, x, H, W, interpolate_pos_encoding)
+        if fmt is None and not (_FUSED and x.is_cuda):
             assert stats_out is None
             pos = self.position_embeddings
             if interpolate_pos_encoding:
@@ -362,20 +380,7 @@ class Embeddings(packing.PackedMixin, nn.Module):
             out[:, 1:, :] = tokens
             packing.finalize_embeddings(self, out, pos, bool_masked_pos)
             return out
-        return packing.patch_embed(self, x, stats_out, interpolate=interpolate_pos_encoding, mask=bool_masked_pos)
-
-    def forward_uint8(self, x, image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
-                      rescale_factor: float = 1.0 / 255.0, stats_out: Optional[torch.Tensor] = None,
-                      interpolate_pos_encoding: bool = False,
-                      bool_masked_pos: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """Raw uint8 NHWC pixels (B, H, W, C) -> embeddings: the image processor's rescale and
-        normalisation (defaults: HF ``ViTImageProcessor`` of google/vit-base-patch16-224) are folded
-        into the patch projection, see ``packing.pack_embeddings_u8``.  ``interpolate_pos_encoding`` and
-        ``bool_masked_pos`` as for ``forward``."""
-        if bool_masked_pos is not None:
-            self.check_mask(bool_masked_pos, x, x.shape[1], x.shape[2], interpolate_pos_encoding)
-        return packing.patch_embed_u8(self, x, image_mean, image_std, rescale_factor, stats_out,
-                                      interpolate=interpolate_pos_encoding, mask=bool_masked_pos)
+        return packing.patch_embed(self, x, fmt, stats_out, interpolate=interpolate_pos_encoding, mask=bool_masked_pos)
 
     def check_mask(self, bool_masked_pos, x, height: int, width: int, interpolate_pos_encoding: bool) -> None:
         """AssertionError, before anything is launched, unless ``bool_masked_pos`` fits pixels ``x`` of that size."""
@@ -404,6 +409,9 @@ class Embeddings(packing.PackedMixin, nn.Module):
 
     def _build_packed(self):
         return packing.pack_embeddings(self)
+
+    def _build_packed_u8(self, fmt):
+        return packing.pack_embeddings(self, fmt)
 
 
 def _head_on_cls(hidden: torch.Tensor, dense: "LinearWithBias", act: int) -> torch.Tensor:
@@ -543,7 +551,6 @@ class VIT(nn.Module):
         for m in self.modules():
             if isinstance(m, packing.PackedMixin):
                 m.invalidate_packed()
-            m.__dict__.pop("_u8_pack", None)
         clear_derived_cache()
 
     @property
@@ -569,22 +576,7 @@ class VIT(nn.Module):
         path with head dim 64 or 80 each block's probabilities take one ``vt_attn_probs`` launch, elsewhere they are
         the ones the attention materialises.  Not for a list of images."""
         self._check_outputs(x, output_hidden_states, output_attentions)
-        if bool_masked_pos is not None:
-            assert not isinstance(x, (list, tuple)), "bool_masked_pos is not supported with a list of images"
-        if interpolate_pos_encoding:
-            assert x.dim() == 4, f"Expected (B, C, H, W) pixels, provided: {tuple(x.shape)}"
-            packing.check_any_size(self.embeddings, *x.shape[1:])
-            n_tok = 1 + math.prod(packing.patch_grid(self.embeddings, x.shape[2], x.shape[3]))
-        else:
-            assert x.shape[1:] == (self.channels, self.height, self.width), f"Image size {x.shape[1:]} not matching with the model input size: {self.channels, self.height, self.width}"
-            n_tok = None
-        if bool_masked_pos is not None:
-            self.embeddings.check_mask(bool_masked_pos, x, x.shape[2], x.shape[3], interpolate_pos_encoding)
-        stats = self._embed_stats(x, n_tok)
-        kw = dict(interpolate_pos_encoding=True) if interpolate_pos_encoding else {}
-        if bool_masked_pos is not None:
-            kw["bool_masked_pos"] = bool_masked_pos
-        x = self.embeddings(x, stats, **kw) if stats is not None else self.embeddings(x, **kw)
+        x, stats = self._embed(x, None, interpolate_pos_encoding, bool_masked_pos)
         return self._encode(x, stats, output_hidden_states, output_attentions)
 
     @staticmethod
@@ -639,22 +631,37 @@ class VIT(nn.Module):
         ``forward_uint8(resize_uint8(x, height, width, resample), ...)`` bit for bit."""
         x = self._resized(x, do_resize, resample)
         self._check_outputs(x, output_hidden_states, output_attentions)
+        x, stats = self._embed(x, packing.pixel_format(image_mean, image_std, rescale_factor), interpolate_pos_encoding,
+                               bool_masked_pos)
+        return self._encode(x, stats, output_hidden_states, output_attentions)
+
+    def _embed(self, x, fmt, interpolate_pos_encoding: bool, bool_masked_pos: Optional[torch.Tensor]) -> tuple:
+        """(embeddings, row-statistics buffer or None) of pixels of format ``fmt`` (``packing.patch_embed``), after the
+        checks of ``forward`` / ``forward_uint8``, which raise before anything is launched."""
         if bool_masked_pos is not None:
             assert not isinstance(x, (list, tuple)), "bool_masked_pos is not supported with a list of images"
-        if interpolate_pos_encoding:
-            assert x.dim() == 4, f"Expected (B, H, W, C) pixels, provided: {tuple(x.shape)}"
-            packing.check_any_size(self.embeddings, x.shape[3], x.shape[1], x.shape[2])
-            n_tok = 1 + math.prod(packing.patch_grid(self.embeddings, x.shape[1], x.shape[2]))
+        if fmt is None:
+            layout, size = "(B, C, H, W)", (self.channels, self.height, self.width)
         else:
-            assert tuple(x.shape[1:]) == (self.height, self.width, self.channels), f"Image size {x.shape[1:]} not matching with the model input size: {self.height, self.width, self.channels}"
+            layout, size = "(B, H, W, C)", (self.height, self.width, self.channels)
+        if interpolate_pos_encoding:
+            assert x.dim() == 4, f"Expected {layout} pixels, provided: {tuple(x.shape)}"
+            _, C, H, W = packing.pixel_dims(x, fmt)
+            packing.check_any_size(self.embeddings, C, H, W)
+            n_tok = 1 + math.prod(packing.patch_grid(self.embeddings, H, W))
+        else:
+            assert tuple(x.shape[1:]) == size, f"Image size {x.shape[1:]} not matching with the model input size: {size}"
             n_tok = None
         if bool_masked_pos is not None:
-            self.embeddings.check_mask(bool_masked_pos, x, x.shape[1], x.shape[2], interpolate_pos_encoding)
+            _, _, H, W = packing.pixel_dims(x, fmt)
+            self.embeddings.check_mask(bool_masked_pos, x, H, W, interpolate_pos_encoding)
         stats = self._embed_stats(x, n_tok)
-        x = self.embeddings.forward_uint8(x, image_mean, image_std, rescale_factor, stats,
-                                          interpolate_pos_encoding=interpolate_pos_encoding,
-                                          bool_masked_pos=bool_masked_pos)
-        return self._encode(x, stats, output_hidden_states, output_attentions)
+        if fmt is not None:
+            return self.embeddings._embed(x, fmt, stats, interpolate_pos_encoding, bool_masked_pos), stats
+        kw = dict(interpolate_pos_encoding=True) if interpolate_pos_encoding else {}
+        if bool_masked_pos is not None:
+            kw["bool_masked_pos"] = bool_masked_pos
+        return (self.embeddings(x, stats, **kw) if stats is not None else self.embeddings(x, **kw)), stats
 
     def _resized(self, x, do_resize: bool, resample: int):
         """x itself, or with ``do_resize`` the uint8 (B, height, width, C) batch ``resize_uint8`` makes of x (a batch already

@@ -1,5 +1,5 @@
 // extern "C" surface of libvitb200.so (declared in include/vitb200.h and its companions
-// vitb200_resolution.h, vitb200_ragged.h, vitb200_mask.h).  Thin: argument plumbing
+// vitb200_resolution.h, vitb200_ragged.h, vitb200_mask.h, vitb200_tokens.h).  Thin: argument plumbing
 // only, all kernels live in the other translation units.
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -9,6 +9,7 @@
 #include "../../include/vitb200_resolution.h"
 #include "../../include/vitb200_ragged.h"
 #include "../../include/vitb200_mask.h"
+#include "../../include/vitb200_tokens.h"
 
 namespace vt {
 int layernorm_rows(const void*, const void*, const void*, void*, long long, int, long long,
@@ -44,18 +45,19 @@ int gemm2_fp8_tcgen05(const void*, long long, const void*, long long, void*, lon
 int layernorm_e4m3(const void*, const void*, const void*, void*, long long, int, long long, long long, float, float,
                    cudaStream_t);
 int quantize_rows_e4m3(const void*, long long, void*, long long, float*, int, int, cudaStream_t);
-int patch_gather(const void*, int, void*, int, int, int, int, int, int, int, cudaStream_t);
-int pos_resample(const void*, int, float*, int, int, int, int, cudaStream_t);
-int patch_gather_ragged(const void*, int, int, int, int, void*, long long, void*, int, long long, cudaStream_t);
+int patch_gather(const void*, int, void*, int, int, int, int, int, int, int, int, cudaStream_t);
+int pos_resample(const void*, int, float*, int, int, int, int, int, cudaStream_t);
+int patch_gather_ragged(const void*, int, int, int, int, void*, long long, void*, int, long long, int, cudaStream_t);
 int gather_rows(const void*, long long, const long long*, void*, long long, int, int, int, cudaStream_t);
 int gemm2_patch_tokens(const void*, long long, const void*, long long, void*, const float*, const void*, float*, int, int,
                        int, int, int, int, cudaStream_t);
 int ln_fold(const void*, long long, const float*, const float*, const float*, void*, long long, float*, float*, int,
             int, int, cudaStream_t);
-int embed_finalize(void*, const void*, const void*, int, int, int, int, cudaStream_t);
+int embed_finalize(void*, const void*, const void*, int, int, int, int, int, cudaStream_t);
 int patch_gather_masked(const void*, int, const void*, const void*, const void*, void*, long long, void*, int, int, int,
-                        int, int, int, cudaStream_t);
-int embed_finalize_masked(void*, const void*, const void*, const void*, const void*, int, int, int, int, cudaStream_t);
+                        int, int, int, int, cudaStream_t);
+int embed_finalize_masked(void*, const void*, const void*, const void*, const void*, int, int, int, int, int,
+                          cudaStream_t);
 int mim_reconstruct(const void*, void*, int, int, int, int, int, int, const void*, int, const float*, float, const void*,
                     float*, float*, cudaStream_t);
 int conv2d_nchw(const void*, const void*, const void*, void*, int, int, int, int, int, int, int,
@@ -234,14 +236,22 @@ int vt_patch_embed_gemm(const void* pixels, int32_t pix_dtype, const void* w, in
 int vt_patch_embed_gemm_hw(const void* pixels, int32_t pix_dtype, const void* w, int64_t ldw, const float* bias,
                            const void* posb, void* out, float* stats_out, void* workspace, int32_t B, int32_t C,
                            int32_t H, int32_t W, int32_t P, int32_t D, void* stream) {
-  if (P <= 0 || H < P || W < P || !workspace) return VT_ERR_ARG;
+  return vt_patch_embed_gemm_hw_prefix(pixels, pix_dtype, w, ldw, bias, posb, out, stats_out, workspace, B, C, H, W, P,
+                                       D, 1, stream);
+}
+
+int vt_patch_embed_gemm_hw_prefix(const void* pixels, int32_t pix_dtype, const void* w, int64_t ldw, const float* bias,
+                                  const void* posb, void* out, float* stats_out, void* workspace, int32_t B, int32_t C,
+                                  int32_t H, int32_t W, int32_t P, int32_t D, int32_t prefix, void* stream) {
+  if (P <= 0 || H < P || W < P || !workspace || prefix < 1 || prefix > 2) return VT_ERR_ARG;
   const long long n = static_cast<long long>(H / P) * (W / P);
   if (n + 32 > 0x7fffffffLL) return VT_ERR_UNSUPPORTED;
-  const int tokens = static_cast<int>(n) + 1;
+  const int tokens = static_cast<int>(n) + prefix;
   const int tok_pad = (tokens + 31) & ~31;
   const int K = C * P * P;
   if (ldw < K || (ldw % 8)) return VT_ERR_ALIGN;
-  const int rc = vt::patch_gather(pixels, pix_dtype, workspace, B, C, H, W, P, tok_pad, static_cast<int>(ldw), S(stream));
+  const int rc = vt::patch_gather(pixels, pix_dtype, workspace, B, C, H, W, P, tok_pad, static_cast<int>(ldw), prefix,
+                                  S(stream));
   if (rc) return rc;
   return vt::gemm2_patch_tokens(workspace, ldw, w, ldw, out, bias, posb, stats_out, B, tok_pad, tokens, D,
                                 static_cast<int>(ldw), next_direction(), S(stream));
@@ -249,13 +259,24 @@ int vt_patch_embed_gemm_hw(const void* pixels, int32_t pix_dtype, const void* w,
 
 int vt_pos_embed_resample(const void* pos, int32_t pos_dtype, float* out, int32_t D, int32_t g_in, int32_t gh,
                           int32_t gw, void* stream) {
-  return vt::pos_resample(pos, pos_dtype, out, D, g_in, gh, gw, S(stream));
+  return vt_pos_embed_resample_prefix(pos, pos_dtype, out, D, g_in, gh, gw, 1, stream);
+}
+
+int vt_pos_embed_resample_prefix(const void* pos, int32_t pos_dtype, float* out, int32_t D, int32_t g_in, int32_t gh,
+                                 int32_t gw, int32_t prefix, void* stream) {
+  return vt::pos_resample(pos, pos_dtype, out, D, g_in, gh, gw, prefix, S(stream));
 }
 
 int vt_patch_embed_ragged_gather(const vt_ragged_image* images, int32_t n_images, int32_t pix_dtype, int32_t C,
                                  int32_t P, void* patches, int64_t ldw, void* table, int32_t D, int64_t M,
                                  void* stream) {
-  return vt::patch_gather_ragged(images, n_images, pix_dtype, C, P, patches, ldw, table, D, M, S(stream));
+  return vt_patch_embed_ragged_gather_prefix(images, n_images, pix_dtype, C, P, patches, ldw, table, D, M, 1, stream);
+}
+
+int vt_patch_embed_ragged_gather_prefix(const vt_ragged_image* images, int32_t n_images, int32_t pix_dtype, int32_t C,
+                                        int32_t P, void* patches, int64_t ldw, void* table, int32_t D, int64_t M,
+                                        int32_t prefix, void* stream) {
+  return vt::patch_gather_ragged(images, n_images, pix_dtype, C, P, patches, ldw, table, D, M, prefix, S(stream));
 }
 
 int vt_gather_rows(const void* x, int64_t ldx, const int64_t* idx, void* out, int64_t ldo, int32_t rows, int32_t cols,
@@ -270,18 +291,38 @@ int vt_patching(const void* image, void* out, int32_t B, int32_t C, int32_t H, i
 
 int vt_embed_finalize(void* x, const void* pos, const void* cls, int32_t B, int32_t N, int32_t D,
                       int32_t dtype, void* stream) {
-  return vt::embed_finalize(x, pos, cls, B, N, D, dtype, S(stream));
+  return vt_embed_finalize_prefix(x, pos, cls, B, N, D, dtype, 1, stream);
+}
+
+int vt_embed_finalize_prefix(void* x, const void* pos, const void* prefix_rows, int32_t B, int32_t N, int32_t D,
+                             int32_t dtype, int32_t prefix, void* stream) {
+  return vt::embed_finalize(x, pos, prefix_rows, B, N, D, dtype, prefix, S(stream));
 }
 
 int vt_patch_embed_masked_gather(const void* pixels, int32_t pix_dtype, const void* mask, const void* pos,
                                  const void* posm, void* patches, int64_t ldw, void* table, int32_t B, int32_t C,
                                  int32_t H, int32_t W, int32_t P, int32_t D, void* stream) {
-  return vt::patch_gather_masked(pixels, pix_dtype, mask, pos, posm, patches, ldw, table, B, C, H, W, P, D, S(stream));
+  return vt_patch_embed_masked_gather_prefix(pixels, pix_dtype, mask, pos, posm, patches, ldw, table, B, C, H, W, P, D,
+                                             1, stream);
+}
+
+int vt_patch_embed_masked_gather_prefix(const void* pixels, int32_t pix_dtype, const void* mask, const void* pos,
+                                        const void* posm, void* patches, int64_t ldw, void* table, int32_t B,
+                                        int32_t C, int32_t H, int32_t W, int32_t P, int32_t D, int32_t prefix,
+                                        void* stream) {
+  return vt::patch_gather_masked(pixels, pix_dtype, mask, pos, posm, patches, ldw, table, B, C, H, W, P, D, prefix,
+                                 S(stream));
 }
 
 int vt_embed_finalize_masked(void* x, const void* pos, const void* cls, const void* mask_token, const void* mask,
                              int32_t B, int32_t N, int32_t D, int32_t dtype, void* stream) {
-  return vt::embed_finalize_masked(x, pos, cls, mask_token, mask, B, N, D, dtype, S(stream));
+  return vt_embed_finalize_masked_prefix(x, pos, cls, mask_token, mask, B, N, D, dtype, 1, stream);
+}
+
+int vt_embed_finalize_masked_prefix(void* x, const void* pos, const void* prefix_rows, const void* mask_token,
+                                    const void* mask, int32_t B, int32_t N, int32_t D, int32_t dtype, int32_t prefix,
+                                    void* stream) {
+  return vt::embed_finalize_masked(x, pos, prefix_rows, mask_token, mask, B, N, D, dtype, prefix, S(stream));
 }
 
 int vt_mim_reconstruct(const void* dec, void* rec, int32_t dtype, int32_t B, int32_t C, int32_t gh, int32_t gw,

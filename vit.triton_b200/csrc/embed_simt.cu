@@ -2,7 +2,8 @@
 //   patching        (B,C,H,W) -> (B, n, C*P*P) patch rows in (c, i, j) order.  Same contract as the
 //                   reference's exported-but-unused `patching` entry point
 //                   (vit/kernels/patching.py:54-92, torch restatement :95-105).
-//   embed_finalize  x[b,0,:] = cls + pos[0] ; x[b,t,:] += pos[t]  (vit/vit.py:195-200)
+//   embed_finalize  x[b,t,:] = prefix_rows[t] + pos[t] for t < prefix ; x[b,t,:] += pos[t]  (vit/vit.py:195-200);
+//                   prefix_rows = [cls] (ViT) or [cls; distillation token] (DeiT)
 //   conv2d_nchw     generic strided conv with stride == kernel (vit/kernels/conv2d.py:100-150),
 //                   output (B, O, H/kh, W/kw) like the reference; used by the standalone entry point.
 #include "common.cuh"
@@ -37,22 +38,22 @@ __global__ void patching_kernel(const T* __restrict__ img, T* __restrict__ out, 
 
 template <typename T>
 __global__ void embed_finalize_kernel(T* __restrict__ x, const T* __restrict__ pos,
-                                      const T* __restrict__ cls, int B, int N, int D) {
+                                      const T* __restrict__ prefix_rows, int B, int N, int D, int prefix) {
   const long long total = static_cast<long long>(B) * N * D;
   const long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (idx >= total) return;
   const int d = static_cast<int>(idx % D);
   const int t = static_cast<int>((idx / D) % N);
   const float pv = ldf(pos + static_cast<long long>(t) * D + d);
-  const float v = (t == 0) ? ldf(cls + d) : ldf(x + idx);
+  const float v = (t < prefix) ? ldf(prefix_rows + static_cast<long long>(t) * D + d) : ldf(x + idx);
   stf(x + idx, v + pv);
 }
 
 // embed_finalize with bool_masked_pos: a masked patch's projection is replaced by the mask token before pos is added
 template <typename T>
-__global__ void embed_finalize_masked_kernel(T* __restrict__ x, const T* __restrict__ pos, const T* __restrict__ cls,
-                                             const T* __restrict__ mask_token, const uint8_t* __restrict__ mask,
-                                             int B, int N, int D) {
+__global__ void embed_finalize_masked_kernel(T* __restrict__ x, const T* __restrict__ pos,
+                                             const T* __restrict__ prefix_rows, const T* __restrict__ mask_token,
+                                             const uint8_t* __restrict__ mask, int B, int N, int D, int prefix) {
   const long long total = static_cast<long long>(B) * N * D;
   const long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (idx >= total) return;
@@ -62,8 +63,8 @@ __global__ void embed_finalize_masked_kernel(T* __restrict__ x, const T* __restr
   const long long b = bt / N;
   const float pv = ldf(pos + static_cast<long long>(t) * D + d);
   float v;
-  if (t == 0) v = ldf(cls + d);
-  else if (mask[b * (N - 1) + t - 1]) v = ldf(mask_token + d);
+  if (t < prefix) v = ldf(prefix_rows + static_cast<long long>(t) * D + d);
+  else if (mask[b * (N - prefix) + t - prefix]) v = ldf(mask_token + d);
   else v = ldf(x + idx);
   stf(x + idx, v + pv);
 }
@@ -112,40 +113,42 @@ int patching(const void* img, void* out, int B, int C, int H, int W, int P, int 
   return static_cast<int>(cudaGetLastError());
 }
 
-int embed_finalize(void* x, const void* pos, const void* cls, int B, int N, int D, int dtype,
+int embed_finalize(void* x, const void* pos, const void* prefix_rows, int B, int N, int D, int dtype, int prefix,
                    cudaStream_t stream) {
-  if (!x || !pos || !cls || B < 0 || N <= 0 || D <= 0) return VT_ERR_ARG;
+  if (!x || !pos || !prefix_rows || B < 0 || N < prefix || D <= 0 || prefix < 1 || prefix > 2) return VT_ERR_ARG;
   const long long total = static_cast<long long>(B) * N * D;
   if (total == 0) return VT_OK;
   const unsigned grid = static_cast<unsigned>((total + 255) / 256);
   if (dtype == VT_F32)
     embed_finalize_kernel<float><<<grid, 256, 0, stream>>>(
-        static_cast<float*>(x), static_cast<const float*>(pos), static_cast<const float*>(cls), B,
-        N, D);
+        static_cast<float*>(x), static_cast<const float*>(pos), static_cast<const float*>(prefix_rows), B,
+        N, D, prefix);
   else if (dtype == VT_BF16)
     embed_finalize_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(
         static_cast<__nv_bfloat16*>(x), static_cast<const __nv_bfloat16*>(pos),
-        static_cast<const __nv_bfloat16*>(cls), B, N, D);
+        static_cast<const __nv_bfloat16*>(prefix_rows), B, N, D, prefix);
   else
     return VT_ERR_DTYPE;
   return static_cast<int>(cudaGetLastError());
 }
 
-int embed_finalize_masked(void* x, const void* pos, const void* cls, const void* mask_token, const void* mask, int B,
-                          int N, int D, int dtype, cudaStream_t stream) {
-  if (!x || !pos || !cls || !mask_token || !mask || B < 0 || N <= 0 || D <= 0) return VT_ERR_ARG;
+int embed_finalize_masked(void* x, const void* pos, const void* prefix_rows, const void* mask_token, const void* mask,
+                          int B, int N, int D, int dtype, int prefix, cudaStream_t stream) {
+  if (!x || !pos || !prefix_rows || !mask_token || !mask || B < 0 || N < prefix || D <= 0 || prefix < 1 || prefix > 2)
+    return VT_ERR_ARG;
   const long long total = static_cast<long long>(B) * N * D;
   if (total == 0) return VT_OK;
   const unsigned grid = static_cast<unsigned>((total + 255) / 256);
   const uint8_t* m = static_cast<const uint8_t*>(mask);
   if (dtype == VT_F32)
     embed_finalize_masked_kernel<float><<<grid, 256, 0, stream>>>(
-        static_cast<float*>(x), static_cast<const float*>(pos), static_cast<const float*>(cls),
-        static_cast<const float*>(mask_token), m, B, N, D);
+        static_cast<float*>(x), static_cast<const float*>(pos), static_cast<const float*>(prefix_rows),
+        static_cast<const float*>(mask_token), m, B, N, D, prefix);
   else if (dtype == VT_BF16)
     embed_finalize_masked_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(
         static_cast<__nv_bfloat16*>(x), static_cast<const __nv_bfloat16*>(pos),
-        static_cast<const __nv_bfloat16*>(cls), static_cast<const __nv_bfloat16*>(mask_token), m, B, N, D);
+        static_cast<const __nv_bfloat16*>(prefix_rows), static_cast<const __nv_bfloat16*>(mask_token), m, B, N, D,
+        prefix);
   else
     return VT_ERR_DTYPE;
   return static_cast<int>(cudaGetLastError());

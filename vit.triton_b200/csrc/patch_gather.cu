@@ -1,10 +1,12 @@
 // K2a: patch gather — pixels -> padded bf16 patch rows, the A operand of the patch-embedding GEMM (K2b = the
 // 2-CTA tcgen05 GEMM of gemm2_sm100.cu in token mode).  Bandwidth-bound, every pixel is read ONCE:
 //
-//   A[b, 0, :]        = 0                                   (CLS slot: the GEMM adds bias + (cls + pos[0] - bias))
-//   A[b, 1 + p, k]    = pixel k of patch p of image b       k = (c, i, j) for NCHW fp32 / bf16 pixels,
+//   A[b, t, :]        = 0 for t < prefix                    (CLS / distillation slots: the GEMM adds bias + posb[t])
+//   A[b, prefix + p, k] = pixel k of patch p of image b     k = (c, i, j) for NCHW fp32 / bf16 pixels,
 //                                                           k = (i, j, c) for NHWC uint8 pixels
-//   A[b, t, :]        = 0 for n < t < Tpad,  A[.., k] = 0 for K <= k < Kpad
+//   A[b, t, :]        = 0 for prefix + n <= t < Tpad,  A[.., k] = 0 for K <= k < Kpad
+//
+// prefix = the tokens in front of the patches: 1 (CLS, ViT) or 2 (CLS and distillation token, DeiT).
 //
 // Tpad = tokens rounded up to 32: no 32-row tile of the GEMM's epilogue straddles two images, so its output and
 // position-table coordinates are (token, image) and TMA clips the padding rows.  Gather + GEMM need one pass over the
@@ -22,7 +24,7 @@ namespace {
 struct GatherParams {
   const void* pixels;
   __nv_bfloat16* out;
-  int B, C, H, W, P, grid_w, n_patches, K, Kpad, Tpad;
+  int B, C, H, W, P, grid_w, n_patches, K, Kpad, Tpad, prefix;
   long long total_chunks;    // B * Tpad * Kpad / 8
 };
 
@@ -90,9 +92,9 @@ patch_gather_kernel(const GatherParams p) {
   const int chunks_per_row = p.Kpad >> 3;
   const int t = blockIdx.x;
   const int b = blockIdx.y;
-  const int patch = t - 1;
+  const int patch = t - p.prefix;
   const int py = patch / p.grid_w, px = patch - py * p.grid_w;      // block-uniform
-  const bool real_row = t >= 1 && t <= p.n_patches;
+  const bool real_row = patch >= 0 && patch < p.n_patches;
   const TPix* img = static_cast<const TPix*>(p.pixels) + static_cast<long long>(b) * p.C * p.H * p.W;
   uint4* out_row = reinterpret_cast<uint4*>(p.out) + (static_cast<long long>(b) * p.Tpad + t) * chunks_per_row;
   for (int kc = threadIdx.x; kc < chunks_per_row; kc += blockDim.x) {
@@ -114,10 +116,10 @@ int launch_gather(const GatherParams& p, cudaStream_t stream) {
 
 // pixels: [B, C, H, W] (f32 | bf16) or [B, H, W, C] (VT_U8); the patch grid is (H / P) x (W / P) rounded down, the
 // pixels of the last H % P rows and W % P columns belong to no patch (a stride-P convolution drops them too).
-// out: bf16 [B, Tpad, Kpad] (Kpad % 8 == 0, Tpad >= n_patches + 1), 16-byte aligned.
+// out: bf16 [B, Tpad, Kpad] (Kpad % 8 == 0, Tpad >= n_patches + prefix), 16-byte aligned.
 int patch_gather(const void* pixels, int pix_dtype, void* out, int B, int C, int H, int W, int P, int Tpad, int Kpad,
-                 cudaStream_t stream) {
-  if (!pixels || !out || B <= 0 || C <= 0 || P <= 0 || H < P || W < P) return VT_ERR_ARG;
+                 int prefix, cudaStream_t stream) {
+  if (!pixels || !out || B <= 0 || C <= 0 || P <= 0 || H < P || W < P || prefix < 1 || prefix > 2) return VT_ERR_ARG;
   GatherParams p;
   p.pixels = pixels;
   p.out = static_cast<__nv_bfloat16*>(out);
@@ -127,7 +129,8 @@ int patch_gather(const void* pixels, int pix_dtype, void* out, int B, int C, int
   p.K = C * P * P;
   p.Kpad = Kpad;
   p.Tpad = Tpad;
-  if ((Kpad % 8) || Kpad < p.K || Tpad < p.n_patches + 1) return VT_ERR_ARG;
+  p.prefix = prefix;
+  if ((Kpad % 8) || Kpad < p.K || Tpad < p.n_patches + prefix) return VT_ERR_ARG;
   if ((reinterpret_cast<uintptr_t>(pixels) | reinterpret_cast<uintptr_t>(out)) & 15) return VT_ERR_ALIGN;
   p.total_chunks = static_cast<long long>(B) * Tpad * (Kpad / 8);
   // vector loads need every 8-element chunk inside one patch row and 8-element aligned: image rows of a multiple of
@@ -155,7 +158,7 @@ struct RaggedParams {
   const vt_ragged_image* images;
   __nv_bfloat16* patches;
   __nv_bfloat16* table;
-  int n_images, C, P, K, Kpad, D;
+  int n_images, C, P, K, Kpad, D, prefix;
 };
 
 template <typename TPix>
@@ -176,8 +179,8 @@ patch_gather_ragged_kernel(const RaggedParams p) {
   const int t = covered ? static_cast<int>(t64) : 0;
   const int grid_w = W / p.P;
   const int n_patches = (H / p.P) * grid_w;
-  const bool real_row = covered && t >= 1 && t <= n_patches;
-  const int patch = real_row ? t - 1 : 0;
+  const bool real_row = covered && t >= p.prefix && t - p.prefix < n_patches;
+  const int patch = real_row ? t - p.prefix : 0;
   const int py = patch / grid_w, px = patch - py * grid_w;
   const TPix* img = static_cast<const TPix*>(d->pixels);
   const bool aligned = (reinterpret_cast<uintptr_t>(img) & 15) == 0;
@@ -218,8 +221,10 @@ patch_gather_ragged_kernel(const RaggedParams p) {
 }  // namespace
 
 int patch_gather_ragged(const void* images, int n_images, int pix_dtype, int C, int P, void* patches, long long ldw,
-                        void* table, int D, long long M, cudaStream_t stream) {
-  if (!images || !patches || !table || n_images <= 0 || C <= 0 || P <= 0 || D <= 0 || M <= 0) return VT_ERR_ARG;
+                        void* table, int D, long long M, int prefix, cudaStream_t stream) {
+  if (!images || !patches || !table || n_images <= 0 || C <= 0 || P <= 0 || D <= 0 || M <= 0 || prefix < 1 ||
+      prefix > 2)
+    return VT_ERR_ARG;
   if (M > 0x7fffffffLL) return VT_ERR_UNSUPPORTED;
   const long long K = static_cast<long long>(C) * P * P;
   if (ldw < K || ldw > 0x7fffffffLL) return VT_ERR_ARG;
@@ -230,6 +235,7 @@ int patch_gather_ragged(const void* images, int n_images, int pix_dtype, int C, 
   p.patches = static_cast<__nv_bfloat16*>(patches);
   p.table = static_cast<__nv_bfloat16*>(table);
   p.n_images = n_images; p.C = C; p.P = P; p.K = static_cast<int>(K); p.Kpad = static_cast<int>(ldw); p.D = D;
+  p.prefix = prefix;
   const dim3 grid(static_cast<unsigned int>(M));
   if (pix_dtype == VT_U8) patch_gather_ragged_kernel<uint8_t><<<grid, 128, 0, stream>>>(p);
   else if (pix_dtype == VT_BF16) patch_gather_ragged_kernel<__nv_bfloat16><<<grid, 128, 0, stream>>>(p);
@@ -242,6 +248,7 @@ int patch_gather_ragged(const void* images, int n_images, int pix_dtype, int C, 
 // bool_masked_pos (vt_patch_embed_masked_gather): one block per unpadded output row (blockIdx.x = token, blockIdx.y =
 // image).  A masked patch's row is zero and its table row carries mask_token + pos - bias, so the plain-mode GEMM's
 // bias + residual epilogue turns it into mask_token + pos; an unmasked row is the batched gather's row and pos[t].
+// The first `prefix` rows of an image are the CLS (and distillation) slots: zero rows, table rows from pos.
 namespace {
 
 struct MaskedParams {
@@ -251,7 +258,7 @@ struct MaskedParams {
   const uint4* posm;
   uint4* patches;
   uint4* table;
-  int C, H, W, P, grid_w, n_patches, K, Kpad, D;
+  int C, H, W, P, grid_w, n_patches, K, Kpad, D, prefix;
 };
 
 template <typename TPix, bool kVec>
@@ -259,10 +266,11 @@ __global__ void __launch_bounds__(128)
 patch_gather_masked_kernel(const MaskedParams p) {
   const int t = blockIdx.x;
   const int b = blockIdx.y;
-  const int N = p.n_patches + 1;
-  const int patch = t > 0 ? t - 1 : 0;
-  const bool masked = t > 0 && p.mask[static_cast<long long>(b) * p.n_patches + patch] != 0;   // block-uniform
-  const bool real_row = t > 0 && !masked;
+  const int N = p.n_patches + p.prefix;
+  const bool patch_row = t >= p.prefix;
+  const int patch = patch_row ? t - p.prefix : 0;
+  const bool masked = patch_row && p.mask[static_cast<long long>(b) * p.n_patches + patch] != 0;   // block-uniform
+  const bool real_row = patch_row && !masked;
   const int py = patch / p.grid_w, px = patch - py * p.grid_w;
   const TPix* img = static_cast<const TPix*>(p.pixels) + static_cast<long long>(b) * p.C * p.H * p.W;
   const long long row = static_cast<long long>(b) * N + t;
@@ -284,23 +292,23 @@ patch_gather_masked_kernel(const MaskedParams p) {
 
 template <typename TPix, bool kVec>
 int launch_masked(const MaskedParams& p, int B, cudaStream_t stream) {
-  patch_gather_masked_kernel<TPix, kVec><<<dim3(p.n_patches + 1, B), 128, 0, stream>>>(p);
+  patch_gather_masked_kernel<TPix, kVec><<<dim3(p.n_patches + p.prefix, B), 128, 0, stream>>>(p);
   return static_cast<int>(cudaGetLastError());
 }
 
 }  // namespace
 
 int patch_gather_masked(const void* pixels, int pix_dtype, const void* mask, const void* pos, const void* posm,
-                        void* patches, long long ldw, void* table, int B, int C, int H, int W, int P, int D,
+                        void* patches, long long ldw, void* table, int B, int C, int H, int W, int P, int D, int prefix,
                         cudaStream_t stream) {
   if (!pixels || !mask || !pos || !posm || !patches || !table || B <= 0 || C <= 0 || P <= 0 || D <= 0 || H < P ||
-      W < P)
+      W < P || prefix < 1 || prefix > 2)
     return VT_ERR_ARG;
   const long long K = static_cast<long long>(C) * P * P;
   if (ldw < K || ldw > 0x7fffffffLL) return VT_ERR_ARG;
   if ((ldw % 8) || (D % 8)) return VT_ERR_ALIGN;
   const long long n = static_cast<long long>(H / P) * (W / P);
-  if (B > 65535 || static_cast<long long>(B) * (n + 1) > 0x7fffffffLL) return VT_ERR_UNSUPPORTED;
+  if (B > 65535 || static_cast<long long>(B) * (n + prefix) > 0x7fffffffLL) return VT_ERR_UNSUPPORTED;
   if ((reinterpret_cast<uintptr_t>(pixels) | reinterpret_cast<uintptr_t>(patches) | reinterpret_cast<uintptr_t>(table) |
        reinterpret_cast<uintptr_t>(pos) | reinterpret_cast<uintptr_t>(posm)) & 15)
     return VT_ERR_ALIGN;
@@ -317,6 +325,7 @@ int patch_gather_masked(const void* pixels, int pix_dtype, const void* mask, con
   p.K = static_cast<int>(K);
   p.Kpad = static_cast<int>(ldw);
   p.D = D;
+  p.prefix = prefix;
   // the vector-load conditions of patch_gather
   if (pix_dtype == VT_U8) {
     const bool vec = ((P * C) % 8 == 0) && ((W * C) % 8 == 0);

@@ -2,8 +2,10 @@
 // other than the one it was trained at (HF ViTEmbeddings.interpolate_pos_encoding).  Pack-time work: one launch per
 // (weights, grid), the result is cached by the host (vit/vit.py Embeddings.interpolate_pos_encoding).
 //
-//   out[0, :]               = pos[0, :]                                         (CLS position, copied)
-//   out[1 + y * gw + x, :]  = bicubic(grid, y, x)  of the g_in x g_in grid pos[1 + i * g_in + j, :]
+//   out[t, :]                    = pos[t, :]  for t < prefix                    (CLS / distillation positions, copied)
+//   out[prefix + y * gw + x, :]  = bicubic(grid, y, x)  of the g_in x g_in grid pos[prefix + i * g_in + j, :]
+//
+// prefix = 1 (ViT) or 2 (DeiT: CLS and distillation token).
 //
 // bicubic = torch.nn.functional.interpolate(mode="bicubic", align_corners=False) with the channel stored last, in
 // fp32 with torch's CPU arithmetic: src = (in / out) * (dst + 0.5) - 0.5 (not clamped), i = floor(src),
@@ -48,14 +50,14 @@ __device__ __forceinline__ float ldp(const __nv_bfloat16* p) { return __bfloat16
 template <typename T>
 __global__ void __launch_bounds__(256)
 pos_resample_kernel(const T* __restrict__ pos, float* __restrict__ out, int D, int g_in, int gh, int gw,
-                    float scale_h, float scale_w) {
+                    float scale_h, float scale_w, int prefix) {
   const int t = blockIdx.x;
   float* dst = out + static_cast<long long>(t) * D;
-  if (t == 0) {
-    for (int d = threadIdx.x; d < D; d += blockDim.x) dst[d] = ldp(pos + d);
+  if (t < prefix) {
+    for (int d = threadIdx.x; d < D; d += blockDim.x) dst[d] = ldp(pos + static_cast<long long>(t) * D + d);
     return;
   }
-  const int y = (t - 1) / gw, x = (t - 1) - y * gw;
+  const int y = (t - prefix) / gw, x = (t - prefix) - y * gw;
   float wy[4], wx[4];
   const int y0 = source_taps(y, scale_h, wy);
   const int x0 = source_taps(x, scale_w, wx);
@@ -65,7 +67,7 @@ pos_resample_kernel(const T* __restrict__ pos, float* __restrict__ out, int D, i
     rows[a] = min(max(y0 + a, 0), g_in - 1);
     cols[a] = min(max(x0 + a, 0), g_in - 1);
   }
-  const T* grid = pos + D;   // row 1 of the table = grid position (0, 0)
+  const T* grid = pos + static_cast<long long>(prefix) * D;   // row prefix of the table = grid position (0, 0)
   for (int d = threadIdx.x; d < D; d += blockDim.x) {
     float h[4];
 #pragma unroll
@@ -80,10 +82,11 @@ pos_resample_kernel(const T* __restrict__ pos, float* __restrict__ out, int D, i
 
 }  // namespace
 
-// pos: [1 + g_in^2, D] (f32 | bf16), out: f32 [1 + gh * gw, D]; distinct buffers.
-int pos_resample(const void* pos, int pos_dtype, float* out, int D, int g_in, int gh, int gw, cudaStream_t stream) {
-  if (!pos || !out || D <= 0 || g_in <= 0 || gh <= 0 || gw <= 0) return VT_ERR_ARG;
-  const long long tokens = 1 + static_cast<long long>(gh) * gw;
+// pos: [prefix + g_in^2, D] (f32 | bf16), out: f32 [prefix + gh * gw, D]; distinct buffers.
+int pos_resample(const void* pos, int pos_dtype, float* out, int D, int g_in, int gh, int gw, int prefix,
+                 cudaStream_t stream) {
+  if (!pos || !out || D <= 0 || g_in <= 0 || gh <= 0 || gw <= 0 || prefix < 1 || prefix > 2) return VT_ERR_ARG;
+  const long long tokens = prefix + static_cast<long long>(gh) * gw;
   if (tokens > 0x7fffffffLL) return VT_ERR_UNSUPPORTED;
   const float scale_h = static_cast<float>(g_in) / static_cast<float>(gh);
   const float scale_w = static_cast<float>(g_in) / static_cast<float>(gw);
@@ -91,10 +94,10 @@ int pos_resample(const void* pos, int pos_dtype, float* out, int D, int g_in, in
   const dim3 grid(static_cast<unsigned>(tokens));
   if (pos_dtype == VT_F32)
     pos_resample_kernel<float><<<grid, threads, 0, stream>>>(static_cast<const float*>(pos), out, D, g_in, gh, gw,
-                                                               scale_h, scale_w);
+                                                               scale_h, scale_w, prefix);
   else if (pos_dtype == VT_BF16)
     pos_resample_kernel<__nv_bfloat16><<<grid, threads, 0, stream>>>(static_cast<const __nv_bfloat16*>(pos), out, D,
-                                                                       g_in, gh, gw, scale_h, scale_w);
+                                                                       g_in, gh, gw, scale_h, scale_w, prefix);
   else
     return VT_ERR_DTYPE;
   return static_cast<int>(cudaGetLastError());

@@ -1,5 +1,6 @@
 """ctypes binding of libvitb200.so (C ABI declared in include/vitb200.h, include/vitb200_resolution.h,
-include/vitb200_ragged.h, include/vitb200_mask.h, include/vitb200_attn.h and include/vitb200_preprocess.h).
+include/vitb200_ragged.h, include/vitb200_mask.h, include/vitb200_attn.h, include/vitb200_preprocess.h and
+include/vitb200_tokens.h).
 
 There is deliberately no fallback: if the shared library is missing or a tensor is not on a CUDA
 device the entry points raise.  The oracle under /oracle is test infrastructure and is never
@@ -102,6 +103,29 @@ PREPROCESS_SIGNATURES = {
     "vt_resize_u8_list": [_c_ptr, _c_i32, _c_i32, _c_ptr, _c_ptr, _c_i32, _c_i32, _c_ptr],
 }
 
+# name -> argtypes of the entry points with a prefix-token count (1 = CLS, 2 = CLS + distillation token); mirrors
+# include/vitb200_tokens.h one to one (tests/test_abi_tokens.py checks both directions).  Each is an entry point of
+# another table with an int32 prefix in front of the stream.
+TOKENS_SIGNATURES = {
+    "vt_patch_embed_gemm_hw_prefix": RESOLUTION_SIGNATURES["vt_patch_embed_gemm_hw"][:-1] + [_c_i32, _c_ptr],
+    "vt_patch_embed_masked_gather_prefix": MASK_SIGNATURES["vt_patch_embed_masked_gather"][:-1] + [_c_i32, _c_ptr],
+    "vt_patch_embed_ragged_gather_prefix": RAGGED_SIGNATURES["vt_patch_embed_ragged_gather"][:-1] + [_c_i32, _c_ptr],
+    "vt_pos_embed_resample_prefix": RESOLUTION_SIGNATURES["vt_pos_embed_resample"][:-1] + [_c_i32, _c_ptr],
+    "vt_embed_finalize_prefix": SIGNATURES["vt_embed_finalize"][:-1] + [_c_i32, _c_ptr],
+    "vt_embed_finalize_masked_prefix": MASK_SIGNATURES["vt_embed_finalize_masked"][:-1] + [_c_i32, _c_ptr],
+}
+
+
+def call_prefix(name: str, prefix: int, *args) -> None:
+    """One host path for every prefix-token count: ``name + "_prefix"`` (include/vitb200_tokens.h) with ``prefix`` right
+    before the stream (the last of ``args``).  At prefix 1 (CLS only) the call goes to ``name`` itself, the one-line
+    wrapper that passes 1: the same kernel and bits, and a ViT model's launches keep the names that launch counts and
+    per-kernel timings are keyed on."""
+    if prefix == 1:
+        call(name, *args)
+    else:
+        call(name + "_prefix", *args[:-1], prefix, args[-1])
+
 
 class RaggedImage(ctypes.Structure):
     """``vt_ragged_image`` of include/vitb200_ragged.h: one image of a ragged batch."""
@@ -136,7 +160,8 @@ def load() -> ctypes.CDLL:
     lib = ctypes.CDLL(path)
     for name, argtypes in (list(SIGNATURES.items()) + list(RESOLUTION_SIGNATURES.items())
                            + list(RAGGED_SIGNATURES.items()) + list(MASK_SIGNATURES.items())
-                           + list(ATTN_SIGNATURES.items()) + list(PREPROCESS_SIGNATURES.items())):
+                           + list(ATTN_SIGNATURES.items()) + list(PREPROCESS_SIGNATURES.items())
+                           + list(TOKENS_SIGNATURES.items())):
         fn = getattr(lib, name)
         fn.argtypes = argtypes
         fn.restype = ctypes.c_int

@@ -205,18 +205,29 @@ def linear_fp8(x8: torch.Tensor, w8: torch.Tensor, colscale: torch.Tensor, bias3
     return out
 
 
-def _posb16(pos32: torch.Tensor, cls_token: torch.Tensor, bias32: torch.Tensor) -> torch.Tensor:
+def _posb16(pos32: torch.Tensor, prefix32: torch.Tensor, bias32: torch.Tensor) -> torch.Tensor:
     """bf16 [N, D] position table of the two-launch patch embedding (``vt_patch_embed_gemm``): the GEMM adds the
-    conv bias to EVERY row, so row 0 (CLS: a zero patch row) carries cls + pos[0] - bias."""
+    conv bias to EVERY row, so row t < prefix (CLS, distillation token: zero patch rows) carries
+    token_t + pos[t] - bias, with ``prefix32`` the fp32 [prefix, D] token rows (``prefix_rows32``)."""
     t = pos32.clone()
-    t[0] += cls_token.detach().float().reshape(-1) - bias32
+    t[:prefix32.shape[0]] += prefix32 - bias32
     return t.to(torch.bfloat16).contiguous()
+
+
+def prefix_tokens(emb) -> list:
+    """The learned tokens in front of the patches, (1, 1, D) each: [cls_token], or [cls_token, distillation_token]."""
+    return [emb.cls_token] if emb.distillation_token is None else [emb.cls_token, emb.distillation_token]
+
+
+def prefix_rows32(emb) -> torch.Tensor:
+    """fp32 [prefix, D] rows of the tokens in front of the patches, [cls; dist]."""
+    return torch.cat([t.detach().float().reshape(1, -1) for t in prefix_tokens(emb)])
 
 
 def _posm16(pos32: torch.Tensor, mask_token: Optional[torch.Tensor], bias32: torch.Tensor) -> Optional[torch.Tensor]:
     """bf16 [N, D] table of masked patches (``vt_patch_embed_masked_gather``): a masked patch's row is zero, so the GEMM
-    gives bias + this row, which must come out as mask_token + pos.  One rounding from fp32; row 0 is not read.  None
-    for a model without a mask token."""
+    gives bias + this row, which must come out as mask_token + pos.  One rounding from fp32; the prefix rows are not
+    read.  None for a model without a mask token."""
     if mask_token is None:
         return None
     return (pos32 + mask_token.detach().float().reshape(-1) - bias32).to(torch.bfloat16).contiguous()
@@ -238,8 +249,9 @@ def pixel_dims(x: torch.Tensor, fmt: Optional[tuple]) -> tuple:
 
 def pack_embeddings(emb, fmt: Optional[tuple] = None) -> SimpleNamespace:
     """Patch-projection operands for pixels of format ``fmt``: the bf16 | fp32 weight ``w`` [D, ldw] (K = C*P*P columns,
-    zero padding to a multiple of 8), the fp32 bias ``bias32`` [D] and the bf16 position tables ``posb16`` /
-    ``posm16`` of the trained grid.  Float pixels: the conv weight in the reference's (c, i, j) order and the conv bias.
+    zero padding to a multiple of 8), the fp32 bias ``bias32`` [D], the fp32 prefix-token rows ``prefix32`` [prefix, D]
+    and the bf16 position tables ``posb16`` / ``posm16`` of the trained grid.  Float pixels: the conv weight in the
+    reference's (c, i, j) order and the conv bias.
 
     Raw uint8 NHWC pixels (``fmt`` = ``pixel_format``): the image processor's ``(x * rescale - mean_c) / std_c`` (HF
     ViTImageProcessor: 1/255, 0.5, 0.5) is folded into the operands, so the kernel multiplies bytes:
@@ -264,8 +276,28 @@ def pack_embeddings(emb, fmt: Optional[tuple] = None) -> SimpleNamespace:
     w2d = torch.zeros((D, kpad), device=w.device, dtype=w.dtype)
     w2d[:, :K] = w.reshape(D, K)
     pos = emb.position_embeddings.detach().float()[0]          # [N, D]
-    return SimpleNamespace(w=w2d, ldw=kpad, K=K, bias32=bias32, posb16=_posb16(pos, emb.cls_token, bias32),
-                           posm16=_posm16(pos, emb.mask_token, bias32))
+    prefix32 = prefix_rows32(emb)
+    return SimpleNamespace(w=w2d, ldw=kpad, K=K, bias32=bias32, prefix32=prefix32,
+                           posb16=_posb16(pos, prefix32, bias32), posm16=_posm16(pos, emb.mask_token, bias32))
+
+
+def pack_teacher_head(cls_head, dist_head, pieces: int) -> SimpleNamespace:
+    """DeiT's two classifiers (``LinearWithBias``, weight (D, L)) as ONE GEMM over each image's rows 0 and 1 (2D
+    contiguous elements): the K-major [3L, 2D] weight [[Wc, 0], [0, Wd], [Wc / 2, Wd / 2]] packed for ``bg.dense_rows``
+    with ``pieces`` (``w``), and the fp32 bias [bc, bd, (bc + bd) / 2] (``bias32``).  The outputs are the cls logits,
+    the distillation logits and their mean; halving is exact."""
+    wc = cls_head.weight.detach().t()                          # [L, D]
+    wd = dist_head.weight.detach().t()
+    L, D = wc.shape
+    w = torch.zeros((3 * L, 2 * D), device=wc.device, dtype=wc.dtype)
+    w[:L, :D] = wc
+    w[L:2 * L, D:] = wd
+    w[2 * L:, :D] = wc / 2
+    w[2 * L:, D:] = wd / 2
+    bc = cls_head.bias.detach().float()
+    bd = dist_head.bias.detach().float()
+    return SimpleNamespace(w=bg.pack_weight_nk(w, pieces), pieces=pieces, labels=L,
+                           bias32=torch.cat([bc, bd, (bc + bd) / 2]).contiguous())
 
 
 def embed_pack(emb, fmt: Optional[tuple] = None) -> SimpleNamespace:
@@ -379,16 +411,18 @@ def _embed_batch_step(n_patches: int) -> int:
 
 
 def _embed_call(stats, b0, n_tok, dim, pk, pos, pixels_ptr, pix_code, out_ptr, nb, C, H, W, P, stream, device,
-                interpolate):
+                interpolate, prefix):
     """Patch embedding of images b0 .. b0 + nb: gather + 2-CTA GEMM in token mode with the bf16 position table ``pos``;
     row statistics of those images go into ``stats`` when given.  ``vt_patch_embed_gemm`` for a square input at the
-    model's size, ``vt_patch_embed_gemm_hw`` for any (H, W) with ``interpolate``."""
+    model's size with one prefix token, ``vt_patch_embed_gemm_hw`` (``_prefix``) for any (H, W) with ``interpolate`` or
+    ``prefix`` tokens in front of the patches."""
     s_ptr = None if stats is None else stats.data_ptr() + b0 * n_tok * (dim // STATS_COLS) * 2 * 4
     tok_pad = (n_tok + 31) // 32 * 32
     work = torch.empty((nb, tok_pad, pk.ldw), device=device, dtype=torch.bfloat16)
-    if interpolate:
-        _lib.call("vt_patch_embed_gemm_hw", pixels_ptr, pix_code, pk.w.data_ptr(), pk.ldw, pk.bias32.data_ptr(),
-                  pos.data_ptr(), out_ptr, s_ptr, work.data_ptr(), nb, C, H, W, P, dim, stream)
+    if interpolate or prefix != 1:
+        _lib.call_prefix("vt_patch_embed_gemm_hw", prefix, pixels_ptr, pix_code, pk.w.data_ptr(), pk.ldw,
+                         pk.bias32.data_ptr(), pos.data_ptr(), out_ptr, s_ptr, work.data_ptr(), nb, C, H, W, P, dim,
+                         stream)
     else:
         _lib.call("vt_patch_embed_gemm", pixels_ptr, pix_code, pk.w.data_ptr(), pk.ldw, pk.bias32.data_ptr(),
                   pos.data_ptr(), out_ptr, s_ptr, work.data_ptr(), nb, C, H, P, dim, stream)
@@ -396,10 +430,11 @@ def _embed_call(stats, b0, n_tok, dim, pk, pos, pixels_ptr, pix_code, out_ptr, n
 
 def patch_embed(emb, x: torch.Tensor, fmt: Optional[tuple] = None, stats: Optional[torch.Tensor] = None,
                 interpolate: bool = False, mask: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """Pixels of format ``fmt`` -> token embeddings (B, n+1, D) including CLS and position embeddings.  ``fmt`` None:
+    """Pixels of format ``fmt`` -> token embeddings (B, prefix + n, D) including CLS (and distillation token) and
+    position embeddings, prefix = ``emb.num_prefix_tokens``.  ``fmt`` None:
     float pixels (B, C, S, S); ``pixel_format``: raw uint8 NHWC pixels (B, S, S, C), rescale + normalise + patch
     projection in the same launches (bf16 models on the tensor-core path only).
-    ``stats``: optional (B * (n+1), D/128, 2) fp32 buffer for the row statistics the LayerNorm folded
+    ``stats``: optional (B * (prefix + n), D/128, 2) fp32 buffer for the row statistics the LayerNorm folded
     into the first QKV GEMM consumes (bf16 tensor-core path only).  ``interpolate``: pixels at any
     H, W >= patch size, n = (H // P) * (W // P), position table resampled to that grid (``pos_grid``).
     ``mask``: checked bool_masked_pos (B, n): masked patches take the mask token (``embed_masked`` on the bf16
@@ -432,7 +467,8 @@ def patch_embed(emb, x: torch.Tensor, fmt: Optional[tuple] = None, stats: Option
         posm = None if mask is None else grid_table(emb, grid, fmt, True)
     else:
         pos = emb.position_embeddings if grid is None or grid == native_grid(emb) else pos_grid(emb, *grid).pos
-    n_tok = n + 1
+    prefix = emb.num_prefix_tokens
+    n_tok = prefix + n
     x = x.contiguous()
     out = torch.empty((B, n_tok, D), device=x.device, dtype=w.dtype)
     if B == 0:
@@ -448,12 +484,12 @@ def patch_embed(emb, x: torch.Tensor, fmt: Optional[tuple] = None, stats: Option
         for b0 in range(0, B, step):
             nb = min(step, B - b0)
             _embed_call(stats, b0, n_tok, D, pk, pos, x[b0:].data_ptr(), code, out[b0:].data_ptr(), nb, C, H, W, P,
-                        stream, x.device, interpolate)
+                        stream, x.device, interpolate, prefix)
         return out
     assert stats is None, "Row statistics come out of the bf16 tensor-core patch embedding only"
 
     # fp32 / odd-width path: im2col rows, tensor-core GEMM (fp32 operands split into bf16 pieces) straight
-    # into rows 1..n of every image, then CLS / position embeddings
+    # into rows prefix .. prefix + n - 1 of every image, then the prefix tokens and position embeddings
     from .kernels.patching import patching
     if x.dtype != w.dtype:
         x = x.to(w.dtype)
@@ -468,7 +504,7 @@ def patch_embed(emb, x: torch.Tensor, fmt: Optional[tuple] = None, stats: Option
         for b0 in range(0, B, 32768):
             nb = min(32768, B - b0)
             _lib.call("vt_gemm_strided", patches[b0:].data_ptr(), pk.w.data_ptr(),
-                      out[b0:].data_ptr() + D * es, bias.data_ptr(), n, D, K, nb, 1,
+                      out[b0:].data_ptr() + prefix * D * es, bias.data_ptr(), n, D, K, nb, 1,
                       _lib.i64x4(n * K, 0, K, 1), _lib.i64x4(0, 0, 1, pk.ldw), _lib.i64x4(n_tok * D, 0, D, 1),
                       1.0, 0, code, stream)
     else:
@@ -476,23 +512,25 @@ def patch_embed(emb, x: torch.Tensor, fmt: Optional[tuple] = None, stats: Option
         wp = split_weight(pk.w, pieces)                    # [D, pieces * ldw]: pk.w rows are already padded to 8
         a = bg.pack(patches, patches.data_ptr(), n, K, B, 1, (n * K, 0, K, 1), pieces, pattern=0)
         kk = a.shape[2]
-        bg.bgemm(a.data_ptr(), wp.data_ptr(), out, out.data_ptr() + D * es, n, D, kk, B, 1, (n * kk, 0, kk),
+        bg.bgemm(a.data_ptr(), wp.data_ptr(), out, out.data_ptr() + prefix * D * es, n, D, kk, B, 1, (n * kk, 0, kk),
                  (0, 0, kk), (n_tok * D, 0, D), bias32=pk.bias32)
     finalize_embeddings(emb, out, pos, mask)
     return out
 
 
 def finalize_embeddings(emb, out: torch.Tensor, pos: torch.Tensor, mask: Optional[torch.Tensor]) -> None:
-    """CLS row and position add of embeddings (B, N, D) whose rows 1.. hold the patch projections, in place:
-    ``vt_embed_finalize``, or ``vt_embed_finalize_masked`` (masked patches take the mask token) with a mask."""
+    """Prefix-token rows and position add of embeddings (B, N, D) whose rows prefix.. hold the patch projections, in
+    place: ``vt_embed_finalize``, or ``vt_embed_finalize_masked`` (masked patches take the mask token) with a mask."""
     B, n_tok, D = out.shape
     code, stream = _lib.dtype_code(out), _lib.stream_ptr(out)
+    rows = emb.prefix_rows()
     if mask is None:
-        _lib.call("vt_embed_finalize", out.data_ptr(), pos.data_ptr(), emb.cls_token.data_ptr(), B, n_tok, D, code,
-                  stream)
+        _lib.call_prefix("vt_embed_finalize", emb.num_prefix_tokens, out.data_ptr(), pos.data_ptr(), rows.data_ptr(), B,
+                         n_tok, D, code, stream)
     else:
-        _lib.call("vt_embed_finalize_masked", out.data_ptr(), pos.data_ptr(), emb.cls_token.data_ptr(),
-                  emb.mask_token.data_ptr(), mask.contiguous().data_ptr(), B, n_tok, D, code, stream)
+        _lib.call_prefix("vt_embed_finalize_masked", emb.num_prefix_tokens, out.data_ptr(), pos.data_ptr(),
+                         rows.data_ptr(), emb.mask_token.data_ptr(), mask.contiguous().data_ptr(), B, n_tok, D, code,
+                         stream)
 
 
 # ------------------------------------------------------------------------------------------------ bool_masked_pos
@@ -526,9 +564,9 @@ def embed_masked(emb, x: torch.Tensor, pix_code: int, H: int, W: int, mask: torc
         rows = nb * n_tok
         patches = torch.empty((rows, pk.ldw), device=out.device, dtype=torch.bfloat16)
         table = torch.empty((rows, D), device=out.device, dtype=torch.bfloat16)
-        _lib.call("vt_patch_embed_masked_gather", x[b0:].data_ptr(), pix_code, mask[b0:].data_ptr(), pos.data_ptr(),
-                  posm.data_ptr(), patches.data_ptr(), pk.ldw, table.data_ptr(), nb, emb.channels, H, W,
-                  emb.patch_size, D, stream)
+        _lib.call_prefix("vt_patch_embed_masked_gather", emb.num_prefix_tokens, x[b0:].data_ptr(), pix_code,
+                         mask[b0:].data_ptr(), pos.data_ptr(), posm.data_ptr(), patches.data_ptr(), pk.ldw,
+                         table.data_ptr(), nb, emb.channels, H, W, emb.patch_size, D, stream)
         s_ptr = None if stats is None else stats[b0 * n_tok:].data_ptr()
         _lib.call("vt_gemm_bf16_ln", patches.data_ptr(), pk.ldw, pk.w.data_ptr(), pk.ldw, out[b0:].data_ptr(), D,
                   pk.bias32.data_ptr(), table.data_ptr(), D, rows, D, pk.ldw, 0, None, None, 0, 0.0, s_ptr, stream)
@@ -580,44 +618,45 @@ def check_any_size(emb, channels: int, height: int, width: int) -> None:
         f"Image size {(channels, height, width)} needs {emb.channels} channels and sides of at least the patch size {P}"
 
 
-def resample_pos_table(pos: torch.Tensor, g_in: int, gh: int, gw: int) -> torch.Tensor:
-    """[1 + g_in^2, D] position table (fp32 | bf16, CUDA) -> fp32 [1 + gh * gw, D]: row 0 copied, the grid resampled
-    bicubically like HF ``ViTEmbeddings.interpolate_pos_encoding`` (one ``vt_pos_embed_resample`` launch)."""
-    assert pos.is_cuda and pos.dim() == 2 and pos.shape[0] == 1 + g_in * g_in, \
-        f"Expected a CUDA [1 + {g_in}^2, D] position table, provided: {tuple(pos.shape)} on {pos.device}"
+def resample_pos_table(pos: torch.Tensor, g_in: int, gh: int, gw: int, prefix: int = 1) -> torch.Tensor:
+    """[prefix + g_in^2, D] position table (fp32 | bf16, CUDA) -> fp32 [prefix + gh * gw, D]: the ``prefix`` rows of
+    the tokens in front of the patches (CLS, distillation token) copied, the grid resampled bicubically like HF
+    ``ViTEmbeddings`` / ``DeiTEmbeddings.interpolate_pos_encoding`` (one ``vt_pos_embed_resample`` launch)."""
+    assert pos.is_cuda and pos.dim() == 2 and pos.shape[0] == prefix + g_in * g_in, \
+        f"Expected a CUDA [{prefix} + {g_in}^2, D] position table, provided: {tuple(pos.shape)} on {pos.device}"
     pos = pos.contiguous()
-    out = torch.empty((1 + gh * gw, pos.shape[1]), device=pos.device, dtype=torch.float32)
-    _lib.call("vt_pos_embed_resample", pos.data_ptr(), _lib.dtype_code(pos), out.data_ptr(), pos.shape[1], g_in, gh, gw,
-              _lib.stream_ptr(pos))
+    out = torch.empty((prefix + gh * gw, pos.shape[1]), device=pos.device, dtype=torch.float32)
+    _lib.call_prefix("vt_pos_embed_resample", prefix, pos.data_ptr(), _lib.dtype_code(pos), out.data_ptr(),
+                     pos.shape[1], g_in, gh, gw, _lib.stream_ptr(pos))
     return out
 
 
 class PosGrid:
     """Position tables of one non-native patch grid, all derived from one resample of the model's table:
-    ``pos32`` fp32 [1 + n, D]; ``pos`` (1, 1 + n, D) in the model's dtype (``Embeddings.interpolate_pos_encoding``,
-    and ``vt_embed_finalize`` of the fp32 / unfused paths); ``table`` the bf16 tables of the tensor-core patch
-    embedding for each pixel format.  A table, once built, is never replaced while this object lives: CUDA graphs keep
+    ``pos32`` fp32 [prefix + n, D]; ``pos`` (1, prefix + n, D) in the model's dtype (``Embeddings.interpolate_pos_encoding``
+    and ``vt_embed_finalize`` of the fp32 / unfused paths); ``table`` the bf16 tables of the tensor-core patch embedding
+    for each pixel format.  A table, once built, is never replaced while this object lives: CUDA graphs keep
     reading it (see ``pos_grid``)."""
 
     def __init__(self, emb, gh: int, gw: int):
         source = emb.position_embeddings.detach()
-        self.pos32 = resample_pos_table(source[0], native_grid(emb)[0], gh, gw)
+        self.pos32 = resample_pos_table(source[0], native_grid(emb)[0], gh, gw, emb.num_prefix_tokens)
         self.pos = self.pos32.to(source.dtype)[None]
         self._tables = {}
 
     def table(self, emb, fmt: Optional[tuple], masked: bool) -> torch.Tensor:
-        """bf16 table for pixels of format ``fmt`` (the pack ``embed_pack(emb, fmt)``): of every token (row 0 = cls +
-        pos[0] - the pack's bias), or with ``masked`` of masked patches (mask_token + pos - the pack's bias,
+        """bf16 table for pixels of format ``fmt`` (the pack ``embed_pack(emb, fmt)``): of every token (row t < prefix =
+        token_t + pos[t] - the pack's bias), or with ``masked`` of masked patches (mask_token + pos - the pack's bias,
         ``embed_masked``)."""
         table = self._tables.get((fmt, masked))
         if table is None:
             _assert_not_capturing()
-            bias32 = embed_pack(emb, fmt).bias32
+            pk = embed_pack(emb, fmt)
             with torch.no_grad():
                 if masked:
-                    table = _posm16(self.pos32, emb.mask_token, bias32)
+                    table = _posm16(self.pos32, emb.mask_token, pk.bias32)
                 else:
-                    table = _posb16(self.pos32, emb.cls_token, bias32)
+                    table = _posb16(self.pos32, pk.prefix32, pk.bias32)
             self._tables[(fmt, masked)] = table
         return table
 
@@ -658,7 +697,7 @@ def pos_grid(emb, gh: int, gw: int, keep: int = POS_GRIDS_KEPT) -> PosGrid:
 
 def grid_table(emb, grid: Optional[tuple], fmt: Optional[tuple], masked: bool,
                keep: int = POS_GRIDS_KEPT) -> torch.Tensor:
-    """bf16 [1 + gh * gw, D] position table of the tensor-core patch embedding for patch grid ``grid`` (None: the
+    """bf16 [prefix + gh * gw, D] position table of the tensor-core patch embedding for patch grid ``grid`` (None: the
     model's own) and pixels of format ``fmt``; with ``masked`` the table of masked patches.  The pack's ``posb16`` /
     ``posm16`` at the trained grid, else ``PosGrid.table`` of the resampled grid; ``keep``: grids ``pos_grid`` keeps."""
     if grid is None or grid == native_grid(emb):
@@ -675,11 +714,13 @@ class RaggedLayout:
     """Where the images of a ragged batch go in the packed (M, D) activation.  Images are grouped by token count, so
     that images with the same count occupy one contiguous row range (one attention call each); inside a group they keep
     the caller's order.  ``order``: caller indices in packed order; ``row0[i]`` / ``tokens[i]``: first row (CLS) and
-    token count of caller image i; ``groups``: (first row, images, tokens) per distinct token count; ``rows`` = M."""
+    token count of caller image i, ``prefix`` tokens in front of its patches; ``groups``: (first row, images, tokens) per
+    distinct token count; ``rows`` = M."""
 
-    def __init__(self, grids):
+    def __init__(self, grids, prefix: int = 1):
         self.grids = [tuple(g) for g in grids]
-        self.tokens = [1 + gh * gw for gh, gw in self.grids]
+        self.prefix = prefix
+        self.tokens = [prefix + gh * gw for gh, gw in self.grids]
         self.order = sorted(range(len(self.grids)), key=lambda i: (self.tokens[i], i))
         self.row0 = [0] * len(self.grids)
         self.groups = []
@@ -783,8 +824,8 @@ def patch_embed_ragged(emb, images, layout: RaggedLayout, stats: Optional[torch.
         desc_dev = _to_device_async(bytes(desc), device)
         patches = torch.empty((rows, pk.ldw), device=device, dtype=torch.bfloat16)
         table = torch.empty((rows, D), device=device, dtype=torch.bfloat16)
-        _lib.call("vt_patch_embed_ragged_gather", desc_dev.data_ptr(), len(chunk), code, emb.channels, emb.patch_size,
-                  patches.data_ptr(), pk.ldw, table.data_ptr(), D, rows, stream)
+        _lib.call_prefix("vt_patch_embed_ragged_gather", layout.prefix, desc_dev.data_ptr(), len(chunk), code,
+                         emb.channels, emb.patch_size, patches.data_ptr(), pk.ldw, table.data_ptr(), D, rows, stream)
         s_ptr = None if stats is None else stats[base:].data_ptr()
         _lib.call("vt_gemm_bf16_ln", patches.data_ptr(), pk.ldw, pk.w.data_ptr(), pk.ldw, out[0, base:].data_ptr(), D,
                   pk.bias32.data_ptr(), table.data_ptr(), D, rows, D, pk.ldw, 0, None, None, 0, 0.0, s_ptr, stream)

@@ -132,7 +132,8 @@ class DataParallelVIT(torch.nn.Module):
                  output: str = "pooled", interpolate_pos_encoding: bool = False):
         """``output``: "pooled" gathers the CLS embeddings (B, D); "pooler" the HF pooler output
         tanh(dense(CLS)) (B, D) of a model built with ``add_pooling_layer=True``; "logits" the class
-        logits (B, num_labels) of a model built with a classifier head (``VIT(num_labels=...)``).
+        logits (B, num_labels) of a model built with a classifier head (``VIT(num_labels=...)``, or the mean of the
+        two DeiT heads of ``VIT(..., distillation_head=True)``).
         ``peer_gather``: None = use the fused pool + peer-store kernel whenever it applies (CUDA,
         NCCL group, equal shards, symmetric memory available; VT_PEER_GATHER=0 disables), True =
         require it, False = always all-gather through torch.distributed.  Which one runs is decided
@@ -241,7 +242,8 @@ class DataParallelVIT(torch.nn.Module):
     # ------------------------------------------------------------------ collective plan (cold path)
     def _out_dim(self) -> int:
         if self.output == "logits":
-            return self.model.classifier.weight.shape[1]
+            head = self.model.classifier if self.model.classifier is not None else self.model.cls_classifier
+            return head.weight.shape[1]
         return int(getattr(self.model, "hidden_dim", 0))
 
     def _local_want(self, x_local: torch.Tensor, global_batch: int) -> bool:

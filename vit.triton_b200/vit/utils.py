@@ -43,6 +43,11 @@ def _dense_mapping(num_layers: int) -> dict:
         'embeddings.mask_token': 'embeddings.mask_token',   # ViTModel(use_mask_token=True), VIT(use_mask_token=True)
         'decoder.0.weight': 'decoder.0.weight',             # ViTForMaskedImageModeling, VIT(add_decoder=True)
         'decoder.0.bias': 'decoder.0.bias',
+        'embeddings.distillation_token': 'embeddings.distillation_token',   # DeiTModel, VIT(distillation_token=True)
+        'cls_classifier.weight': 'cls_classifier.weight',   # DeiTForImageClassificationWithTeacher,
+        'cls_classifier.bias': 'cls_classifier.bias',       # VIT(distillation_head=True)
+        'distillation_classifier.weight': 'distillation_classifier.weight',
+        'distillation_classifier.bias': 'distillation_classifier.bias',
     }
     for i in range(num_layers):
         pre = f'encoder.layer.{i}.'
@@ -59,13 +64,21 @@ _HF_QKV = re.compile(r"^encoder\.layer\.(\d+)\.attention\.attention\.(query|key|
 
 def transfer_pretrained_weights(pretrained_model: torch.nn.Module, custom_model: torch.nn.Module,
                                 verbose: bool = True) -> torch.nn.Module:
-    """Copy every weight of a HuggingFace ``ViTModel`` into ``custom_model`` (a ``vit.vit.VIT``).
+    """Copy every weight of a HuggingFace ``ViTModel`` or ``DeiTModel`` into ``custom_model`` (a ``vit.vit.VIT``).
 
     Same call and result as the reference (utils.py:45-113); the layer count comes from the models.
-    Keys of the source may carry a ``vit.`` prefix (``ViTForImageClassification``, ``ViTForMaskedImageModeling``).
+    Keys of the source may carry a ``vit.`` prefix (``ViTForImageClassification``, ``ViTForMaskedImageModeling``) or a
+    ``deit.`` prefix (``DeiTForImageClassification``, ``DeiTForImageClassificationWithTeacher``).  A DeiT checkpoint
+    needs a model built with ``distillation_token=True``, and only a DeiT checkpoint fits such a model: anything else
+    raises an AssertionError before a tensor is copied.
     """
-    source = {(k[4:] if k.startswith('vit.') else k): v for k, v in pretrained_model.state_dict().items()}
+    source = {re.sub(r'^(vit|deit)\.', '', k): v for k, v in pretrained_model.state_dict().items()}
     dest = custom_model.state_dict()
+    has_token = 'embeddings.distillation_token' in source
+    wants_token = 'embeddings.distillation_token' in dest
+    assert has_token == wants_token, (
+        "The checkpoint has a distillation token (DeiT): build the model with distillation_token=True" if has_token else
+        "The model was built with distillation_token=True but the checkpoint has no distillation token (not DeiT)")
 
     layer_ids = [int(m.group(1)) for m in map(_HF_QKV.match, source) if m]
     num_layers = (max(layer_ids) + 1) if layer_ids else 0

@@ -319,20 +319,27 @@ class Encoder(nn.Module):
 
 
 class Embeddings(packing.PackedMixin, nn.Module):
-    """Patch projection + CLS token + position embeddings (reference vit.py:173-200)."""
+    """Patch projection + CLS token + position embeddings (reference vit.py:173-200).  With ``distillation_token``
+    (HF ``DeiTEmbeddings``) a second learned token follows CLS: the sequence is [CLS, DIST, patches].
+    ``num_prefix_tokens`` (1, or 2 with the distillation token) is the number of tokens in front of the patches; every
+    token count, row offset and position-table shape of the patch embedding derives from it."""
 
-    def __init__(self, patch_size, num_patches, patch_dim, hidden_dim, channels: int = 3, use_mask_token: bool = False):
+    def __init__(self, patch_size, num_patches, patch_dim, hidden_dim, channels: int = 3, use_mask_token: bool = False,
+                 distillation_token: bool = False):
         super().__init__()
         self.patch_size = patch_size
         self.num_patches = num_patches
         self.patch_dim = patch_dim
         self.hidden_dim = hidden_dim
         self.channels = channels
+        self.num_prefix_tokens = 2 if distillation_token else 1
 
         self.cls_token = nn.Parameter(torch.zeros((1, 1, hidden_dim)))
+        # HF DeiTEmbeddings: the token of the distillation (teacher) head, row 1 of every image
+        self.distillation_token = nn.Parameter(torch.zeros(1, 1, hidden_dim)) if distillation_token else None
         # HF ViTEmbeddings(use_mask_token=True): the embedding of a patch masked by bool_masked_pos
         self.mask_token = nn.Parameter(torch.zeros(1, 1, hidden_dim)) if use_mask_token else None
-        self.position_embeddings = nn.Parameter(torch.zeros(1, num_patches + 1, hidden_dim))
+        self.position_embeddings = nn.Parameter(torch.zeros(1, num_patches + self.num_prefix_tokens, hidden_dim))
         self.projection = Conv2DTriton(
             in_channels=channels,
             out_channels=hidden_dim,
@@ -343,10 +350,10 @@ class Embeddings(packing.PackedMixin, nn.Module):
                 bool_masked_pos: Optional[torch.Tensor] = None) -> torch.Tensor:
         """``stats_out`` (optional, fused bf16 path only): (B * N, D/128, 2) fp32 buffer that receives the
         row statistics of the output for the LayerNorm folded into block 0's QKV GEMM.
-        ``interpolate_pos_encoding``: (B, C, H, W) at any H, W >= patch size, N = 1 + (H // P) * (W // P), the
-        position table resampled to that grid (``interpolate_pos_encoding(H, W)``), like HF ``ViTEmbeddings``.
-        ``bool_masked_pos``: bool (B, N - 1), needs ``use_mask_token=True``: a masked patch's embedding is the mask token
-        (plus its position embedding), like HF ``ViTEmbeddings``."""
+        ``interpolate_pos_encoding``: (B, C, H, W) at any H, W >= patch size, N = num_prefix_tokens + (H // P) * (W // P),
+        the position table resampled to that grid (``interpolate_pos_encoding(H, W)``), like HF ``ViTEmbeddings``.
+        ``bool_masked_pos``: bool (B, N - num_prefix_tokens), needs ``use_mask_token=True``: a masked patch's embedding is
+        the mask token (plus its position embedding), like HF ``ViTEmbeddings``."""
         return self._embed(x, None, stats_out, interpolate_pos_encoding, bool_masked_pos)
 
     def forward_uint8(self, x, image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
@@ -377,7 +384,7 @@ class Embeddings(packing.PackedMixin, nn.Module):
             tokens = self.projection(x.to(self.projection.weight.dtype)).flatten(2).transpose(1, 2)
             out = torch.empty((x.shape[0], pos.shape[1], self.hidden_dim), device=x.device,
                               dtype=tokens.dtype)
-            out[:, 1:, :] = tokens
+            out[:, self.num_prefix_tokens:, :] = tokens
             packing.finalize_embeddings(self, out, pos, bool_masked_pos)
             return out
         return packing.patch_embed(self, x, fmt, stats_out, interpolate=interpolate_pos_encoding, mask=bool_masked_pos)
@@ -388,9 +395,10 @@ class Embeddings(packing.PackedMixin, nn.Module):
         packing.check_mask(self, bool_masked_pos, x, grid[0] * grid[1] if interpolate_pos_encoding else self.num_patches)
 
     def interpolate_pos_encoding(self, height: int, width: int) -> torch.Tensor:
-        """(1, 1 + gh * gw, D) position table for a (height, width) input, gh = height // P, gw = width // P:
-        HF ``ViTEmbeddings.interpolate_pos_encoding``.  The stored parameter itself at the trained grid; otherwise
-        its patch grid resampled bicubically (align_corners=False) by one ``vt_pos_embed_resample`` launch, cached
+        """(1, num_prefix_tokens + gh * gw, D) position table for a (height, width) input, gh = height // P,
+        gw = width // P: HF ``ViTEmbeddings`` / ``DeiTEmbeddings.interpolate_pos_encoding``.  The stored parameter itself
+        at the trained grid; otherwise its patch grid resampled bicubically (align_corners=False) by one
+        ``vt_pos_embed_resample`` launch, cached
         per grid for the last few grids (``packing.pos_grid``) with the tables the patch embedding derives from it.
         A new grid's tables are built outside CUDA-graph capture."""
         grid = packing.patch_grid(self, height, width)
@@ -404,8 +412,22 @@ class Embeddings(packing.PackedMixin, nn.Module):
         self.__dict__.pop("_pos_grids", None)
 
     def _packed_sources(self):
-        sources = [self.cls_token, self.position_embeddings, self.projection.weight, self.projection.bias]
+        sources = packing.prefix_tokens(self) + [self.position_embeddings, self.projection.weight, self.projection.bias]
         return sources if self.mask_token is None else sources + [self.mask_token]
+
+    def prefix_rows(self) -> torch.Tensor:
+        """[num_prefix_tokens, D] rows of the tokens in front of the patches in the model's dtype, [cls; dist]: the
+        ``cls_token`` parameter itself, or a copy cached with the packs (``vt_embed_finalize`` of the fp32 / unfused
+        paths)."""
+        if self.distillation_token is None:
+            return self.cls_token
+        return self.packed("prefix")
+
+    def _packed_sources_prefix(self):
+        return packing.prefix_tokens(self)
+
+    def _build_packed_prefix(self):
+        return torch.cat(packing.prefix_tokens(self), dim=1)[0].detach().contiguous()
 
     def _build_packed(self):
         return packing.pack_embeddings(self)
@@ -434,6 +456,22 @@ def _head_on_cls(hidden: torch.Tensor, dense: "LinearWithBias", act: int) -> tor
     bg.dense_rows(hidden, hidden.data_ptr(), B, D, hidden.stride(0), wp, pieces, n_out, bias32, act, out,
                   out.data_ptr(), n_out)
     return out
+
+
+def _distilled_head(hidden: torch.Tensor, pk: SimpleNamespace) -> "DistilledLogits":
+    """DeiT's teacher head over rows 0 (CLS) and 1 (distillation token) of every image of ``hidden`` (B, N, D): ONE
+    tensor-core launch (``vt_bgemm``, K = 2D) that reads each image's two rows in place as one 2D-element row at row
+    stride N * D, with the packed [3L, 2D] weight of ``packing.pack_teacher_head``; the three results are views into
+    one (B, 3L) output.  fp32 models pack the rows into split bf16 pieces first."""
+    from .kernels import bgemm as bg
+    assert hidden.is_cuda and hidden.dim() == 3 and hidden.stride(2) == 1 and hidden.stride(1) == hidden.shape[2]
+    B, _, D = hidden.shape
+    L = pk.labels
+    out = torch.empty((B, 3 * L), device=hidden.device, dtype=hidden.dtype)
+    if B:
+        bg.dense_rows(hidden, hidden.data_ptr(), B, 2 * D, hidden.stride(0), pk.w, pk.pieces, 3 * L, pk.bias32,
+                      bg.ACT_NONE, out, out.data_ptr(), 3 * L)
+    return DistilledLogits(out[:, 2 * L:], out[:, :L], out[:, L:2 * L])
 
 
 class Pooler(nn.Module):
@@ -478,6 +516,14 @@ class VITOutput(NamedTuple):
     attentions: Optional[Tuple[torch.Tensor, ...]] = None
 
 
+class DistilledLogits(NamedTuple):
+    """What ``VIT.distillation_logits`` returns, like HF ``DeiTForImageClassificationWithTeacherOutput``: (B, num_labels)
+    each; ``logits`` = (cls_logits + distillation_logits) / 2."""
+    logits: torch.Tensor
+    cls_logits: torch.Tensor
+    distillation_logits: torch.Tensor
+
+
 def _refuse_outputs(what: str, output_hidden_states: bool, output_attentions: bool) -> None:
     assert not (output_hidden_states or output_attentions), \
         f"output_hidden_states / output_attentions are not supported by {what}: call the model itself with them"
@@ -485,7 +531,12 @@ def _refuse_outputs(what: str, output_hidden_states: bool, output_attentions: bo
 
 class VIT(nn.Module):
     """ViT encoder returning the final-LayerNorm hidden states (B, N, D) — no pooler, like the
-    reference (vit.py:203-247) and HF ``ViTModel(add_pooling_layer=False).last_hidden_state``."""
+    reference (vit.py:203-247) and HF ``ViTModel(add_pooling_layer=False).last_hidden_state``.
+
+    ``distillation_token=True`` builds a DeiT encoder (HF ``DeiTModel``): a learned distillation token follows CLS, so
+    N = 2 + gh * gw and the position table has num_patches + 2 rows.  ``distillation_head=True`` (needs ``num_labels``
+    and the token) adds HF ``DeiTForImageClassificationWithTeacher``'s ``cls_classifier`` and
+    ``distillation_classifier`` in place of ``classifier`` (``distillation_logits``)."""
 
     def __init__(
         self,
@@ -502,6 +553,8 @@ class VIT(nn.Module):
         use_mask_token: bool = False,
         add_decoder: bool = False,
         encoder_stride: Optional[int] = None,
+        distillation_token: bool = False,
+        distillation_head: bool = False,
     ):
         super().__init__()
         assert height == width, "Height and width should be the same"
@@ -517,6 +570,8 @@ class VIT(nn.Module):
         self.num_layers = num_layers
 
         assert self.hidden_dim % self.num_heads == 0, f"Hidden dimension should be divisible by number of heads, provided: {self.hidden_dim} {self.num_heads}"
+        assert not distillation_head or (num_labels and distillation_token), \
+            "distillation_head=True needs num_labels and distillation_token=True"
 
         num_patches = (self.height // self.patch_size) * (self.width // self.patch_size)
         patch_dim = self.patch_size * self.patch_size * self.channels
@@ -524,7 +579,8 @@ class VIT(nn.Module):
 
         self.embeddings = Embeddings(patch_size=self.patch_size, num_patches=num_patches, patch_dim=patch_dim,
                                      hidden_dim=self.hidden_dim, channels=self.channels,
-                                     use_mask_token=use_mask_token or add_decoder)
+                                     use_mask_token=use_mask_token or add_decoder,
+                                     distillation_token=distillation_token)
         self.encoder = Encoder(num_layers=self.num_layers, num_heads=self.num_heads, hidden_dim=self.hidden_dim,
                                d_out=d_out, mlp_dim=mlp_dim)
         self.layernorm = LayerNormTriton(dim=self.hidden_dim, eps=1e-12)
@@ -532,7 +588,13 @@ class VIT(nn.Module):
         self.pooler = Pooler(self.hidden_dim) if add_pooling_layer else None
         # optional HF ViTForImageClassification head (Linear on the CLS row of the final hidden states):
         # state-dict keys classifier.{weight,bias}
-        self.classifier = LinearWithBias(self.hidden_dim, num_labels) if num_labels else None
+        self.classifier = LinearWithBias(self.hidden_dim, num_labels) if num_labels and not distillation_head else None
+        # optional HF DeiTForImageClassificationWithTeacher heads, on the CLS and the distillation-token rows: state-dict
+        # keys cls_classifier.{weight,bias}, distillation_classifier.{weight,bias}
+        self.cls_classifier = self.distillation_classifier = None
+        if distillation_head:
+            self.cls_classifier = LinearWithBias(self.hidden_dim, num_labels)
+            self.distillation_classifier = LinearWithBias(self.hidden_dim, num_labels)
         # optional HF ViTForMaskedImageModeling (SimMIM) decoder, Conv2d(D, s^2 C, 1) + PixelShuffle(s) with s =
         # encoder_stride (default: the patch size): state-dict keys decoder.0.{weight,bias}; implies the mask token
         self.encoder_stride = patch_size if encoder_stride is None else encoder_stride
@@ -551,6 +613,7 @@ class VIT(nn.Module):
         for m in self.modules():
             if isinstance(m, packing.PackedMixin):
                 m.invalidate_packed()
+        self.__dict__.pop("_teacher_packed", None)
         clear_derived_cache()
 
     @property
@@ -565,8 +628,9 @@ class VIT(nn.Module):
                 output_hidden_states: bool = False, output_attentions: bool = False):
         """(B, C, H, W) -> final hidden states (B, N, D).  ``interpolate_pos_encoding`` (HF ``ViTModel``'s flag): any
         H, W >= patch size, square or not; N = 1 + (H // P) * (W // P), the position table resampled bicubically to
-        that grid (``Embeddings.interpolate_pos_encoding``).  Without it the input must be the model's size.
-        ``bool_masked_pos`` (HF ``ViTModel``'s argument, needs ``use_mask_token=True``): bool (B, N - 1) on x's device,
+        that grid (``Embeddings.interpolate_pos_encoding``).  Without it the input must be the model's size.  With a
+        distillation token N counts two tokens in front of the patches instead of one.
+        ``bool_masked_pos`` (HF ``ViTModel``'s argument, needs ``use_mask_token=True``): bool (B, patches) on x's device,
         True = the patch's embedding is replaced by the mask token.  Masked inputs take the gather + GEMM patch
         embedding (``packing.embed_masked``); an all-false mask gives the unmasked result bit for bit.
 
@@ -603,7 +667,7 @@ class VIT(nn.Module):
     def _embed_stats(self, x: torch.Tensor, n_tok: Optional[int] = None) -> Optional[torch.Tensor]:
         """Buffer for the row statistics of the embeddings when block 0's layernorm_before is folded
         into its QKV GEMM (fused bf16 tensor-core path, hidden size a multiple of 128); None otherwise.
-        ``n_tok``: tokens per image (default: the model's own, num_patches + 1)."""
+        ``n_tok``: tokens per image (default: the model's own, num_patches + num_prefix_tokens)."""
         w = self.embeddings.projection.weight
         batch = x.shape[0]
         if not (x.is_cuda and w.is_cuda and w.dtype == torch.bfloat16 and batch > 0 and self.hidden_dim % 8 == 0
@@ -612,7 +676,7 @@ class VIT(nn.Module):
         probe = torch.empty((1,), device=x.device, dtype=w.dtype)
         if not self.encoder.folding_active(probe):
             return None
-        n_tok = self.embeddings.num_patches + 1 if n_tok is None else n_tok
+        n_tok = self.embeddings.num_patches + self.embeddings.num_prefix_tokens if n_tok is None else n_tok
         return torch.empty((batch * n_tok, self.hidden_dim // packing.STATS_COLS, 2), device=x.device,
                            dtype=torch.float32)
 
@@ -648,7 +712,7 @@ class VIT(nn.Module):
             assert x.dim() == 4, f"Expected {layout} pixels, provided: {tuple(x.shape)}"
             _, C, H, W = packing.pixel_dims(x, fmt)
             packing.check_any_size(self.embeddings, C, H, W)
-            n_tok = 1 + math.prod(packing.patch_grid(self.embeddings, H, W))
+            n_tok = self.embeddings.num_prefix_tokens + math.prod(packing.patch_grid(self.embeddings, H, W))
         else:
             assert tuple(x.shape[1:]) == size, f"Image size {x.shape[1:]} not matching with the model input size: {size}"
             n_tok = None
@@ -680,7 +744,7 @@ class VIT(nn.Module):
                        rescale_factor: float = 1.0 / 255.0) -> list:
         """Images of different resolutions in one batch: a list of (C, H_i, W_i) float32 / bfloat16 or raw (H_i, W_i, C)
         uint8 tensors (one dtype, the model's channel count, sides of at least one patch) -> the list of final hidden
-        states (N_i, D), N_i = 1 + (H_i // P) * (W_i // P), in the caller's order.  Image i gives what
+        states (N_i, D), N_i = num_prefix_tokens + (H_i // P) * (W_i // P), in the caller's order.  Image i gives what
         ``self(images[i][None], interpolate_pos_encoding=True)[0]`` (``forward_uint8`` for uint8, with these image-processor
         constants) gives, bit for bit: each image takes its own patch grid and position table.
 
@@ -697,7 +761,7 @@ class VIT(nn.Module):
         """(packed final hidden states (M, D), ``packing.RaggedLayout``) of a ragged batch."""
         grids, u8 = packing.check_ragged(self.embeddings, images)
         assert not torch.cuda.is_current_stream_capturing(), "A ragged batch cannot be captured into a CUDA graph"
-        layout = packing.RaggedLayout(grids)
+        layout = packing.RaggedLayout(grids, self.embeddings.num_prefix_tokens)
         first = images[0]
         if not (_FUSED and first.is_cuda and self.dtype == torch.bfloat16 and self.hidden_dim % 8 == 0):
             hidden = None
@@ -718,10 +782,11 @@ class VIT(nn.Module):
         x = self.layernorm(x)
         return x[0], layout
 
-    def _ragged_cls(self, images) -> torch.Tensor:
-        """(B, D) CLS rows of the final hidden states of a ragged batch, in the caller's order (``vt_gather_rows``)."""
+    def _ragged_cls(self, images, rows: int = 1) -> torch.Tensor:
+        """(B * rows, D): the first ``rows`` rows (CLS, then the distillation token) of every image's final hidden states
+        of a ragged batch, in the caller's order (one ``vt_gather_rows``)."""
         hidden, layout = self._ragged_hidden(images, (0.5, 0.5, 0.5), (0.5, 0.5, 0.5), 1.0 / 255.0)
-        return packing.gather_rows(hidden, layout.row0)
+        return packing.gather_rows(hidden, [r + j for r in layout.row0 for j in range(rows)])
 
     def _hidden(self, x, interpolate_pos_encoding: bool, bool_masked_pos: Optional[torch.Tensor] = None,
                 image_mean=(0.5, 0.5, 0.5), image_std=(0.5, 0.5, 0.5),
@@ -737,11 +802,12 @@ class VIT(nn.Module):
             return self.forward_uint8(x, image_mean, image_std, rescale_factor, **kw)
         return self.forward(x, **kw)
 
-    def _cls_hidden(self, x, interpolate_pos_encoding: bool, bool_masked_pos) -> torch.Tensor:
-        """(B, N, D) final hidden states, or (B, 1, D) CLS rows of a list of images (ragged batch)."""
+    def _cls_hidden(self, x, interpolate_pos_encoding: bool, bool_masked_pos, rows: int = 1) -> torch.Tensor:
+        """(B, N, D) final hidden states, or (B, rows, D) first rows of every image of a list of images (ragged
+        batch)."""
         if isinstance(x, (list, tuple)):
             assert bool_masked_pos is None, "bool_masked_pos is not supported with a list of images"
-            return self._ragged_cls(x)[:, None, :]
+            return self._ragged_cls(x, rows).view(len(x), rows, -1)
         return self._hidden(x, interpolate_pos_encoding, bool_masked_pos)
 
     def pooler_output(self, x, interpolate_pos_encoding: bool = False,
@@ -765,13 +831,48 @@ class VIT(nn.Module):
         ``ViTForImageClassification(...).logits``; needs ``VIT(..., num_labels=...)``.  One tensor-core
         launch over the CLS rows of the final hidden states.  ``x`` may also be a list of images of different sizes
         (``forward_ragged``), each with its own patch grid (without a mask).  ``do_resize`` / ``resample`` as for
-        ``forward_uint8``: the images are resized to the model's size first (a list then runs as one batch, not ragged)."""
+        ``forward_uint8``: the images are resized to the model's size first (a list then runs as one batch, not ragged).
+        On a model with ``distillation_head=True``: ``distillation_logits(...).logits``."""
         _refuse_outputs("logits", output_hidden_states, output_attentions)
+        if self.cls_classifier is not None:
+            return self.distillation_logits(x, interpolate_pos_encoding, bool_masked_pos, do_resize=do_resize,
+                                            resample=resample).logits
         assert self.classifier is not None, "VIT was built without a classifier head (num_labels)"
         x = self._resized(x, do_resize, resample)
         hidden = self._cls_hidden(x, interpolate_pos_encoding, bool_masked_pos)
         from .kernels import bgemm as bg
         return _head_on_cls(hidden, self.classifier, bg.ACT_NONE)
+
+    def distillation_logits(self, x, interpolate_pos_encoding: bool = False,
+                            bool_masked_pos: Optional[torch.Tensor] = None, output_hidden_states: bool = False,
+                            output_attentions: bool = False, do_resize: bool = False,
+                            resample: int = 2) -> DistilledLogits:
+        """HF ``DeiTForImageClassificationWithTeacher``: ``DistilledLogits(logits, cls_logits, distillation_logits)``,
+        (B, num_labels) each, cls_logits = cls_classifier(final hidden states[:, 0]), distillation_logits =
+        distillation_classifier(final hidden states[:, 1]), logits their mean; needs ``VIT(..., distillation_head=True)``.
+        One tensor-core launch after the encoder for all three (``_distilled_head``).  Arguments as for ``logits``; a
+        list of images first collects rows 0 and 1 of every image with one ``vt_gather_rows``."""
+        _refuse_outputs("distillation_logits", output_hidden_states, output_attentions)
+        assert self.cls_classifier is not None, "VIT was built without the distillation head (distillation_head=True)"
+        x = self._resized(x, do_resize, resample)
+        hidden = self._cls_hidden(x, interpolate_pos_encoding, bool_masked_pos, rows=2)
+        from .kernels import bgemm as bg
+        pieces = 1 if hidden.dtype == torch.bfloat16 else bg.split_pieces()
+        return _distilled_head(hidden, self._teacher_pack(pieces))
+
+    def _teacher_pack(self, pieces: int) -> SimpleNamespace:
+        """``packing.pack_teacher_head`` of the two classifiers, cached on the model: rebuilt when either classifier's
+        storage pointer or version counter changes, dropped by ``invalidate_packed``."""
+        params = [self.cls_classifier.weight, self.cls_classifier.bias, self.distillation_classifier.weight,
+                  self.distillation_classifier.bias]
+        key = (pieces, packing.PackedMixin._packed_key(params))
+        hit = self.__dict__.get("_teacher_packed")
+        if hit is not None and hit[0] == key:
+            return hit[1]
+        with torch.no_grad():
+            value = packing.pack_teacher_head(self.cls_classifier, self.distillation_classifier, pieces)
+        self.__dict__["_teacher_packed"] = (key, value)
+        return value
 
     def pooled(self, x, interpolate_pos_encoding: bool = False,
                bool_masked_pos: Optional[torch.Tensor] = None, output_hidden_states: bool = False,
@@ -806,6 +907,10 @@ class VIT(nn.Module):
         fp32 device tensor reduced in a fixed order (no host synchronisation, the same bits on every call).  The loss
         needs s == P and H, W multiples of P; the reconstruction works on any grid (HF only defines square ones)."""
         _refuse_outputs("masked_image_modeling", output_hidden_states, output_attentions)
+        # HF DeiTForMaskedImageModeling drops the last patch row (sequence_output[:, 1:-1]) instead of the distillation
+        # token; that layout is not reproduced
+        assert self.embeddings.distillation_token is None, \
+            "masked_image_modeling is not supported on a model with distillation_token=True"
         assert self.decoder is not None, "VIT was built without the masked image modeling decoder (add_decoder=True)"
         assert not isinstance(x, (list, tuple)), "masked_image_modeling takes a batch tensor, not a list of images"
         u8 = x.dtype == torch.uint8

@@ -56,7 +56,8 @@ int vt_softmax(const void* x, void* out, int64_t rows, int32_t cols, int64_t in_
 
 /* K1 — tensor-core GEMM (tcgen05 + TMEM + TMA):  out[M,N] = epi(A[M,K] . Bt[N,K]^T + bias).
  * A, Bt bf16, K-major (row strides lda / ldb in elements, multiples of 8; K, N multiples of 8).
- * out / residual: bf16 or f32 (out_dtype); bias: f32 or NULL; gelu: exact-erf GELU;
+ * out / residual: bf16 or f32 (out_dtype); bias: f32 or NULL; gelu: epilogue activation, VT_ACT_NONE /
+ * VT_ACT_GELU (exact erf) / VT_ACT_QUICK_GELU of vitb200_clip.h (0 / 1 / 3; others: VT_ERR_ARG);
  * residual (nullable) is added after the bias and may alias out.
  * Replaces matmul_triton (vit/kernels/matmul.py:111-156) for the model's dense layers and folds
  * add_triton (vit/vit.py:140,147) into the epilogue. */
@@ -73,7 +74,8 @@ int vt_gemm_bf16(const void* A, int64_t lda, const void* Bt, int64_t ldb, void* 
  *     variance is exactly 0 yields out = bias_n (= LN's beta through the dense layer).
  *     ln_dim % 128 == 0; Bt must carry gamma
  *     (Bt[n,k] = W[n,k] * gamma[k]), bias must carry beta (bias[n] + sum_k beta[k] W[n,k]) and
- *     colsum[n] = sum_k Bt[n,k]:   out = rstd_m * acc - rstd_m * mean_m * colsum_n + bias_n  (then GELU).
+ *     colsum[n] = sum_k Bt[n,k]:   out = rstd_m * acc - rstd_m * mean_m * colsum_n + bias_n  (then the activation:
+ *     gelu as for vt_gemm_bf16).
  *     colsum == NULL: the rows of Bt sum to zero (Bt[n,k] = W[n,k]*gamma[k] - mean_k(W[n,k]*gamma[k])), the
  *     mean term is then part of acc and   out = rstd_m * acc + bias_n.
  *   stats_out != NULL (needs residual, N % 128 == 0): writes the (sum, M2) of every 128-column group
@@ -101,7 +103,7 @@ int vt_ln_fold(const void* w, int64_t ldw, const float* bias, const float* gamma
 /* Generic strided batched GEMM on the FP32 pipe (exact-fp32 path and odd shapes):
  *   C[z] = scale * act(A[z] . B[z] + bias),  z = zo * batch_inner + zi
  * strides (elements): sA = {outer, inner, m, k}, sB = {outer, inner, k, n}, sC = {outer, inner, m, n}.
- * All tensors share `dtype`; bias nullable.
+ * All tensors share `dtype`; bias nullable; gelu: VT_ACT_NONE / VT_ACT_GELU / VT_ACT_QUICK_GELU (vitb200_clip.h).
  * Replaces matmul_triton (matmul.py:111-156) and matmul3's matmul_triton (matmul3.py:111-156)
  * wherever the tensor-core path's alignment rules do not hold. */
 int vt_gemm_strided(const void* A, const void* B, void* C, const void* bias, int32_t M, int32_t N,
@@ -113,7 +115,8 @@ int vt_gemm_strided(const void* A, const void* B, void* C, const void* bias, int
  *   out[M,N] = act( (A8[M,K] . B8[N,K]^T) * colscale[n] + bias[n] ) (+ residual)
  * A8, B8: e4m3 bytes, K-major, row strides lda / ldb in BYTES (multiples of 16, K % 16 == 0); colscale f32 [N] =
  * per-output-channel weight scale x activation scale; bias f32 [N] (nullable); residual bf16 (nullable, ldr in elements);
- * out_dtype VT_BF16 (ldo in elements) or VT_E4M3: out8 = e4m3(out * out_scale), ldo in bytes, N % 128 == 0, no residual.
+ * out_dtype VT_BF16 (ldo in elements) or VT_E4M3: out8 = e4m3(out * out_scale), ldo in bytes, N % 128 == 0, no residual;
+ * gelu (act): VT_ACT_NONE / VT_ACT_GELU / VT_ACT_QUICK_GELU (vitb200_clip.h).
  * Replaces matmul_triton (vit/kernels/matmul.py:111-156) for the QKV / fc1 / fc2 layers when the FP8 path is on. */
 int vt_gemm_fp8(const void* A, int64_t lda, const void* Bt, int64_t ldb, void* out, int64_t ldo, int32_t out_dtype,
                 const float* bias, const float* colscale, const void* residual, int64_t ldr, int32_t M, int32_t N,
@@ -138,7 +141,7 @@ int vt_quantize_rows_fp8(const void* w, int64_t ldw, void* out, int64_t ldo, flo
  *    A batch stride of 0 broadcasts the operand along that level (A and B alike); both batch strides 0 =
  *    one matrix shared by all batches (weights).
  * C / residual: out_dtype (bf16 | f32) [M, N] per batch, sC = {outer, inner, row}; bias f32 [N] (nullable);
- * act: 0 none, 1 exact-erf GELU, 2 tanh.  Any M, N, K; every A / B stride a multiple of 8 elements and
+ * act: VT_ACT_* of vitb200_clip.h: 0 none, 1 exact-erf GELU, 2 tanh, 3 quick GELU.  Any M, N, K; every A / B stride a multiple of 8 elements and
  * both bases 16-byte aligned (pack with vt_pack_bf16 otherwise).
  * Replaces matmul3's matmul_triton (vit/kernels/matmul3.py:111-156); with split fp32 operands
  * (vt_pack_bf16, pieces = 3) also matmul_triton (vit/kernels/matmul.py:111-156) for the fp32 model, whose

@@ -1,5 +1,5 @@
 // extern "C" surface of libvitb200.so (declared in include/vitb200.h and its companions
-// vitb200_resolution.h, vitb200_ragged.h, vitb200_mask.h, vitb200_tokens.h).  Thin: argument plumbing
+// vitb200_resolution.h, vitb200_ragged.h, vitb200_mask.h, vitb200_tokens.h, vitb200_clip.h).  Thin: argument plumbing
 // only, all kernels live in the other translation units.
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -10,10 +10,13 @@
 #include "../../include/vitb200_ragged.h"
 #include "../../include/vitb200_mask.h"
 #include "../../include/vitb200_tokens.h"
+#include "../../include/vitb200_clip.h"
 
 namespace vt {
 int layernorm_rows(const void*, const void*, const void*, void*, long long, int, long long,
                    long long, float, int, int, int, cudaStream_t);
+int layernorm_stats(const void*, const void*, const void*, void*, float*, long long, int, long long, long long, float, int,
+                    cudaStream_t);
 int add_elementwise(const void*, const void*, void*, long long, int, cudaStream_t);
 int softmax_rows(const void*, void*, long long, int, long long, int, cudaStream_t);
 int pool_cls(const void*, void*, int, int, long long, int, cudaStream_t);
@@ -121,6 +124,12 @@ int vt_layernorm(const void* x, const void* gamma, const void* beta, void* out, 
                  int32_t in_dtype, int32_t out_dtype, void* stream) {
   return vt::layernorm_rows(x, gamma, beta, out, rows, dim, in_row_stride, out_row_stride, eps,
                             in_dtype, out_dtype, next_direction(), S(stream));
+}
+
+int vt_layernorm_stats(const void* x, const void* gamma, const void* beta, void* out, float* stats, int64_t rows,
+                       int32_t dim, int64_t in_row_stride, int64_t out_row_stride, float eps, void* stream) {
+  return vt::layernorm_stats(x, gamma, beta, out, stats, rows, dim, in_row_stride, out_row_stride, eps,
+                             next_direction(), S(stream));
 }
 
 int vt_add(const void* a, const void* b, void* out, int64_t n, int32_t dtype, void* stream) {

@@ -34,7 +34,7 @@ constexpr int GB_BK = 64;
 constexpr int GB_EPI_WARPS = 8;
 constexpr int GB_THREADS = 128 + GB_EPI_WARPS * 32;
 
-enum : int { ACT_NONE = 0, ACT_GELU = 1, ACT_TANH = 2 };
+enum : int { ACT_NONE = kActNone, ACT_GELU = kActGelu, ACT_TANH = kActTanh, ACT_QUICK_GELU = kActQuickGelu };
 
 struct BgemmParams {
   int M, N, K;
@@ -227,6 +227,9 @@ bgemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_con
         } else if (p.act == ACT_TANH) {
 #pragma unroll
           for (int i = 0; i < 32; ++i) v[i] = tanhf(v[i]);
+        } else if (p.act == ACT_QUICK_GELU) {
+#pragma unroll
+          for (int i = 0; i < 32; ++i) v[i] = quick_gelu(v[i]);
         }
         const bool full_chunk = (col + 32 <= p.N) && p.vec_ok;
         if (p.out_f32) {
@@ -334,7 +337,7 @@ int bgemm_tcgen05(const void* A, const void* B, void* C, const float* bias, cons
   if (!A || !B || !C || !sA || !sB || !sC || M <= 0 || N <= 0 || K <= 0 || batch_outer <= 0 || batch_inner <= 0)
     return VT_ERR_ARG;
   if (out_dtype != VT_BF16 && out_dtype != VT_F32) return VT_ERR_DTYPE;
-  if (act < ACT_NONE || act > ACT_TANH) return VT_ERR_ARG;
+  if (act < ACT_NONE || act > ACT_QUICK_GELU) return VT_ERR_ARG;
   if (static_cast<long long>(batch_outer) * batch_inner >= (1LL << 30)) return VT_ERR_UNSUPPORTED;
   // TMA: base 16-byte aligned, every stride a multiple of 16 bytes
   if ((sA[0] % 8) || (sA[1] % 8) || (sA[2] % 8) || (sB[0] % 8) || (sB[1] % 8) || (sB[2] % 8)) return VT_ERR_ALIGN;

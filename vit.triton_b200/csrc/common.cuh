@@ -27,6 +27,11 @@ enum : int {
 
 enum : int { VT_F32 = 0, VT_BF16 = 1, VT_U8 = 2, VT_E4M3 = 3 };
 
+// GEMM epilogue activations: the VT_ACT_* codes of include/vitb200_clip.h.  vt_bgemm takes all four; the `gelu`
+// argument of vt_gemm_bf16, vt_gemm_bf16_ln, vt_gemm_fp8 and vt_gemm_strided takes none, GELU or quick GELU.
+enum : int { kActNone = 0, kActGelu = 1, kActTanh = 2, kActQuickGelu = 3 };
+inline bool gemm_act_ok(int act) { return act == kActNone || act == kActGelu || act == kActQuickGelu; }
+
 // ----------------------------------------------------------------------------------------------
 // host: opt-in dynamic shared memory.  cudaFuncAttributeMaxDynamicSharedMemorySize is a PER-DEVICE
 // attribute; `granted` is the call site's own per-device cache (one static array per kernel).
@@ -493,6 +498,39 @@ __device__ __forceinline__ float2 gelu_erf_poly_x2(float2 x) {
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e.y) : "f"(p.y));
   const float2 nh = __fmul2_rn(a, make_float2(-0.5f, -0.5f));
   return __ffma2_rn(nh, e, make_float2(fmaxf(x.x, 0.0f), fmaxf(x.y, 0.0f)));
+}
+
+// Quick GELU (CLIP's hidden_act="quick_gelu", VT_ACT_QUICK_GELU) for fp32 outputs: x * sigmoid(1.702 x) with expf and
+// an IEEE division, within 2e-6 relative + 1e-7 absolute of the fp64 value for every finite x (for x < -52 the
+// exponential overflows to +inf and the result is -0, off by less than 1e-36).
+__device__ __forceinline__ float quick_gelu(float x) {
+  return x / (1.0f + expf(-1.702f * x));
+}
+
+// Quick GELU for results that are immediately rounded to bf16 (fc1 epilogue), ONE MUFU operation per element:
+// with a = |x| and e2 = 2^(-1.702 a log2(e) / 2), e = e2^2 = exp(-1.702 a),
+//   x * sigmoid(1.702 x) = relu(x) - a * e / (1 + e)         (both signs: x - x e/(1+e) for x >= 0, x e/(1+e) below)
+// and 1 / (1 + e) on e in [0, 1] is a degree-4 minimax polynomial (relative error <= 3.0e-4; the coefficients below
+// are negated so that a * e2 * (e2 * -r) is one FFMA2 into relu(x)).  The product keeps the two factors a * e2 and
+// e2 * r apart so that neither underflows before the final FMA: results down to the fp32 subnormal range (x to about
+// -60) keep their relative accuracy, and ex2.approx.ftz only flushes e2 where the result is below bf16's range.
+// Relative error <= 3.1e-4, under a tenth of a bf16 ulp: within one bf16 ulp of the correctly rounded fp64
+// x * sigmoid(1.702 x) for every finite bf16 input (tests/test_abi_clip.py restates the arithmetic in numpy and
+// checks all of them).  tanh.approx.f32 (0.5 x + 0.5 x tanh(0.851 x)) needs no second MUFU either, but its
+// 2^-11 relative error is amplified by the cancellation at x < 0 and misses that bound.  15 instructions per PAIR,
+// two of them MUFU (gelu_erf_poly_x2: 13 and two).
+__device__ __forceinline__ float2 quick_gelu_bf16_x2(float2 x) {
+  const float2 a = make_float2(fabsf(x.x), fabsf(x.y));
+  const float2 t = __fmul2_rn(a, make_float2(-1.2277335f, -1.2277335f));   // -1.702 log2(e) / 2
+  float2 e2;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e2.x) : "f"(t.x));
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e2.y) : "f"(t.y));
+  const float2 e = __fmul2_rn(e2, e2);
+  float2 r = __ffma2_rn(e, make_float2(-0.15224545f, -0.15224545f), make_float2(0.53285909f, 0.53285909f));
+  r = __ffma2_rn(e, r, make_float2(-0.86589509f, -0.86589509f));
+  r = __ffma2_rn(e, r, make_float2(0.98483551f, 0.98483551f));
+  r = __ffma2_rn(e, r, make_float2(-0.99970269f, -0.99970269f));                // r = -1 / (1 + e)
+  return __ffma2_rn(__fmul2_rn(a, e2), __fmul2_rn(e2, r), make_float2(fmaxf(x.x, 0.0f), fmaxf(x.y, 0.0f)));
 }
 
 __device__ __forceinline__ float ex2_approx(float x) {

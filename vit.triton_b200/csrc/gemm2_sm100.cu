@@ -75,7 +75,8 @@ constexpr uint32_t kPeerMask = 0xFEFFFFFFu;             // clears the CTA-rank b
 
 // EPI_NOCS (with EPI_LNF): the folded weights have zero-sum rows (packing._fold_layernorm_zero_sum), so the
 // mean term is already inside the accumulator and the epilogue needs no column sums.
-enum : int { EPI_GELU = 1, EPI_RES = 2, EPI_LNF = 4, EPI_STATS = 8, EPI_NOCS = 16, EPI_CSCALE = 32 };
+enum : int { EPI_GELU = 1, EPI_RES = 2, EPI_LNF = 4, EPI_STATS = 8, EPI_NOCS = 16, EPI_CSCALE = 32, EPI_QGELU = 64 };
+// EPI_QGELU: quick GELU x * sigmoid(1.702 x) (CLIP) where EPI_GELU applies exact GELU; the two never combine.
 // EPI_CSCALE (FP8 operands): out = acc * colscale_n + bias_n — the per-output-channel dequantisation scale of the
 // e4m3 weights times the activation scale (Gemm2Params::colsum carries it).
 // PREC: 0 = bf16 operands, bf16 output (kind::f16); 1 = e4m3 operands, bf16 output; 2 = e4m3 operands, e4m3 output
@@ -675,6 +676,10 @@ gemm2_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_consta
 #pragma unroll
               for (int q = 0; q < 4; ++q) v[q] = gelu_epi2(v[q]);
             }
+            if (EPI & EPI_QGELU) {
+#pragma unroll
+              for (int q = 0; q < 4; ++q) v[q] = quick_gelu_bf16_x2(v[q]);
+            }
             if (EPI & EPI_STATS) {
               if (c == 0 && hh == 0 && jj == 0) st_npiv2 = make_float2(-v[0].x, -v[0].x);
 #pragma unroll
@@ -834,7 +839,7 @@ int gemm2_bf16_tcgen05(const void* A, long long lda, const void* Bt, long long l
                        long long ldo, const float* bias, const void* residual, long long ldr, int M,
                        int N, int K, int gelu, const float* rowstats, const float* colsum, int ln_dim,
                        float ln_eps, float* stats_out, int reverse, cudaStream_t stream) {
-  if (!A || !Bt || !out || M <= 0 || N <= 0 || K <= 0) return VT_ERR_ARG;
+  if (!A || !Bt || !out || M <= 0 || N <= 0 || K <= 0 || !gemm_act_ok(gelu)) return VT_ERR_ARG;
   if (gelu && residual) return VT_ERR_UNSUPPORTED;
   if (colsum && !rowstats) return VT_ERR_ARG;
   if (rowstats && (residual || stats_out || ln_dim <= 0)) return VT_ERR_UNSUPPORTED;
@@ -900,7 +905,7 @@ int gemm2_bf16_tcgen05(const void* A, long long lda, const void* Bt, long long l
   // everything else takes the sixth operand stage — with the paced epilogue and the prefetched
   // operands that now also holds for GELU (215.7k -> 209.4k cycles per fc1 launch) and the LayerNorm
   // fold (7947 -> 7050 cycles per tile).  VT_GEMM_STAGES=5|6 forces one for every launch,
-  // VT_LNF_STAGES=5|6 for the LayerNorm-fold launches only, VT_GELU_STAGES=5|6 for the GELU launches.
+  // VT_LNF_STAGES=5|6 for the LayerNorm-fold launches only, VT_GELU_STAGES=5|6 for the GELU and quick-GELU launches.
   static const int forced = [] {
     const char* e = getenv("VT_GEMM_STAGES");
     return (e && (e[0] == '5' || e[0] == '6')) ? (e[0] - '0') : 0;
@@ -918,9 +923,16 @@ int gemm2_bf16_tcgen05(const void* A, long long lda, const void* Bt, long long l
   }();
   if (gelu && forced_gelu) deep = (forced_gelu == 6);
 #define VT_G2_LAUNCH(E) (deep ? launch2<E, G2Deep>(ta, tb, to, tr, ta64, tb64, p, stream) : launch2<E, G2Wide>(ta, tb, to, tr, ta64, tb64, p, stream))
-  if (rowstats && !colsum) return gelu ? VT_G2_LAUNCH(EPI_LNF | EPI_NOCS | EPI_GELU) : VT_G2_LAUNCH(EPI_LNF | EPI_NOCS);
-  if (rowstats) return gelu ? VT_G2_LAUNCH(EPI_LNF | EPI_GELU) : VT_G2_LAUNCH(EPI_LNF);
-  if (gelu) return VT_G2_LAUNCH(EPI_GELU);
+  const bool quick = gelu == kActQuickGelu;
+  if (rowstats && !colsum) {
+    if (!gelu) return VT_G2_LAUNCH(EPI_LNF | EPI_NOCS);
+    return quick ? VT_G2_LAUNCH(EPI_LNF | EPI_NOCS | EPI_QGELU) : VT_G2_LAUNCH(EPI_LNF | EPI_NOCS | EPI_GELU);
+  }
+  if (rowstats) {
+    if (!gelu) return VT_G2_LAUNCH(EPI_LNF);
+    return quick ? VT_G2_LAUNCH(EPI_LNF | EPI_QGELU) : VT_G2_LAUNCH(EPI_LNF | EPI_GELU);
+  }
+  if (gelu) return quick ? VT_G2_LAUNCH(EPI_QGELU) : VT_G2_LAUNCH(EPI_GELU);
   if (residual) return stats_out ? VT_G2_LAUNCH(EPI_RES | EPI_STATS) : VT_G2_LAUNCH(EPI_RES);
   return VT_G2_LAUNCH(0);
 #undef VT_G2_LAUNCH
@@ -989,7 +1001,7 @@ int gemm2_patch_tokens(const void* A, long long lda, const void* W, long long ld
 int gemm2_fp8_tcgen05(const void* A, long long lda, const void* Bt, long long ldb, void* out, long long ldo,
                       int out_e4m3, const float* bias, const float* colscale, const void* residual, long long ldr,
                       int M, int N, int K, int gelu, float out_scale, int reverse, cudaStream_t stream) {
-  if (!A || !Bt || !out || !colscale || M <= 0 || N <= 0 || K <= 0) return VT_ERR_ARG;
+  if (!A || !Bt || !out || !colscale || M <= 0 || N <= 0 || K <= 0 || !gemm_act_ok(gelu)) return VT_ERR_ARG;
   if (gelu && residual) return VT_ERR_UNSUPPORTED;
   if (out_e4m3 && (residual || (N % 128))) return VT_ERR_UNSUPPORTED;
   if ((K % 16) || (lda % 16) || (ldb % 16) || (N % 8) || (ldo % (out_e4m3 ? 16 : 8)) || (residual && (ldr % 8)))
@@ -1038,10 +1050,14 @@ int gemm2_fp8_tcgen05(const void* A, long long lda, const void* Bt, long long ld
   if (ideal > 6144) ideal = 6144;
   p.pace = static_cast<int>(ideal * 210 / 1000);
   p.pace_q = static_cast<int>(ideal * 50 / 1000);
-  if (out_e4m3)
+  const bool quick = gelu == kActQuickGelu;
+  if (out_e4m3) {
+    if (quick) return launch2<EPI_CSCALE | EPI_QGELU, G2Deep, 2>(ta, tb, to, tr, ta64, tb64, p, stream);
     return gelu ? launch2<EPI_CSCALE | EPI_GELU, G2Deep, 2>(ta, tb, to, tr, ta64, tb64, p, stream)
                 : launch2<EPI_CSCALE, G2Deep, 2>(ta, tb, to, tr, ta64, tb64, p, stream);
+  }
   if (residual) return launch2<EPI_CSCALE | EPI_RES, G2Deep, 1>(ta, tb, to, tr, ta64, tb64, p, stream);
+  if (quick) return launch2<EPI_CSCALE | EPI_QGELU, G2Deep, 1>(ta, tb, to, tr, ta64, tb64, p, stream);
   if (gelu) return launch2<EPI_CSCALE | EPI_GELU, G2Deep, 1>(ta, tb, to, tr, ta64, tb64, p, stream);
   return launch2<EPI_CSCALE, G2Deep, 1>(ta, tb, to, tr, ta64, tb64, p, stream);
 }

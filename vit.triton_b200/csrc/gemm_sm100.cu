@@ -24,7 +24,7 @@ constexpr int BK = 64;
 constexpr int kEpiWarps = 8;
 constexpr int kThreads = 128 + kEpiWarps * 32;
 
-enum : int { EPI_GELU = 1, EPI_RES = 2, EPI_F32 = 4 };
+enum : int { EPI_GELU = 1, EPI_RES = 2, EPI_F32 = 4, EPI_QGELU = 8 };   // EPI_QGELU: quick GELU (CLIP)
 
 struct GemmParams {
   int M, N, K;
@@ -196,6 +196,10 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a,
 #pragma unroll
           for (int i = 0; i < 32; ++i) v[i] = gelu_erf(v[i]);
         }
+        if (EPI & EPI_QGELU) {
+#pragma unroll
+          for (int i = 0; i < 32; ++i) v[i] = quick_gelu(v[i]);
+        }
         if (row < p.M) {
           const bool full_chunk = (col + 32 <= p.N);
           if (EPI & EPI_F32) {
@@ -303,6 +307,8 @@ int launch_bn(const CUtensorMap& ta, const CUtensorMap& tb, const GemmParams& p,
     case EPI_RES: return launch_cfg<BN, EPI_RES>(ta, tb, p, stream);
     case EPI_F32: return launch_cfg<BN, EPI_F32>(ta, tb, p, stream);
     case EPI_F32 | EPI_GELU: return launch_cfg<BN, EPI_F32 | EPI_GELU>(ta, tb, p, stream);
+    case EPI_QGELU: return launch_cfg<BN, EPI_QGELU>(ta, tb, p, stream);
+    case EPI_F32 | EPI_QGELU: return launch_cfg<BN, EPI_F32 | EPI_QGELU>(ta, tb, p, stream);
     case EPI_F32 | EPI_RES: return launch_cfg<BN, EPI_F32 | EPI_RES>(ta, tb, p, stream);
     default: return VT_ERR_UNSUPPORTED;
   }
@@ -315,7 +321,7 @@ int launch_bn(const CUtensorMap& ta, const CUtensorMap& tb, const GemmParams& p,
 int gemm_bf16_tcgen05(const void* A, long long lda, const void* Bt, long long ldb, void* out,
                       long long ldo, int out_dtype, const float* bias, const void* residual,
                       long long ldr, int M, int N, int K, int gelu, cudaStream_t stream) {
-  if (!A || !Bt || !out || M <= 0 || N <= 0 || K <= 0) return VT_ERR_ARG;
+  if (!A || !Bt || !out || M <= 0 || N <= 0 || K <= 0 || !gemm_act_ok(gelu)) return VT_ERR_ARG;
   if (gelu && residual) return VT_ERR_UNSUPPORTED;
   if ((K % 8) || (lda % 8) || (ldb % 8) || (N % 8) || (ldo % 8) || (residual && (ldr % 8)))
     return VT_ERR_ALIGN;
@@ -339,7 +345,7 @@ int gemm_bf16_tcgen05(const void* A, long long lda, const void* Bt, long long ld
   p.out = out; p.ldo = ldo;
   p.bias = bias;
   p.residual = residual; p.ldr = ldr;
-  int epi = (gelu ? EPI_GELU : 0) | (residual ? EPI_RES : 0) | (out_dtype == VT_F32 ? EPI_F32 : 0);
+  int epi = (gelu == kActGelu ? EPI_GELU : gelu == kActQuickGelu ? EPI_QGELU : 0) | (residual ? EPI_RES : 0) | (out_dtype == VT_F32 ? EPI_F32 : 0);
   return bn == 256 ? launch_bn<256>(ta, tb, p, epi, stream) : launch_bn<128>(ta, tb, p, epi, stream);
 }
 

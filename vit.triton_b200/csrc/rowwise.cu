@@ -134,12 +134,17 @@ layernorm_rows_kernel(const T* __restrict__ x, const T* __restrict__ gamma,
 // unpacked in each of the three passes: <= 32 registers per thread, i.e. 64 resident warps per SM
 // instead of 40 for layernorm_rows_kernel.  Same formula; the sums run over even / odd elements
 // separately (packed pairs), so the last bit can differ from layernorm_rows_kernel.
-template <int VPL>
-__global__ void __launch_bounds__(256, 8)
+// STATS (vt_layernorm_stats, dim % 128 == 0): also writes the (sum, M2 about the group mean) of every 128-column group of
+// every OUTPUT row, computed from the bf16 values stored, to stats[(row * dim/128 + group) * 2 .. +1] — the rowstats
+// layout of vt_gemm_bf16_ln.  A group is the 16 vectors of one half-warp, reduced in a fixed shuffle order (no
+// atomics: bit-reproducible); the normalised output is the same arithmetic, so the same bits, as without STATS.  The
+// statistics keep the stored row in registers: up to 64 per thread (4 blocks per SM) instead of 32, which spill.
+template <int VPL, bool STATS = false>
+__global__ void __launch_bounds__(256, STATS ? 4 : 8)
 layernorm_bf16_packed_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ gamma,
                              const __nv_bfloat16* __restrict__ beta, __nv_bfloat16* __restrict__ out,
                              long long rows, int dim, long long in_stride, long long out_stride, float eps,
-                             int reverse) {
+                             int reverse, float* __restrict__ stats = nullptr) {
   const int lane = threadIdx.x & 31;
   long long row = static_cast<long long>(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (row >= rows) return;
@@ -195,6 +200,36 @@ layernorm_bf16_packed_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfl
       o.z = nrm(d[i].z, g.z, b.z);
       o.w = nrm(d[i].w, g.w, b.w);
       orow[vi] = o;
+      if constexpr (STATS) d[i] = o;    // keep the stored bf16 values for the statistics
+    }
+  }
+  if constexpr (STATS) {
+    // dim % 128 == 0: a half-warp's 16 vectors (one group) are all valid or all past the row; the shuffles run on every
+    // lane, invalid ones contributing zeros
+    auto half_sum = [](float v) {
+#pragma unroll
+      for (int o = 8; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+      return v;
+    };
+    const int parts = dim >> 7;
+    float2* srow = reinterpret_cast<float2*>(stats) + row * parts;
+#pragma unroll
+    for (int i = 0; i < VPL; ++i) {
+      const bool valid = lane + i * 32 < nvec;
+      float2 s = make_float2(0.f, 0.f);
+      if (valid) {
+        s = __fadd2_rn(up(d[i].x), up(d[i].y));
+        s = __fadd2_rn(s, __fadd2_rn(up(d[i].z), up(d[i].w)));
+      }
+      const float sum = half_sum(s.x + s.y);
+      const float2 ng = make_float2(-sum * (1.0f / 128.0f), -sum * (1.0f / 128.0f));
+      float2 q = make_float2(0.f, 0.f);
+      if (valid) {
+        auto sq = [&](uint32_t w) { const float2 c = __fadd2_rn(up(w), ng); q = __ffma2_rn(c, c, q); };
+        sq(d[i].x); sq(d[i].y); sq(d[i].z); sq(d[i].w);
+      }
+      const float m2 = half_sum(q.x + q.y);
+      if (valid && (lane & 15) == 0) srow[2 * i + (lane >> 4)] = make_float2(sum, m2);
     }
   }
 }
@@ -530,6 +565,33 @@ int layernorm_rows(const void* x, const void* gamma, const void* beta, void* out
     return launch_layernorm<float, __nv_bfloat16>(x, gamma, beta, out, rows, dim, in_stride,
                                                   out_stride, eps, reverse, stream);
   return VT_ERR_DTYPE;
+}
+
+// vt_layernorm_stats: the packed kernel vt_layernorm runs for these rows (bf16, dim <= 1280, 16-byte aligned) with the
+// row statistics of its output written as well.
+int layernorm_stats(const void* x, const void* gamma, const void* beta, void* out, float* stats, long long rows, int dim,
+                    long long in_stride, long long out_stride, float eps, int reverse, cudaStream_t stream) {
+  if (!x || !gamma || !beta || !out || !stats || rows < 0 || dim <= 0 || (dim % 128)) return VT_ERR_ARG;
+  if (dim > 5 * 32 * 8) return VT_ERR_UNSUPPORTED;
+  if ((in_stride % 8) || (out_stride % 8) ||
+      ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(gamma) | reinterpret_cast<uintptr_t>(beta) |
+        reinterpret_cast<uintptr_t>(out)) & 15) || (reinterpret_cast<uintptr_t>(stats) & 7))
+    return VT_ERR_ALIGN;
+  if (rows == 0) return VT_OK;
+  const int warps = 8;
+  const unsigned grid = static_cast<unsigned>((rows + warps - 1) / warps);
+  const auto* xp = static_cast<const __nv_bfloat16*>(x);
+  const auto* gp = static_cast<const __nv_bfloat16*>(gamma);
+  const auto* bp = static_cast<const __nv_bfloat16*>(beta);
+  auto* op = static_cast<__nv_bfloat16*>(out);
+#define VT_LNS_CASE(V)                                                                                               \
+  case V:                                                                                                            \
+    layernorm_bf16_packed_kernel<V, true><<<grid, warps * 32, 0, stream>>>(xp, gp, bp, op, rows, dim, in_stride,     \
+                                                                           out_stride, eps, reverse, stats);         \
+    break;
+  switch ((dim / 8 + 31) / 32) { VT_LNS_CASE(1) VT_LNS_CASE(2) VT_LNS_CASE(3) VT_LNS_CASE(4) VT_LNS_CASE(5) }
+#undef VT_LNS_CASE
+  return static_cast<int>(cudaGetLastError());
 }
 
 int add_elementwise(const void* a, const void* b, void* out, long long n, int dtype,

@@ -2,7 +2,7 @@
 //
 // This is the exact-fp32 and odd-shape path behind the `matmul` / `matmul3` entry points
 // (reference vit/kernels/matmul.py:111-156, matmul3.py:111-156): arbitrary strides, any M/N/K,
-// fp32 or bf16 storage, fp32 accumulation, optional bias / exact-erf GELU / scale epilogue.
+// fp32 or bf16 storage, fp32 accumulation, optional bias / exact-erf or quick GELU / scale epilogue.
 // The bf16 model path never comes here for its dense layers (those run on tcgen05, see
 // gemm_sm100.cu); the fp32 parity configuration (C1, <=1e-3 vs HF) does, because single-pass
 // TF32 tensor-core math misses that tolerance (SURVEY.md 7.2).
@@ -105,7 +105,8 @@ simt_gemm_kernel(const SimtGemmParams p) {
       if (gn >= p.N) continue;
       float v = acc[i][j];
       if (bias) v += ldf(bias + gn);
-      if (p.gelu) v = gelu_erf(v);
+      if (p.gelu == kActGelu) v = gelu_erf(v);
+      else if (p.gelu == kActQuickGelu) v = quick_gelu(v);
       v *= p.scale;
       stf(C + gm * p.sCm + gn * p.sCn, v);
     }
@@ -117,7 +118,7 @@ simt_gemm_kernel(const SimtGemmParams p) {
 int simt_gemm(const void* A, const void* B, void* C, const void* bias, int M, int N, int K,
               int batch_outer, int batch_inner, const long long* sA, const long long* sB,
               const long long* sC, float scale, int gelu, int dtype, cudaStream_t stream) {
-  if (!A || !B || !C || M < 0 || N < 0 || K < 0 || batch_outer < 0 || batch_inner <= 0)
+  if (!A || !B || !C || M < 0 || N < 0 || K < 0 || batch_outer < 0 || batch_inner <= 0 || !gemm_act_ok(gelu))
     return VT_ERR_ARG;
   if (M == 0 || N == 0 || batch_outer == 0) return VT_OK;
   const long long nz = static_cast<long long>(batch_outer) * batch_inner;

@@ -1,6 +1,6 @@
 """ctypes binding of libvitb200.so (C ABI declared in include/vitb200.h, include/vitb200_resolution.h,
-include/vitb200_ragged.h, include/vitb200_mask.h, include/vitb200_attn.h, include/vitb200_preprocess.h and
-include/vitb200_tokens.h).
+include/vitb200_ragged.h, include/vitb200_mask.h, include/vitb200_attn.h, include/vitb200_preprocess.h,
+include/vitb200_tokens.h and include/vitb200_clip.h).
 
 There is deliberately no fallback: if the shared library is missing or a tensor is not on a CUDA
 device the entry points raise.  The oracle under /oracle is test infrastructure and is never
@@ -21,6 +21,11 @@ VT_U8 = 2     # raw NHWC pixels (patch embeddings, masked-image-modeling loss)
 VT_E4M3 = 3   # FP8 path (vt_gemm_fp8 / vt_layernorm_fp8)
 VT_PG_PUT = 1  # vt_pool_cls_allgather modes
 VT_PG_GET = 2
+# GEMM epilogue activations (VT_ACT_* of include/vitb200_clip.h): vt_bgemm's act, the gelu argument of the other GEMMs
+VT_ACT_NONE = 0
+VT_ACT_GELU = 1
+VT_ACT_TANH = 2
+VT_ACT_QUICK_GELU = 3
 
 _c_i32 = ctypes.c_int32
 _c_i64 = ctypes.c_int64
@@ -115,6 +120,12 @@ TOKENS_SIGNATURES = {
     "vt_embed_finalize_masked_prefix": MASK_SIGNATURES["vt_embed_finalize_masked"][:-1] + [_c_i32, _c_ptr],
 }
 
+# name -> argtypes of the CLIP entry points; mirrors include/vitb200_clip.h one to one (tests/test_abi_clip.py checks both
+# directions)
+CLIP_SIGNATURES = {
+    "vt_layernorm_stats": [_c_ptr, _c_ptr, _c_ptr, _c_ptr, _c_ptr, _c_i64, _c_i32, _c_i64, _c_i64, _c_f32, _c_ptr],
+}
+
 
 def call_prefix(name: str, prefix: int, *args) -> None:
     """One host path for every prefix-token count: ``name + "_prefix"`` (include/vitb200_tokens.h) with ``prefix`` right
@@ -161,7 +172,7 @@ def load() -> ctypes.CDLL:
     for name, argtypes in (list(SIGNATURES.items()) + list(RESOLUTION_SIGNATURES.items())
                            + list(RAGGED_SIGNATURES.items()) + list(MASK_SIGNATURES.items())
                            + list(ATTN_SIGNATURES.items()) + list(PREPROCESS_SIGNATURES.items())
-                           + list(TOKENS_SIGNATURES.items())):
+                           + list(TOKENS_SIGNATURES.items()) + list(CLIP_SIGNATURES.items())):
         fn = getattr(lib, name)
         fn.argtypes = argtypes
         fn.restype = ctypes.c_int

@@ -12,8 +12,8 @@ import torch
 
 from . import _lib
 
-ACT_NONE, ACT_GELU, ACT_TANH = 0, 1, 2
-_ACT = {None: ACT_NONE, "": ACT_NONE, "gelu": ACT_GELU, "tanh": ACT_TANH}
+ACT_NONE, ACT_GELU, ACT_TANH, ACT_QUICK_GELU = _lib.VT_ACT_NONE, _lib.VT_ACT_GELU, _lib.VT_ACT_TANH, _lib.VT_ACT_QUICK_GELU
+_ACT = {None: ACT_NONE, "": ACT_NONE, "gelu": ACT_GELU, "tanh": ACT_TANH, "quick_gelu": ACT_QUICK_GELU}
 
 
 def split_pieces() -> int:

@@ -66,7 +66,8 @@ def matmul(A: torch.Tensor, B: torch.Tensor, bias: Optional[torch.Tensor] = None
     """O[b] = act(A[b] @ B + bias) with fp32 accumulation.
 
     Args / errors follow the reference's ``matmul_triton`` (matmul.py:124-133): A is (B, T, Cin) with
-    any strides, B is (Cin, Cout), bias is (Cout,), activation is None or "gelu" (exact erf).
+    any strides, B is (Cin, Cout), bias is (Cout,), activation is None, "gelu" (exact erf) or "quick_gelu"
+    (x * sigmoid(1.702 x), CLIP).
     Returns a fresh (B, T, Cout) tensor in A's dtype.
     """
     assert len(A.shape) == 3, "First input matrix needs to have 3 dimensions (B, T, C)"
@@ -77,7 +78,9 @@ def matmul(A: torch.Tensor, B: torch.Tensor, bias: Optional[torch.Tensor] = None
         assert bias.is_cuda, "Bias is not on GPU"
         assert bias.numel() == B.shape[1], "Bias shape does not match output feature dimension shape"
     if activation:
-        assert activation in ["gelu"], f"Only GELU activation supported as of now! Provided: {activation}"
+        assert activation in ["gelu", "quick_gelu"], \
+            f"Only the gelu and quick_gelu activations are supported, provided: {activation}"
+    act = bg._ACT[activation]
 
     batch, M, K = A.shape
     N = B.shape[1]
@@ -90,7 +93,7 @@ def matmul(A: torch.Tensor, B: torch.Tensor, bias: Optional[torch.Tensor] = None
         Bt = _cached(B, "kmajor", _k_major)
         bias32 = None if bias is None else _cached(bias, "f32", lambda b: b.detach().float().contiguous())
         _lib.call("vt_gemm_bf16", A.data_ptr(), A.stride(1), Bt.data_ptr(), K, O.data_ptr(), N,
-                  _lib.VT_BF16, _lib.ptr(bias32), None, 0, batch * M, N, K, 1 if activation else 0, stream)
+                  _lib.VT_BF16, _lib.ptr(bias32), None, 0, batch * M, N, K, act, stream)
         return O
 
     assert A.dtype == B.dtype, f"Input dtypes need to be same, provided {A.dtype}, {B.dtype}"
@@ -102,7 +105,7 @@ def matmul(A: torch.Tensor, B: torch.Tensor, bias: Optional[torch.Tensor] = None
                   _lib.i64x4(A.stride(0), 0, A.stride(1), A.stride(2)),
                   _lib.i64x4(0, 0, B.stride(0), B.stride(1)),
                   _lib.i64x4(M * N, 0, N, 1),
-                  1.0, 1 if activation else 0, _lib.dtype_code(A), stream)
+                  1.0, act, _lib.dtype_code(A), stream)
         return O
 
     # tensor cores for everything else: pack A (any strides) and W^T into K-major bf16 rows — fp32 split
@@ -114,5 +117,5 @@ def matmul(A: torch.Tensor, B: torch.Tensor, bias: Optional[torch.Tensor] = None
     a = bg.pack(A, A.data_ptr(), M, K, batch, 1, (A.stride(0), 0, A.stride(1), A.stride(2)), pieces, pattern=0)
     kk = a.shape[2]
     bg.bgemm(a.data_ptr(), wp.data_ptr(), O, O.data_ptr(), M, N, kk, batch, 1, (M * kk, 0, kk), (0, 0, kk),
-             (M * N, 0, N), bias32=bias32, act=bg.ACT_GELU if activation else bg.ACT_NONE)
+             (M * N, 0, N), bias32=bias32, act=act)
     return O

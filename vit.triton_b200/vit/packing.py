@@ -192,16 +192,17 @@ def layernorm_fp8(x: torch.Tensor, ln, scale: float = FP8_ACT_SCALE) -> torch.Te
     return out
 
 
-def linear_fp8(x8: torch.Tensor, w8: torch.Tensor, colscale: torch.Tensor, bias32: torch.Tensor, gelu: bool = False,
+def linear_fp8(x8: torch.Tensor, w8: torch.Tensor, colscale: torch.Tensor, bias32: torch.Tensor, gelu: int = 0,
                residual: Optional[torch.Tensor] = None, out_fp8: bool = False, out_scale: float = 1.0) -> torch.Tensor:
-    """out = act((x8 @ w8^T) * colscale + bias) (+ residual) on tcgen05.mma kind::f8f6f4; x8 / w8 are e4m3 bytes."""
+    """out = act((x8 @ w8^T) * colscale + bias) (+ residual) on tcgen05.mma kind::f8f6f4; x8 / w8 are e4m3 bytes.
+    ``gelu``: the activation code (``_lib.VT_ACT_*``: 0 none, 1 exact GELU, 3 quick GELU; False / True are 0 / 1)."""
     B, N, K = x8.shape
     n_out = w8.shape[0]
     out = torch.empty((B, N, n_out), device=x8.device, dtype=torch.uint8 if out_fp8 else torch.bfloat16)
     if out.numel():
         _lib.call("vt_gemm_fp8", x8.data_ptr(), K, w8.data_ptr(), K, out.data_ptr(), n_out,
                   _lib.VT_E4M3 if out_fp8 else _lib.VT_BF16, bias32.data_ptr(), colscale.data_ptr(),
-                  _lib.ptr(residual), n_out, B * N, n_out, K, 1 if gelu else 0, float(out_scale), _lib.stream_ptr(x8))
+                  _lib.ptr(residual), n_out, B * N, n_out, K, int(gelu), float(out_scale), _lib.stream_ptr(x8))
     return out
 
 
@@ -307,6 +308,7 @@ def embed_pack(emb, fmt: Optional[tuple] = None) -> SimpleNamespace:
 
 
 STATS_COLS = 128   # columns per (sum, M2) partial of the row statistics (VT_LN_STATS_COLS in include/vitb200.h)
+LN_STATS_MAX_DIM = 1280   # widest row vt_layernorm_stats takes (include/vitb200_clip.h)
 
 
 def folding_supported(x: torch.Tensor, dim: int, mlp_dim: int) -> bool:
@@ -315,16 +317,29 @@ def folding_supported(x: torch.Tensor, dim: int, mlp_dim: int) -> bool:
 
 
 def linear_ln(x: torch.Tensor, w_fold: torch.Tensor, b_fold: torch.Tensor, colsum: Optional[torch.Tensor],
-              rowstats: torch.Tensor, eps: float, gelu: bool = False) -> torch.Tensor:
+              rowstats: torch.Tensor, eps: float, gelu: int = 0) -> torch.Tensor:
     """out = act(LN(x) @ W^T + b) computed as a GEMM on the un-normalised x with the normalisation
     applied per row in the epilogue; ``rowstats`` is the (M, K/128, 2) fp32 table of per-128-column
-    (sum, M2) partials of x's rows written by ``linear_res_stats``."""
+    (sum, M2) partials of x's rows written by ``linear_res_stats`` (or ``layernorm_stats``).  ``gelu``: the activation
+    code, as for ``linear``."""
     B, N, K = x.shape
     n_out = w_fold.shape[0]
     out = torch.empty((B, N, n_out), device=x.device, dtype=x.dtype)
     _lib.call("vt_gemm_bf16_ln", x.data_ptr(), K, w_fold.data_ptr(), K, out.data_ptr(), n_out,
-              b_fold.data_ptr(), None, 0, B * N, n_out, K, 1 if gelu else 0, rowstats.data_ptr(),
+              b_fold.data_ptr(), None, 0, B * N, n_out, K, int(gelu), rowstats.data_ptr(),
               _lib.ptr(colsum), K, float(eps), None, _lib.stream_ptr(x))
+    return out
+
+
+def layernorm_stats(x: torch.Tensor, ln, stats_out: torch.Tensor) -> torch.Tensor:
+    """LayerNorm ``ln`` of bf16 (B, N, D) rows that also writes every output row's per-128-column (sum, M2) partials
+    into the (B * N, D/128, 2) fp32 ``stats_out`` for the LayerNorm folded into the next GEMM (``vt_layernorm_stats``:
+    the same bits as ``ln(x)``)."""
+    B, N, D = x.shape
+    x = x.contiguous()
+    out = torch.empty_like(x)
+    _lib.call("vt_layernorm_stats", x.data_ptr(), ln.weight.data_ptr(), ln.bias.data_ptr(), out.data_ptr(),
+              stats_out.data_ptr(), B * N, D, D, D, float(ln.eps), _lib.stream_ptr(x))
     return out
 
 
@@ -341,9 +356,10 @@ def linear_res_stats(x: torch.Tensor, w_nk: torch.Tensor, bias32: torch.Tensor, 
     return out
 
 
-def linear(x: torch.Tensor, w_nk: torch.Tensor, bias32: torch.Tensor, gelu: bool = False,
+def linear(x: torch.Tensor, w_nk: torch.Tensor, bias32: torch.Tensor, gelu: int = 0,
            residual: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """out = epi(x @ w_nk^T + bias) over the flattened (B*N, K) activation.
+    """out = epi(x @ w_nk^T + bias) over the flattened (B*N, K) activation.  ``gelu``: the activation code of the
+    epilogue (``_lib.VT_ACT_*``: 0 none, 1 exact GELU, 3 quick GELU; False / True are 0 / 1).
 
     bf16 -> tcgen05 GEMM with bias / GELU / residual fused into the epilogue;
     fp32 -> exact FP32-pipe GEMM (bias / GELU fused, residual added by the add kernel).
@@ -358,7 +374,7 @@ def linear(x: torch.Tensor, w_nk: torch.Tensor, bias32: torch.Tensor, gelu: bool
     if x.dtype == torch.bfloat16 and K % 8 == 0 and n_out % 8 == 0:
         _lib.call("vt_gemm_bf16", x.data_ptr(), K, w_nk.data_ptr(), K, out.data_ptr(), n_out,
                   _lib.VT_BF16, bias32.data_ptr(), _lib.ptr(residual), n_out, M, n_out, K,
-                  1 if gelu else 0, stream)
+                  int(gelu), stream)
         return out
 
     if os.environ.get("VT_EXACT_FP32") == "1":      # FP32-pipe kernel, A/B comparisons only
@@ -371,7 +387,7 @@ def linear(x: torch.Tensor, w_nk: torch.Tensor, bias32: torch.Tensor, gelu: bool
             _lib.call("vt_gemm_strided", x.data_ptr() + m0 * K * es, w_nk.data_ptr(),
                       out.data_ptr() + m0 * n_out * es, bias.data_ptr(), mm, n_out, K, 1, 1,
                       _lib.i64x4(0, 0, K, 1), _lib.i64x4(0, 0, 1, K), _lib.i64x4(0, 0, n_out, 1),
-                      1.0, 1 if gelu else 0, code, stream)
+                      1.0, int(gelu), code, stream)
         if residual is not None:
             _lib.call("vt_add", out.data_ptr(), residual.data_ptr(), out.data_ptr(), out.numel(), code, stream)
         return out
@@ -380,7 +396,7 @@ def linear(x: torch.Tensor, w_nk: torch.Tensor, bias32: torch.Tensor, gelu: bool
     # fp32 operands split into bf16 pieces (kernels/bgemm.py), bias / GELU / residual fused
     pieces = 1 if x.dtype == torch.bfloat16 else bg.split_pieces()
     wp = split_weight(w_nk, pieces)
-    bg.dense_rows(x, x.data_ptr(), M, K, K, wp, pieces, n_out, bias32, bg.ACT_GELU if gelu else bg.ACT_NONE, out,
+    bg.dense_rows(x, x.data_ptr(), M, K, K, wp, pieces, n_out, bias32, int(gelu), out,
                   out.data_ptr(), n_out, residual_ptr=_lib.ptr(residual))
     return out
 

@@ -133,7 +133,9 @@ class DataParallelVIT(torch.nn.Module):
         """``output``: "pooled" gathers the CLS embeddings (B, D); "pooler" the HF pooler output
         tanh(dense(CLS)) (B, D) of a model built with ``add_pooling_layer=True``; "logits" the class
         logits (B, num_labels) of a model built with a classifier head (``VIT(num_labels=...)``, or the mean of the
-        two DeiT heads of ``VIT(..., distillation_head=True)``).
+        two DeiT heads of ``VIT(..., distillation_head=True)``); "image_embeds" the CLIP image embeddings
+        (B, projection_dim) of ``VIT(..., clip=True, projection_dim=...)`` (on a CLIP model "pooler" gathers its
+        ``pooler_output``, post_layernorm of the CLS rows).
         ``peer_gather``: None = use the fused pool + peer-store kernel whenever it applies (CUDA,
         NCCL group, equal shards, symmetric memory available; VT_PEER_GATHER=0 disables), True =
         require it, False = always all-gather through torch.distributed.  Which one runs is decided
@@ -147,7 +149,8 @@ class DataParallelVIT(torch.nn.Module):
         self.model = model
         self.group = group
         self.peer_gather = peer_gather
-        assert output in ("pooled", "pooler", "logits"), f"output must be 'pooled', 'pooler' or 'logits', provided: {output}"
+        assert output in ("pooled", "pooler", "logits", "image_embeds"), \
+            f"output must be 'pooled', 'pooler', 'logits' or 'image_embeds', provided: {output}"
         self.output = output
         self.interpolate_pos_encoding = bool(interpolate_pos_encoding)
         self._peer = None          # PeerGather of the current plan
@@ -174,6 +177,8 @@ class DataParallelVIT(torch.nn.Module):
             return self.model.logits(x_local, **kw)
         if self.output == "pooler":
             return self.model.pooler_output(x_local, **kw)
+        if self.output == "image_embeds":
+            return self.model.image_embeds(x_local, **kw)
         return self.model.pooled(x_local, **kw)
 
     def _model_kwargs(self) -> dict:
@@ -244,6 +249,8 @@ class DataParallelVIT(torch.nn.Module):
         if self.output == "logits":
             head = self.model.classifier if self.model.classifier is not None else self.model.cls_classifier
             return head.weight.shape[1]
+        if self.output == "image_embeds":
+            return self.model.visual_projection.weight.shape[1]
         return int(getattr(self.model, "hidden_dim", 0))
 
     def _local_want(self, x_local: torch.Tensor, global_batch: int) -> bool:

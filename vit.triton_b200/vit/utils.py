@@ -48,6 +48,8 @@ def _dense_mapping(num_layers: int) -> dict:
         'cls_classifier.bias': 'cls_classifier.bias',       # VIT(distillation_head=True)
         'distillation_classifier.weight': 'distillation_classifier.weight',
         'distillation_classifier.bias': 'distillation_classifier.bias',
+        'pre_layernorm.weight': 'pre_layernorm.weight',     # CLIP pre_layrnorm, VIT(clip=True)
+        'pre_layernorm.bias': 'pre_layernorm.bias',
     }
     for i in range(num_layers):
         pre = f'encoder.layer.{i}.'
@@ -61,18 +63,81 @@ def _dense_mapping(num_layers: int) -> dict:
 
 _HF_QKV = re.compile(r"^encoder\.layer\.(\d+)\.attention\.attention\.(query|key|value)\.(weight|bias)$")
 
+# HF CLIP vision-tower names (after ``vision_model.``) -> the HF ViT names the mapping above takes
+_CLIP_RENAMES = [
+    (re.compile(r"^embeddings\.patch_embedding\.weight$"), "embeddings.patch_embeddings.projection.weight"),
+    (re.compile(r"^pre_layrnorm\.(weight|bias)$"), r"pre_layernorm.\1"),
+    (re.compile(r"^post_layernorm\.(weight|bias)$"), r"layernorm.\1"),
+    (re.compile(r"^encoder\.layers\.(\d+)\.self_attn\.(q|k|v)_proj\.(weight|bias)$"),
+     lambda m: f"encoder.layer.{m.group(1)}.attention.attention.{dict(q='query', k='key', v='value')[m.group(2)]}."
+               f"{m.group(3)}"),
+    (re.compile(r"^encoder\.layers\.(\d+)\.self_attn\.out_proj\.(weight|bias)$"),
+     r"encoder.layer.\1.attention.output.dense.\2"),
+    (re.compile(r"^encoder\.layers\.(\d+)\.layer_norm1\.(weight|bias)$"), r"encoder.layer.\1.layernorm_before.\2"),
+    (re.compile(r"^encoder\.layers\.(\d+)\.layer_norm2\.(weight|bias)$"), r"encoder.layer.\1.layernorm_after.\2"),
+    (re.compile(r"^encoder\.layers\.(\d+)\.mlp\.fc1\.(weight|bias)$"), r"encoder.layer.\1.intermediate.dense.\2"),
+    (re.compile(r"^encoder\.layers\.(\d+)\.mlp\.fc2\.(weight|bias)$"), r"encoder.layer.\1.output.dense.\2"),
+]
+
+
+def _clip_source(pretrained_model: torch.nn.Module, custom_model: torch.nn.Module) -> tuple:
+    """(ViT-named source state dict, visual projection (P, D) or None) of an HF ``CLIPVisionModel``,
+    ``CLIPVisionModelWithProjection`` or ``CLIPModel``: ``vision_model.`` stripped, text-tower keys ignored.
+    AssertionError, before anything is copied, when the checkpoint's hidden_act / layer_norm_eps differ from the model's
+    or the model has a projection the checkpoint lacks."""
+    config = pretrained_model.config
+    config = getattr(config, "vision_config", config)           # CLIPModel: the vision tower's config
+    for name in ("hidden_act", "layer_norm_eps"):
+        want, have = getattr(config, name), getattr(custom_model, name)
+        assert want == have, f"The checkpoint has {name}={want!r}: build the model with {name}={want!r} (it has {have!r})"
+    source, proj = {}, None
+    for key, t in pretrained_model.state_dict().items():
+        if key == "visual_projection.weight":
+            proj = t
+            continue
+        if not key.startswith("vision_model."):
+            continue                                            # text tower, logit_scale, text_projection
+        key = key[len("vision_model."):]
+        if key == "embeddings.class_embedding":
+            source["embeddings.cls_token"] = t.reshape(1, 1, -1)
+        elif key == "embeddings.position_embedding.weight":
+            source["embeddings.position_embeddings"] = t.unsqueeze(0)
+        else:
+            for pattern, repl in _CLIP_RENAMES:
+                new, n = pattern.subn(repl, key)
+                if n:
+                    source[new] = t
+                    break
+    assert proj is not None or custom_model.visual_projection is None, \
+        "The checkpoint has no visual_projection (not CLIPVisionModelWithProjection / CLIPModel): build the model " \
+        "without projection_dim"
+    return source, proj
+
 
 def transfer_pretrained_weights(pretrained_model: torch.nn.Module, custom_model: torch.nn.Module,
                                 verbose: bool = True) -> torch.nn.Module:
-    """Copy every weight of a HuggingFace ``ViTModel`` or ``DeiTModel`` into ``custom_model`` (a ``vit.vit.VIT``).
+    """Copy every weight of a HuggingFace ``ViTModel``, ``DeiTModel`` or CLIP vision tower into ``custom_model`` (a
+    ``vit.vit.VIT``).
 
     Same call and result as the reference (utils.py:45-113); the layer count comes from the models.
     Keys of the source may carry a ``vit.`` prefix (``ViTForImageClassification``, ``ViTForMaskedImageModeling``) or a
     ``deit.`` prefix (``DeiTForImageClassification``, ``DeiTForImageClassificationWithTeacher``).  A DeiT checkpoint
-    needs a model built with ``distillation_token=True``, and only a DeiT checkpoint fits such a model: anything else
+    needs a model built with ``distillation_token=True``, and only a DeiT checkpoint fits such a model.
+    ``CLIPVisionModel``, ``CLIPVisionModelWithProjection`` and ``CLIPModel`` (whose text tower is ignored) need a model
+    built with ``clip=True`` and the checkpoint's ``hidden_act`` and ``layer_norm_eps``, and only they fit such a model;
+    the projection is loaded into a model built with ``projection_dim`` and ignored by one without.  Anything else
     raises an AssertionError before a tensor is copied.
     """
-    source = {re.sub(r'^(vit|deit)\.', '', k): v for k, v in pretrained_model.state_dict().items()}
+    is_clip = any(k.startswith("vision_model.") for k in pretrained_model.state_dict())
+    wants_clip = bool(getattr(custom_model, "clip", False))
+    assert is_clip == wants_clip, (
+        "The checkpoint is a CLIP vision tower: build the model with clip=True" if is_clip else
+        "The model was built with clip=True but the checkpoint is not a CLIP vision tower")
+    proj = None
+    if is_clip:
+        source, proj = _clip_source(pretrained_model, custom_model)
+    else:
+        source = {re.sub(r'^(vit|deit)\.', '', k): v for k, v in pretrained_model.state_dict().items()}
     dest = custom_model.state_dict()
     has_token = 'embeddings.distillation_token' in source
     wants_token = 'embeddings.distillation_token' in dest
@@ -89,6 +154,8 @@ def transfer_pretrained_weights(pretrained_model: torch.nn.Module, custom_model:
             dest = map_attn_layers(m.group(1), m.group(2), m.group(3), tensor, dest)
     dest = map_non_attn_layers(source_state_dict=source, dest_state_dict=dest,
                                weight_mapping=_dense_mapping(num_layers))
+    if proj is not None and "visual_projection.weight" in dest:
+        dest["visual_projection.weight"] = proj.t().clone()     # HF (P, D) -> (in, out)
 
     custom_model.load_state_dict(dest, strict=False)
 

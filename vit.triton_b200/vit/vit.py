@@ -86,6 +86,12 @@ def set_layernorm_folding(enabled: bool, mlp: bool = True) -> None:
     _FOLD_LN_MLP = bool(enabled and mlp)
 
 
+def _act_code(hidden_act: str) -> int:
+    """Epilogue activation code (``_lib.VT_ACT_*``) of an HF ``hidden_act``: "gelu" or "quick_gelu"."""
+    assert hidden_act in ("gelu", "quick_gelu"), f"hidden_act must be 'gelu' or 'quick_gelu', provided: {hidden_act}"
+    return _lib.VT_ACT_GELU if hidden_act == "gelu" else _lib.VT_ACT_QUICK_GELU
+
+
 class LinearWithBias(nn.Module):
     """y = act(x @ weight + bias); weight is stored (in, out) like the reference (vit.py:25-35)."""
 
@@ -172,20 +178,23 @@ class MultiHeadAttention(packing.PackedMixin, nn.Module):
 
 class Transformer(packing.PackedMixin, nn.Module):
     """Pre-LN encoder block (reference vit.py:114-149): res = x + MHA(LN1(x));
-    out = res + W2 . GELU(W1 . LN2(res)).  LayerNorm eps is 1e-12 like HF ViT."""
+    out = res + W2 . act(W1 . LN2(res)).  ``hidden_act``: "gelu" (exact erf, HF ViT) or "quick_gelu"
+    (x * sigmoid(1.702 x), OpenAI CLIP); ``layer_norm_eps``: 1e-12 like HF ViT by default (CLIP: 1e-5)."""
 
-    def __init__(self, num_heads: int, d_in: int, d_out: int, mlp_dim: Optional[int] = None):
+    def __init__(self, num_heads: int, d_in: int, d_out: int, mlp_dim: Optional[int] = None, hidden_act: str = "gelu",
+                 layer_norm_eps: float = 1e-12):
         super().__init__()
         self.num_heads = num_heads
         self.d_in = d_in
         self.d_out = d_out
         self.mlp_dim = 4 * self.d_in if mlp_dim is None else mlp_dim
+        self.act = _act_code(hidden_act)     # epilogue activation code of fc1 (_lib.VT_ACT_*)
 
-        self.layernorm_before = LayerNormTriton(self.d_in, eps=1e-12)
+        self.layernorm_before = LayerNormTriton(self.d_in, eps=layer_norm_eps)
         self.attention = MultiHeadAttention(self.num_heads, self.d_in, self.d_out)
-        self.intermediate = LinearWithBias(self.d_in, self.mlp_dim, activation='gelu')
+        self.intermediate = LinearWithBias(self.d_in, self.mlp_dim, activation=hidden_act)
         self.output = LinearWithBias(self.mlp_dim, self.d_in)
-        self.layernorm_after = LayerNormTriton(self.d_in, eps=1e-12)
+        self.layernorm_after = LayerNormTriton(self.d_in, eps=layer_norm_eps)
 
     def forward(self, x, groups=None, attn: Optional[list] = None):
         """``attn``: a list that receives the block's attention probabilities (B, H, N, N)."""
@@ -198,7 +207,7 @@ class Transformer(packing.PackedMixin, nn.Module):
         pk = self.packed()
         x = x.contiguous()
         res = self.attention(self.layernorm_before(x), residual=x, groups=groups, attn=attn)
-        mid = packing.linear(self.layernorm_after(res), pk.w1, pk.b1, gelu=True)
+        mid = packing.linear(self.layernorm_after(res), pk.w1, pk.b1, gelu=self.act)
         return packing.linear(mid, pk.w2, pk.b2, residual=res)
 
     def _packed_sources(self):
@@ -231,7 +240,7 @@ class Transformer(packing.PackedMixin, nn.Module):
         ctx = _attention(qkv, self.num_heads, 1.0 / math.sqrt(self.d_out), groups, attn)
         res = packing.linear(ctx, att.wo, att.bo, residual=x)
         mid8 = packing.linear_fp8(packing.layernorm_fp8(res, self.layernorm_after, q8.ln2_scale), q8.w18, q8.c1,
-                                  mlp.b1, gelu=True, out_fp8=True, out_scale=packing.FP8_MID_SCALE)
+                                  mlp.b1, gelu=self.act, out_fp8=True, out_scale=packing.FP8_MID_SCALE)
         return packing.linear_fp8(mid8, q8.w28, q8.c2, mlp.b2, residual=res)
 
     def forward_folded(self, x: torch.Tensor, ln1_stats: Optional[torch.Tensor], groups=None,
@@ -256,10 +265,10 @@ class Transformer(packing.PackedMixin, nn.Module):
             stats2 = torch.empty((x.shape[0] * x.shape[1], self.d_in // packing.STATS_COLS, 2), device=x.device,
                                  dtype=torch.float32)
             res = packing.linear_res_stats(ctx, att.wo, att.bo, x, stats2)
-            mid = packing.linear_ln(res, pk.w1, pk.b1, pk.c1, stats2, self.layernorm_after.eps, gelu=True)
+            mid = packing.linear_ln(res, pk.w1, pk.b1, pk.c1, stats2, self.layernorm_after.eps, gelu=self.act)
         else:
             res = packing.linear(ctx, att.wo, att.bo, residual=x)
-            mid = packing.linear(self.layernorm_after(res), mlp.w1, mlp.b1, gelu=True)
+            mid = packing.linear(self.layernorm_after(res), mlp.w1, mlp.b1, gelu=self.act)
         stats = torch.empty((x.shape[0] * x.shape[1], self.d_in // packing.STATS_COLS, 2), device=x.device, dtype=torch.float32)
         out = packing.linear_res_stats(mid, mlp.w2, mlp.b2, res, stats)
         return out, stats
@@ -269,14 +278,15 @@ class Encoder(nn.Module):
     """Stack of blocks (reference vit.py:152-170)."""
 
     def __init__(self, num_layers: int, num_heads: int, hidden_dim: int, d_out: int,
-                 mlp_dim: Optional[int] = None):
+                 mlp_dim: Optional[int] = None, hidden_act: str = "gelu", layer_norm_eps: float = 1e-12):
         super().__init__()
         self.num_layers = num_layers
         self.num_heads = num_heads
         self.hidden_dim = hidden_dim
         self.d_out = d_out
         self.layer = nn.ModuleList(
-            Transformer(num_heads=self.num_heads, d_in=self.hidden_dim, d_out=d_out, mlp_dim=mlp_dim)
+            Transformer(num_heads=self.num_heads, d_in=self.hidden_dim, d_out=d_out, mlp_dim=mlp_dim,
+                        hidden_act=hidden_act, layer_norm_eps=layer_norm_eps)
             for _ in range(self.num_layers)
         )
 
@@ -452,7 +462,7 @@ def _head_on_cls(hidden: torch.Tensor, dense: "LinearWithBias", act: int) -> tor
     pieces = 1 if hidden.dtype == torch.bfloat16 else bg.split_pieces()
     wp = _cached(w, f"packed{pieces}", lambda p_: bg.pack(p_, p_.data_ptr(), n_out, D, 1, 1,
                                                           (0, 0, p_.stride(1), p_.stride(0)), pieces, pattern=1)[0])
-    bias32 = _cached(dense.bias, "f32", lambda b: b.detach().float().contiguous())
+    bias32 = None if dense.bias is None else _cached(dense.bias, "f32", lambda b: b.detach().float().contiguous())
     bg.dense_rows(hidden, hidden.data_ptr(), B, D, hidden.stride(0), wp, pieces, n_out, bias32, act, out,
                   out.data_ptr(), n_out)
     return out
@@ -506,6 +516,18 @@ class DecoderConv(packing.PackedMixin, nn.Module):
                                b32=self.bias.detach().float().contiguous())
 
 
+class VisualProjection(nn.Module):
+    """HF ``CLIPVisionModelWithProjection.visual_projection``: a bias-free Linear(D, projection_dim), weight stored
+    (in, out) like every dense weight here (state-dict key visual_projection.weight).  ``VIT.image_embeds`` runs it
+    as one tensor-core launch over the pooled rows (``_head_on_cls``)."""
+
+    bias = None
+
+    def __init__(self, hidden_dim: int, projection_dim: int):
+        super().__init__()
+        self.weight = nn.Parameter(torch.zeros(hidden_dim, projection_dim))
+
+
 class VITOutput(NamedTuple):
     """What ``VIT.forward`` / ``forward_uint8`` return when ``output_hidden_states`` or ``output_attentions`` is set, like
     HF ``BaseModelOutput``; an unrequested field is None.  ``hidden_states``: num_layers + 1 tensors (B, N, D), the
@@ -536,7 +558,15 @@ class VIT(nn.Module):
     ``distillation_token=True`` builds a DeiT encoder (HF ``DeiTModel``): a learned distillation token follows CLS, so
     N = 2 + gh * gw and the position table has num_patches + 2 rows.  ``distillation_head=True`` (needs ``num_labels``
     and the token) adds HF ``DeiTForImageClassificationWithTeacher``'s ``cls_classifier`` and
-    ``distillation_classifier`` in place of ``classifier`` (``distillation_logits``)."""
+    ``distillation_classifier`` in place of ``classifier`` (``distillation_logits``).
+
+    ``hidden_act`` ("gelu" or "quick_gelu") and ``layer_norm_eps`` are HF's config values of those names; every MLP and
+    every LayerNorm of the model uses them.  ``clip=True`` builds a CLIP image encoder (HF ``CLIPVisionModel``): a
+    LayerNorm ``pre_layernorm`` (HF ``pre_layrnorm``) normalises the embeddings before block 0, the forward returns the
+    encoder output with no final LayerNorm, and ``layernorm`` is CLIP's ``post_layernorm``, applied to the CLS rows
+    only (``pooler_output``).  The patch convolution keeps its bias parameter (zero in a CLIP checkpoint).
+    ``projection_dim`` (with ``clip``) adds ``visual_projection`` (HF ``CLIPVisionModelWithProjection``,
+    ``image_embeds``)."""
 
     def __init__(
         self,
@@ -555,6 +585,10 @@ class VIT(nn.Module):
         encoder_stride: Optional[int] = None,
         distillation_token: bool = False,
         distillation_head: bool = False,
+        hidden_act: str = "gelu",
+        layer_norm_eps: float = 1e-12,
+        clip: bool = False,
+        projection_dim: Optional[int] = None,
     ):
         super().__init__()
         assert height == width, "Height and width should be the same"
@@ -572,6 +606,16 @@ class VIT(nn.Module):
         assert self.hidden_dim % self.num_heads == 0, f"Hidden dimension should be divisible by number of heads, provided: {self.hidden_dim} {self.num_heads}"
         assert not distillation_head or (num_labels and distillation_token), \
             "distillation_head=True needs num_labels and distillation_token=True"
+        _act_code(hidden_act)
+        # HF has no CLIP vision model with these; CLIPForImageClassification's mean-pooled head is not implemented
+        for flag, value in (("use_mask_token", use_mask_token), ("add_decoder", add_decoder),
+                            ("distillation_token", distillation_token), ("add_pooling_layer", add_pooling_layer),
+                            ("num_labels", num_labels)):
+            assert not (clip and value), f"clip=True does not combine with {flag}"
+        assert projection_dim is None or clip, "projection_dim needs clip=True"
+        self.clip = bool(clip)
+        self.hidden_act = hidden_act
+        self.layer_norm_eps = layer_norm_eps
 
         num_patches = (self.height // self.patch_size) * (self.width // self.patch_size)
         patch_dim = self.patch_size * self.patch_size * self.channels
@@ -582,8 +626,13 @@ class VIT(nn.Module):
                                      use_mask_token=use_mask_token or add_decoder,
                                      distillation_token=distillation_token)
         self.encoder = Encoder(num_layers=self.num_layers, num_heads=self.num_heads, hidden_dim=self.hidden_dim,
-                               d_out=d_out, mlp_dim=mlp_dim)
-        self.layernorm = LayerNormTriton(dim=self.hidden_dim, eps=1e-12)
+                               d_out=d_out, mlp_dim=mlp_dim, hidden_act=hidden_act, layer_norm_eps=layer_norm_eps)
+        # CLIP: pre_layrnorm in front of block 0 (state-dict keys pre_layernorm.{weight,bias})
+        self.pre_layernorm = LayerNormTriton(dim=self.hidden_dim, eps=layer_norm_eps) if clip else None
+        # the final LayerNorm; on a CLIP model its post_layernorm, applied to the CLS rows only
+        self.layernorm = LayerNormTriton(dim=self.hidden_dim, eps=layer_norm_eps)
+        # CLIPVisionModelWithProjection.visual_projection: state-dict key visual_projection.weight (D, projection_dim)
+        self.visual_projection = VisualProjection(self.hidden_dim, projection_dim) if projection_dim else None
         # optional HF pooler (tanh(dense(CLS))): state-dict keys pooler.dense.{weight,bias}
         self.pooler = Pooler(self.hidden_dim) if add_pooling_layer else None
         # optional HF ViTForImageClassification head (Linear on the CLS row of the final hidden states):
@@ -651,14 +700,16 @@ class VIT(nn.Module):
 
     def _encode(self, x: torch.Tensor, stats: Optional[torch.Tensor], output_hidden_states: bool,
                 output_attentions: bool):
-        """Encoder + final LayerNorm over the embeddings x: the final hidden states, or a ``VITOutput`` when a flag is set."""
+        """Encoder + final LayerNorm over the embeddings x (CLIP: the encoder alone): the final hidden states, or a
+        ``VITOutput`` when a flag is set."""
         kw = {}
         if output_hidden_states:
             kw["hidden"] = []
         if output_attentions:
             kw["attn"] = []
         x = self.encoder(x, stats, **kw) if stats is not None else self.encoder(x, **kw)
-        x = self.layernorm(x)
+        if not self.clip:
+            x = self.layernorm(x)
         if not kw:
             return x
         return VITOutput(x, tuple(kw["hidden"]) if output_hidden_states else None,
@@ -676,6 +727,8 @@ class VIT(nn.Module):
         probe = torch.empty((1,), device=x.device, dtype=w.dtype)
         if not self.encoder.folding_active(probe):
             return None
+        if self.clip and self.hidden_dim > packing.LN_STATS_MAX_DIM:
+            return None                  # pre_layernorm cannot write the statistics: block 0's LayerNorm runs as a kernel
         n_tok = self.embeddings.num_patches + self.embeddings.num_prefix_tokens if n_tok is None else n_tok
         return torch.empty((batch * n_tok, self.hidden_dim // packing.STATS_COLS, 2), device=x.device,
                            dtype=torch.float32)
@@ -720,12 +773,25 @@ class VIT(nn.Module):
             _, _, H, W = packing.pixel_dims(x, fmt)
             self.embeddings.check_mask(bool_masked_pos, x, H, W, interpolate_pos_encoding)
         stats = self._embed_stats(x, n_tok)
+        emb_stats = None if self.clip else stats        # CLIP: the statistics are those of pre_layernorm's output
         if fmt is not None:
-            return self.embeddings._embed(x, fmt, stats, interpolate_pos_encoding, bool_masked_pos), stats
+            x = self.embeddings._embed(x, fmt, emb_stats, interpolate_pos_encoding, bool_masked_pos)
+            return self._pre_layernorm(x, stats), stats
         kw = dict(interpolate_pos_encoding=True) if interpolate_pos_encoding else {}
         if bool_masked_pos is not None:
             kw["bool_masked_pos"] = bool_masked_pos
-        return (self.embeddings(x, stats, **kw) if stats is not None else self.embeddings(x, **kw)), stats
+        x = self.embeddings(x, emb_stats, **kw) if emb_stats is not None else self.embeddings(x, **kw)
+        return self._pre_layernorm(x, stats), stats
+
+    def _pre_layernorm(self, x: torch.Tensor, stats: Optional[torch.Tensor]) -> torch.Tensor:
+        """CLIP's pre_layrnorm of the embeddings x (x itself on a model without ``clip``): with ``stats`` (the fold is
+        active) one ``vt_layernorm_stats`` launch that also writes the row statistics block 0's folded
+        layernorm_before reads, otherwise the LayerNorm module."""
+        if not self.clip:
+            return x
+        if stats is not None:
+            return packing.layernorm_stats(x, self.pre_layernorm, stats)
+        return self.pre_layernorm(x)
 
     def _resized(self, x, do_resize: bool, resample: int):
         """x itself, or with ``do_resize`` the uint8 (B, height, width, C) batch ``resize_uint8`` makes of x (a batch already
@@ -776,10 +842,11 @@ class VIT(nn.Module):
                 hidden[layout.row0[i]:layout.row0[i] + layout.tokens[i]].copy_(h[0])
             return hidden, layout
         stats = self._embed_stats(first[None], layout.rows)       # one "image" of M rows
-        x = packing.patch_embed_ragged(self.embeddings, images, layout, stats, u8, image_mean, image_std,
-                                       rescale_factor)
-        x = self.encoder(x, stats, groups=layout.groups)
-        x = self.layernorm(x)
+        x = packing.patch_embed_ragged(self.embeddings, images, layout, None if self.clip else stats, u8, image_mean,
+                                       image_std, rescale_factor)
+        x = self.encoder(self._pre_layernorm(x, stats), stats, groups=layout.groups)
+        if not self.clip:
+            x = self.layernorm(x)
         return x[0], layout
 
     def _ragged_cls(self, images, rows: int = 1) -> torch.Tensor:
@@ -814,14 +881,41 @@ class VIT(nn.Module):
                       bool_masked_pos: Optional[torch.Tensor] = None, output_hidden_states: bool = False,
                       output_attentions: bool = False, do_resize: bool = False,
                       resample: int = 2) -> torch.Tensor:
-        """HF ``ViTModel(...).pooler_output``: tanh(dense(final hidden state of CLS)), (B, D).  ``x`` may also be a list
-        of images of different sizes (``forward_ragged``), each with its own patch grid (without a mask).  ``do_resize`` /
-        ``resample`` as for ``forward_uint8``: the images are resized to the model's size first (a list then runs as
-        one batch, not ragged)."""
+        """HF ``ViTModel(...).pooler_output``: tanh(dense(final hidden state of CLS)), (B, D); on a ``clip=True`` model
+        HF ``CLIPVisionModel(...).pooler_output``, post_layernorm of the CLS rows (``_clip_pooled``).  ``x`` may also be
+        a list of images of different sizes (``forward_ragged``), each with its own patch grid (without a mask).
+        ``do_resize`` / ``resample`` as for ``forward_uint8``: the images are resized to the model's size first (a list
+        then runs as one batch, not ragged)."""
         _refuse_outputs("pooler_output", output_hidden_states, output_attentions)
-        assert self.pooler is not None, "Model was built without add_pooling_layer=True"
+        assert self.clip or self.pooler is not None, "Model was built without add_pooling_layer=True"
         x = self._resized(x, do_resize, resample)
-        return self.pooler(self._cls_hidden(x, interpolate_pos_encoding, bool_masked_pos))
+        hidden = self._cls_hidden(x, interpolate_pos_encoding, bool_masked_pos)
+        return self._clip_pooled(hidden) if self.clip else self.pooler(hidden)
+
+    def _clip_pooled(self, hidden: torch.Tensor) -> torch.Tensor:
+        """(B, D) post_layernorm (``layernorm``) of the CLS rows of ``hidden`` (B, N, D): ONE ``vt_layernorm`` launch that
+        reads row 0 of every image in place through its input row stride (N * D)."""
+        B, _, D = hidden.shape
+        assert hidden.is_cuda and hidden.stride(2) == 1
+        out = torch.empty((B, D), device=hidden.device, dtype=hidden.dtype)
+        ln = self.layernorm
+        code = _lib.dtype_code(hidden)
+        _lib.call("vt_layernorm", hidden.data_ptr(), ln.weight.data_ptr(), ln.bias.data_ptr(), out.data_ptr(), B, D,
+                  hidden.stride(0), D, float(ln.eps), code, code, _lib.stream_ptr(hidden))
+        return out
+
+    def image_embeds(self, x, interpolate_pos_encoding: bool = False,
+                     bool_masked_pos: Optional[torch.Tensor] = None, output_hidden_states: bool = False,
+                     output_attentions: bool = False, do_resize: bool = False, resample: int = 2) -> torch.Tensor:
+        """HF ``CLIPVisionModelWithProjection(...).image_embeds``: visual_projection(pooler_output), (B, projection_dim),
+        not normalised; needs ``VIT(..., clip=True, projection_dim=...)``.  The LayerNorm launch of ``pooler_output``
+        and one tensor-core launch (``vt_bgemm``) over its rows.  Arguments as for ``pooler_output``."""
+        _refuse_outputs("image_embeds", output_hidden_states, output_attentions)
+        assert self.visual_projection is not None, "VIT was built without a projection (clip=True, projection_dim=...)"
+        pooled = self.pooler_output(x, interpolate_pos_encoding, bool_masked_pos, do_resize=do_resize,
+                                    resample=resample)
+        from .kernels import bgemm as bg
+        return _head_on_cls(pooled[:, None, :], self.visual_projection, bg.ACT_NONE)
 
     def logits(self, x, interpolate_pos_encoding: bool = False,
                bool_masked_pos: Optional[torch.Tensor] = None, output_hidden_states: bool = False,

@@ -163,10 +163,17 @@ int vt_pack_bf16(const void* src, int32_t src_dtype, void* dst, int32_t rows, in
                  int32_t batch_inner, const int64_t* s_src, const int64_t* s_dst, int32_t cpad, int32_t pieces,
                  int32_t pattern, void* stream);
 
-/* K3 — fused attention forward (tcgen05, flash style, no materialised scores), bf16, head dim 64.
- * q/k/v: [B, N, H*dh] views with common row / batch strides (e.g. slices of a fused-QKV buffer);
- * out: [B, N, H*dh].  Replaces the per-head matmul3 -> softmax -> matmul3 -> slice-assign chain
- * (vit/vit.py:60-72,101-108). */
+/* K3 — fused attention forward (tcgen05, flash style, no materialised scores), bf16:
+ *   out[b, i, h*dh:(h+1)*dh] = softmax_j( scale * q[b,i,h] . k[b,j,h] ) v[b,j,h]
+ * head dim 64 or 80, any N >= 1, scale > 0 and finite.
+ * q/k/v: [B, N, H*dh] views with common row / batch strides (e.g. slices of a fused-QKV buffer, or three
+ * allocations); out: [B, N, H*dh] with its own row / batch strides.  Every pointer 16-byte aligned, every stride a
+ * multiple of 8 elements.  Nothing outside out's [B, N, H*dh] view is written, and nothing outside the q/k/v views
+ * is read.
+ * Returns VT_ERR_ARG for a null pointer or B, H, N <= 0; VT_ERR_ALIGN for a misaligned pointer or stride;
+ * VT_ERR_UNSUPPORTED, before anything is launched, for another head dim, a scale that is not positive and finite
+ * (the kernels take the row maximum of the raw scores), or a batch too large for one launch.
+ * Replaces the per-head matmul3 -> softmax -> matmul3 -> slice-assign chain (vit/vit.py:60-72,101-108). */
 int vt_flash_attn(const void* q, const void* k, const void* v, void* out, int32_t B, int32_t H,
                   int32_t N, int32_t dh, int64_t qkv_row_stride, int64_t qkv_batch_stride,
                   int64_t out_row_stride, int64_t out_batch_stride, float scale, void* stream);

@@ -139,7 +139,8 @@ __device__ __forceinline__ float max_groups5(uint32_t a, int nv) {
 
 // exp2 of two BOUNDED arguments (|x| <= 64: the bounded-logit path) on the FMA pipe instead of the MUFU:
 // x = n + f with n = rint(x) read out of the mantissa of x + 1.5 * 2^23, 2^f by a degree-3 polynomial on
-// [-0.5, 0.5] (max relative error 7.5e-5, far below the bf16 rounding of P), 2^n added into the exponent field.
+// [-0.5, 0.5] (max relative error 7.52e-5, far below the bf16 rounding of P; valid for -126 < x < 128,
+// tests/test_abi_attn.py), 2^n added into the exponent field.
 // Six packed-fp32 instructions + two integer ones per pair against two MUFU slots (16 cycles of the
 // quarter-rate pipe): VT_ATTN5_POLY pairs of every eight take this route.
 __device__ __forceinline__ float2 ex2_poly_x2(float2 x) {
@@ -1171,6 +1172,8 @@ int attn5_fwd_tcgen05(const void* q, const void* k, const void* v, void* out, in
                       cudaStream_t stream) {
   if (!q || !k || !v || !out || B <= 0 || H <= 0 || N <= 0) return VT_ERR_ARG;
   if (dh != kDH5 || N > kMaxN5) return VT_ERR_UNSUPPORTED;
+  // the row max is taken over the raw scores and then scaled: the maximum of the scaled logits only for scale > 0
+  if (!(scale > 0.f) || !(scale < INFINITY)) return VT_ERR_UNSUPPORTED;
   if ((qkv_row_stride % 8) || (qkv_batch_stride % 8) || (out_row_stride % 8) || (out_batch_stride % 8))
     return VT_ERR_ALIGN;
   if ((reinterpret_cast<uintptr_t>(q) | reinterpret_cast<uintptr_t>(k) | reinterpret_cast<uintptr_t>(v) |
@@ -1268,6 +1271,7 @@ int attn5mb_fwd_tcgen05(const void* q, const void* k, const void* v, void* out, 
                         cudaStream_t stream) {
   if (!q || !k || !v || !out || B <= 0 || H <= 0 || N <= 0) return VT_ERR_ARG;
   if (dh != 64 && dh != 80) return VT_ERR_UNSUPPORTED;
+  if (!(scale > 0.f) || !(scale < INFINITY)) return VT_ERR_UNSUPPORTED;   // as attn5_fwd_tcgen05
   if ((qkv_row_stride % 8) || (qkv_batch_stride % 8) || (out_row_stride % 8) || (out_batch_stride % 8))
     return VT_ERR_ALIGN;
   if ((reinterpret_cast<uintptr_t>(q) | reinterpret_cast<uintptr_t>(k) | reinterpret_cast<uintptr_t>(v) |
